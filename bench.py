@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path (one process per GPU under torchrun)
   python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU path (oracle port + cv2), rank 0 only
+  python bench.py ... --dump-outputs DIR                   # also writes the last timed step's outputs (.npy) to compare builds
 
 A "step" is one pass of the hot path over one batch of 64 synthetic 1920x1080 BGR frames per GPU (BASELINE.json
 configs[1]) with synthetic RetinaFace head tensors of the exact output shapes (no CNN / model server offline):
@@ -458,9 +459,36 @@ class Workload:
                 "rows_max_rel_err": max_rel, "tolerance": "tensor/crops bit-exact, rows 1e-5 relative (BASELINE north_star)"}, counts
 
 
-def measure(ctx, ext, wk, steps, warmup, world, barrier, sample_every=1, profile_steps=20):
+DUMP_TENSOR_VALUES = 1 << 20     # seeded draws from the B x 3 x 640 x 640 CNN input tensor (78.6 M values at batch 64)
+DUMP_CROPS = 128                 # seeded sample of the aligned 112 x 112 x 3 crops
+
+
+def dump_outputs(ctx, wk, det_scale, out_dir):
+    """Writes what the last timed step handed its caller as float32 / float64 .npy files under out_dir (about 32 MB):
+    detections per image (`counts`), `det_scale`, every detection row (`det`: x1 y1 x2 y2 score) and its landmarks (`lmk`),
+    and seeded samples of the CNN input tensor and of the crops together with the flat tensor indices / crop rows they
+    were taken at.  The inputs are seeded too, so two builds run with the same arguments can be compared file by file."""
+    import torch
+    counts, det, lmk = ctx.detect_fetch(wk.B)
+    total = int(counts.sum())
+    rng = np.random.default_rng(0)
+    t_idx = np.unique(rng.integers(0, wk.tensor_t.numel(), DUMP_TENSOR_VALUES))
+    c_idx = np.sort(rng.choice(total, min(total, DUMP_CROPS), replace=False))
+    dev = wk.tensor_t.device
+    out = {"counts": counts.astype(np.float64), "det_scale": np.asarray(det_scale, np.float32), "det": det, "lmk": lmk,
+           "tensor_sample": wk.tensor_t.view(-1)[torch.from_numpy(t_idx).to(dev)].cpu().numpy(),
+           "tensor_sample_index": t_idx.astype(np.float64),
+           "crops_sample": wk.crops_t[torch.from_numpy(c_idx).to(dev)].float().cpu().numpy(),
+           "crops_sample_index": c_idx.astype(np.float64)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
+def measure(ctx, ext, wk, steps, warmup, world, barrier, sample_every=1, profile_steps=20, dump_dir=None):
     """Times `steps` serial steps of workload `wk` with CUDA events on the ctx stream; per-kernel events on every
-    `sample_every`-th step of the timed region.  Returns a dict (rank-local values already max-reduced over ranks)."""
+    `sample_every`-th step of the timed region.  Returns a dict (rank-local values already max-reduced over ranks).
+    With dump_dir, rank 0 then writes the last timed step's outputs there (dump_outputs)."""
     import ctypes as C
     import torch
     for _ in range(max(warmup, 3)):
@@ -494,6 +522,8 @@ def measure(ctx, ext, wk, steps, warmup, world, barrier, sample_every=1, profile
     secs = dist_max(ev0.elapsed_time(ev1) / 1e3)
     live_us = {name: 1e3 * float(np.mean([m[i].elapsed_time(m[i + 1]) for m in marks.values()]))
                for i, name in enumerate(("preprocess", "detect", "align"))}
+    if dump_dir and int(os.environ.get("RANK", "0")) == 0:
+        dump_outputs(ctx, wk, ds, dump_dir)
 
     # ---- per-kernel device times through the ABI's per-launch events (separate untimed loop) + algorithmic bytes (SURVEY 8d):
     #      preprocess min(H*W*3, 640*360*12) + 4,915,200 B/frame; decode 1,008,000 B/image + 64 B/candidate; warp
@@ -604,7 +634,7 @@ def run_ours(args):
     # ---- timed region: device-resident ----
     sampler = ClockSampler(local_rank)
     sampler.start()
-    res = measure(ctx, ext, wk, args.steps, warmup, world, barrier, sample_every=args.roofline_sample)
+    res = measure(ctx, ext, wk, args.steps, warmup, world, barrier, sample_every=args.roofline_sample, dump_dir=args.dump_outputs)
     clocks = sampler.stop()
     secs, launches = res["secs"], res["launches"]
 
@@ -878,7 +908,10 @@ def main():
     ap.add_argument("--no-nms", action="store_true")
     ap.add_argument("--no-pipelined", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip BASELINE configs 4 and 5 (extra_workloads)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as .npy files to DIR (rank 0)")
     args = ap.parse_args()
+    if args.dump_outputs and args.steps < 1:
+        ap.error("--dump-outputs needs at least one timed step")
     if args.impl == "reference":
         return run_reference(args)
     world = int(os.environ.get("WORLD_SIZE", "1"))

@@ -157,7 +157,7 @@ def test_build_recipes_compile_every_translation_unit():
         assert not sym.startswith(("fd_", "_ZN2fd")), "undefined in libfd_b200.so: " + sym
 
 
-REFERENCE_SIGNATURES = {   # file under rust/src -> signatures that must appear verbatim (whitespace-normalised), reference file:line
+REFERENCE_SIGNATURES = {   # file under rust/src -> signatures copied verbatim from the reference (file:line), whitespace-normalised
     "processing/nms.rs": ["pub fn nms(dets: &Array2<f32>, thresh: f32) -> Vec<usize>"],                                   # nms.rs:3
     "processing/bbox_transform.rs": [
         "pub fn bbox_overlaps_py(boxes: &Array2<f32>, query_boxes: &Array2<f32>) -> Array2<f32>",                          # :2
@@ -193,9 +193,3 @@ def test_rust_wrappers_keep_the_reference_signatures():
         txt = norm(open(os.path.join(ROOT, "rust", "src", rel)).read())
         for sig in sigs:
             assert norm(sig) in txt, "%s: missing `%s`" % (rel, sig)
-    if os.path.isdir("/root/reference/src"):           # in this container the signatures are also checked against the reference itself
-        ref = norm(open("/root/reference/src/processing/bbox_transform.rs").read())
-        for sig in REFERENCE_SIGNATURES["processing/bbox_transform.rs"]:
-            assert norm(sig) in ref, sig
-        assert norm(REFERENCE_SIGNATURES["processing/nms.rs"][0]) in norm(open("/root/reference/src/processing/nms.rs").read())
-        assert norm(REFERENCE_SIGNATURES["rcnn/anchors.rs"][0]) in norm(open("/root/reference/src/rcnn/anchors.rs").read())

@@ -161,12 +161,12 @@ def test_argsort_descending(ctx, oracle, n):
     np.testing.assert_array_equal(ctx.argsort_descending(s), oracle.argsort_descending(s))
 
 
-def test_vs_reference_cuda_nms(ctx, oracle):
-    """The reference's own (vestigial, never built) CUDA NMS compiled from /root/reference into oracle/_ref: an A/B
-    cross-check on non-degenerate data, where `ovr > thr` == `!(ovr <= thr)`."""
+def reference_cuda_nms(srt, thresh):
+    """Keep list of the reference's own CUDA NMS (`_nms`, src/nms_kernel.cu) on score-sorted boxes, or None when
+    oracle/_ref has not been built from a reference checkout (`make -C oracle ref REF=<checkout>`)."""
     path = os.path.join(ROOT, "oracle", "_ref", "libref_gpu_nms.so")
     if not os.path.exists(path):
-        pytest.skip("oracle/_ref not built")
+        return None
     ref = C.CDLL(path)
     # nms_kernel.cu:91 defines _nms(.., const float*, ..) while gpu_nms.hpp:7 declares float*: the definition is a
     # C++ overload, not the extern "C" symbol, so look the mangled name up.
@@ -175,13 +175,24 @@ def test_vs_reference_cuda_nms(ctx, oracle):
              if "_nms" in l and "kernel" not in l]
     assert names, "no _nms symbol in oracle/_ref"
     ref_nms = getattr(ref, names[0])
-    dets = _random_dets(5000, 99, canvas=1200)
-    srt = np.ascontiguousarray(dets[oracle.argsort_descending(dets[:, 4])])
+    srt = np.ascontiguousarray(srt, np.float32)
     keep = np.zeros(len(srt), np.int32)
     num = C.c_int(0)
     ref_nms(keep.ctypes.data_as(C.POINTER(C.c_int32)), C.byref(num), srt.ctypes.data_as(C.POINTER(C.c_float)), len(srt), 5,
-            C.c_float(0.4), 0)
-    np.testing.assert_array_equal(ctx.nms_sorted(srt, 0.4), keep[:num.value])
+            C.c_float(thresh), 0)
+    return keep[:num.value]
+
+
+def test_vs_reference_cuda_nms(ctx):
+    """The reference's own (vestigial, never built) CUDA NMS: an A/B cross-check on non-degenerate data, where
+    `ovr > thr` == `!(ovr <= thr)`.  Its keep list is stored in tests/golden/ref_nms_golden.npz
+    (tests/golden/make_ref_nms_golden.py); when oracle/_ref is built, the stored list is checked against the library too."""
+    g = np.load(os.path.join(ROOT, "tests", "golden", "ref_nms_golden.npz"))
+    srt, keep, thresh = g["dets_sorted"], g["keep"], float(g["thresh"])
+    np.testing.assert_array_equal(ctx.nms_sorted(srt, thresh), keep)
+    live = reference_cuda_nms(srt, thresh)
+    if live is not None:
+        np.testing.assert_array_equal(live, keep)
 
 
 def test_property_random_small(ctx, oracle):
