@@ -276,13 +276,17 @@ __global__ void __launch_bounds__(WARP_THREADS, 4) warp_kernel(WarpArgs a) {
     int2 *xy0 = dxy + a.cw;      // [WARP_BAND]  (X0, Y0) per row
     __shared__ int s_item[2];
     const int tid = threadIdx.x;
+    pdl_wait();
     const int F = a.count_dev ? min(*a.count_dev, a.F) : a.F;
     const int n_items = F * a.bands;
     if (tid == 0) s_item[0] = atomicAdd(a.ticket, 1);
     __syncthreads();
     for (int par = 0;; par ^= 1) {
         const int item = s_item[par];
-        if (item >= n_items) break;
+        if (item >= n_items) {
+            pdl_trigger();   // out of tickets: the next step kernel may take this CTA's place
+            break;
+        }
         if (tid == 0) s_item[par ^ 1] = atomicAdd(a.ticket, 1);
         const int f = item / a.bands, band_y0 = (item - f * a.bands) * WARP_BAND;
         const int rows = min(WARP_BAND, a.ch - band_y0);
@@ -411,6 +415,7 @@ __global__ void __launch_bounds__(2 * CW) warp_fixed_kernel(WarpArgs a) {
     __shared__ int s_item[2];
     const int tid = threadIdx.x;
     const int r = tid / CW, x = tid - r * CW;
+    pdl_wait();
     const int F = a.count_dev ? min(*a.count_dev, a.F) : a.F;
     const int n_items = F * ITEMS;
     long long t_entry = 0, t_prev = 0, t_sum = 0;
@@ -423,7 +428,10 @@ __global__ void __launch_bounds__(2 * CW) warp_fixed_kernel(WarpArgs a) {
         const int item = s_item[par];
         if (a.dbg && tid == 0 && par == 1 && n_done == 1) a.dbg[blockIdx.x * 8 + 2] = warp_now();
         if (a.dbg && tid == 0) { const long long t = warp_now(); if (n_done) t_sum += t - t_prev; t_prev = t; ++n_done; }
-        if (item >= n_items) break;
+        if (item >= n_items) {
+            pdl_trigger();   // out of tickets: the next step kernel may take this CTA's place
+            break;
+        }
         if (tid == 0) s_item[par ^ 1] = atomicAdd(a.ticket, 1);
         const int f = item / ITEMS, y0 = (item - f * ITEMS) * IR;
         uint8_t *band_out = a.crops + ((size_t)f * CH + y0) * CW * 3;
@@ -611,7 +619,7 @@ int warp_launch(fd_ctx *ctx, const FrameDev *frames_dev, const int32_t *frame_id
         if (!per_sm_fixed) FD_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm_fixed, kern, 224, 0));
         const long long items = (long long)F_cap * (112 / IR);
         const int grid = (int)std::min<long long>(items, (long long)ctx->num_sms * std::max(per_sm_fixed, 1));
-        kern<<<grid, 224, 0, ctx->stream>>>(a);
+        FD_TRY(launch_pdl(ctx, kern, dim3(grid), dim3(224), 0, a));
         FD_LAUNCH_CHECK_NAMED(ctx, "warp_fixed_kernel");
         if (dbg_on) {   // in-kernel timeline (globaltimer): where a launch's time goes beyond the per-item work
             std::vector<long long> h(8 * (size_t)std::min(grid, 4096));
@@ -635,7 +643,7 @@ int warp_launch(fd_ctx *ctx, const FrameDev *frames_dev, const int32_t *frame_id
     FD_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, warp_kernel, WARP_THREADS, smem));
     const long long items = (long long)F_cap * a.bands;
     const int grid = (int)std::min<long long>(items, (long long)ctx->num_sms * std::max(per_sm, 1));
-    warp_kernel<<<grid, WARP_THREADS, smem, ctx->stream>>>(a);
+    FD_TRY(launch_pdl(ctx, warp_kernel, dim3(grid), dim3(WARP_THREADS), smem, a));
     FD_LAUNCH_CHECK_NAMED(ctx, "warp_kernel");
     return FD_OK;
 }

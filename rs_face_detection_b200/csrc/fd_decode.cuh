@@ -50,14 +50,13 @@ __device__ __forceinline__ AnchorGeo anchor_geo(const DecodeCfg &c, int s, int l
     g.cy = __fadd_rn(ay1, __fmul_rn(0.5f, __fsub_rn(g.ah, 1.0f)));
     return g;
 }
-// bbox_pred (face_detection.rs:516-549) + clip_boxes to the padded detector image (:373, bbox_transform.rs:36-42)
-__device__ __forceinline__ float4 decode_box(const DecodeCfg &c, const HeadPtrs &hp, int b, int s, int local, int a, const AnchorGeo &g) {
-    const int hw = c.fh[s] * c.fw[s];
-    const float *bb = hp.p[3 * s + 1] + (size_t)b * 4 * c.A * hw;
-    const float dx = __fmul_rn(__ldg(bb + (size_t)(4 * a + 0) * hw + local), c.bbox_stds[0]);  // :366-371
-    const float dy = __fmul_rn(__ldg(bb + (size_t)(4 * a + 1) * hw + local), c.bbox_stds[1]);
-    const float dw = __fmul_rn(__ldg(bb + (size_t)(4 * a + 2) * hw + local), c.bbox_stds[2]);
-    const float dh = __fmul_rn(__ldg(bb + (size_t)(4 * a + 3) * hw + local), c.bbox_stds[3]);
+// bbox_pred (face_detection.rs:516-549) + clip_boxes to the padded detector image (:373, bbox_transform.rs:36-42) from the
+// anchor's 4 raw box deltas
+__device__ __forceinline__ float4 decode_box(const DecodeCfg &c, const float *raw4, const AnchorGeo &g) {
+    const float dx = __fmul_rn(raw4[0], c.bbox_stds[0]);  // :366-371
+    const float dy = __fmul_rn(raw4[1], c.bbox_stds[1]);
+    const float dw = __fmul_rn(raw4[2], c.bbox_stds[2]);
+    const float dh = __fmul_rn(raw4[3], c.bbox_stds[3]);
     // :532-535.  exp through fp64 is correctly rounded to <=0.5 ulp; the reference's f32::exp is the platform expf.
     const float pcx = __fadd_rn(__fmul_rn(dx, g.aw), g.cx), pcy = __fadd_rn(__fmul_rn(dy, g.ah), g.cy);
     const float pw = __fmul_rn((float)exp((double)dw), g.aw), ph = __fmul_rn((float)exp((double)dh), g.ah);
@@ -70,7 +69,22 @@ __device__ __forceinline__ float4 decode_box(const DecodeCfg &c, const HeadPtrs 
     box.w = fmaxf(fminf(__fadd_rn(pcy, hwy), c.clip_h), 0.0f);
     return box;
 }
-// landmark_pred from the ANCHOR box, never clipped (face_detection.rs:399, :551-570)
+__device__ __forceinline__ float4 decode_box(const DecodeCfg &c, const HeadPtrs &hp, int b, int s, int local, int a, const AnchorGeo &g) {
+    const int hw = c.fh[s] * c.fw[s];
+    const float *bb = hp.p[3 * s + 1] + (size_t)b * 4 * c.A * hw;
+    float raw[4];
+#pragma unroll
+    for (int k = 0; k < 4; ++k) raw[k] = __ldg(bb + (size_t)(4 * a + k) * hw + local);
+    return decode_box(c, raw, g);
+}
+// landmark_pred from the ANCHOR box, never clipped (face_detection.rs:399, :551-570), from the anchor's 10 raw deltas
+__device__ __forceinline__ void decode_landmarks(const DecodeCfg &c, const float *lraw, const AnchorGeo &g, float *out10) {
+#pragma unroll
+    for (int p = 0; p < 5; ++p) {
+        out10[2 * p] = __fadd_rn(__fmul_rn(__fmul_rn(lraw[2 * p], c.landmark_std), g.aw), g.cx);
+        out10[2 * p + 1] = __fadd_rn(__fmul_rn(__fmul_rn(lraw[2 * p + 1], c.landmark_std), g.ah), g.cy);
+    }
+}
 __device__ __forceinline__ void decode_landmarks(const DecodeCfg &c, const HeadPtrs &hp, int b, int s, int local, int a,
                                                  const AnchorGeo &g, float *out10) {
     const int hw = c.fh[s] * c.fw[s];
@@ -78,11 +92,7 @@ __device__ __forceinline__ void decode_landmarks(const DecodeCfg &c, const HeadP
     float lraw[10];
 #pragma unroll
     for (int k = 0; k < 10; ++k) lraw[k] = __ldg(lm + (size_t)(10 * a + k) * hw + local);
-#pragma unroll
-    for (int p = 0; p < 5; ++p) {
-        out10[2 * p] = __fadd_rn(__fmul_rn(__fmul_rn(lraw[2 * p], c.landmark_std), g.aw), g.cx);
-        out10[2 * p + 1] = __fadd_rn(__fmul_rn(__fmul_rn(lraw[2 * p + 1], c.landmark_std), g.ah), g.cy);
-    }
+    decode_landmarks(c, lraw, g, out10);
 }
 #endif  // __CUDACC__
 

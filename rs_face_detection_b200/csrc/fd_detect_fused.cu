@@ -3,9 +3,12 @@
 //
 //   score scan      the 2A foreground score planes of the image, 128-bit loads, `>= conf_thr` (face_detection.rs:374-379),
 //                   warp-aggregated compaction of sort keys (score desc | anchor id) into shared memory;
-//   sort            register bitonic network (fd_nms_tiny.cuh) — ascending keys == the reference's stable descending sort
-//                   over the 32|16|8 concatenation (utils.rs:87-95, face_detection.rs:410-430);
-//   decode          bbox_pred + clip_boxes for the candidates only, by the thread that holds their sorted rank;
+//   head fetch      as soon as the keys are compacted, every candidate's box deltas, landmark deltas and score are copied
+//                   into shared memory (cp.async), in flight during the sort; decode and gather read them from there;
+//   sort            rank sort: keys are unique, so a key's rank is the number of smaller keys — sorted runs of 32 per warp,
+//                   then binary searches of the other runs; ascending keys == the reference's stable descending sort over
+//                   the 32|16|8 concatenation (utils.rs:87-95, face_detection.rs:410-430);
+//   decode          bbox_pred + clip_boxes for the candidates only, scattered to their sorted rank;
 //   NMS             exact greedy (nms.rs:3-65) in shared memory / registers (fd_nms_tiny.cuh);
 //   offsets         every CTA publishes its kept count (epoch-tagged) and sums its predecessors' — no chain, no second launch;
 //   gather          kept boxes / landmark_pred / `÷ det_scale` (face_detection.rs:432-493) straight to the compact outputs;
@@ -75,10 +78,18 @@ constexpr int FUSED_CTRL_BYTES = 256;
 static_assert(sizeof(FusedCtrl) <= FUSED_CTRL_BYTES, "control block");
 struct FusedSmem {
     TinySmem t;
-    u64 ckey[TINY_CAP];          // candidate keys in arrival order
-    float flmk[TINY_CAP * 10];   // rescaled landmarks of the kept faces (output rows, input of the estimate)
-    float fdet[TINY_CAP * 5];    // rescaled boxes + score of the kept faces (output rows)
+    u64 ckey[TINY_CAP];          // candidate keys in arrival order (slot)
+    int rank[TINY_CAP];          // sorted rank of slot i
+    int slot[TINY_CAP];          // slot of rank r
+    union {
+        float head[TINY_CAP][15];   // until the gather has read it: raw box deltas [0..3], landmark deltas [4..13], fg score [14] of slot i
+        struct {
+            float flmk[TINY_CAP * 10];   // rescaled landmarks of the kept faces (output rows, input of the estimate)
+            float fdet[TINY_CAP * 5];    // rescaled boxes + score of the kept faces (output rows)
+        };
+    };
 };
+static_assert(FUSED_CTRL_BYTES + sizeof(FusedSmem) <= 227 * 1024, "fused detect shared memory");
 
 __device__ __forceinline__ u64 ld_acquire_u64(const u64 *p) {
     u64 v;
@@ -87,6 +98,35 @@ __device__ __forceinline__ u64 ld_acquire_u64(const u64 *p) {
 }
 __device__ __forceinline__ void st_release_u64(u64 *p, u64 v) {
     asm volatile("st.release.gpu.global.u64 [%0], %1;" ::"l"(p), "l"(v) : "memory");
+}
+__device__ __forceinline__ void cp_async4(float *dst_smem, const float *src) {
+    asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"((unsigned)__cvta_generic_to_shared(dst_smem)), "l"(src) : "memory");
+}
+__device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_all;" ::: "memory"); }
+
+// ascending bitonic network over the 32 keys of a warp; each key's slot moves with it
+__device__ __forceinline__ void warp_sort_slots(u64 &key, int &slot, int lane) {
+#pragma unroll
+    for (int k = 2; k <= 32; k <<= 1) {
+#pragma unroll
+        for (int j = k >> 1; j > 0; j >>= 1) {
+            const u64 okey = __shfl_xor_sync(0xffffffffu, key, j);
+            const int oslot = __shfl_xor_sync(0xffffffffu, slot, j);
+            const bool take_min = ((lane & j) == 0) == ((lane & k) == 0);
+            if (take_min == (okey < key)) {
+                key = okey;
+                slot = oslot;
+            }
+        }
+    }
+}
+// number of keys below `key` in an ascending run of 32
+__device__ __forceinline__ int count_below(const u64 *run, u64 key) {
+    int p = 0;
+#pragma unroll
+    for (int s = 16; s > 0; s >>= 1)
+        if (run[p + s - 1] < key) p += s;
+    return p + (run[p] < key ? 1 : 0);
 }
 
 // Score scan of image b: UN items (4 consecutive positions of one stride each) per thread are loaded before any is
@@ -179,12 +219,15 @@ __device__ __forceinline__ void detect_fused_body(const FusedArgs &a) {
     FusedSmem &sm = *reinterpret_cast<FusedSmem *>(fused_raw + FUSED_CTRL_BYTES);
     const DecodeCfg &c = a.c;
     const int tid = threadIdx.x, lane = tid & 31;
+    pdl_trigger();   // the warp kernel's CTAs may take the SMs this grid leaves idle (they wait for its completion)
     if (tid == 0) {
-        ctl.b = atomicAdd(a.ticket, 1);   // images in ticket order: every predecessor of this image is already running
         ctl.cnt = 0;
         ctl.kept = 0;
         ctl.general = 0;
     }
+    sm.rank[tid] = 0;   // (FT == TINY_CAP)
+    pdl_wait();
+    if (tid == 0) ctl.b = atomicAdd(a.ticket, 1);   // images in ticket order: every predecessor of this image is already running
     __syncthreads();
     const int b = ctl.b;
     fused_stamp(a, b, 0);
@@ -198,6 +241,19 @@ __device__ __forceinline__ void detect_fused_body(const FusedArgs &a) {
     fused_stamp(a, b, 1);
     const int K = ctl.cnt;
     if (tid == 0) a.counts[b] = K;
+    if (K <= TINY_CAP && tid < K) {   // head fetch of slot tid: in flight during the sort, waited for by this thread only
+        int s, local, aa;
+        split_anchor_id(c, (int)(unsigned)sm.ckey[tid], s, local, aa);
+        const int hw = c.fh[s] * c.fw[s];
+        const float *bb = a.hp.p[3 * s + 1] + (size_t)b * 4 * A * hw + local;
+        const float *lm = a.hp.p[3 * s + 2] + (size_t)b * 10 * A * hw + local;
+        float *dst = sm.head[tid];
+#pragma unroll
+        for (int k = 0; k < 4; ++k) cp_async4(dst + k, bb + (size_t)(4 * aa + k) * hw);
+#pragma unroll
+        for (int k = 0; k < 10; ++k) cp_async4(dst + 4 + k, lm + (size_t)(10 * aa + k) * hw);
+        cp_async4(dst + 14, a.hp.p[3 * s] + (size_t)b * 2 * A * hw + (size_t)(A + aa) * hw + local);
+    }
 
     // ---- 2. sort + decode + NMS (K <= 1024), or decode everything and defer ----
     int *keep = a.keep + img_base;
@@ -251,31 +307,51 @@ __device__ __forceinline__ void detect_fused_body(const FusedArgs &a) {
     } else if (K > 0) {
         int n2 = 32;
         while (n2 < K) n2 <<= 1;
+        {   // rank of slot i.  Every warp sorts the keys of its 32 slots (shuffle network, carrying the slot) into a run; a key's
+            // rank is its place in its run plus, for every other run, the number of that run's keys below it (binary search).
+            // The FT / (32 runs) parts of the block take every parts-th run each.
+            const int nruns = (K + 31) >> 5, ne = nruns * 32, parts = FT / ne;
+            u64 *run_key = sm.t.xch[0], *run_slot = sm.t.xch[1];
+            if (tid < ne) {
+                u64 key = tid < K ? sm.ckey[tid] : ~0ull;
+                int slot = tid;
+                warp_sort_slots(key, slot, lane);
+                run_key[tid] = key;
+                run_slot[tid] = (u64)slot;
+            }
+            __syncthreads();
+            const int part = tid / ne, e = tid - part * ne;
+            if (part < parts && run_key[e] != ~0ull) {
+                const u64 key = run_key[e];
+                const int w = e >> 5;
+                int cnt = part == 0 ? (e & 31) : 0;
+#pragma unroll 4
+                for (int r = part; r < nruns; r += parts)
+                    if (r != w) cnt += count_below(run_key + 32 * r, key);
+                const int slot = (int)run_slot[e];
+                if (parts == 1) sm.rank[slot] = cnt;
+                else atomicAdd(&sm.rank[slot], cnt);
+            }
+        }
+        __syncthreads();
+        fused_stamp(a, b, 2);
+        bool ok = true;
+        if (tid < K) {   // decode slot tid into rank order
+            const int r = sm.rank[tid], id = (int)(unsigned)sm.ckey[tid];
+            int s, local, aa;
+            split_anchor_id(c, id, s, local, aa);
+            cp_async_wait_all();
+            const float4 bx = decode_box(c, sm.head[tid], anchor_geo(c, s, local, aa));
+            sm.t.sbox[r] = bx;
+            sm.t.sarea[r] = box_area(bx);
+            sm.t.sidx[r] = id;
+            sm.slot[r] = tid;
+            ok = box_is_fast_ok(bx);
+        }
+        const bool fast = !__syncthreads_or(!ok) && a.iou.fast;   // also publishes sbox / sidx / slot
+        fused_stamp(a, b, 3);
         if (tid < n2) {   // whole warps; their barriers are named barrier 2 over n2 threads
-            u64 key = tid < K ? sm.ckey[tid] : ~0ull;
-            switch (n2) {
-                case 32: tiny_sort<32>(key, sm.t, tid); break;
-                case 64: tiny_sort<64>(key, sm.t, tid); break;
-                case 128: tiny_sort<128>(key, sm.t, tid); break;
-                case 256: tiny_sort<256>(key, sm.t, tid); break;
-                case 512: tiny_sort<512>(key, sm.t, tid); break;
-                default: tiny_sort<1024>(key, sm.t, tid); break;
-            }
-            fused_stamp(a, b, 2);
-            float4 my = make_float4(0.f, 0.f, 0.f, 0.f);
-            bool ok = true;
-            if (tid < K) {
-                const int id = (int)(unsigned)key;
-                int s, local, aa;
-                split_anchor_id(c, id, s, local, aa);
-                my = decode_box(c, a.hp, b, s, local, aa, anchor_geo(c, s, local, aa));
-                sm.t.sbox[tid] = my;
-                sm.t.sarea[tid] = box_area(my);
-                sm.t.sidx[tid] = id;
-                ok = box_is_fast_ok(my);
-            }
-            const bool fast = !named_bar_or(2, n2, !ok) && a.iou.fast;   // also publishes sbox / sidx
-            fused_stamp(a, b, 3);
+            const float4 my = tid < K ? sm.t.sbox[tid] : make_float4(0.f, 0.f, 0.f, 0.f);
             const int nk = fast ? tiny_greedy<0, true>(sm.t, a.iou, K, n2, keep, my, nullptr)
                                 : tiny_greedy<0, false>(sm.t, a.iou, K, n2, keep, my, nullptr);
             if (tid == 0) {
@@ -296,9 +372,10 @@ __device__ __forceinline__ void detect_fused_body(const FusedArgs &a) {
 
     // ---- 4. gather + rescale (division, face_detection.rs:477-483) into shared memory: needs no offset yet ----
     const float ds = a.det_scale[b];
-    for (int m = tid; m < M; m += FT) {
-        float4 bx;
-        float rec[CAND_REC];
+    float4 bx;
+    float rec[CAND_REC];
+    const int m = tid;   // M <= TINY_CAP == FT: one kept face per thread at most
+    if (m < M) {
         if (general) {   // kept anchor ids from the general path; boxes / landmarks / score were decoded to global memory
             const int id = keep[m];
             bx = a.cand_box[img_base + id];
@@ -309,12 +386,12 @@ __device__ __forceinline__ void detect_fused_body(const FusedArgs &a) {
         } else {
             const int rank = sm.t.krank[m];
             const int id = sm.t.sidx[rank];
+            const float *raw = sm.head[sm.slot[rank]];
             bx = sm.t.sbox[rank];
             int s, local, aa;
             split_anchor_id(c, id, s, local, aa);
-            decode_landmarks(c, a.hp, b, s, local, aa, anchor_geo(c, s, local, aa), rec);
-            const int hw = c.fh[s] * c.fw[s];
-            rec[10] = __ldg(a.hp.p[3 * s] + (size_t)b * 2 * A * hw + (size_t)(A + aa) * hw + local);
+            decode_landmarks(c, raw + 4, anchor_geo(c, s, local, aa), rec);
+            rec[10] = raw[14];
             rec[11] = 0.0f;
             a.cand_box[img_base + id] = bx;   // the lazily-run general finalize reads these for every image of the batch
             float4 *dst = reinterpret_cast<float4 *>(a.cand_rec + (img_base + id) * CAND_REC);
@@ -322,6 +399,9 @@ __device__ __forceinline__ void detect_fused_body(const FusedArgs &a) {
             dst[1] = make_float4(rec[4], rec[5], rec[6], rec[7]);
             dst[2] = make_float4(rec[8], rec[9], rec[10], rec[11]);
         }
+    }
+    __syncthreads();   // every kept face's head values are read: fdet / flmk may overwrite them
+    if (m < M) {
         float *d = sm.fdet + m * 5;
         d[0] = __fdiv_rn(bx.x, ds);
         d[1] = __fdiv_rn(bx.y, ds);
@@ -471,7 +551,7 @@ int detect_fused_launch(fd_ctx *ctx, const float *const *heads_dev, int B, float
     }
     void (*kern)(const FusedArgs) = ctx->share_sms ? detect_fused_shared_kernel : detect_fused_kernel;
     FD_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    kern<<<B, FT, smem, ctx->stream>>>(a);
+    FD_TRY(launch_pdl(ctx, kern, dim3(B), dim3(FT), smem, a));
     FD_LAUNCH_CHECK_NAMED(ctx, "detect_fused_kernel");
     if (dbg_on) {
         std::vector<long long> h(16 * (size_t)std::min(B, FUSED_DBG_IMAGES));

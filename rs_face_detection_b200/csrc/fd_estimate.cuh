@@ -19,9 +19,17 @@ struct EstConst {
 int make_est_const(const fd_ctx *ctx, EstConst *out);   // host
 
 #ifdef __CUDACC__
+// v[2 * i + o] for a runtime point index i < 5, by selects: indexing the caller's register arrays directly would move them
+// to local memory
+__device__ __forceinline__ float pick_pt(const float *v, int i, int o) {
+    float r = v[o];
+#pragma unroll
+    for (int k = 1; k < 5; ++k) r = i == k ? v[2 * k + o] : r;
+    return r;
+}
 __device__ __forceinline__ void fit2(const float *f, const float *t, int i0, int i1, double *M) {
-    double x1 = f[2 * i0], y1 = f[2 * i0 + 1], x2 = f[2 * i1], y2 = f[2 * i1 + 1];
-    double X1 = t[2 * i0], Y1 = t[2 * i0 + 1], X2 = t[2 * i1], Y2 = t[2 * i1 + 1];
+    double x1 = pick_pt(f, i0, 0), y1 = pick_pt(f, i0, 1), x2 = pick_pt(f, i1, 0), y2 = pick_pt(f, i1, 1);
+    double X1 = pick_pt(t, i0, 0), Y1 = pick_pt(t, i0, 1), X2 = pick_pt(t, i1, 0), Y2 = pick_pt(t, i1, 1);
     double d = 1. / ((x1 - x2) * (x1 - x2) + (y1 - y2) * (y1 - y2));
     double S0 = d * ((X1 - X2) * (x1 - x2) + (Y1 - Y2) * (y1 - y2));
     double S1 = d * ((Y1 - Y2) * (x1 - x2) - (X1 - X2) * (y1 - y2));

@@ -136,7 +136,7 @@ __device__ int tiny_greedy(TinySmem &sm, const IouParams iou, int K, int nthr, i
 }
 
 // Bitonic network over N2 keys, one per thread, fully unrolled: partner distance < 32 by shuffle, otherwise through the
-// double-buffered exchange array (one barrier per such stage).
+// double-buffered exchange array (one barrier per such stage).  Used by nms_cta_kernel; the fused detect kernel rank-sorts.
 template <int N2>
 __device__ __forceinline__ void tiny_sort(u64 &key, TinySmem &sm, int tid) {
     int pbuf = 0;

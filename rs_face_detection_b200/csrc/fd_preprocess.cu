@@ -45,7 +45,6 @@ __device__ __forceinline__ const uint8_t *stage_row(uint8_t *buf, const uint8_t 
 
 __global__ void preprocess_kernel(PreArgs a) {
     extern __shared__ __align__(16) unsigned char smem[];
-    const FrameDev f = a.frames[blockIdx.y];
     const int ow = a.out_w;
     float *lut = reinterpret_cast<float *>(smem);                  // [3][256], indexed by BGR channel
     int *xo0 = reinterpret_cast<int *>(lut + 768);                 // [ow]
@@ -61,6 +60,8 @@ __global__ void preprocess_kernel(PreArgs a) {
         int c = i >> 8, v = i & 255;
         lut[i] = __fdiv_rn(__fsub_rn(__fdiv_rn((float)v, a.pixel_scale), a.means[c]), a.stds[c]);  // face_detection.rs:227
     }
+    pdl_wait();   // (no early trigger: the detect kernel's CTAs would take SMs this grid still needs)
+    const FrameDev f = a.frames[blockIdx.y];
     for (int x = threadIdx.x; x < f.new_w; x += blockDim.x) x_taps(x, f.scale_x, f.w, &xo0[x], &xo1[x], &xa0[x], &xa1[x]);
     __syncthreads();
     const float pad_r = lut[2 * 256], pad_g = lut[1 * 256], pad_b = lut[0];
@@ -152,7 +153,6 @@ __global__ void __launch_bounds__(256) preprocess_tma_kernel(PreArgs a) {
     uint64_t *full = reinterpret_cast<uint64_t *>(smem);        // [PRE2_STAGES]
     float *lut = reinterpret_cast<float *>(smem + 64);          // [3][256]
     uint8_t *bufs = smem + 64 + 3072;                           // [PRE2_STAGES][2][row_buf_bytes]
-    const FrameDev f = a.frames[blockIdx.y];
     const int tid = threadIdx.x;
     const int ow = a.out_w;
     const int rb = a.row_buf_bytes;
@@ -168,6 +168,8 @@ __global__ void __launch_bounds__(256) preprocess_tma_kernel(PreArgs a) {
             lut[i] = __fdiv_rn(__fsub_rn(__fdiv_rn((float)v, a.pixel_scale), a.means[c]), a.stds[c]);
         }
     }
+    pdl_wait();   // (no early trigger: the detect kernel's CTAs would take SMs this grid still needs)
+    const FrameDev f = a.frames[blockIdx.y];
     // x taps of this thread's 4 pixels, in registers
     int x0[4];
     short wa0[4], wa1[4];
@@ -382,13 +384,9 @@ int preprocess_launch(fd_ctx *ctx, const FrameDev *frames_dev, int B, float *out
         if (smem <= (size_t)ctx->max_smem_optin) {
             int threads = std::max(32, ((ngroups + 31) / 32) * 32);
             dim3 grid((a.out_h + PRE2_ROWS - 1) / PRE2_ROWS, B);
-            if (ident) {
-                FD_CUDA(cudaFuncSetAttribute(preprocess_tma_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-                preprocess_tma_kernel<true><<<grid, threads, smem, ctx->stream>>>(a);
-            } else {
-                FD_CUDA(cudaFuncSetAttribute(preprocess_tma_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-                preprocess_tma_kernel<false><<<grid, threads, smem, ctx->stream>>>(a);
-            }
+            void (*kern)(PreArgs) = ident ? preprocess_tma_kernel<true> : preprocess_tma_kernel<false>;
+            FD_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            FD_TRY(launch_pdl(ctx, kern, grid, dim3(threads), smem, a));
             FD_LAUNCH_CHECK_NAMED(ctx, "preprocess_tma_kernel");
             return FD_OK;
         }
@@ -400,7 +398,7 @@ int preprocess_launch(fd_ctx *ctx, const FrameDev *frames_dev, int B, float *out
     FD_CUDA(cudaFuncSetAttribute(preprocess_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int threads = std::min(1024, std::max(64, ((ngroups + 31) / 32) * 32));
     dim3 grid((a.out_h + PRE_ROWS - 1) / PRE_ROWS, B);
-    preprocess_kernel<<<grid, threads, smem, ctx->stream>>>(a);
+    FD_TRY(launch_pdl(ctx, preprocess_kernel, grid, dim3(threads), smem, a));
     FD_LAUNCH_CHECK_NAMED(ctx, "preprocess_kernel");
     return FD_OK;
 }
