@@ -59,6 +59,16 @@ typedef struct fd_frame {
     int32_t height, width, pitch;
 } fd_frame;
 
+/* Frame descriptor: NV12 video frame (a hardware decoder's output): a height x width Y plane and a height/2 x width plane of
+ * interleaved U,V pairs, each row `pitch_*` bytes apart.  Device pointers; the planes may be separate allocations.  Width and
+ * height must be even (cv::cvtColor rejects odd sizes).  The *_nv12 calls give the results of their BGR counterparts on the
+ * frame cv::cvtColor(COLOR_YUV2BGR_NV12) makes (BT.601 limited range), without building it. */
+struct fd_frame_nv12 {
+    const uint8_t *y, *uv;
+    int32_t height, width, pitch_y, pitch_uv;
+};
+typedef struct fd_frame_nv12 fd_frame_nv12;
+
 /* ---- library / context ---------------------------------------------------------------------------- */
 int fd_abi_version(void);
 const char *fd_last_error(void);
@@ -181,6 +191,10 @@ int fd_nms_device(fd_ctx *ctx, const float *dets_dev, int K, float thresh, int32
 /* frames: HOST array of B descriptors whose .data are DEV pointers.  out_nchw_dev (B,3,image_h,image_w) f32.
  * det_scale_host (B) is written before return (pure host arithmetic). */
 int fd_preprocess_batch(fd_ctx *ctx, const fd_frame *frames, int B, float *out_nchw_dev, float *det_scale_host);
+/* fd_preprocess_batch on NV12 frames: the tensor and det_scale of cv::cvtColor(COLOR_YUV2BGR_NV12) followed by
+ * fd_preprocess_batch, reading only the Y and UV rows the resize taps.  FD_ERR_INVALID for an odd width or height, a pitch
+ * below the width or a null plane. */
+int fd_preprocess_batch_nv12(fd_ctx *ctx, const fd_frame_nv12 *frames, int B, float *out_nchw_dev, float *det_scale_host);
 /* heads_dev[3*s+0..2]: (B,2A,H,W), (B,4A,H,W), (B,10A,H,W) dev tensors of stride s.  Results stay on the device
  * inside the ctx until fd_detect_fetch / fd_align_detections.  Asynchronous.  Images with more than 4096 candidates
  * (and, the first time a ctx meets one, images with more than 1024) are completed by fd_detect_fetch / fd_detect_view;
@@ -211,10 +225,18 @@ int fd_detect_last_stats(fd_ctx *ctx, int32_t *out);
  * 1 = similarity warp, 2 = bbox-crop fallback (face_alignment.rs:64-116), 0 = the reference returns Err (crop zero-filled). */
 int fd_align_batch(fd_ctx *ctx, const fd_frame *frames, int B, const float *landmarks_dev, const int32_t *frame_idx_dev,
                    const float *bbox_dev, int F, uint8_t *crops_dev, double *M_dev, uint8_t *ok_dev);
+/* fd_align_batch on NV12 frames: crops, M and modes of cv::cvtColor(COLOR_YUV2BGR_NV12) followed by fd_align_batch
+ * (BORDER_CONSTANT is black in BGR). */
+int fd_align_batch_nv12(fd_ctx *ctx, const fd_frame_nv12 *frames, int B, const float *landmarks_dev, const int32_t *frame_idx_dev,
+                        const float *bbox_dev, int F, uint8_t *crops_dev, double *M_dev, uint8_t *ok_dev);
 /* Aligns every detection of the last fd_detect_batch without a host round trip (fallback box = the detection's own box).
  * crops_dev has room for cap_faces crops; detections beyond cap_faces are not aligned (fd_detect_fetch still reports them). */
 int fd_align_detections(fd_ctx *ctx, const fd_frame *frames, int B, uint8_t *crops_dev, int cap_faces, double *M_dev,
                         uint8_t *ok_dev);
+/* fd_align_detections on NV12 frames: the results of cv::cvtColor(COLOR_YUV2BGR_NV12) followed by fd_align_detections,
+ * re-run on the NV12 frames by fd_detect_fetch / fd_detect_view when deferred images change the detections. */
+int fd_align_detections_nv12(fd_ctx *ctx, const fd_frame_nv12 *frames, int B, uint8_t *crops_dev, int cap_faces, double *M_dev,
+                             uint8_t *ok_dev);
 
 /* ---- SURVEY 8(f) N1: post-align model preprocessors, fused onto the aligned crops ----------------------- */
 /* FaceExtraction::_preprocess (face_extraction.rs:38-77: mean 127.5, mul 0.0078125), FaceQuality::call
@@ -254,10 +276,16 @@ int fd_face_selection(fd_ctx *ctx, int img_h, int img_w, const float *face_boxes
  * {row of the selected detection, row of its key points} as rows of the fd_detect_fetch arrays (-1 = None).  With sel_host
  * the call blocks (and first completes images the detect kernel deferred); without it nothing leaves the device. */
 int fd_select_detections(fd_ctx *ctx, const fd_frame *frames, int B, int is_enroll, const fd_select_params *params, int32_t *sel_host);
+/* fd_select_detections on NV12 frames (the selection reads only their sizes): the selections of
+ * cv::cvtColor(COLOR_YUV2BGR_NV12) followed by fd_select_detections. */
+int fd_select_detections_nv12(fd_ctx *ctx, const fd_frame_nv12 *frames, int B, int is_enroll, const fd_select_params *params,
+                              int32_t *sel_host);
 /* FaceAlignment::call on the selection of the last fd_select_detections (face_pipeline/pipeline.rs:216-232): one crop per
  * image, crops_dev (B,crop_h,crop_w,3); images without a selection or without key points (the reference's call(.., None)
  * returns Err) get ok = 0 and a zero crop; ok = 2 marks the bbox-crop fallback on the selected box.  M_dev (B,6) / ok_dev (B) optional. */
 int fd_align_selected(fd_ctx *ctx, const fd_frame *frames, int B, uint8_t *crops_dev, double *M_dev, uint8_t *ok_dev);
+/* fd_align_selected on NV12 frames: the results of cv::cvtColor(COLOR_YUV2BGR_NV12) followed by fd_align_selected. */
+int fd_align_selected_nv12(fd_ctx *ctx, const fd_frame_nv12 *frames, int B, uint8_t *crops_dev, double *M_dev, uint8_t *ok_dev);
 
 /* ---- SURVEY 8(f) N4: utils::byte_data_to_opencv (utils.rs:8-52 = cv::imdecode(bytes, IMREAD_UNCHANGED)), baseline JPEG ------- */
 /* Host-only header parse: image size and luma sampling (11 = 4:4:4, 21 = 4:2:2, 22 = 4:2:0).  FD_ERR_INVALID for streams the

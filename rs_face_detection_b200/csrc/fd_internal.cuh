@@ -48,10 +48,12 @@ struct PinnedBuf {
 
 // Per-frame descriptor as the kernels see it.
 struct FrameDev {
-    const uint8_t *data;
+    const uint8_t *data;     // BGR pixels, or the Y plane of an NV12 frame
     int h, w, pitch;
     int new_w, new_h;        // letterbox content size
     double scale_x, scale_y; // cv::resize inverse scales
+    const uint8_t *uv;       // NV12: the interleaved U,V plane (h/2 rows of w bytes); nullptr for a BGR frame
+    int pitch_uv;
 };
 
 // Decode geometry passed by value to kernels.
@@ -92,6 +94,7 @@ struct fd_ctx {
 
     // batched pipeline state
     fd::DevBuf frames_dev;       // FrameDev[B]
+    bool frames_nv12 = false;    // frames_dev describes NV12 frames (the kernels reading it take their NV12 variants)
     fd::DevBuf det_scale_dev;    // float[B]
     fd::DevBuf cand_count;       // int[B] (+ error flags)
     fd::DevBuf cand_keys;        // u64[B][total_anchors]
@@ -254,7 +257,8 @@ __device__ __forceinline__ bool box_is_fast_ok(float4 b) {
 #endif  // __CUDACC__
 
 // stage entry points implemented across the .cu files
-int preprocess_launch(fd_ctx *ctx, const FrameDev *frames_dev, int B, float *out_nchw_dev, int max_row_bytes, bool rows_aligned16);
+int preprocess_launch(fd_ctx *ctx, const FrameDev *frames_dev, int B, float *out_nchw_dev, int max_row_bytes, bool rows_aligned16,
+                      bool nv12);
 int resize_launch(fd_ctx *ctx, const FrameDev &frame, uint8_t *out_dev, int out_h, int out_w);
 int crops_to_tensor_launch(fd_ctx *ctx, const uint8_t *crops_dev, const int *count_dev, int F, int in_h, int in_w, int out_h,
                            int out_w, const float *mean_rgb, const float *mul_rgb, float *out_dev);
@@ -283,6 +287,7 @@ struct WarpFallback {
     uint8_t *mode_out = nullptr;   // optional device (F): 1 warp, 2 fallback crop, 0 the reference returns Err (zero crop)
 };
 int warp_launch(fd_ctx *ctx, const FrameDev *frames_dev, const int32_t *frame_idx_dev, const double *M12_dev,
-                const uint8_t *ok_dev, const int *count_dev, int F_cap, uint8_t *crops_dev, int cw, int ch, const WarpFallback &fb);
+                const uint8_t *ok_dev, const int *count_dev, int F_cap, uint8_t *crops_dev, int cw, int ch, const WarpFallback &fb,
+                bool nv12);
 
 }  // namespace fd

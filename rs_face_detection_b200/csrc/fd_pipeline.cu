@@ -41,37 +41,66 @@ static void letterbox(int h, int w, int size_w, int size_h, int *new_w, int *new
     *det_scale = ds;
 }
 
-static int fill_frame(const fd_ctx *ctx, const fd_frame &fr, const uint8_t *data_dev, FrameDev *out, float *det_scale) {
-    FD_REQUIRE(fr.height > 0 && fr.width > 0 && fr.pitch >= fr.width * 3, "frame: bad geometry");
-    out->data = data_dev;
-    out->h = fr.height;
-    out->w = fr.width;
-    out->pitch = fr.pitch;
+// letterbox geometry of an h x w frame (out->h, out->w, new_w, new_h, scales)
+static int fill_geometry(const fd_ctx *ctx, int height, int width, FrameDev *out, float *det_scale) {
+    out->h = height;
+    out->w = width;
     float ds;
-    letterbox(fr.height, fr.width, ctx->cfg.image_w, ctx->cfg.image_h, &out->new_w, &out->new_h, &ds);
+    letterbox(height, width, ctx->cfg.image_w, ctx->cfg.image_h, &out->new_w, &out->new_h, &ds);
     // cv::resize rejects an empty destination size (the reference returns Err, face_detection.rs:156-159)
     FD_REQUIRE(out->new_w > 0 && out->new_h > 0, "frame: letterbox size is empty (extreme aspect ratio)");
     out->new_w = std::min(out->new_w, ctx->cfg.image_w);
     out->new_h = std::min(out->new_h, ctx->cfg.image_h);
-    out->scale_x = 1.0 / ((double)out->new_w / fr.width);
-    out->scale_y = 1.0 / ((double)out->new_h / fr.height);
+    out->scale_x = 1.0 / ((double)out->new_w / width);
+    out->scale_y = 1.0 / ((double)out->new_h / height);
     if (det_scale) *det_scale = ds;
     return FD_OK;
 }
 
-// uploads B descriptors (frames[].data are device pointers); returns the widest source row in bytes
-static int upload_frame_table(fd_ctx *ctx, const fd_frame *frames, int B, float *det_scale_host, int *max_row_bytes) {
+static int fill_frame(const fd_ctx *ctx, const fd_frame &fr, const uint8_t *data_dev, FrameDev *out, float *det_scale) {
+    FD_REQUIRE(fr.height > 0 && fr.width > 0 && fr.pitch >= fr.width * 3, "frame: bad geometry");
+    out->data = data_dev;
+    out->pitch = fr.pitch;
+    return fill_geometry(ctx, fr.height, fr.width, out, det_scale);
+}
+
+// cv::cvtColor(COLOR_YUV2BGR_NV12) accepts even sizes only
+static int fill_frame_nv12(const fd_ctx *ctx, const fd_frame_nv12 &fr, FrameDev *out, float *det_scale) {
+    FD_REQUIRE(fr.y && fr.uv, "frame (NV12): null plane");
+    FD_REQUIRE(fr.height > 0 && fr.width > 0 && fr.height % 2 == 0 && fr.width % 2 == 0 && fr.pitch_y >= fr.width && fr.pitch_uv >= fr.width,
+               "frame (NV12): bad geometry (width and height must be even, pitches at least the width)");
+    out->data = fr.y;
+    out->pitch = fr.pitch_y;
+    out->uv = fr.uv;
+    out->pitch_uv = fr.pitch_uv;
+    return fill_geometry(ctx, fr.height, fr.width, out, det_scale);
+}
+
+// The frames of a batched call: BGR (bgr) or NV12 (nv12), device pointers; exactly one is set.
+struct FrameList {
+    const fd_frame *bgr = nullptr;
+    const fd_frame_nv12 *nv12 = nullptr;
+};
+
+// uploads B descriptors; returns the widest staged source row in bytes (BGR: 3w, NV12: w)
+static int upload_frame_table(fd_ctx *ctx, FrameList frames, int B, float *det_scale_host, int *max_row_bytes) {
     std::vector<FrameDev> tab(B);
     int mrb = 0;
     for (int i = 0; i < B; ++i) {
-        FD_REQUIRE(frames[i].data != nullptr, "frame: null data");
         float ds;
         memset(&tab[i], 0, sizeof(FrameDev));
-        FD_TRY(fill_frame(ctx, frames[i], frames[i].data, &tab[i], &ds));
+        if (frames.nv12) {
+            FD_TRY(fill_frame_nv12(ctx, frames.nv12[i], &tab[i], &ds));
+            mrb = std::max(mrb, frames.nv12[i].width);
+        } else {
+            FD_REQUIRE(frames.bgr[i].data != nullptr, "frame: null data");
+            FD_TRY(fill_frame(ctx, frames.bgr[i], frames.bgr[i].data, &tab[i], &ds));
+            mrb = std::max(mrb, frames.bgr[i].width * 3);
+        }
         if (det_scale_host) det_scale_host[i] = ds;
-        mrb = std::max(mrb, frames[i].width * 3);
     }
     if (max_row_bytes) *max_row_bytes = mrb;
+    ctx->frames_nv12 = frames.nv12 != nullptr;
     const size_t bytes = sizeof(FrameDev) * (size_t)B;
     // the table already on the device is reused when nothing changed (steady-state streaming over a frame ring)
     if (ctx->frames_shadow.size() == bytes && memcmp(ctx->frames_shadow.data(), tab.data(), bytes) == 0) return FD_OK;
@@ -88,7 +117,8 @@ static int upload_frame_table(fd_ctx *ctx, const fd_frame *frames, int B, float 
 // from_detect: the faces are the detections of the last fd_detect_batch; when the fused detect kernel already estimated
 // their transforms (ctx->est_valid) and they all fit, the estimate launch is skipped.
 // fb: the bbox rows / selection of the fallback (face_alignment.rs:64-116); ok_dev receives the per-face mode (0/1/2).
-static int align_enqueue(fd_ctx *ctx, const FrameDev *frames_dev, const float *lmk_dev, const int32_t *frame_idx_dev,
+// The frames are those of the table in ctx->frames_dev, in its format (ctx->frames_nv12).
+static int align_enqueue(fd_ctx *ctx, const float *lmk_dev, const int32_t *frame_idx_dev,
                          const int *count_dev, int F_cap, uint8_t *crops_dev, double *M_dev, uint8_t *ok_dev, bool from_detect,
                          WarpFallback fb) {
     if (F_cap <= 0) return FD_OK;
@@ -101,8 +131,8 @@ static int align_enqueue(fd_ctx *ctx, const FrameDev *frames_dev, const float *l
         FD_TRY(estimate_launch(ctx, lmk_dev, nullptr, count_dev, F_cap, ctx->align_M.as<double>(), M_dev, ctx->align_ok.as<uint8_t>(), nullptr));
     }
     fb.mode_out = ok_dev;
-    FD_TRY(warp_launch(ctx, frames_dev, frame_idx_dev, ctx->align_M.as<double>(), ctx->align_ok.as<uint8_t>(), count_dev, F_cap,
-                       crops_dev, ctx->cfg.crop_w, ctx->cfg.crop_h, fb));
+    FD_TRY(warp_launch(ctx, ctx->frames_dev.as<FrameDev>(), frame_idx_dev, ctx->align_M.as<double>(), ctx->align_ok.as<uint8_t>(), count_dev,
+                       F_cap, crops_dev, ctx->cfg.crop_w, ctx->cfg.crop_h, fb, ctx->frames_nv12));
     return FD_OK;
 }
 
@@ -133,8 +163,8 @@ static int detect_resolve(fd_ctx *ctx) {
         }
         FD_TRY(finalize_launch(ctx, B));
         ctx->est_valid = false;
-        if (ctx->align_replay)  // the crops were produced from incomplete detections: align again
-            FD_TRY(align_enqueue(ctx, ctx->frames_dev.as<FrameDev>(), ctx->out_lmk.as<float>(), ctx->out_frame_idx.as<int32_t>(),
+        if (ctx->align_replay)  // the crops were produced from incomplete detections: align again (BGR or NV12, as the table)
+            FD_TRY(align_enqueue(ctx, ctx->out_lmk.as<float>(), ctx->out_frame_idx.as<int32_t>(),
                                  ctx->status() + 2, ctx->align_cap, ctx->align_crops, ctx->align_M_out, ctx->align_ok_out, true,
                                  detect_fallback(ctx)));
         FD_TRY(wait_stream(ctx));
@@ -208,17 +238,36 @@ FD_EXPORT int fd_letterbox_geometry(const fd_ctx *ctx, int img_h, int img_w, int
     return FD_OK;
 }
 
-FD_EXPORT int fd_preprocess_batch(fd_ctx *ctx, const fd_frame *frames, int B, float *out_nchw_dev, float *det_scale_host) {
+static int preprocess_batch(fd_ctx *ctx, FrameList frames, int B, float *out_nchw_dev, float *det_scale_host) {
     FD_TRY(check_ctx(ctx));
-    FD_REQUIRE(B >= 0 && (B == 0 || (frames && out_nchw_dev)), "fd_preprocess_batch: bad arguments");
+    FD_REQUIRE(B >= 0 && (B == 0 || ((frames.bgr || frames.nv12) && out_nchw_dev)), "fd_preprocess_batch: bad arguments");
     if (B == 0) return FD_OK;
     int mrb = 0;
     FD_TRY(upload_frame_table(ctx, frames, B, det_scale_host, &mrb));
     bool aligned = true;  // bulk-TMA staging needs 16-byte aligned rows that can be over-read to a 16-byte multiple
-    for (int i = 0; i < B; ++i)
-        aligned = aligned && (reinterpret_cast<uintptr_t>(frames[i].data) % 16 == 0) && (frames[i].pitch % 16 == 0) &&
-                  (((frames[i].width * 3 + 15) & ~15) <= frames[i].pitch);
-    return preprocess_launch(ctx, ctx->frames_dev.as<FrameDev>(), B, out_nchw_dev, mrb, aligned);
+    auto row_ok = [](const uint8_t *p, int pitch, int row_bytes) {
+        return reinterpret_cast<uintptr_t>(p) % 16 == 0 && pitch % 16 == 0 && ((row_bytes + 15) & ~15) <= pitch;
+    };
+    for (int i = 0; i < B; ++i) {
+        if (frames.nv12) {
+            const fd_frame_nv12 &f = frames.nv12[i];
+            aligned = aligned && row_ok(f.y, f.pitch_y, f.width) && row_ok(f.uv, f.pitch_uv, f.width);
+        } else {
+            aligned = aligned && row_ok(frames.bgr[i].data, frames.bgr[i].pitch, frames.bgr[i].width * 3);
+        }
+    }
+    return preprocess_launch(ctx, ctx->frames_dev.as<FrameDev>(), B, out_nchw_dev, mrb, aligned, frames.nv12 != nullptr);
+}
+
+FD_EXPORT int fd_preprocess_batch(fd_ctx *ctx, const fd_frame *frames, int B, float *out_nchw_dev, float *det_scale_host) {
+    FrameList fl;
+    fl.bgr = frames;
+    return preprocess_batch(ctx, fl, B, out_nchw_dev, det_scale_host);
+}
+FD_EXPORT int fd_preprocess_batch_nv12(fd_ctx *ctx, const fd_frame_nv12 *frames, int B, float *out_nchw_dev, float *det_scale_host) {
+    FrameList fl;
+    fl.nv12 = frames;
+    return preprocess_batch(ctx, fl, B, out_nchw_dev, det_scale_host);
 }
 
 FD_EXPORT int fd_detect_batch(fd_ctx *ctx, const float *const *heads_dev, int n_heads, int B, const float *det_scale_host,
@@ -285,22 +334,34 @@ FD_EXPORT int fd_detect_last_stats(fd_ctx *ctx, int32_t *out) {
     return FD_OK;
 }
 
-FD_EXPORT int fd_align_batch(fd_ctx *ctx, const fd_frame *frames, int B, const float *landmarks_dev, const int32_t *frame_idx_dev,
-                             const float *bbox_dev, int F, uint8_t *crops_dev, double *M_dev, uint8_t *ok_dev) {
+static int align_batch(fd_ctx *ctx, FrameList frames, int B, const float *landmarks_dev, const int32_t *frame_idx_dev,
+                       const float *bbox_dev, int F, uint8_t *crops_dev, double *M_dev, uint8_t *ok_dev) {
     FD_TRY(check_ctx(ctx));
-    FD_REQUIRE(B > 0 && frames && F >= 0 && (F == 0 || (landmarks_dev && crops_dev)), "fd_align_batch: bad arguments");
+    FD_REQUIRE(B > 0 && (frames.bgr || frames.nv12) && F >= 0 && (F == 0 || (landmarks_dev && crops_dev)), "fd_align_batch: bad arguments");
     if (F == 0) return FD_OK;
     FD_TRY(upload_frame_table(ctx, frames, B, nullptr, nullptr));
     WarpFallback fb;
     fb.bbox = bbox_dev;
     fb.bbox_stride = 4;
-    return align_enqueue(ctx, ctx->frames_dev.as<FrameDev>(), landmarks_dev, frame_idx_dev, nullptr, F, crops_dev, M_dev, ok_dev, false, fb);
+    return align_enqueue(ctx, landmarks_dev, frame_idx_dev, nullptr, F, crops_dev, M_dev, ok_dev, false, fb);
 }
 
-FD_EXPORT int fd_align_detections(fd_ctx *ctx, const fd_frame *frames, int B, uint8_t *crops_dev, int cap_faces, double *M_dev,
-                                  uint8_t *ok_dev) {
+FD_EXPORT int fd_align_batch(fd_ctx *ctx, const fd_frame *frames, int B, const float *landmarks_dev, const int32_t *frame_idx_dev,
+                             const float *bbox_dev, int F, uint8_t *crops_dev, double *M_dev, uint8_t *ok_dev) {
+    FrameList fl;
+    fl.bgr = frames;
+    return align_batch(ctx, fl, B, landmarks_dev, frame_idx_dev, bbox_dev, F, crops_dev, M_dev, ok_dev);
+}
+FD_EXPORT int fd_align_batch_nv12(fd_ctx *ctx, const fd_frame_nv12 *frames, int B, const float *landmarks_dev, const int32_t *frame_idx_dev,
+                                  const float *bbox_dev, int F, uint8_t *crops_dev, double *M_dev, uint8_t *ok_dev) {
+    FrameList fl;
+    fl.nv12 = frames;
+    return align_batch(ctx, fl, B, landmarks_dev, frame_idx_dev, bbox_dev, F, crops_dev, M_dev, ok_dev);
+}
+
+static int align_detections(fd_ctx *ctx, FrameList frames, int B, uint8_t *crops_dev, int cap_faces, double *M_dev, uint8_t *ok_dev) {
     FD_TRY(check_ctx(ctx));
-    FD_REQUIRE(B > 0 && frames && B == ctx->last_B && crops_dev && cap_faces > 0, "fd_align_detections: bad arguments");
+    FD_REQUIRE(B > 0 && (frames.bgr || frames.nv12) && B == ctx->last_B && crops_dev && cap_faces > 0, "fd_align_detections: bad arguments");
     // No host synchronisation here: images needing the big NMS path are detected lazily at
     // fd_detect_fetch / fd_detect_view / fd_ctx-level fetch, which replays this align if the detections changed.
     FD_TRY(upload_frame_table(ctx, frames, B, nullptr, nullptr));
@@ -309,8 +370,21 @@ FD_EXPORT int fd_align_detections(fd_ctx *ctx, const fd_frame *frames, int B, ui
     ctx->align_cap = cap_faces;
     ctx->align_M_out = M_dev;
     ctx->align_ok_out = ok_dev;
-    return align_enqueue(ctx, ctx->frames_dev.as<FrameDev>(), ctx->out_lmk.as<float>(), ctx->out_frame_idx.as<int32_t>(),
-                         ctx->status() + 2, cap_faces, crops_dev, M_dev, ok_dev, true, detect_fallback(ctx));
+    return align_enqueue(ctx, ctx->out_lmk.as<float>(), ctx->out_frame_idx.as<int32_t>(), ctx->status() + 2, cap_faces, crops_dev, M_dev,
+                         ok_dev, true, detect_fallback(ctx));
+}
+
+FD_EXPORT int fd_align_detections(fd_ctx *ctx, const fd_frame *frames, int B, uint8_t *crops_dev, int cap_faces, double *M_dev,
+                                  uint8_t *ok_dev) {
+    FrameList fl;
+    fl.bgr = frames;
+    return align_detections(ctx, fl, B, crops_dev, cap_faces, M_dev, ok_dev);
+}
+FD_EXPORT int fd_align_detections_nv12(fd_ctx *ctx, const fd_frame_nv12 *frames, int B, uint8_t *crops_dev, int cap_faces, double *M_dev,
+                                       uint8_t *ok_dev) {
+    FrameList fl;
+    fl.nv12 = frames;
+    return align_detections(ctx, fl, B, crops_dev, cap_faces, M_dev, ok_dev);
 }
 
 // ---- single-image host wrappers -----------------------------------------------------------------------------------
@@ -447,7 +521,7 @@ static int warp_host(fd_ctx *ctx, const uint8_t *img, int h, int w, int pitch, c
     const size_t n = (size_t)out_h * out_w * 3;
     FD_TRY(ctx->scratch[4].reserve(n));
     FD_TRY(warp_launch(ctx, ctx->scratch[5].as<FrameDev>(), nullptr, ctx->align_M.as<double>(), ctx->align_ok.as<uint8_t>(), nullptr, 1,
-                       ctx->scratch[4].as<uint8_t>(), out_w, out_h, fb));
+                       ctx->scratch[4].as<uint8_t>(), out_w, out_h, fb, false));
     uint8_t mode = 0;
     double M12[12];
     FD_CUDA(cudaMemcpyAsync(out, ctx->scratch[4].p, n, cudaMemcpyDeviceToHost, ctx->stream));
@@ -572,9 +646,9 @@ FD_EXPORT int fd_face_selection(fd_ctx *ctx, int img_h, int img_w, const float *
     return FD_OK;
 }
 
-FD_EXPORT int fd_select_detections(fd_ctx *ctx, const fd_frame *frames, int B, int is_enroll, const fd_select_params *params, int32_t *sel_host) {
+static int select_detections(fd_ctx *ctx, FrameList frames, int B, int is_enroll, const fd_select_params *params, int32_t *sel_host) {
     FD_TRY(check_ctx(ctx));
-    FD_REQUIRE(frames && B > 0 && B == ctx->last_B, "fd_select_detections: needs the frames of the last fd_detect_batch");
+    FD_REQUIRE((frames.bgr || frames.nv12) && B > 0 && B == ctx->last_B, "fd_select_detections: needs the frames of the last fd_detect_batch");
     if (sel_host) FD_TRY(detect_resolve(ctx));
     fd_select_params p;
     if (params) p = *params;
@@ -593,17 +667,40 @@ FD_EXPORT int fd_select_detections(fd_ctx *ctx, const fd_frame *frames, int B, i
     return FD_OK;
 }
 
-FD_EXPORT int fd_align_selected(fd_ctx *ctx, const fd_frame *frames, int B, uint8_t *crops_dev, double *M_dev, uint8_t *ok_dev) {
+FD_EXPORT int fd_select_detections(fd_ctx *ctx, const fd_frame *frames, int B, int is_enroll, const fd_select_params *params, int32_t *sel_host) {
+    FrameList fl;
+    fl.bgr = frames;
+    return select_detections(ctx, fl, B, is_enroll, params, sel_host);
+}
+FD_EXPORT int fd_select_detections_nv12(fd_ctx *ctx, const fd_frame_nv12 *frames, int B, int is_enroll, const fd_select_params *params,
+                                        int32_t *sel_host) {
+    FrameList fl;
+    fl.nv12 = frames;
+    return select_detections(ctx, fl, B, is_enroll, params, sel_host);
+}
+
+static int align_selected(fd_ctx *ctx, FrameList frames, int B, uint8_t *crops_dev, double *M_dev, uint8_t *ok_dev) {
     FD_TRY(check_ctx(ctx));
-    FD_REQUIRE(frames && B > 0 && B == ctx->select_B && crops_dev, "fd_align_selected: needs the frames of the last fd_select_detections");
+    FD_REQUIRE((frames.bgr || frames.nv12) && B > 0 && B == ctx->select_B && crops_dev,
+               "fd_align_selected: needs the frames of the last fd_select_detections");
     FD_TRY(upload_frame_table(ctx, frames, B, nullptr, nullptr));
     // Images without a selection (or whose selection has no key points) carry NaN key points: the estimate fails there and,
     // as the reference's call(&image, box, None) errs on the empty landmark Mat, the crop is zero-filled with ok = 0; a
     // selection whose key points are degenerate takes the bbox-crop fallback on its selected box (ok = 2).
     WarpFallback fb = detect_fallback(ctx);
     fb.sel = ctx->select_sel.as<int>();
-    return align_enqueue(ctx, ctx->frames_dev.as<FrameDev>(), ctx->select_lmk.as<float>(), ctx->select_fidx.as<int32_t>(), nullptr, B, crops_dev,
-                         M_dev, ok_dev, false, fb);
+    return align_enqueue(ctx, ctx->select_lmk.as<float>(), ctx->select_fidx.as<int32_t>(), nullptr, B, crops_dev, M_dev, ok_dev, false, fb);
+}
+
+FD_EXPORT int fd_align_selected(fd_ctx *ctx, const fd_frame *frames, int B, uint8_t *crops_dev, double *M_dev, uint8_t *ok_dev) {
+    FrameList fl;
+    fl.bgr = frames;
+    return align_selected(ctx, fl, B, crops_dev, M_dev, ok_dev);
+}
+FD_EXPORT int fd_align_selected_nv12(fd_ctx *ctx, const fd_frame_nv12 *frames, int B, uint8_t *crops_dev, double *M_dev, uint8_t *ok_dev) {
+    FrameList fl;
+    fl.nv12 = frames;
+    return align_selected(ctx, fl, B, crops_dev, M_dev, ok_dev);
 }
 
 // ---- end-to-end with host buffers ------------------------------------------------------------------------------------
@@ -918,10 +1015,12 @@ static int pipeline_host_impl(fd_ctx *ctx, const fd_frame *frames, const fd_fram
                     }
                 }
             }
-            FD_TRY(upload_frame_table(ctx, dframes.data(), B, nullptr, nullptr));
+            FrameList fl;
+            fl.bgr = dframes.data();
+            FD_TRY(upload_frame_table(ctx, fl, B, nullptr, nullptr));
             fb.mode_out = mode_dev;
             FD_TRY(warp_launch(ctx, frames_dev, fidx_dev, ctx->align_M.as<double>(), ctx->align_ok.as<uint8_t>(), nullptr,
-                               std::min(F, (int)out->cap_rows), crops_dev, cw, ch, fb));
+                               std::min(F, (int)out->cap_rows), crops_dev, cw, ch, fb, false));
             ctx->align_replay = false;
         }
         if (select && out->sel) {

@@ -43,6 +43,9 @@ __device__ __forceinline__ const uint8_t *stage_row(uint8_t *buf, const uint8_t 
     return dst;
 }
 
+// NV: the frame is NV12 (FrameDev::uv); each tap is converted to BGR (yuv_bgr24) before the resize arithmetic, and the
+// staged rows are the Y rows and the UV row(s) of the taps.
+template <bool NV>
 __global__ void preprocess_kernel(PreArgs a) {
     extern __shared__ __align__(16) unsigned char smem[];
     const int ow = a.out_w;
@@ -55,6 +58,7 @@ __global__ void preprocess_kernel(PreArgs a) {
     tab_bytes = (tab_bytes + 15) & ~(size_t)15;
     uint8_t *rowbuf0 = smem + tab_bytes;
     uint8_t *rowbuf1 = rowbuf0 + a.row_buf_bytes;
+    uint8_t *rowbuf2 = rowbuf1 + a.row_buf_bytes, *rowbuf3 = rowbuf2 + a.row_buf_bytes;   // NV: UV rows
 
     for (int i = threadIdx.x; i < 768; i += blockDim.x) {
         int c = i >> 8, v = i & 255;
@@ -62,7 +66,10 @@ __global__ void preprocess_kernel(PreArgs a) {
     }
     pdl_wait();   // (no early trigger: the detect kernel's CTAs would take SMs this grid still needs)
     const FrameDev f = a.frames[blockIdx.y];
-    for (int x = threadIdx.x; x < f.new_w; x += blockDim.x) x_taps(x, f.scale_x, f.w, &xo0[x], &xo1[x], &xa0[x], &xa1[x]);
+    for (int x = threadIdx.x; x < f.new_w; x += blockDim.x) {
+        x_taps(x, f.scale_x, f.w, &xo0[x], &xo1[x], &xa0[x], &xa1[x]);
+        if (NV) { xo0[x] /= 3; xo1[x] /= 3; }   // pixel, not byte, offsets
+    }
     __syncthreads();
     const float pad_r = lut[2 * 256], pad_g = lut[1 * 256], pad_b = lut[0];
     const size_t plane = (size_t)a.out_h * ow;
@@ -70,20 +77,24 @@ __global__ void preprocess_kernel(PreArgs a) {
     const int ngroups = (ow + 3) >> 2;
     const int row_begin = blockIdx.x * PRE_ROWS;
     const int row_end = min(row_begin + PRE_ROWS, a.out_h);
-    const int src_row_bytes = f.w * 3;
+    const int src_row_bytes = NV ? f.w : f.w * 3;
 
     for (int dy = row_begin; dy < row_end; ++dy) {
         float *o_r = out_img + (size_t)dy * ow;  // plane 0 = R (BGR channel 2), face_detection.rs:226-227
         float *o_g = o_r + plane;
         float *o_b = o_g + plane;
         const bool content = dy < f.new_h;
-        const uint8_t *r0 = nullptr, *r1 = nullptr;
+        const uint8_t *r0 = nullptr, *r1 = nullptr, *c0 = nullptr, *c1 = nullptr;
         int b0 = 0, b1 = 0;
         if (content) {
             int y0, y1;
             y_taps(dy, f.scale_y, f.h, &y0, &y1, &b0, &b1);
             r0 = stage_row(rowbuf0, f.data + (size_t)y0 * f.pitch, src_row_bytes);
             r1 = b1 != 0 ? stage_row(rowbuf1, f.data + (size_t)y1 * f.pitch, src_row_bytes) : r0;
+            if (NV) {   // one UV row when both taps share it (or the second tap has weight 0)
+                c0 = stage_row(rowbuf2, f.uv + (size_t)(y0 >> 1) * f.pitch_uv, src_row_bytes);
+                c1 = b1 != 0 && (y1 >> 1) != (y0 >> 1) ? stage_row(rowbuf3, f.uv + (size_t)(y1 >> 1) * f.pitch_uv, src_row_bytes) : c0;
+            }
             __syncthreads();
         }
         for (int g = threadIdx.x; g < ngroups; g += blockDim.x) {
@@ -93,9 +104,17 @@ __global__ void preprocess_kernel(PreArgs a) {
                 const int x = 4 * g + j;
                 if (content && x < f.new_w) {
                     const int x0 = xo0[x], x1 = xo1[x], a0 = xa0[x], a1 = xa1[x];
-                    vb[j] = lut[resize_px(r0, r1, x0, x1, a0, a1, b0, b1)];
-                    vg[j] = lut[256 + resize_px(r0, r1, x0 + 1, x1 + 1, a0, a1, b0, b1)];
-                    vr[j] = lut[512 + resize_px(r0, r1, x0 + 2, x1 + 2, a0, a1, b0, b1)];
+                    if (NV) {
+                        const unsigned p = resize_px24(nv12_px24(r0, c0, x0), nv12_px24(r0, c0, x1), b1 != 0 ? nv12_px24(r1, c1, x0) : 0u,
+                                                       b1 != 0 ? nv12_px24(r1, c1, x1) : 0u, a0, a1, b0, b1);
+                        vb[j] = lut[p & 255u];
+                        vg[j] = lut[256 + ((p >> 8) & 255u)];
+                        vr[j] = lut[512 + (p >> 16)];
+                    } else {
+                        vb[j] = lut[resize_px(r0, r1, x0, x1, a0, a1, b0, b1)];
+                        vg[j] = lut[256 + resize_px(r0, r1, x0 + 1, x1 + 1, a0, a1, b0, b1)];
+                        vr[j] = lut[512 + resize_px(r0, r1, x0 + 2, x1 + 2, a0, a1, b0, b1)];
+                    }
                 } else {
                     vb[j] = pad_b; vg[j] = pad_g; vr[j] = pad_r;
                 }
@@ -147,12 +166,15 @@ __device__ __forceinline__ void bulk_g2s(void *dst_smem, const void *src_gmem, u
                  : "memory");
 }
 
-template <bool IDENT>
+// NV: NV12 frame; a stage holds the Y rows of the taps and their UV row(s) — one when both taps map to the same UV row
+// (4K -> 640x360: rows 6y+2 and 6y+3 both read UV row 3y+1).
+template <bool IDENT, bool NV>
 __global__ void __launch_bounds__(256) preprocess_tma_kernel(PreArgs a) {
+    constexpr int SLOTS = NV ? 4 : 2;                           // rows per stage: Y0, Y1 (BGR: row 0, row 1), UV0, UV1
     extern __shared__ __align__(128) unsigned char smem[];
     uint64_t *full = reinterpret_cast<uint64_t *>(smem);        // [PRE2_STAGES]
     float *lut = reinterpret_cast<float *>(smem + 64);          // [3][256]
-    uint8_t *bufs = smem + 64 + 3072;                           // [PRE2_STAGES][2][row_buf_bytes]
+    uint8_t *bufs = smem + 64 + 3072;                           // [PRE2_STAGES][SLOTS][row_buf_bytes]
     const int tid = threadIdx.x;
     const int ow = a.out_w;
     const int rb = a.row_buf_bytes;
@@ -183,6 +205,7 @@ __global__ void __launch_bounds__(256) preprocess_tma_kernel(PreArgs a) {
         if (x < f.new_w) {
             int o1;
             x_taps(x, f.scale_x, f.w, &x0[j], &o1, &wa0[j], &wa1[j]);
+            if (NV) x0[j] /= 3;   // pixel, not byte, offset
             point &= (wa1[j] == 0);
         }
     }
@@ -194,17 +217,20 @@ __global__ void __launch_bounds__(256) preprocess_tma_kernel(PreArgs a) {
     const int row_begin = blockIdx.x * PRE2_ROWS;
     const int row_end = min(row_begin + PRE2_ROWS, a.out_h);
     const int n_content = max(0, min(f.new_h, row_end) - row_begin);
-    const uint32_t copy_bytes = (uint32_t)((f.w * 3 + 15) & ~15);
+    const uint32_t copy_bytes = (uint32_t)(((NV ? f.w : f.w * 3) + 15) & ~15);
     const bool active = 4 * tid < ow;
 
     auto issue = [&](int it) {
         int y0, y1, b0, b1;
         y_taps(row_begin + it, f.scale_y, f.h, &y0, &y1, &b0, &b1);
         const int st = it % PRE2_STAGES;
-        uint8_t *dst = bufs + (size_t)st * 2 * rb;
-        mbar_expect_tx(&full[st], b1 != 0 ? 2 * copy_bytes : copy_bytes);
+        uint8_t *dst = bufs + (size_t)st * SLOTS * rb;
+        const bool uv1 = NV && b1 != 0 && (y1 >> 1) != (y0 >> 1);
+        mbar_expect_tx(&full[st], copy_bytes * ((b1 != 0 ? 2 : 1) + (NV ? 1 : 0) + (uv1 ? 1 : 0)));
         bulk_g2s(dst, f.data + (size_t)y0 * f.pitch, copy_bytes, &full[st]);
         if (b1 != 0) bulk_g2s(dst + rb, f.data + (size_t)y1 * f.pitch, copy_bytes, &full[st]);
+        if (NV) bulk_g2s(dst + 2 * rb, f.uv + (size_t)(y0 >> 1) * f.pitch_uv, copy_bytes, &full[st]);
+        if (uv1) bulk_g2s(dst + 3 * rb, f.uv + (size_t)(y1 >> 1) * f.pitch_uv, copy_bytes, &full[st]);
     };
     if (tid == 0)
         for (int it = 0; it < PRE2_STAGES - 1 && it < n_content; ++it) issue(it);
@@ -215,8 +241,9 @@ __global__ void __launch_bounds__(256) preprocess_tma_kernel(PreArgs a) {
         int y0, y1, b0, b1;
         y_taps(dy, f.scale_y, f.h, &y0, &y1, &b0, &b1);
         const int st = it % PRE2_STAGES;
-        const uint8_t *r0 = bufs + (size_t)st * 2 * rb;
+        const uint8_t *r0 = bufs + (size_t)st * SLOTS * rb;
         const uint8_t *r1 = b1 != 0 ? r0 + rb : r0;
+        const uint8_t *c0 = r0 + 2 * rb, *c1 = b1 != 0 && (y1 >> 1) != (y0 >> 1) ? r0 + 3 * rb : c0;   // NV only
         mbar_wait(&full[st], (uint32_t)((it / PRE2_STAGES) & 1));
         if (active) {
             float vr[4], vg[4], vb[4];
@@ -224,8 +251,14 @@ __global__ void __launch_bounds__(256) preprocess_tma_kernel(PreArgs a) {
 #pragma unroll
                 for (int j = 0; j < 4; ++j) {
                     if (x0[j] >= 0) {
-                        const uint8_t *p = r0 + x0[j];
-                        const int pb = p[0], pg = p[1], pr = p[2];
+                        int pb, pg, pr;
+                        if (NV) {
+                            const unsigned p = nv12_px24(r0, c0, x0[j]);
+                            pb = p & 255u; pg = (p >> 8) & 255u; pr = p >> 16;
+                        } else {
+                            const uint8_t *p = r0 + x0[j];
+                            pb = p[0]; pg = p[1]; pr = p[2];
+                        }
                         vb[j] = IDENT ? (float)pb : lut[pb];
                         vg[j] = IDENT ? (float)pg : lut[256 + pg];
                         vr[j] = IDENT ? (float)pr : lut[512 + pr];
@@ -237,10 +270,17 @@ __global__ void __launch_bounds__(256) preprocess_tma_kernel(PreArgs a) {
 #pragma unroll
                 for (int j = 0; j < 4; ++j) {
                     if (x0[j] >= 0) {
-                        const int o0 = x0[j], o1 = x0[j] + (wa1[j] != 0 ? 3 : 0), q0 = wa0[j], q1 = wa1[j];
-                        const int pb = resize_px(r0, r1, o0, o1, q0, q1, b0, b1);
-                        const int pg = resize_px(r0, r1, o0 + 1, o1 + 1, q0, q1, b0, b1);
-                        const int pr = resize_px(r0, r1, o0 + 2, o1 + 2, q0, q1, b0, b1);
+                        const int o0 = x0[j], o1 = x0[j] + (wa1[j] != 0 ? (NV ? 1 : 3) : 0), q0 = wa0[j], q1 = wa1[j];
+                        int pb, pg, pr;
+                        if (NV) {
+                            const unsigned p = resize_px24(nv12_px24(r0, c0, o0), nv12_px24(r0, c0, o1), b1 != 0 ? nv12_px24(r1, c1, o0) : 0u,
+                                                           b1 != 0 ? nv12_px24(r1, c1, o1) : 0u, q0, q1, b0, b1);
+                            pb = p & 255u; pg = (p >> 8) & 255u; pr = p >> 16;
+                        } else {
+                            pb = resize_px(r0, r1, o0, o1, q0, q1, b0, b1);
+                            pg = resize_px(r0, r1, o0 + 1, o1 + 1, q0, q1, b0, b1);
+                            pr = resize_px(r0, r1, o0 + 2, o1 + 2, q0, q1, b0, b1);
+                        }
                         vb[j] = IDENT ? (float)pb : lut[pb];
                         vg[j] = IDENT ? (float)pg : lut[256 + pg];
                         vr[j] = IDENT ? (float)pr : lut[512 + pr];
@@ -361,7 +401,10 @@ int crops_to_tensor_launch(fd_ctx *ctx, const uint8_t *crops_dev, const int *cou
     return FD_OK;
 }
 
-int preprocess_launch(fd_ctx *ctx, const FrameDev *frames_dev, int B, float *out_nchw_dev, int max_row_bytes, bool rows_aligned16) {
+// max_row_bytes: widest staged row (BGR: 3w, NV12: w); nv12: frames_dev describes NV12 frames
+int preprocess_launch(fd_ctx *ctx, const FrameDev *frames_dev, int B, float *out_nchw_dev, int max_row_bytes, bool rows_aligned16,
+                      bool nv12) {
+    constexpr int SLOTS_NV = 4;
     PreArgs a;
     a.frames = frames_dev;
     a.out = out_nchw_dev;
@@ -380,26 +423,28 @@ int preprocess_launch(fd_ctx *ctx, const FrameDev *frames_dev, int B, float *out
     // v2 (bulk-TMA staging): 16-byte aligned source rows, vector stores, one 4-pixel group per thread
     if (rows_aligned16 && a.vec_store && ngroups <= 256) {
         a.row_buf_bytes = (max_row_bytes + 15) & ~15;
-        size_t smem = 64 + 3072 + (size_t)PRE2_STAGES * 2 * a.row_buf_bytes;
+        size_t smem = 64 + 3072 + (size_t)PRE2_STAGES * (nv12 ? SLOTS_NV : 2) * a.row_buf_bytes;
         if (smem <= (size_t)ctx->max_smem_optin) {
             int threads = std::max(32, ((ngroups + 31) / 32) * 32);
             dim3 grid((a.out_h + PRE2_ROWS - 1) / PRE2_ROWS, B);
-            void (*kern)(PreArgs) = ident ? preprocess_tma_kernel<true> : preprocess_tma_kernel<false>;
+            void (*kern)(PreArgs) = nv12 ? (ident ? preprocess_tma_kernel<true, true> : preprocess_tma_kernel<false, true>)
+                                         : (ident ? preprocess_tma_kernel<true, false> : preprocess_tma_kernel<false, false>);
             FD_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
             FD_TRY(launch_pdl(ctx, kern, grid, dim3(threads), smem, a));
-            FD_LAUNCH_CHECK_NAMED(ctx, "preprocess_tma_kernel");
+            FD_LAUNCH_CHECK_NAMED(ctx, nv12 ? "preprocess_tma_kernel_nv12" : "preprocess_tma_kernel");
             return FD_OK;
         }
     }
     size_t tab_bytes = 768 * 4 + (size_t)a.out_w * 12;
     tab_bytes = (tab_bytes + 15) & ~(size_t)15;
-    size_t smem = tab_bytes + 2 * (size_t)a.row_buf_bytes;
+    size_t smem = tab_bytes + (nv12 ? SLOTS_NV : 2) * (size_t)a.row_buf_bytes;
     if (smem > (size_t)ctx->max_smem_optin) return fail(FD_ERR_INVALID, "fd_preprocess: source row too wide for shared-memory staging");
-    FD_CUDA(cudaFuncSetAttribute(preprocess_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    void (*kern)(PreArgs) = nv12 ? preprocess_kernel<true> : preprocess_kernel<false>;
+    FD_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int threads = std::min(1024, std::max(64, ((ngroups + 31) / 32) * 32));
     dim3 grid((a.out_h + PRE_ROWS - 1) / PRE_ROWS, B);
-    FD_TRY(launch_pdl(ctx, preprocess_kernel, grid, dim3(threads), smem, a));
-    FD_LAUNCH_CHECK_NAMED(ctx, "preprocess_kernel");
+    FD_TRY(launch_pdl(ctx, kern, grid, dim3(threads), smem, a));
+    FD_LAUNCH_CHECK_NAMED(ctx, nv12 ? "preprocess_kernel_nv12" : "preprocess_kernel");
     return FD_OK;
 }
 

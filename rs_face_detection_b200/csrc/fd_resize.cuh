@@ -89,4 +89,54 @@ __device__ __forceinline__ unsigned resize_pixel24(const uint8_t *roi, int pitch
     return pb | (pg << 8) | (pr << 16);
 }
 
+// ---- NV12 sources: every tap is converted as cv::cvtColor(COLOR_YUV2BGR_NV12) would have converted the whole frame ----
+// OpenCV's BT.601 limited-range conversion (imgproc color_yuv: 20-bit fixed point, round half up, saturate), restated in
+// int32 and equal to cv2 4.13 on all 2^24 (Y,U,V) triples.  Returns b | g << 8 | r << 16.
+__device__ __forceinline__ unsigned yuv_bgr24(int Y, int U, int V) {
+    const int y = max(Y - 16, 0) * 1220542 + (1 << 19), u = U - 128, v = V - 128;
+    const int r = (y + 1673527 * v) >> 20, g = (y - 852492 * v - 409993 * u) >> 20, b = (y + 2116026 * u) >> 20;
+    return (unsigned)min(max(b, 0), 255) | ((unsigned)min(max(g, 0), 255) << 8) | ((unsigned)min(max(r, 0), 255) << 16);
+}
+// pixel x of an NV12 row: its own Y and the U,V pair of its 2x2 block (uvrow = UV plane row y/2)
+__device__ __forceinline__ unsigned nv12_px24(const uint8_t *yrow, const uint8_t *uvrow, int x) {
+    return yuv_bgr24(yrow[x], uvrow[x & ~1], uvrow[x | 1]);
+}
+
+// resize_px on the three channels of packed pixels: taps (p00, p01) of the first row, (p10, p11) of the second (read only
+// when b1 != 0)
+__device__ __forceinline__ unsigned resize_px24(unsigned p00, unsigned p01, unsigned p10, unsigned p11, int a0, int a1, int b0, int b1) {
+    unsigned out = 0;
+#pragma unroll
+    for (int c = 0; c < 24; c += 8) {
+        const int t0 = (int)((p00 >> c) & 255u) * a0 + (int)((p01 >> c) & 255u) * a1;
+        int v = (b0 * (t0 >> 4)) >> 16;
+        if (b1 != 0) {
+            const int t1 = (int)((p10 >> c) & 255u) * a0 + (int)((p11 >> c) & 255u) * a1;
+            v += (b1 * (t1 >> 4)) >> 16;
+        }
+        out |= (unsigned)((v + 2) >> 2) << c;
+    }
+    return out;
+}
+
+// resize_pixel24 of the ROI (rx0, ry0)..(rx0 + rw, ry0 + rh) of an NV12 frame: taps in ROI coordinates, chroma of the
+// frame's own 2x2 blocks (rx0, ry0 may be odd)
+__device__ __forceinline__ unsigned resize_pixel24_nv12(const uint8_t *yp, int pitch, const uint8_t *uvp, int pitch_uv, int rx0, int ry0,
+                                                        int rw, int rh, int ow, int oh, int x, int y) {
+    if (rw == ow && rh == oh) {
+        const int sy = ry0 + y;
+        return nv12_px24(yp + (size_t)sy * pitch, uvp + (size_t)(sy >> 1) * pitch_uv, rx0 + x);
+    }
+    const double scale_x = 1.0 / ((double)ow / rw), scale_y = 1.0 / ((double)oh / rh);
+    int o0, o1, y0, y1, b0, b1;
+    short a0, a1;
+    x_taps(x, scale_x, rw, &o0, &o1, &a0, &a1);
+    y_taps(y, scale_y, rh, &y0, &y1, &b0, &b1);
+    const int x0 = rx0 + o0 / 3, x1 = rx0 + o1 / 3, sy0 = ry0 + y0, sy1 = ry0 + y1;
+    const uint8_t *r0 = yp + (size_t)sy0 * pitch, *c0 = uvp + (size_t)(sy0 >> 1) * pitch_uv;
+    const uint8_t *r1 = yp + (size_t)sy1 * pitch, *c1 = uvp + (size_t)(sy1 >> 1) * pitch_uv;
+    const unsigned p10 = b1 != 0 ? nv12_px24(r1, c1, x0) : 0u, p11 = b1 != 0 ? nv12_px24(r1, c1, x1) : 0u;
+    return resize_px24(nv12_px24(r0, c0, x0), nv12_px24(r0, c0, x1), p10, p11, a0, a1, b0, b1);
+}
+
 }  // namespace fd

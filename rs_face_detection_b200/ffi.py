@@ -45,6 +45,11 @@ class FdFrame(C.Structure):
     _fields_ = [("data", C.c_void_p), ("height", C.c_int32), ("width", C.c_int32), ("pitch", C.c_int32)]
 
 
+class FdFrameNV12(C.Structure):
+    _fields_ = [("y", C.c_void_p), ("uv", C.c_void_p), ("height", C.c_int32), ("width", C.c_int32), ("pitch_y", C.c_int32),
+                ("pitch_uv", C.c_int32)]
+
+
 class FdAnchorCfg(C.Structure):
     _fields_ = [("stride", C.c_int32), ("base_size", C.c_int32), ("n_ratios", C.c_int32), ("n_scales", C.c_int32),
                 ("ratios", C.c_float * 8), ("scales", C.c_float * 8), ("allowed_border", C.c_int32)]
@@ -89,6 +94,7 @@ SYMBOLS = [
     "fd_nms_device", "fd_preprocess_batch", "fd_detect_batch", "fd_detect_fetch", "fd_detect_view", "fd_detect_last_stats", "fd_align_batch",
     "fd_align_detections", "fd_crops_to_tensor", "fd_model_preprocess", "fd_detect_batch_raw", "fd_select_params_default", "fd_face_selection",
     "fd_select_detections", "fd_align_selected", "fd_jpeg_info", "fd_decode_jpeg_batch", "fd_jpeg_last_stats", "fd_imdecode", "fd_pipeline_opts_default", "fd_pipeline_host", "fd_pipeline_host_jpeg", "fd_pipeline_tensor_dev",
+    "fd_preprocess_batch_nv12", "fd_align_batch_nv12", "fd_align_detections_nv12", "fd_select_detections_nv12", "fd_align_selected_nv12",
 ]
 
 _lib = None
@@ -495,6 +501,19 @@ class Context:
             arr[i].data, arr[i].height, arr[i].width, arr[i].pitch = _devptr(p), h, w, pitch
         return arr
 
+    @staticmethod
+    def _frames_nv12(frames):
+        """frames: list of (y_dev_ptr, uv_dev_ptr, h, w, pitch_y, pitch_uv), or an fd_frame_nv12 array from frame_table_nv12()"""
+        if isinstance(frames, C.Array):
+            return frames
+        arr = (FdFrameNV12 * len(frames))()
+        for i, (y, uv, h, w, py, puv) in enumerate(frames):
+            arr[i].y, arr[i].uv, arr[i].height, arr[i].width, arr[i].pitch_y, arr[i].pitch_uv = _devptr(y), _devptr(uv), h, w, py, puv
+        return arr
+
+    def frame_table_nv12(self, frames):
+        return self._frames_nv12(frames)
+
     def frame_table(self, frames):
         """Builds the fd_frame array once (a streaming caller reuses it: filling 64 ctypes structs per call costs more
         host time than the kernels they describe)."""
@@ -555,6 +574,37 @@ class Context:
         arr = self._frames(frames)
         _chk(self.lib.fd_align_detections(self.handle, arr, len(frames), C.c_void_p(_devptr(crops_dev)), cap_faces,
                                           C.c_void_p(_devptr(M_dev)), C.c_void_p(_devptr(ok_dev))))
+
+    # ---- NV12 video frames: the results of cv2.cvtColor(COLOR_YUV2BGR_NV12) followed by the BGR call
+    def preprocess_batch_nv12(self, frames, out_dev):
+        arr = self._frames_nv12(frames)
+        ds = np.empty(len(frames), np.float32)
+        _chk(self.lib.fd_preprocess_batch_nv12(self.handle, arr, len(frames), C.c_void_p(_devptr(out_dev)), _ptr(ds, c_f32p)))
+        return ds
+
+    def align_batch_nv12(self, frames, landmarks_dev, frame_idx_dev, F, crops_dev, M_dev=None, ok_dev=None, bbox_dev=None):
+        arr = self._frames_nv12(frames)
+        _chk(self.lib.fd_align_batch_nv12(self.handle, arr, len(frames), C.c_void_p(_devptr(landmarks_dev)),
+                                          C.c_void_p(_devptr(frame_idx_dev)), C.c_void_p(_devptr(bbox_dev)), F,
+                                          C.c_void_p(_devptr(crops_dev)), C.c_void_p(_devptr(M_dev)), C.c_void_p(_devptr(ok_dev))))
+
+    def align_detections_nv12(self, frames, crops_dev, cap_faces, M_dev=None, ok_dev=None):
+        arr = self._frames_nv12(frames)
+        _chk(self.lib.fd_align_detections_nv12(self.handle, arr, len(frames), C.c_void_p(_devptr(crops_dev)), cap_faces,
+                                               C.c_void_p(_devptr(M_dev)), C.c_void_p(_devptr(ok_dev))))
+
+    def select_detections_nv12(self, frames, is_enroll=False, params=None, fetch=True):
+        arr = self._frames_nv12(frames)
+        prm = None if params is None else (C.c_float * 4)(*params)
+        sel = np.empty((len(frames), 2), np.int32) if fetch else None
+        _chk(self.lib.fd_select_detections_nv12(self.handle, arr, len(frames), int(bool(is_enroll)), prm,
+                                                None if sel is None else _ptr(sel, c_i32p)))
+        return sel
+
+    def align_selected_nv12(self, frames, crops_dev, M_dev=None, ok_dev=None):
+        arr = self._frames_nv12(frames)
+        _chk(self.lib.fd_align_selected_nv12(self.handle, arr, len(frames), C.c_void_p(_devptr(crops_dev)), C.c_void_p(_devptr(M_dev)),
+                                             C.c_void_p(_devptr(ok_dev))))
 
     # ---- N2: Triton raw_output_contents
     def detect_batch_raw(self, raw, shapes, det_scale, conf_thr, iou_thr):

@@ -91,28 +91,13 @@ def parse_header(src):
         enums.append((m.group(2), [(k, int(v)) for k, v in re.findall(r"(\w+)\s*=\s*(\d+)", m.group(1))]))
     for m in re.finditer(r"(?<!typedef\s)enum\s*\{(.*?)\}\s*;", src, flags=re.S):
         enums.append((None, [(k, int(v)) for k, v in re.findall(r"(\w+)\s*=\s*(\d+)", m.group(1))]))
-    structs = []
-    for m in re.finditer(r"typedef\s+struct\s+(\w+)\s*\{(.*?)\}\s*(\w+)\s*;", src, flags=re.S):
-        fields = []
-        for decl in m.group(2).split(";"):
-            decl = " ".join(decl.split())
-            if not decl:
-                continue
-            first, *rest = split_params(decl)
-            fm = re.match(r"^(.*?)([A-Za-z_][A-Za-z0-9_]*)((?:\s*\[\s*\w+\s*\])*)$", first)
-            ctype_full = fm.group(1).strip()
-            base = ctype_full.replace("*", "").strip()
-            for d in [fm.group(2) + fm.group(3)] + [r.strip() for r in rest]:
-                stars = d.count("*") + (ctype_full.count("*") if d == fm.group(2) + fm.group(3) else 0)
-                dm = re.match(r"^\**\s*([A-Za-z_][A-Za-z0-9_]*)((?:\s*\[\s*\w+\s*\])*)$", d.replace(" ", ""))
-                name, dims = dm.group(1), re.findall(r"\[\s*(\w+)\s*\]", dm.group(2))
-                t = rust_type(base + " " + "*" * stars, consts)
-                for n in reversed(dims):
-                    t = "[%s; %s]" % (t, n if not n.isdigit() else n)
-                fields.append((name, t))
-        structs.append((m.group(3), fields))
-    opaque = re.findall(r"typedef\s+struct\s+(\w+)\s+(\w+)\s*;", src)
+    structs = [(m.group(3), parse_fields(m.group(2), consts))
+               for m in re.finditer(r"typedef\s+struct\s+(\w+)\s*\{(.*?)\}\s*(\w+)\s*;", src, flags=re.S)]
+    # `typedef struct X X;` names an opaque type unless `struct X {...};` defines it (parse_plain_structs)
+    defined = {name for name, _ in parse_plain_structs(src)}
+    opaque = [o for o in re.findall(r"typedef\s+struct\s+(\w+)\s+(\w+)\s*;", src) if o[0] not in defined]
     body = re.sub(r"typedef\s+(struct|enum)\s+\w+\s*\{.*?\}\s*\w+\s*;", "", src, flags=re.S)
+    body = re.sub(r"(?<!typedef\s)struct\s+\w+\s*\{.*?\}\s*;", "", body, flags=re.S)
     body = re.sub(r"enum\s*\{.*?\}\s*;", "", body, flags=re.S)
     body = re.sub(r"typedef[^;]*;", "", body)
     body = re.sub(r"#[^\n]*", "", body)
@@ -129,8 +114,40 @@ def parse_header(src):
     return consts, enums, structs, [o[1] for o in opaque], funcs
 
 
+def parse_plain_structs(src):
+    """structs defined as `struct X {...};` and named by a separate `typedef struct X X;` -> [(name, fields)]"""
+    src = strip_comments(src)
+    consts = dict(re.findall(r"#define\s+(FD_[A-Z_]+)\s+(\d+)", src))
+    return [(m.group(1), parse_fields(m.group(2), consts))
+            for m in re.finditer(r"(?<!typedef\s)struct\s+(\w+)\s*\{(.*?)\}\s*;", src, flags=re.S)]
+
+
+def parse_fields(body, consts):
+    """the field declarations of one struct body -> [(name, rust type)]"""
+    fields = []
+    for decl in body.split(";"):
+        decl = " ".join(decl.split())
+        if not decl:
+            continue
+        first, *rest = split_params(decl)
+        fm = re.match(r"^(.*?)([A-Za-z_][A-Za-z0-9_]*)((?:\s*\[\s*\w+\s*\])*)$", first)
+        ctype_full = fm.group(1).strip()
+        base = ctype_full.replace("*", "").strip()
+        for d in [fm.group(2) + fm.group(3)] + [r.strip() for r in rest]:
+            stars = d.count("*") + (ctype_full.count("*") if d == fm.group(2) + fm.group(3) else 0)
+            dm = re.match(r"^\**\s*([A-Za-z_][A-Za-z0-9_]*)((?:\s*\[\s*\w+\s*\])*)$", d.replace(" ", ""))
+            name, dims = dm.group(1), re.findall(r"\[\s*(\w+)\s*\]", dm.group(2))
+            t = rust_type(base + " " + "*" * stars, consts)
+            for n in reversed(dims):
+                t = "[%s; %s]" % (t, n if not n.isdigit() else n)
+            fields.append((name, t))
+    return fields
+
+
 def generate():
-    consts, enums, structs, opaque, funcs = parse_header(open(HEADER).read())
+    src = open(HEADER).read()
+    consts, enums, structs, opaque, funcs = parse_header(src)
+    structs = structs + parse_plain_structs(src)
     o = []
     o.append("//! src/ffi.rs — `extern \"C\"` declarations of include/fd_b200.h (the only unsafe surface of the crate).")
     o.append("//! Replaces the commented-out binding in src/rcnn/gpu_nms.rs:9-19.")
