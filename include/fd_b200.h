@@ -69,6 +69,18 @@ struct fd_frame_nv12 {
 };
 typedef struct fd_frame_nv12 fd_frame_nv12;
 
+/* Layouts of a 4:2:0 frame for the *_yuv420 calls, which describe every layout with fd_frame_nv12.  `y` is always the
+ * height x width luma plane.  What `uv` points to (H = height, W = width, all rows `pitch_uv` bytes apart):
+ *   FD_YUV420_NV12  interleaved U,V: H/2 rows of W bytes; pitch_uv >= W (NVDEC output)
+ *   FD_YUV420_NV21  interleaved V,U: H/2 rows of W bytes; pitch_uv >= W (Android camera preview)
+ *   FD_YUV420_I420  the U plane, H/2 rows of W/2 bytes; the V plane starts at uv + (H/2) * pitch_uv; pitch_uv >= W/2
+ *                   (FFmpeg yuv420p, WebRTC I420Buffer)
+ *   FD_YUV420_YV12  the V plane, H/2 rows of W/2 bytes; the U plane starts at uv + (H/2) * pitch_uv; pitch_uv >= W/2
+ * I420 and YV12 are thus the single buffer cv::cvtColor reads, with pitches added; (H/2) * pitch_uv must stay below 2 GB.  The calls give the results of their
+ * BGR counterparts on the frame cv::cvtColor(COLOR_YUV2BGR_NV12 / _NV21 / _I420 / _YV12) makes (BT.601 limited range),
+ * without building it. */
+enum { FD_YUV420_NV12 = 0, FD_YUV420_NV21 = 1, FD_YUV420_I420 = 2, FD_YUV420_YV12 = 3 };
+
 /* ---- library / context ---------------------------------------------------------------------------- */
 int fd_abi_version(void);
 const char *fd_last_error(void);
@@ -195,6 +207,11 @@ int fd_preprocess_batch(fd_ctx *ctx, const fd_frame *frames, int B, float *out_n
  * fd_preprocess_batch, reading only the Y and UV rows the resize taps.  FD_ERR_INVALID for an odd width or height, a pitch
  * below the width or a null plane. */
 int fd_preprocess_batch_nv12(fd_ctx *ctx, const fd_frame_nv12 *frames, int B, float *out_nchw_dev, float *det_scale_host);
+/* fd_preprocess_batch_nv12 for any FD_YUV420_* layout (layout FD_YUV420_NV12 is fd_preprocess_batch_nv12).  FD_ERR_INVALID
+ * for an odd width or height, a null plane, pitch_y below the width, pitch_uv below the layout's minimum or an unknown
+ * layout.  The same for the other *_yuv420 calls. */
+int fd_preprocess_batch_yuv420(fd_ctx *ctx, const fd_frame_nv12 *frames, int32_t layout, int B, float *out_nchw_dev,
+                               float *det_scale_host);
 /* heads_dev[3*s+0..2]: (B,2A,H,W), (B,4A,H,W), (B,10A,H,W) dev tensors of stride s.  Results stay on the device
  * inside the ctx until fd_detect_fetch / fd_align_detections.  Asynchronous.  Images with more than 4096 candidates
  * (and, the first time a ctx meets one, images with more than 1024) are completed by fd_detect_fetch / fd_detect_view;
@@ -229,6 +246,9 @@ int fd_align_batch(fd_ctx *ctx, const fd_frame *frames, int B, const float *land
  * (BORDER_CONSTANT is black in BGR). */
 int fd_align_batch_nv12(fd_ctx *ctx, const fd_frame_nv12 *frames, int B, const float *landmarks_dev, const int32_t *frame_idx_dev,
                         const float *bbox_dev, int F, uint8_t *crops_dev, double *M_dev, uint8_t *ok_dev);
+/* fd_align_batch_nv12 for any FD_YUV420_* layout. */
+int fd_align_batch_yuv420(fd_ctx *ctx, const fd_frame_nv12 *frames, int32_t layout, int B, const float *landmarks_dev,
+                          const int32_t *frame_idx_dev, const float *bbox_dev, int F, uint8_t *crops_dev, double *M_dev, uint8_t *ok_dev);
 /* Aligns every detection of the last fd_detect_batch without a host round trip (fallback box = the detection's own box).
  * crops_dev has room for cap_faces crops; detections beyond cap_faces are not aligned (fd_detect_fetch still reports them). */
 int fd_align_detections(fd_ctx *ctx, const fd_frame *frames, int B, uint8_t *crops_dev, int cap_faces, double *M_dev,
@@ -237,6 +257,10 @@ int fd_align_detections(fd_ctx *ctx, const fd_frame *frames, int B, uint8_t *cro
  * re-run on the NV12 frames by fd_detect_fetch / fd_detect_view when deferred images change the detections. */
 int fd_align_detections_nv12(fd_ctx *ctx, const fd_frame_nv12 *frames, int B, uint8_t *crops_dev, int cap_faces, double *M_dev,
                              uint8_t *ok_dev);
+/* fd_align_detections_nv12 for any FD_YUV420_* layout; a replay at fd_detect_fetch / fd_detect_view reads the frames in
+ * the layout given here. */
+int fd_align_detections_yuv420(fd_ctx *ctx, const fd_frame_nv12 *frames, int32_t layout, int B, uint8_t *crops_dev, int cap_faces,
+                               double *M_dev, uint8_t *ok_dev);
 
 /* ---- SURVEY 8(f) N1: post-align model preprocessors, fused onto the aligned crops ----------------------- */
 /* FaceExtraction::_preprocess (face_extraction.rs:38-77: mean 127.5, mul 0.0078125), FaceQuality::call
@@ -280,12 +304,18 @@ int fd_select_detections(fd_ctx *ctx, const fd_frame *frames, int B, int is_enro
  * cv::cvtColor(COLOR_YUV2BGR_NV12) followed by fd_select_detections. */
 int fd_select_detections_nv12(fd_ctx *ctx, const fd_frame_nv12 *frames, int B, int is_enroll, const fd_select_params *params,
                               int32_t *sel_host);
+/* fd_select_detections_nv12 for any FD_YUV420_* layout. */
+int fd_select_detections_yuv420(fd_ctx *ctx, const fd_frame_nv12 *frames, int32_t layout, int B, int is_enroll,
+                                const fd_select_params *params, int32_t *sel_host);
 /* FaceAlignment::call on the selection of the last fd_select_detections (face_pipeline/pipeline.rs:216-232): one crop per
  * image, crops_dev (B,crop_h,crop_w,3); images without a selection or without key points (the reference's call(.., None)
  * returns Err) get ok = 0 and a zero crop; ok = 2 marks the bbox-crop fallback on the selected box.  M_dev (B,6) / ok_dev (B) optional. */
 int fd_align_selected(fd_ctx *ctx, const fd_frame *frames, int B, uint8_t *crops_dev, double *M_dev, uint8_t *ok_dev);
 /* fd_align_selected on NV12 frames: the results of cv::cvtColor(COLOR_YUV2BGR_NV12) followed by fd_align_selected. */
 int fd_align_selected_nv12(fd_ctx *ctx, const fd_frame_nv12 *frames, int B, uint8_t *crops_dev, double *M_dev, uint8_t *ok_dev);
+/* fd_align_selected_nv12 for any FD_YUV420_* layout. */
+int fd_align_selected_yuv420(fd_ctx *ctx, const fd_frame_nv12 *frames, int32_t layout, int B, uint8_t *crops_dev, double *M_dev,
+                             uint8_t *ok_dev);
 
 /* ---- SURVEY 8(f) N4: utils::byte_data_to_opencv (utils.rs:8-52 = cv::imdecode(bytes, IMREAD_UNCHANGED)), baseline JPEG ------- */
 /* Host-only header parse: image size and luma sampling (11 = 4:4:4, 21 = 4:2:2, 22 = 4:2:0).  FD_ERR_INVALID for streams the

@@ -16,6 +16,7 @@
 #include <cstdlib>
 #include <vector>
 #include <cfloat>
+#include <type_traits>
 #include "fd_internal.cuh"
 #include "fd_estimate.cuh"
 #include "fd_resize.cuh"
@@ -200,15 +201,16 @@ __device__ __forceinline__ unsigned border_tap_blend(const uint8_t *data, int w,
     return blend24(lo0, hi0, lo1, hi1, X & 31, Y & 31);
 }
 
-// ---- NV12 sources: the four taps are converted to BGR (yuv_bgr24) and blended with the same arithmetic ----------------
+// ---- 4:2:0 sources: the four taps are converted to BGR (yuv_bgr24) and blended with the same arithmetic --------------
 // Two horizontally adjacent packed pixels p0, p1 as the (lo, hi) byte pair blend24 takes: bytes b0 g0 r0 b1 | g1 r1.
 __device__ __forceinline__ void pack6(unsigned p0, unsigned p1, unsigned &lo, unsigned &hi) {
     lo = p0 | (p1 << 24);
     hi = p1 >> 8;
 }
-// Interior tap square (sx, sy)..(sx+1, sy+1) of an NV12 frame whose planes and pitches are 4-byte aligned: four bytes at
-// sx of each Y row and at sx & ~1 of each tap row's UV row (the U,V of both columns: one pair when sx is even, two when it
-// is odd; both rows read the same UV row when sy is even), each cut from the two aligned words that cover it.
+// Interior tap square (sx, sy)..(sx+1, sy+1) of an NV12/NV21 frame whose planes and pitches are 4-byte aligned: four bytes
+// at sx of each Y row and at sx & ~1 of each tap row's chroma row (the chroma pairs of both columns: one pair when sx is
+// even, two when it is odd; both rows read the same chroma row when sy is even), each cut from the two aligned words that
+// cover it.
 struct Nv12Quad {
     unsigned y0[2], y1[2], c0[2], c1[2];
     unsigned sy_sh, sc_sh;   // byte phase of the Y and of the UV reads (the two rows of a plane share it)
@@ -229,16 +231,84 @@ __device__ __forceinline__ void nv12_quad_load(const uint8_t *yp, unsigned py, c
     q.sc_sh = (oc0 & 3u) * 8;
     q.odd = (sx & 1) != 0;
 }
+// FMT: SRC_NV12 (chroma bytes U,V) or SRC_NV21 (V,U)
+template <int FMT>
 __device__ __forceinline__ void nv12_row_taps(unsigned yw, unsigned cw, bool odd, unsigned &lo, unsigned &hi) {
-    const unsigned u1 = odd ? (cw >> 16) & 255u : cw & 255u, v1 = odd ? cw >> 24 : (cw >> 8) & 255u;
-    pack6(yuv_bgr24(yw & 255u, cw & 255u, (cw >> 8) & 255u), yuv_bgr24((yw >> 8) & 255u, u1, v1), lo, hi);
+    const unsigned e1 = odd ? (cw >> 16) & 255u : cw & 255u, o1 = odd ? cw >> 24 : (cw >> 8) & 255u;   // chroma pair of column sx+1
+    if (FMT == SRC_NV21) pack6(yuv_bgr24(yw & 255u, (cw >> 8) & 255u, cw & 255u), yuv_bgr24((yw >> 8) & 255u, o1, e1), lo, hi);
+    else pack6(yuv_bgr24(yw & 255u, cw & 255u, (cw >> 8) & 255u), yuv_bgr24((yw >> 8) & 255u, e1, o1), lo, hi);
 }
+template <int FMT>
 __device__ __forceinline__ void nv12_quad_taps(const Nv12Quad &q, unsigned &lo0, unsigned &hi0, unsigned &lo1, unsigned &hi1) {
-    nv12_row_taps(__funnelshift_r(q.y0[0], q.y0[1], q.sy_sh), __funnelshift_r(q.c0[0], q.c0[1], q.sc_sh), q.odd, lo0, hi0);
-    nv12_row_taps(__funnelshift_r(q.y1[0], q.y1[1], q.sy_sh), __funnelshift_r(q.c1[0], q.c1[1], q.sc_sh), q.odd, lo1, hi1);
+    nv12_row_taps<FMT>(__funnelshift_r(q.y0[0], q.y0[1], q.sy_sh), __funnelshift_r(q.c0[0], q.c0[1], q.sc_sh), q.odd, lo0, hi0);
+    nv12_row_taps<FMT>(__funnelshift_r(q.y1[0], q.y1[1], q.sy_sh), __funnelshift_r(q.c1[0], q.c1[1], q.sc_sh), q.odd, lo1, hi1);
 }
-// border_tap_blend for NV12: BORDER_CONSTANT(0) applies to the BGR image, so a tap outside the frame is BGR (0,0,0)
-__device__ __forceinline__ unsigned border_tap_blend_nv12(const uint8_t *yp, int py, const uint8_t *uvp, int puv, int w, int h, int X, int Y) {
+// The same square of a planar (I420/YV12) frame: four bytes at sx of each Y row, and at sx >> 1 of each tap row's U and V
+// rows (byte 0: the chroma of column sx; byte 1: that of column sx+1 when sx is odd).  The U and V planes share the pitch
+// and the 4-byte phase.
+struct PlanarQuad {
+    unsigned y0[2], y1[2], u0[2], v0[2], u1[2], v1[2];
+    unsigned sy_sh, sc_sh;
+    bool odd;
+};
+__device__ __forceinline__ void planar_quad_load(const uint8_t *yp, unsigned py, const uint8_t *up, const uint8_t *vp, unsigned puv, int sx,
+                                                 int sy, PlanarQuad &q) {
+    const unsigned oy = (unsigned)sy * py + (unsigned)sx, xc = (unsigned)(sx >> 1);
+    const unsigned oc0 = (unsigned)(sy >> 1) * puv + xc, oc1 = (unsigned)((sy + 1) >> 1) * puv + xc;
+    const unsigned *ry0 = reinterpret_cast<const unsigned *>(yp + (oy & ~3u));
+    const unsigned *ry1 = reinterpret_cast<const unsigned *>(yp + ((oy + py) & ~3u));
+    const unsigned *ru0 = reinterpret_cast<const unsigned *>(up + (oc0 & ~3u)), *rv0 = reinterpret_cast<const unsigned *>(vp + (oc0 & ~3u));
+    const unsigned *ru1 = reinterpret_cast<const unsigned *>(up + (oc1 & ~3u)), *rv1 = reinterpret_cast<const unsigned *>(vp + (oc1 & ~3u));
+    q.y0[0] = __ldg(ry0); q.y0[1] = __ldg(ry0 + 1);
+    q.y1[0] = __ldg(ry1); q.y1[1] = __ldg(ry1 + 1);
+    q.u0[0] = __ldg(ru0); q.u0[1] = __ldg(ru0 + 1);
+    q.v0[0] = __ldg(rv0); q.v0[1] = __ldg(rv0 + 1);
+    q.u1[0] = __ldg(ru1); q.u1[1] = __ldg(ru1 + 1);
+    q.v1[0] = __ldg(rv1); q.v1[1] = __ldg(rv1 + 1);
+    q.sy_sh = (oy & 3u) * 8;
+    q.sc_sh = (oc0 & 3u) * 8;
+    q.odd = (sx & 1) != 0;
+}
+__device__ __forceinline__ void planar_row_taps(unsigned yw, unsigned uw, unsigned vw, bool odd, unsigned &lo, unsigned &hi) {
+    const unsigned u1 = odd ? (uw >> 8) & 255u : uw & 255u, v1 = odd ? (vw >> 8) & 255u : vw & 255u;
+    pack6(yuv_bgr24(yw & 255u, uw & 255u, vw & 255u), yuv_bgr24((yw >> 8) & 255u, u1, v1), lo, hi);
+}
+__device__ __forceinline__ void planar_quad_taps(const PlanarQuad &q, unsigned &lo0, unsigned &hi0, unsigned &lo1, unsigned &hi1) {
+    planar_row_taps(__funnelshift_r(q.y0[0], q.y0[1], q.sy_sh), __funnelshift_r(q.u0[0], q.u0[1], q.sc_sh),
+                    __funnelshift_r(q.v0[0], q.v0[1], q.sc_sh), q.odd, lo0, hi0);
+    planar_row_taps(__funnelshift_r(q.y1[0], q.y1[1], q.sy_sh), __funnelshift_r(q.u1[0], q.u1[1], q.sc_sh),
+                    __funnelshift_r(q.v1[0], q.v1[1], q.sc_sh), q.odd, lo1, hi1);
+}
+// the tap square of a 4:2:0 format (FMT: SRC_NV12, SRC_NV21 or SRC_PLANAR)
+template <int FMT> using YuvQuad = typename std::conditional<FMT == SRC_PLANAR, PlanarQuad, Nv12Quad>::type;
+template <int FMT>
+__device__ __forceinline__ void yuv_quad_load(const uint8_t *yp, unsigned py, const uint8_t *uvp, const uint8_t *vp, unsigned puv, int sx, int sy,
+                                              YuvQuad<FMT> &q) {
+    if constexpr (FMT == SRC_PLANAR) planar_quad_load(yp, py, uvp, vp, puv, sx, sy, q);
+    else nv12_quad_load(yp, py, uvp, puv, sx, sy, q);
+}
+template <int FMT>
+__device__ __forceinline__ void yuv_quad_taps(const YuvQuad<FMT> &q, unsigned &lo0, unsigned &hi0, unsigned &lo1, unsigned &hi1) {
+    if constexpr (FMT == SRC_PLANAR) planar_quad_taps(q, lo0, hi0, lo1, hi1);
+    else nv12_quad_taps<FMT>(q, lo0, hi0, lo1, hi1);
+}
+// pixel (xx, yy) of a 4:2:0 frame inside it (vp: the V plane, planar only)
+template <int FMT>
+__device__ __forceinline__ unsigned yuv_tap(const uint8_t *yp, int py, const uint8_t *uvp, const uint8_t *vp, int puv, int xx, int yy) {
+    if constexpr (FMT == SRC_PLANAR)
+        return yuv_bgr24(__ldg(yp + (ptrdiff_t)yy * py + xx), __ldg(uvp + (ptrdiff_t)(yy >> 1) * puv + (xx >> 1)),
+                         __ldg(vp + (ptrdiff_t)(yy >> 1) * puv + (xx >> 1)));
+    else if constexpr (FMT == SRC_NV21)
+        return yuv_bgr24(__ldg(yp + (ptrdiff_t)yy * py + xx), __ldg(uvp + (ptrdiff_t)(yy >> 1) * puv + (xx | 1)),
+                         __ldg(uvp + (ptrdiff_t)(yy >> 1) * puv + (xx & ~1)));
+    else
+        return yuv_bgr24(__ldg(yp + (ptrdiff_t)yy * py + xx), __ldg(uvp + (ptrdiff_t)(yy >> 1) * puv + (xx & ~1)),
+                         __ldg(uvp + (ptrdiff_t)(yy >> 1) * puv + (xx | 1)));
+}
+// border_tap_blend for a 4:2:0 frame: BORDER_CONSTANT(0) applies to the BGR image, so a tap outside the frame is BGR (0,0,0)
+template <int FMT>
+__device__ __forceinline__ unsigned border_tap_blend_yuv(const uint8_t *yp, int py, const uint8_t *uvp, const uint8_t *vp, int puv, int w, int h,
+                                                         int X, int Y) {
     const int sx = max(-32768, min(32767, X >> 5)), sy = max(-32768, min(32767, Y >> 5));   // saturate_cast<short>
     unsigned p[2][2];
 #pragma unroll
@@ -246,22 +316,24 @@ __device__ __forceinline__ unsigned border_tap_blend_nv12(const uint8_t *yp, int
 #pragma unroll
         for (int i = 0; i < 2; ++i) {
             const int xx = sx + i, yy = sy + j;
-            p[j][i] = xx >= 0 && xx < w && yy >= 0 && yy < h
-                          ? yuv_bgr24(__ldg(yp + (ptrdiff_t)yy * py + xx), __ldg(uvp + (ptrdiff_t)(yy >> 1) * puv + (xx & ~1)),
-                                      __ldg(uvp + (ptrdiff_t)(yy >> 1) * puv + (xx | 1)))
-                          : 0u;
+            p[j][i] = xx >= 0 && xx < w && yy >= 0 && yy < h ? yuv_tap<FMT>(yp, py, uvp, vp, puv, xx, yy) : 0u;
         }
     unsigned lo0, hi0, lo1, hi1;
     pack6(p[0][0], p[0][1], lo0, hi0);
     pack6(p[1][0], p[1][1], lo1, hi1);
     return blend24(lo0, hi0, lo1, hi1, X & 31, Y & 31);
 }
-// The warp kernels read an NV12 frame's interior taps with nv12_quad_load when its planes and pitches are 4-byte aligned
+// The warp kernels read a 4:2:0 frame's interior taps with yuv_quad_load when its planes and pitches are 4-byte aligned
 // and its offsets fit 32 bits; the reads run up to 7 bytes past a tap, so the interior also keeps two rows from the bottom
-// (the last UV row is then never read there).
+// (the last chroma row is then never read there: the over-read of a chroma row stays in the next row, pitch_uv >= 8).
 __device__ __forceinline__ bool nv12_interior_ok(const FrameDev &f) {
     return ((reinterpret_cast<uintptr_t>(f.data) | reinterpret_cast<uintptr_t>(f.uv)) & 3) == 0 && (f.pitch & 3) == 0 && (f.pitch_uv & 3) == 0 &&
            f.pitch >= 8 && f.pitch_uv >= 8 && (size_t)f.h * f.pitch < 0x7fffffffull && (size_t)f.h * f.pitch_uv < 0x7fffffffull;
+}
+template <int FMT>
+__device__ __forceinline__ bool yuv_interior_ok(const FrameDev &f) {
+    if constexpr (FMT == SRC_PLANAR) return nv12_interior_ok(f) && (f.v_off & 3) == 0;   // the V plane too
+    else return nv12_interior_ok(f);
 }
 
 // Stores the 24-bit pixels of a warp's 32 consecutive output pixels.  packed: the 4 pixels of a lane quad (12 bytes) leave
@@ -284,16 +356,17 @@ struct WarpItem {
     const uint8_t *data;
     int w, h, pitch;
     const uint8_t *lo_lim, *hi_lim;
-    const uint8_t *uv;   // NV12 only
+    const uint8_t *uv;   // 4:2:0 only
     int pitch_uv;
+    const uint8_t *v;    // planar only
 };
 
 // N rounds of WARP_THREADS consecutive output pixels starting at p0: all 4N aligned 64-bit loads of a thread are issued
 // before any is consumed (interior items: no border test anywhere in the band).
-template <int N>
-__device__ __forceinline__ void warp_rounds_interior_nv12(const WarpItem &it, const int2 *__restrict__ dxy, const int2 *__restrict__ xy0,
-                                                          int cw, unsigned cw_magic, int p0, int npix, uint8_t *band_out, bool packed) {
-    Nv12Quad q[N];
+template <int FMT, int N>
+__device__ __forceinline__ void warp_rounds_interior_yuv(const WarpItem &it, const int2 *__restrict__ dxy, const int2 *__restrict__ xy0,
+                                                         int cw, unsigned cw_magic, int p0, int npix, uint8_t *band_out, bool packed) {
+    YuvQuad<FMT> q[N];
     int axy[N];
 #pragma unroll
     for (int u = 0; u < N; ++u) {
@@ -302,13 +375,13 @@ __device__ __forceinline__ void warp_rounds_interior_nv12(const WarpItem &it, co
         const int2 d = dxy[x], r0 = xy0[row];
         const int X = (int)((unsigned)r0.x + (unsigned)d.x) >> 5, Y = (int)((unsigned)r0.y + (unsigned)d.y) >> 5;
         axy[u] = (X & 31) | ((Y & 31) << 8);
-        nv12_quad_load(it.data, (unsigned)it.pitch, it.uv, (unsigned)it.pitch_uv, X >> 5, Y >> 5, q[u]);
+        yuv_quad_load<FMT>(it.data, (unsigned)it.pitch, it.uv, it.v, (unsigned)it.pitch_uv, X >> 5, Y >> 5, q[u]);
     }
 #pragma unroll
     for (int u = 0; u < N; ++u) {
         const int p = p0 + u * WARP_THREADS;
         unsigned lo0, hi0, lo1, hi1;
-        nv12_quad_taps(q[u], lo0, hi0, lo1, hi1);
+        yuv_quad_taps<FMT>(q[u], lo0, hi0, lo1, hi1);
         const unsigned v = blend24(lo0, hi0, lo1, hi1, axy[u] & 31, axy[u] >> 8);
         store_px(band_out, p, v, p < npix, packed);
     }
@@ -346,15 +419,15 @@ __device__ __forceinline__ void warp_rounds_interior(const WarpItem &it, const i
 }
 
 // one round with per-tap BORDER_CONSTANT tests (items that touch the frame border, unaligned or > 2 GB frames)
-template <bool NV>
+template <int FMT>
 __device__ __forceinline__ void warp_round_border(const WarpItem &it, const int2 *__restrict__ dxy, const int2 *__restrict__ xy0, int cw,
                                                   unsigned cw_magic, int p0, int npix, uint8_t *band_out, bool packed) {
     const int p = min(p0, npix - 1);
     const int row = cw_magic ? (int)__umulhi((unsigned)p, cw_magic) : p, x = p - row * cw;
     const int2 d = dxy[x], r0 = xy0[row];
     const int X = (int)((unsigned)r0.x + (unsigned)d.x) >> 5, Y = (int)((unsigned)r0.y + (unsigned)d.y) >> 5;
-    const unsigned v = NV ? border_tap_blend_nv12(it.data, it.pitch, it.uv, it.pitch_uv, it.w, it.h, X, Y)
-                          : border_tap_blend(it.data, it.w, it.h, it.pitch, it.lo_lim, it.hi_lim, X, Y);
+    const unsigned v = FMT != SRC_BGR ? border_tap_blend_yuv<FMT>(it.data, it.pitch, it.uv, it.v, it.pitch_uv, it.w, it.h, X, Y)
+                                      : border_tap_blend(it.data, it.w, it.h, it.pitch, it.lo_lim, it.hi_lim, X, Y);
     store_px(band_out, p0, v, p0 < npix, packed);
 }
 
@@ -362,9 +435,10 @@ __device__ __forceinline__ void warp_round_border(const WarpItem &it, const int2
 // atomic ticket so big faces (more DRAM per item) do not leave a tail.  The next ticket is fetched while the current
 // item is being processed.  Lanes = consecutive output pixels of the band (row-major), so one load instruction's lanes
 // share cache lines and one store instruction writes 96 contiguous bytes.
-// NV: the frames are NV12 (FrameDev::uv)
-template <bool NV>
+// FMT: the source format of the frames (SrcFmt)
+template <int FMT>
 __global__ void __launch_bounds__(WARP_THREADS, 4) warp_kernel(WarpArgs a) {
+    constexpr bool NV = FMT != SRC_BGR;
     extern __shared__ int2 wsm[];
     int2 *dxy = wsm;             // [cw]  (adelta, bdelta)
     int2 *xy0 = dxy + a.cw;      // [WARP_BAND]  (X0, Y0) per row
@@ -396,7 +470,8 @@ __global__ void __launch_bounds__(WARP_THREADS, 4) warp_kernel(WarpArgs a) {
                 const uint8_t *roi = fr.data + (size_t)ry0 * fr.pitch + (size_t)rx0 * 3;
                 for (int p = tid; p < npix; p += WARP_THREADS) {
                     const int row = p / a.cw, x = p - row * a.cw;
-                    const unsigned v = NV ? resize_pixel24_nv12(fr.data, fr.pitch, fr.uv, fr.pitch_uv, rx0, ry0, fr.w - rx0, fr.h - ry0, a.cw, a.ch, x, band_y0 + row)
+                    const unsigned v = NV ? resize_pixel24_yuv<FMT>(fr.data, fr.pitch, fr.uv, fr.v_plane(), fr.pitch_uv, rx0, ry0, fr.w - rx0, fr.h - ry0, a.cw,
+                                                                    a.ch, x, band_y0 + row)
                                           : resize_pixel24(roi, fr.pitch, fr.w - rx0, fr.h - ry0, a.cw, a.ch, x, band_y0 + row);
                     band_out[3 * p] = (uint8_t)v; band_out[3 * p + 1] = (uint8_t)(v >> 8); band_out[3 * p + 2] = (uint8_t)(v >> 16);
                 }
@@ -418,7 +493,7 @@ __global__ void __launch_bounds__(WARP_THREADS, 4) warp_kernel(WarpArgs a) {
         __syncthreads();
         // The map is affine, so the tap coordinates of the band are extremal at its 4 corners: if all 4 corner taps
         // (and their +1 neighbours) are interior, no pixel of the band needs a border test.
-        bool interior = NV ? nv12_interior_ok(fr)
+        bool interior = NV ? yuv_interior_ok<FMT>(fr)
                            : (reinterpret_cast<uintptr_t>(fr.data) & 7) == 0 && (fr.pitch & 7) == 0 && fr.pitch >= 16 &&
                                  (size_t)fr.h * fr.pitch < 0x7fffffffull;
         const int bottom = NV ? 2 : 1;   // rows kept from the bottom: the loads over-read past the last tap row
@@ -438,11 +513,12 @@ __global__ void __launch_bounds__(WARP_THREADS, 4) warp_kernel(WarpArgs a) {
         it.lo_lim = fr.data;
         it.hi_lim = fr.data + (size_t)(fr.h - 1) * fr.pitch + (size_t)fr.w * 3;  // end of valid pixel bytes
         it.uv = fr.uv; it.pitch_uv = fr.pitch_uv;
+        if constexpr (FMT == SRC_PLANAR) it.v = fr.v_plane();
         int p0 = tid;
         if (NV && interior) {
             for (int rounds = (npix + WARP_THREADS - 1) / WARP_THREADS; rounds > 0; rounds -= 2, p0 += 2 * WARP_THREADS) {
-                if (rounds >= 2) warp_rounds_interior_nv12<2>(it, dxy, xy0, a.cw, a.cw_magic, p0, npix, band_out, packed);
-                else warp_rounds_interior_nv12<1>(it, dxy, xy0, a.cw, a.cw_magic, p0, npix, band_out, packed);
+                if (rounds >= 2) warp_rounds_interior_yuv<FMT, 2>(it, dxy, xy0, a.cw, a.cw_magic, p0, npix, band_out, packed);
+                else warp_rounds_interior_yuv<FMT, 1>(it, dxy, xy0, a.cw, a.cw_magic, p0, npix, band_out, packed);
             }
         } else if (interior) {
             int rounds = (npix + WARP_THREADS - 1) / WARP_THREADS;
@@ -453,7 +529,7 @@ __global__ void __launch_bounds__(WARP_THREADS, 4) warp_kernel(WarpArgs a) {
                 else { warp_rounds_interior<1>(it, dxy, xy0, a.cw, a.cw_magic, p0, npix, band_out, packed); rounds = 0; }
             }
         } else {
-            for (; p0 - tid < npix; p0 += WARP_THREADS) warp_round_border<NV>(it, dxy, xy0, a.cw, a.cw_magic, p0, npix, band_out, packed);
+            for (; p0 - tid < npix; p0 += WARP_THREADS) warp_round_border<FMT>(it, dxy, xy0, a.cw, a.cw_magic, p0, npix, band_out, packed);
         }
         __syncthreads();  // tables and s_item[par] are free again
     }
@@ -510,32 +586,33 @@ __device__ __forceinline__ void fixed_rounds_interior(const uint8_t *__restrict_
     }
 }
 
-template <int CW, int N>
-__device__ __forceinline__ void fixed_rounds_interior_nv12(const uint8_t *__restrict__ yp, unsigned py, const uint8_t *__restrict__ uvp,
-                                                           unsigned puv, int2 d, const int2 *__restrict__ xy, unsigned *__restrict__ outw,
-                                                           bool store, unsigned pack_sel) {
-    Nv12Quad q[N];
+template <int CW, int N, int FMT>
+__device__ __forceinline__ void fixed_rounds_interior_yuv(const uint8_t *__restrict__ yp, unsigned py, const uint8_t *__restrict__ uvp,
+                                                          const uint8_t *__restrict__ vp, unsigned puv, int2 d, const int2 *__restrict__ xy,
+                                                          unsigned *__restrict__ outw, bool store, unsigned pack_sel) {
+    YuvQuad<FMT> q[N];
     int axy[N];
 #pragma unroll
     for (int u = 0; u < N; ++u) {
         const int2 r0 = xy[2 * u];
         const int X = (int)((unsigned)r0.x + (unsigned)d.x) >> 5, Y = (int)((unsigned)r0.y + (unsigned)d.y) >> 5;
         axy[u] = (X & 31) | ((Y & 31) << 14);   // ax | ay << 6 << 8
-        nv12_quad_load(yp, py, uvp, puv, X >> 5, Y >> 5, q[u]);
+        yuv_quad_load<FMT>(yp, py, uvp, vp, puv, X >> 5, Y >> 5, q[u]);
     }
 #pragma unroll
     for (int u = 0; u < N; ++u) {
         unsigned lo0, hi0, lo1, hi1;
-        nv12_quad_taps(q[u], lo0, hi0, lo1, hi1);
+        yuv_quad_taps<FMT>(q[u], lo0, hi0, lo1, hi1);
         const unsigned v = blend24_scaled(lo0, hi0, lo1, hi1, axy[u] & 31, axy[u] >> 8);
         const unsigned nv = __shfl_down_sync(0xffffffffu, v, 1);
         if (store) outw[u * (2 * CW * 3 / 4)] = __byte_perm(v, nv, pack_sel);
     }
 }
 
-// NV: the frames are NV12 (FrameDev::uv)
-template <int CW, int CH, int IR, int UN, bool NV>
+// FMT: the source format of the frames (SrcFmt)
+template <int CW, int CH, int IR, int UN, int FMT>
 __global__ void __launch_bounds__(2 * CW) warp_fixed_kernel(WarpArgs a) {
+    constexpr bool NV = FMT != SRC_BGR;
     constexpr int T = 2 * CW, ITEMS = CH / IR, ROUNDS = IR / 2;
     static_assert(CH % IR == 0 && IR % 2 == 0 && T % 32 == 0 && (2 * CW * 3) % 4 == 0 && (IR * CW * 3) % 4 == 0, "fixed warp geometry");
     __shared__ int2 xy0[2][IR];
@@ -568,6 +645,8 @@ __global__ void __launch_bounds__(2 * CW) warp_fixed_kernel(WarpArgs a) {
         const int fw = frp->w, fh = frp->h, pitch = frp->pitch;
         const uint8_t *uvp = NV ? frp->uv : nullptr;
         const int pitch_uv = NV ? frp->pitch_uv : 0;
+        const uint8_t *vp = nullptr;   // planar only
+        if constexpr (FMT == SRC_PLANAR) vp = frp->v_plane();
         int2 d = make_int2(0, 0);
         bool vote = true;
         if (okf) {
@@ -588,7 +667,7 @@ __global__ void __launch_bounds__(2 * CW) warp_fixed_kernel(WarpArgs a) {
                 }
             }
         }
-        const bool interior = __syncthreads_and(vote) && (NV ? nv12_interior_ok(*frp)
+        const bool interior = __syncthreads_and(vote) && (NV ? yuv_interior_ok<FMT>(*frp)
                                                                  : (reinterpret_cast<uintptr_t>(data) & 7) == 0 && (pitch & 7) == 0 && pitch >= 16 &&
                                                                        (size_t)fh * pitch < 0x7fffffffull);
         const bool store = (tid & 3) != 3;
@@ -600,7 +679,7 @@ __global__ void __launch_bounds__(2 * CW) warp_fixed_kernel(WarpArgs a) {
             if (valid) {
                 const uint8_t *roi = data + (size_t)ry0 * pitch + (size_t)rx0 * 3;
                 for (int u = 0; u < ROUNDS; ++u) {
-                    const unsigned v = NV ? resize_pixel24_nv12(data, pitch, uvp, pitch_uv, rx0, ry0, fw - rx0, fh - ry0, CW, CH, x, y0 + r + 2 * u)
+                    const unsigned v = NV ? resize_pixel24_yuv<FMT>(data, pitch, uvp, vp, pitch_uv, rx0, ry0, fw - rx0, fh - ry0, CW, CH, x, y0 + r + 2 * u)
                                           : resize_pixel24(roi, pitch, fw - rx0, fh - ry0, CW, CH, x, y0 + r + 2 * u);
                     const unsigned nv = __shfl_down_sync(0xffffffffu, v, 1);
                     const unsigned word = __funnelshift_r(__byte_perm(v, nv, 0x4210), nv >> 8, 8 * (tid & 3u));
@@ -620,9 +699,10 @@ __global__ void __launch_bounds__(2 * CW) warp_fixed_kernel(WarpArgs a) {
             if (NV) {
 #pragma unroll 1
                 for (; u + UN <= ROUNDS; u += UN)
-                    fixed_rounds_interior_nv12<CW, UN>(data, (unsigned)pitch, uvp, (unsigned)pitch_uv, d, xy + 2 * u, outw + u * (T * 3 / 4), store, pack_sel);
-                if (REM) fixed_rounds_interior_nv12<CW, REM ? REM : 1>(data, (unsigned)pitch, uvp, (unsigned)pitch_uv, d, xy + 2 * (ROUNDS - REM),
-                                                                       outw + (ROUNDS - REM) * (T * 3 / 4), store, pack_sel);
+                    fixed_rounds_interior_yuv<CW, UN, FMT>(data, (unsigned)pitch, uvp, vp, (unsigned)pitch_uv, d, xy + 2 * u, outw + u * (T * 3 / 4),
+                                                           store, pack_sel);
+                if (REM) fixed_rounds_interior_yuv<CW, REM ? REM : 1, FMT>(data, (unsigned)pitch, uvp, vp, (unsigned)pitch_uv, d, xy + 2 * (ROUNDS - REM),
+                                                                           outw + (ROUNDS - REM) * (T * 3 / 4), store, pack_sel);
             } else {
 #pragma unroll 1
                 for (; u + UN <= ROUNDS; u += UN)
@@ -634,7 +714,7 @@ __global__ void __launch_bounds__(2 * CW) warp_fixed_kernel(WarpArgs a) {
             for (int u = 0; u < ROUNDS; ++u) {
                 const int2 r0 = xy[2 * u];
                 const int X = (int)((unsigned)r0.x + (unsigned)d.x) >> 5, Y = (int)((unsigned)r0.y + (unsigned)d.y) >> 5;
-                const unsigned v = NV ? border_tap_blend_nv12(data, pitch, uvp, pitch_uv, fw, fh, X, Y)
+                const unsigned v = NV ? border_tap_blend_yuv<FMT>(data, pitch, uvp, vp, pitch_uv, fw, fh, X, Y)
                                       : border_tap_blend(data, fw, fh, pitch, lo_lim, hi_lim, X, Y);
                 const unsigned nv = __shfl_down_sync(0xffffffffu, v, 1);
                 const unsigned word = __funnelshift_r(__byte_perm(v, nv, 0x4210), nv >> 8, 8 * (tid & 3u));
@@ -719,10 +799,22 @@ int invert_launch(fd_ctx *ctx, const double *M_dev, int F, double *M12_dev, uint
     return FD_OK;
 }
 
-// nv12: frames_dev describes NV12 frames
+// Planar frames keep 2 rounds in flight (12 words a round instead of NV12's 8): with 4 the kernel needs 99 registers and
+// fits 2 CTAs per SM instead of 4.
+template <int IR>
+static void (*fixed_kernel_for(int fmt))(WarpArgs) {
+    return fmt == SRC_NV12 ? warp_fixed_kernel<112, 112, IR, 4, SRC_NV12>
+           : fmt == SRC_NV21 ? warp_fixed_kernel<112, 112, IR, 4, SRC_NV21>
+           : fmt == SRC_PLANAR ? warp_fixed_kernel<112, 112, IR, 2, SRC_PLANAR> : warp_fixed_kernel<112, 112, IR, 4, SRC_BGR>;
+}
+// launch names by source format (I420 and YV12 share the planar instantiations)
+static const char *const FIXED_NAMES[4] = {"warp_fixed_kernel", "warp_fixed_kernel_nv12", "warp_fixed_kernel_nv21", "warp_fixed_kernel_i420"};
+static const char *const WARP_NAMES[4] = {"warp_kernel", "warp_kernel_nv12", "warp_kernel_nv21", "warp_kernel_i420"};
+
+// fmt: the source format of frames_dev (SrcFmt)
 int warp_launch(fd_ctx *ctx, const FrameDev *frames_dev, const int32_t *frame_idx_dev, const double *M12_dev,
                 const uint8_t *ok_dev, const int *count_dev, int F_cap, uint8_t *crops_dev, int cw, int ch, const WarpFallback &fb,
-                bool nv12) {
+                int fmt) {
     if (F_cap <= 0) return FD_OK;
     WarpArgs a;
     a.bbox = fb.bbox;
@@ -756,15 +848,14 @@ int warp_launch(fd_ctx *ctx, const FrameDev *frames_dev, const int32_t *frame_id
         // 4 rounds in flight per thread (72 registers, 4 CTAs/SM); 2, 3 measure the same, 7 (104 registers) is 35 % slower.
         static const int ir_env = getenv("FD_WARP_IR") ? atoi(getenv("FD_WARP_IR")) : 14;   // A/B: 16-row items (7 per face, 8 rounds as 4 + 4): 82.0 vs 78.8 us on C2
         const int IR = ir_env == 16 ? 16 : 14;
-        void (*kern)(WarpArgs) = nv12 ? (IR == 16 ? warp_fixed_kernel<112, 112, 16, 4, true> : warp_fixed_kernel<112, 112, 14, 4, true>)
-                                      : (IR == 16 ? warp_fixed_kernel<112, 112, 16, 4, false> : warp_fixed_kernel<112, 112, 14, 4, false>);
-        static int per_sm_fixed[2] = {0, 0};
-        int &per_sm_k = per_sm_fixed[nv12 ? 1 : 0];
+        void (*kern)(WarpArgs) = IR == 16 ? fixed_kernel_for<16>(fmt) : fixed_kernel_for<14>(fmt);
+        static int per_sm_fixed[4] = {0, 0, 0, 0};
+        int &per_sm_k = per_sm_fixed[fmt];
         if (!per_sm_k) FD_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm_k, kern, 224, 0));
         const long long items = (long long)F_cap * (112 / IR);
         const int grid = (int)std::min<long long>(items, (long long)ctx->num_sms * std::max(per_sm_k, 1));
         FD_TRY(launch_pdl(ctx, kern, dim3(grid), dim3(224), 0, a));
-        FD_LAUNCH_CHECK_NAMED(ctx, nv12 ? "warp_fixed_kernel_nv12" : "warp_fixed_kernel");
+        FD_LAUNCH_CHECK_NAMED(ctx, FIXED_NAMES[fmt]);
         if (dbg_on) {   // in-kernel timeline (globaltimer): where a launch's time goes beyond the per-item work
             std::vector<long long> h(8 * (size_t)std::min(grid, 4096));
             cudaStreamSynchronize(ctx->stream);
@@ -784,12 +875,14 @@ int warp_launch(fd_ctx *ctx, const FrameDev *frames_dev, const int32_t *frame_id
     }
     const size_t smem = sizeof(int2) * ((size_t)cw + WARP_BAND);
     int per_sm = 0;
-    void (*kern)(WarpArgs) = nv12 ? warp_kernel<true> : warp_kernel<false>;
+    void (*kern)(WarpArgs) = fmt == SRC_NV12 ? warp_kernel<SRC_NV12>
+                             : fmt == SRC_NV21 ? warp_kernel<SRC_NV21>
+                             : fmt == SRC_PLANAR ? warp_kernel<SRC_PLANAR> : warp_kernel<SRC_BGR>;
     FD_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, WARP_THREADS, smem));
     const long long items = (long long)F_cap * a.bands;
     const int grid = (int)std::min<long long>(items, (long long)ctx->num_sms * std::max(per_sm, 1));
     FD_TRY(launch_pdl(ctx, kern, dim3(grid), dim3(WARP_THREADS), smem, a));
-    FD_LAUNCH_CHECK_NAMED(ctx, nv12 ? "warp_kernel_nv12" : "warp_kernel");
+    FD_LAUNCH_CHECK_NAMED(ctx, WARP_NAMES[fmt]);
     return FD_OK;
 }
 

@@ -46,15 +46,28 @@ struct PinnedBuf {
     template <class T> T *as() const { return reinterpret_cast<T *>(p); }
 };
 
+// Source pixel format of a frame table; the preprocess and warp kernels are instantiated once per format.
+enum SrcFmt : int {
+    SRC_BGR = 0,
+    SRC_NV12 = 1,     // FrameDev::uv: interleaved U,V
+    SRC_NV21 = 2,     // FrameDev::uv: interleaved V,U
+    SRC_PLANAR = 3,   // I420 and YV12: FrameDev::uv is the U plane, FrameDev::v_plane() the V plane
+};
+
 // Per-frame descriptor as the kernels see it.
 struct FrameDev {
-    const uint8_t *data;     // BGR pixels, or the Y plane of an NV12 frame
+    const uint8_t *data;     // BGR pixels, or the Y plane of a 4:2:0 frame
     int h, w, pitch;
     int new_w, new_h;        // letterbox content size
     double scale_x, scale_y; // cv::resize inverse scales
-    const uint8_t *uv;       // NV12: the interleaved U,V plane (h/2 rows of w bytes); nullptr for a BGR frame
-    int pitch_uv;
+    const uint8_t *uv;       // NV12/NV21: the interleaved chroma plane (h/2 rows of w bytes); planar: the U plane (h/2 rows
+                             // of w/2 bytes); nullptr for a BGR frame
+    int pitch_uv;            // of the chroma plane(s)
+    int v_off;               // planar: start of the V plane minus start of the U plane, in bytes; 0 otherwise (fills the
+                             // padding, so the table keeps its size)
+    __host__ __device__ const uint8_t *v_plane() const { return uv + v_off; }   // planar only
 };
+static_assert(sizeof(FrameDev) == 64, "FrameDev: one 64-byte entry per frame");
 
 // Decode geometry passed by value to kernels.
 struct DecodeCfg {
@@ -94,7 +107,7 @@ struct fd_ctx {
 
     // batched pipeline state
     fd::DevBuf frames_dev;       // FrameDev[B]
-    bool frames_nv12 = false;    // frames_dev describes NV12 frames (the kernels reading it take their NV12 variants)
+    int frames_fmt = fd::SRC_BGR;   // source format of the frames in frames_dev (the kernels reading it take that variant)
     fd::DevBuf det_scale_dev;    // float[B]
     fd::DevBuf cand_count;       // int[B] (+ error flags)
     fd::DevBuf cand_keys;        // u64[B][total_anchors]
@@ -258,7 +271,7 @@ __device__ __forceinline__ bool box_is_fast_ok(float4 b) {
 
 // stage entry points implemented across the .cu files
 int preprocess_launch(fd_ctx *ctx, const FrameDev *frames_dev, int B, float *out_nchw_dev, int max_row_bytes, bool rows_aligned16,
-                      bool nv12);
+                      int fmt);
 int resize_launch(fd_ctx *ctx, const FrameDev &frame, uint8_t *out_dev, int out_h, int out_w);
 int crops_to_tensor_launch(fd_ctx *ctx, const uint8_t *crops_dev, const int *count_dev, int F, int in_h, int in_w, int out_h,
                            int out_w, const float *mean_rgb, const float *mul_rgb, float *out_dev);
@@ -288,6 +301,6 @@ struct WarpFallback {
 };
 int warp_launch(fd_ctx *ctx, const FrameDev *frames_dev, const int32_t *frame_idx_dev, const double *M12_dev,
                 const uint8_t *ok_dev, const int *count_dev, int F_cap, uint8_t *crops_dev, int cw, int ch, const WarpFallback &fb,
-                bool nv12);
+                int fmt);
 
 }  // namespace fd

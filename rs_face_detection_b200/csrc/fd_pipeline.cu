@@ -64,34 +64,68 @@ static int fill_frame(const fd_ctx *ctx, const fd_frame &fr, const uint8_t *data
     return fill_geometry(ctx, fr.height, fr.width, out, det_scale);
 }
 
-// cv::cvtColor(COLOR_YUV2BGR_NV12) accepts even sizes only
-static int fill_frame_nv12(const fd_ctx *ctx, const fd_frame_nv12 &fr, FrameDev *out, float *det_scale) {
-    FD_REQUIRE(fr.y && fr.uv, "frame (NV12): null plane");
-    FD_REQUIRE(fr.height > 0 && fr.width > 0 && fr.height % 2 == 0 && fr.width % 2 == 0 && fr.pitch_y >= fr.width && fr.pitch_uv >= fr.width,
-               "frame (NV12): bad geometry (width and height must be even, pitches at least the width)");
+// the kernels' source format of an FD_YUV420_* layout, or -1
+static int yuv420_format(int32_t layout) {
+    switch (layout) {
+    case FD_YUV420_NV12: return SRC_NV12;
+    case FD_YUV420_NV21: return SRC_NV21;
+    case FD_YUV420_I420:
+    case FD_YUV420_YV12: return SRC_PLANAR;
+    default: return -1;
+    }
+}
+
+// cv::cvtColor(COLOR_YUV2BGR_NV12 / _NV21 / _I420 / _YV12) accepts even sizes only.  The planar layouts' second chroma
+// plane starts (height/2) * pitch_uv bytes after the first: V after U for I420, U after V for YV12.
+static int fill_frame_yuv420(const fd_ctx *ctx, const fd_frame_nv12 &fr, int32_t layout, FrameDev *out, float *det_scale) {
+    const bool planar = yuv420_format(layout) == SRC_PLANAR;
+    FD_REQUIRE(fr.y && fr.uv, "frame (YUV 4:2:0): null plane");
+    FD_REQUIRE(fr.height > 0 && fr.width > 0 && fr.height % 2 == 0 && fr.width % 2 == 0 && fr.pitch_y >= fr.width &&
+                   fr.pitch_uv >= (planar ? fr.width / 2 : fr.width),
+               "frame (YUV 4:2:0): bad geometry (width and height must be even, pitches at least the width, or half of it for "
+               "the planar chroma)");
     out->data = fr.y;
     out->pitch = fr.pitch_y;
     out->uv = fr.uv;
     out->pitch_uv = fr.pitch_uv;
+    if (planar) {   // V - U fits the table's 32-bit offset
+        const size_t plane = (size_t)(fr.height / 2) * fr.pitch_uv;
+        FD_REQUIRE(plane <= 0x7fffffffull, "frame (YUV 4:2:0): chroma plane of 2 GB or more");
+        out->v_off = layout == FD_YUV420_I420 ? (int)plane : -(int)plane;
+        if (layout == FD_YUV420_YV12) out->uv = fr.uv + plane;
+    }
     return fill_geometry(ctx, fr.height, fr.width, out, det_scale);
 }
 
-// The frames of a batched call: BGR (bgr) or NV12 (nv12), device pointers; exactly one is set.
+// The frames of a batched call, device pointers: BGR (bgr) or 4:2:0 (yuv, in the FD_YUV420_* layout `layout`); exactly
+// one is set.
 struct FrameList {
     const fd_frame *bgr = nullptr;
-    const fd_frame_nv12 *nv12 = nullptr;
+    const fd_frame_nv12 *yuv = nullptr;
+    int32_t layout = FD_YUV420_NV12;
 };
 
-// uploads B descriptors; returns the widest staged source row in bytes (BGR: 3w, NV12: w)
+// the FrameList of a *_yuv420 call; an unknown layout is rejected here, before any call can return early
+static int yuv420_frames(const fd_frame_nv12 *frames, int32_t layout, FrameList *fl) {
+    FD_REQUIRE(yuv420_format(layout) >= 0, "frame (YUV 4:2:0): unknown layout");
+    fl->yuv = frames;
+    fl->layout = layout;
+    return FD_OK;
+}
+
+// uploads B descriptors and records their source format in ctx->frames_fmt; returns the widest staged source row in bytes
+// (BGR: 3w, NV12/NV21: w, planar: a U and a V half of round16(w/2) bytes each)
 static int upload_frame_table(fd_ctx *ctx, FrameList frames, int B, float *det_scale_host, int *max_row_bytes) {
+    const int fmt = frames.yuv ? yuv420_format(frames.layout) : SRC_BGR;   // a known layout (yuv420_frames)
     std::vector<FrameDev> tab(B);
     int mrb = 0;
     for (int i = 0; i < B; ++i) {
         float ds;
         memset(&tab[i], 0, sizeof(FrameDev));
-        if (frames.nv12) {
-            FD_TRY(fill_frame_nv12(ctx, frames.nv12[i], &tab[i], &ds));
-            mrb = std::max(mrb, frames.nv12[i].width);
+        if (frames.yuv) {
+            const int w = frames.yuv[i].width;
+            FD_TRY(fill_frame_yuv420(ctx, frames.yuv[i], frames.layout, &tab[i], &ds));
+            mrb = std::max(mrb, fmt == SRC_PLANAR ? 2 * ((w / 2 + 15) & ~15) : w);
         } else {
             FD_REQUIRE(frames.bgr[i].data != nullptr, "frame: null data");
             FD_TRY(fill_frame(ctx, frames.bgr[i], frames.bgr[i].data, &tab[i], &ds));
@@ -100,7 +134,7 @@ static int upload_frame_table(fd_ctx *ctx, FrameList frames, int B, float *det_s
         if (det_scale_host) det_scale_host[i] = ds;
     }
     if (max_row_bytes) *max_row_bytes = mrb;
-    ctx->frames_nv12 = frames.nv12 != nullptr;
+    ctx->frames_fmt = fmt;
     const size_t bytes = sizeof(FrameDev) * (size_t)B;
     // the table already on the device is reused when nothing changed (steady-state streaming over a frame ring)
     if (ctx->frames_shadow.size() == bytes && memcmp(ctx->frames_shadow.data(), tab.data(), bytes) == 0) return FD_OK;
@@ -117,7 +151,7 @@ static int upload_frame_table(fd_ctx *ctx, FrameList frames, int B, float *det_s
 // from_detect: the faces are the detections of the last fd_detect_batch; when the fused detect kernel already estimated
 // their transforms (ctx->est_valid) and they all fit, the estimate launch is skipped.
 // fb: the bbox rows / selection of the fallback (face_alignment.rs:64-116); ok_dev receives the per-face mode (0/1/2).
-// The frames are those of the table in ctx->frames_dev, in its format (ctx->frames_nv12).
+// The frames are those of the table in ctx->frames_dev, in its format (ctx->frames_fmt).
 static int align_enqueue(fd_ctx *ctx, const float *lmk_dev, const int32_t *frame_idx_dev,
                          const int *count_dev, int F_cap, uint8_t *crops_dev, double *M_dev, uint8_t *ok_dev, bool from_detect,
                          WarpFallback fb) {
@@ -132,7 +166,7 @@ static int align_enqueue(fd_ctx *ctx, const float *lmk_dev, const int32_t *frame
     }
     fb.mode_out = ok_dev;
     FD_TRY(warp_launch(ctx, ctx->frames_dev.as<FrameDev>(), frame_idx_dev, ctx->align_M.as<double>(), ctx->align_ok.as<uint8_t>(), count_dev,
-                       F_cap, crops_dev, ctx->cfg.crop_w, ctx->cfg.crop_h, fb, ctx->frames_nv12));
+                       F_cap, crops_dev, ctx->cfg.crop_w, ctx->cfg.crop_h, fb, ctx->frames_fmt));
     return FD_OK;
 }
 
@@ -163,7 +197,7 @@ static int detect_resolve(fd_ctx *ctx) {
         }
         FD_TRY(finalize_launch(ctx, B));
         ctx->est_valid = false;
-        if (ctx->align_replay)  // the crops were produced from incomplete detections: align again (BGR or NV12, as the table)
+        if (ctx->align_replay)  // the crops were produced from incomplete detections: align again (in the table's format)
             FD_TRY(align_enqueue(ctx, ctx->out_lmk.as<float>(), ctx->out_frame_idx.as<int32_t>(),
                                  ctx->status() + 2, ctx->align_cap, ctx->align_crops, ctx->align_M_out, ctx->align_ok_out, true,
                                  detect_fallback(ctx)));
@@ -240,7 +274,7 @@ FD_EXPORT int fd_letterbox_geometry(const fd_ctx *ctx, int img_h, int img_w, int
 
 static int preprocess_batch(fd_ctx *ctx, FrameList frames, int B, float *out_nchw_dev, float *det_scale_host) {
     FD_TRY(check_ctx(ctx));
-    FD_REQUIRE(B >= 0 && (B == 0 || ((frames.bgr || frames.nv12) && out_nchw_dev)), "fd_preprocess_batch: bad arguments");
+    FD_REQUIRE(B >= 0 && (B == 0 || ((frames.bgr || frames.yuv) && out_nchw_dev)), "fd_preprocess_batch: bad arguments");
     if (B == 0) return FD_OK;
     int mrb = 0;
     FD_TRY(upload_frame_table(ctx, frames, B, det_scale_host, &mrb));
@@ -249,14 +283,15 @@ static int preprocess_batch(fd_ctx *ctx, FrameList frames, int B, float *out_nch
         return reinterpret_cast<uintptr_t>(p) % 16 == 0 && pitch % 16 == 0 && ((row_bytes + 15) & ~15) <= pitch;
     };
     for (int i = 0; i < B; ++i) {
-        if (frames.nv12) {
-            const fd_frame_nv12 &f = frames.nv12[i];
-            aligned = aligned && row_ok(f.y, f.pitch_y, f.width) && row_ok(f.uv, f.pitch_uv, f.width);
+        if (frames.yuv) {   // planar: the second chroma plane starts whole pitches after the first
+            const fd_frame_nv12 &f = frames.yuv[i];
+            const bool planar = ctx->frames_fmt == SRC_PLANAR;
+            aligned = aligned && row_ok(f.y, f.pitch_y, f.width) && row_ok(f.uv, f.pitch_uv, planar ? f.width / 2 : f.width);
         } else {
             aligned = aligned && row_ok(frames.bgr[i].data, frames.bgr[i].pitch, frames.bgr[i].width * 3);
         }
     }
-    return preprocess_launch(ctx, ctx->frames_dev.as<FrameDev>(), B, out_nchw_dev, mrb, aligned, frames.nv12 != nullptr);
+    return preprocess_launch(ctx, ctx->frames_dev.as<FrameDev>(), B, out_nchw_dev, mrb, aligned, ctx->frames_fmt);
 }
 
 FD_EXPORT int fd_preprocess_batch(fd_ctx *ctx, const fd_frame *frames, int B, float *out_nchw_dev, float *det_scale_host) {
@@ -264,10 +299,13 @@ FD_EXPORT int fd_preprocess_batch(fd_ctx *ctx, const fd_frame *frames, int B, fl
     fl.bgr = frames;
     return preprocess_batch(ctx, fl, B, out_nchw_dev, det_scale_host);
 }
-FD_EXPORT int fd_preprocess_batch_nv12(fd_ctx *ctx, const fd_frame_nv12 *frames, int B, float *out_nchw_dev, float *det_scale_host) {
+FD_EXPORT int fd_preprocess_batch_yuv420(fd_ctx *ctx, const fd_frame_nv12 *frames, int32_t layout, int B, float *out_nchw_dev, float *det_scale_host) {
     FrameList fl;
-    fl.nv12 = frames;
+    FD_TRY(yuv420_frames(frames, layout, &fl));
     return preprocess_batch(ctx, fl, B, out_nchw_dev, det_scale_host);
+}
+FD_EXPORT int fd_preprocess_batch_nv12(fd_ctx *ctx, const fd_frame_nv12 *frames, int B, float *out_nchw_dev, float *det_scale_host) {
+    return fd_preprocess_batch_yuv420(ctx, frames, FD_YUV420_NV12, B, out_nchw_dev, det_scale_host);
 }
 
 FD_EXPORT int fd_detect_batch(fd_ctx *ctx, const float *const *heads_dev, int n_heads, int B, const float *det_scale_host,
@@ -337,7 +375,7 @@ FD_EXPORT int fd_detect_last_stats(fd_ctx *ctx, int32_t *out) {
 static int align_batch(fd_ctx *ctx, FrameList frames, int B, const float *landmarks_dev, const int32_t *frame_idx_dev,
                        const float *bbox_dev, int F, uint8_t *crops_dev, double *M_dev, uint8_t *ok_dev) {
     FD_TRY(check_ctx(ctx));
-    FD_REQUIRE(B > 0 && (frames.bgr || frames.nv12) && F >= 0 && (F == 0 || (landmarks_dev && crops_dev)), "fd_align_batch: bad arguments");
+    FD_REQUIRE(B > 0 && (frames.bgr || frames.yuv) && F >= 0 && (F == 0 || (landmarks_dev && crops_dev)), "fd_align_batch: bad arguments");
     if (F == 0) return FD_OK;
     FD_TRY(upload_frame_table(ctx, frames, B, nullptr, nullptr));
     WarpFallback fb;
@@ -352,16 +390,20 @@ FD_EXPORT int fd_align_batch(fd_ctx *ctx, const fd_frame *frames, int B, const f
     fl.bgr = frames;
     return align_batch(ctx, fl, B, landmarks_dev, frame_idx_dev, bbox_dev, F, crops_dev, M_dev, ok_dev);
 }
-FD_EXPORT int fd_align_batch_nv12(fd_ctx *ctx, const fd_frame_nv12 *frames, int B, const float *landmarks_dev, const int32_t *frame_idx_dev,
+FD_EXPORT int fd_align_batch_yuv420(fd_ctx *ctx, const fd_frame_nv12 *frames, int32_t layout, int B, const float *landmarks_dev, const int32_t *frame_idx_dev,
                                   const float *bbox_dev, int F, uint8_t *crops_dev, double *M_dev, uint8_t *ok_dev) {
     FrameList fl;
-    fl.nv12 = frames;
+    FD_TRY(yuv420_frames(frames, layout, &fl));
     return align_batch(ctx, fl, B, landmarks_dev, frame_idx_dev, bbox_dev, F, crops_dev, M_dev, ok_dev);
+}
+FD_EXPORT int fd_align_batch_nv12(fd_ctx *ctx, const fd_frame_nv12 *frames, int B, const float *landmarks_dev, const int32_t *frame_idx_dev,
+                                  const float *bbox_dev, int F, uint8_t *crops_dev, double *M_dev, uint8_t *ok_dev) {
+    return fd_align_batch_yuv420(ctx, frames, FD_YUV420_NV12, B, landmarks_dev, frame_idx_dev, bbox_dev, F, crops_dev, M_dev, ok_dev);
 }
 
 static int align_detections(fd_ctx *ctx, FrameList frames, int B, uint8_t *crops_dev, int cap_faces, double *M_dev, uint8_t *ok_dev) {
     FD_TRY(check_ctx(ctx));
-    FD_REQUIRE(B > 0 && (frames.bgr || frames.nv12) && B == ctx->last_B && crops_dev && cap_faces > 0, "fd_align_detections: bad arguments");
+    FD_REQUIRE(B > 0 && (frames.bgr || frames.yuv) && B == ctx->last_B && crops_dev && cap_faces > 0, "fd_align_detections: bad arguments");
     // No host synchronisation here: images needing the big NMS path are detected lazily at
     // fd_detect_fetch / fd_detect_view / fd_ctx-level fetch, which replays this align if the detections changed.
     FD_TRY(upload_frame_table(ctx, frames, B, nullptr, nullptr));
@@ -380,11 +422,15 @@ FD_EXPORT int fd_align_detections(fd_ctx *ctx, const fd_frame *frames, int B, ui
     fl.bgr = frames;
     return align_detections(ctx, fl, B, crops_dev, cap_faces, M_dev, ok_dev);
 }
-FD_EXPORT int fd_align_detections_nv12(fd_ctx *ctx, const fd_frame_nv12 *frames, int B, uint8_t *crops_dev, int cap_faces, double *M_dev,
+FD_EXPORT int fd_align_detections_yuv420(fd_ctx *ctx, const fd_frame_nv12 *frames, int32_t layout, int B, uint8_t *crops_dev, int cap_faces, double *M_dev,
                                        uint8_t *ok_dev) {
     FrameList fl;
-    fl.nv12 = frames;
+    FD_TRY(yuv420_frames(frames, layout, &fl));
     return align_detections(ctx, fl, B, crops_dev, cap_faces, M_dev, ok_dev);
+}
+FD_EXPORT int fd_align_detections_nv12(fd_ctx *ctx, const fd_frame_nv12 *frames, int B, uint8_t *crops_dev, int cap_faces, double *M_dev,
+                                       uint8_t *ok_dev) {
+    return fd_align_detections_yuv420(ctx, frames, FD_YUV420_NV12, B, crops_dev, cap_faces, M_dev, ok_dev);
 }
 
 // ---- single-image host wrappers -----------------------------------------------------------------------------------
@@ -521,7 +567,7 @@ static int warp_host(fd_ctx *ctx, const uint8_t *img, int h, int w, int pitch, c
     const size_t n = (size_t)out_h * out_w * 3;
     FD_TRY(ctx->scratch[4].reserve(n));
     FD_TRY(warp_launch(ctx, ctx->scratch[5].as<FrameDev>(), nullptr, ctx->align_M.as<double>(), ctx->align_ok.as<uint8_t>(), nullptr, 1,
-                       ctx->scratch[4].as<uint8_t>(), out_w, out_h, fb, false));
+                       ctx->scratch[4].as<uint8_t>(), out_w, out_h, fb, SRC_BGR));
     uint8_t mode = 0;
     double M12[12];
     FD_CUDA(cudaMemcpyAsync(out, ctx->scratch[4].p, n, cudaMemcpyDeviceToHost, ctx->stream));
@@ -648,7 +694,7 @@ FD_EXPORT int fd_face_selection(fd_ctx *ctx, int img_h, int img_w, const float *
 
 static int select_detections(fd_ctx *ctx, FrameList frames, int B, int is_enroll, const fd_select_params *params, int32_t *sel_host) {
     FD_TRY(check_ctx(ctx));
-    FD_REQUIRE((frames.bgr || frames.nv12) && B > 0 && B == ctx->last_B, "fd_select_detections: needs the frames of the last fd_detect_batch");
+    FD_REQUIRE((frames.bgr || frames.yuv) && B > 0 && B == ctx->last_B, "fd_select_detections: needs the frames of the last fd_detect_batch");
     if (sel_host) FD_TRY(detect_resolve(ctx));
     fd_select_params p;
     if (params) p = *params;
@@ -672,16 +718,20 @@ FD_EXPORT int fd_select_detections(fd_ctx *ctx, const fd_frame *frames, int B, i
     fl.bgr = frames;
     return select_detections(ctx, fl, B, is_enroll, params, sel_host);
 }
-FD_EXPORT int fd_select_detections_nv12(fd_ctx *ctx, const fd_frame_nv12 *frames, int B, int is_enroll, const fd_select_params *params,
+FD_EXPORT int fd_select_detections_yuv420(fd_ctx *ctx, const fd_frame_nv12 *frames, int32_t layout, int B, int is_enroll, const fd_select_params *params,
                                         int32_t *sel_host) {
     FrameList fl;
-    fl.nv12 = frames;
+    FD_TRY(yuv420_frames(frames, layout, &fl));
     return select_detections(ctx, fl, B, is_enroll, params, sel_host);
+}
+FD_EXPORT int fd_select_detections_nv12(fd_ctx *ctx, const fd_frame_nv12 *frames, int B, int is_enroll, const fd_select_params *params,
+                                        int32_t *sel_host) {
+    return fd_select_detections_yuv420(ctx, frames, FD_YUV420_NV12, B, is_enroll, params, sel_host);
 }
 
 static int align_selected(fd_ctx *ctx, FrameList frames, int B, uint8_t *crops_dev, double *M_dev, uint8_t *ok_dev) {
     FD_TRY(check_ctx(ctx));
-    FD_REQUIRE((frames.bgr || frames.nv12) && B > 0 && B == ctx->select_B && crops_dev,
+    FD_REQUIRE((frames.bgr || frames.yuv) && B > 0 && B == ctx->select_B && crops_dev,
                "fd_align_selected: needs the frames of the last fd_select_detections");
     FD_TRY(upload_frame_table(ctx, frames, B, nullptr, nullptr));
     // Images without a selection (or whose selection has no key points) carry NaN key points: the estimate fails there and,
@@ -697,10 +747,13 @@ FD_EXPORT int fd_align_selected(fd_ctx *ctx, const fd_frame *frames, int B, uint
     fl.bgr = frames;
     return align_selected(ctx, fl, B, crops_dev, M_dev, ok_dev);
 }
-FD_EXPORT int fd_align_selected_nv12(fd_ctx *ctx, const fd_frame_nv12 *frames, int B, uint8_t *crops_dev, double *M_dev, uint8_t *ok_dev) {
+FD_EXPORT int fd_align_selected_yuv420(fd_ctx *ctx, const fd_frame_nv12 *frames, int32_t layout, int B, uint8_t *crops_dev, double *M_dev, uint8_t *ok_dev) {
     FrameList fl;
-    fl.nv12 = frames;
+    FD_TRY(yuv420_frames(frames, layout, &fl));
     return align_selected(ctx, fl, B, crops_dev, M_dev, ok_dev);
+}
+FD_EXPORT int fd_align_selected_nv12(fd_ctx *ctx, const fd_frame_nv12 *frames, int B, uint8_t *crops_dev, double *M_dev, uint8_t *ok_dev) {
+    return fd_align_selected_yuv420(ctx, frames, FD_YUV420_NV12, B, crops_dev, M_dev, ok_dev);
 }
 
 // ---- end-to-end with host buffers ------------------------------------------------------------------------------------
@@ -1020,7 +1073,7 @@ static int pipeline_host_impl(fd_ctx *ctx, const fd_frame *frames, const fd_fram
             FD_TRY(upload_frame_table(ctx, fl, B, nullptr, nullptr));
             fb.mode_out = mode_dev;
             FD_TRY(warp_launch(ctx, frames_dev, fidx_dev, ctx->align_M.as<double>(), ctx->align_ok.as<uint8_t>(), nullptr,
-                               std::min(F, (int)out->cap_rows), crops_dev, cw, ch, fb, false));
+                               std::min(F, (int)out->cap_rows), crops_dev, cw, ch, fb, SRC_BGR));
             ctx->align_replay = false;
         }
         if (select && out->sel) {

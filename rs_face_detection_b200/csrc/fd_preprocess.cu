@@ -43,10 +43,12 @@ __device__ __forceinline__ const uint8_t *stage_row(uint8_t *buf, const uint8_t 
     return dst;
 }
 
-// NV: the frame is NV12 (FrameDev::uv); each tap is converted to BGR (yuv_bgr24) before the resize arithmetic, and the
-// staged rows are the Y rows and the UV row(s) of the taps.
-template <bool NV>
+// FMT: the source format (SrcFmt).  A 4:2:0 frame's taps are converted to BGR (yuv_bgr24) before the resize arithmetic,
+// and the staged rows are the Y rows and the chroma row(s) of the taps; a planar chroma row is staged as its U half and,
+// row_buf_bytes / 2 further, its V half.
+template <int FMT>
 __global__ void preprocess_kernel(PreArgs a) {
+    constexpr bool NV = FMT != SRC_BGR, PL = FMT == SRC_PLANAR;
     extern __shared__ __align__(16) unsigned char smem[];
     const int ow = a.out_w;
     float *lut = reinterpret_cast<float *>(smem);                  // [3][256], indexed by BGR channel
@@ -58,7 +60,8 @@ __global__ void preprocess_kernel(PreArgs a) {
     tab_bytes = (tab_bytes + 15) & ~(size_t)15;
     uint8_t *rowbuf0 = smem + tab_bytes;
     uint8_t *rowbuf1 = rowbuf0 + a.row_buf_bytes;
-    uint8_t *rowbuf2 = rowbuf1 + a.row_buf_bytes, *rowbuf3 = rowbuf2 + a.row_buf_bytes;   // NV: UV rows
+    uint8_t *rowbuf2 = rowbuf1 + a.row_buf_bytes, *rowbuf3 = rowbuf2 + a.row_buf_bytes;   // NV: chroma rows
+    const int half = a.row_buf_bytes >> 1;                                                // PL: V half of a chroma row
 
     for (int i = threadIdx.x; i < 768; i += blockDim.x) {
         int c = i >> 8, v = i & 255;
@@ -84,14 +87,22 @@ __global__ void preprocess_kernel(PreArgs a) {
         float *o_g = o_r + plane;
         float *o_b = o_g + plane;
         const bool content = dy < f.new_h;
-        const uint8_t *r0 = nullptr, *r1 = nullptr, *c0 = nullptr, *c1 = nullptr;
+        const uint8_t *r0 = nullptr, *r1 = nullptr, *c0 = nullptr, *c1 = nullptr, *v0 = nullptr, *v1 = nullptr;
         int b0 = 0, b1 = 0;
         if (content) {
             int y0, y1;
             y_taps(dy, f.scale_y, f.h, &y0, &y1, &b0, &b1);
             r0 = stage_row(rowbuf0, f.data + (size_t)y0 * f.pitch, src_row_bytes);
             r1 = b1 != 0 ? stage_row(rowbuf1, f.data + (size_t)y1 * f.pitch, src_row_bytes) : r0;
-            if (NV) {   // one UV row when both taps share it (or the second tap has weight 0)
+            if (PL) {   // U and V halves of one chroma row when both taps share it (or the second tap has weight 0)
+                const int cb = f.w >> 1;
+                const size_t oc0 = (size_t)(y0 >> 1) * f.pitch_uv, oc1 = (size_t)(y1 >> 1) * f.pitch_uv;
+                c0 = stage_row(rowbuf2, f.uv + oc0, cb);
+                v0 = stage_row(rowbuf2 + half, f.v_plane() + oc0, cb);
+                const bool two = b1 != 0 && (y1 >> 1) != (y0 >> 1);
+                c1 = two ? stage_row(rowbuf3, f.uv + oc1, cb) : c0;
+                v1 = two ? stage_row(rowbuf3 + half, f.v_plane() + oc1, cb) : v0;
+            } else if (NV) {   // one UV row when both taps share it (or the second tap has weight 0)
                 c0 = stage_row(rowbuf2, f.uv + (size_t)(y0 >> 1) * f.pitch_uv, src_row_bytes);
                 c1 = b1 != 0 && (y1 >> 1) != (y0 >> 1) ? stage_row(rowbuf3, f.uv + (size_t)(y1 >> 1) * f.pitch_uv, src_row_bytes) : c0;
             }
@@ -105,8 +116,9 @@ __global__ void preprocess_kernel(PreArgs a) {
                 if (content && x < f.new_w) {
                     const int x0 = xo0[x], x1 = xo1[x], a0 = xa0[x], a1 = xa1[x];
                     if (NV) {
-                        const unsigned p = resize_px24(nv12_px24(r0, c0, x0), nv12_px24(r0, c0, x1), b1 != 0 ? nv12_px24(r1, c1, x0) : 0u,
-                                                       b1 != 0 ? nv12_px24(r1, c1, x1) : 0u, a0, a1, b0, b1);
+                        const unsigned p = resize_px24(yuv_px24<FMT>(r0, c0, v0, x0), yuv_px24<FMT>(r0, c0, v0, x1),
+                                                       b1 != 0 ? yuv_px24<FMT>(r1, c1, v1, x0) : 0u, b1 != 0 ? yuv_px24<FMT>(r1, c1, v1, x1) : 0u,
+                                                       a0, a1, b0, b1);
                         vb[j] = lut[p & 255u];
                         vg[j] = lut[256 + ((p >> 8) & 255u)];
                         vr[j] = lut[512 + (p >> 16)];
@@ -166,10 +178,12 @@ __device__ __forceinline__ void bulk_g2s(void *dst_smem, const void *src_gmem, u
                  : "memory");
 }
 
-// NV: NV12 frame; a stage holds the Y rows of the taps and their UV row(s) — one when both taps map to the same UV row
-// (4K -> 640x360: rows 6y+2 and 6y+3 both read UV row 3y+1).
-template <bool IDENT, bool NV>
+// FMT: the source format (SrcFmt).  4:2:0: a stage holds the Y rows of the taps and their chroma row(s) — one when both
+// taps map to the same chroma row (4K -> 640x360: rows 6y+2 and 6y+3 both read chroma row 3y+1).  A planar chroma row
+// fills its slot as the U half and, row_buf_bytes / 2 further, the V half: bulk copies of round16(w/2) bytes each.
+template <bool IDENT, int FMT>
 __global__ void __launch_bounds__(256) preprocess_tma_kernel(PreArgs a) {
+    constexpr bool NV = FMT != SRC_BGR, PL = FMT == SRC_PLANAR;
     constexpr int SLOTS = NV ? 4 : 2;                           // rows per stage: Y0, Y1 (BGR: row 0, row 1), UV0, UV1
     extern __shared__ __align__(128) unsigned char smem[];
     uint64_t *full = reinterpret_cast<uint64_t *>(smem);        // [PRE2_STAGES]
@@ -218,6 +232,8 @@ __global__ void __launch_bounds__(256) preprocess_tma_kernel(PreArgs a) {
     const int row_end = min(row_begin + PRE2_ROWS, a.out_h);
     const int n_content = max(0, min(f.new_h, row_end) - row_begin);
     const uint32_t copy_bytes = (uint32_t)(((NV ? f.w : f.w * 3) + 15) & ~15);
+    const uint32_t half_bytes = (uint32_t)(((f.w >> 1) + 15) & ~15);   // PL: one U or V row
+    const int half = rb >> 1;
     const bool active = 4 * tid < ow;
 
     auto issue = [&](int it) {
@@ -226,11 +242,22 @@ __global__ void __launch_bounds__(256) preprocess_tma_kernel(PreArgs a) {
         const int st = it % PRE2_STAGES;
         uint8_t *dst = bufs + (size_t)st * SLOTS * rb;
         const bool uv1 = NV && b1 != 0 && (y1 >> 1) != (y0 >> 1);
-        mbar_expect_tx(&full[st], copy_bytes * ((b1 != 0 ? 2 : 1) + (NV ? 1 : 0) + (uv1 ? 1 : 0)));
+        if (PL) mbar_expect_tx(&full[st], copy_bytes * (b1 != 0 ? 2 : 1) + half_bytes * (uv1 ? 4 : 2));
+        else mbar_expect_tx(&full[st], copy_bytes * ((b1 != 0 ? 2 : 1) + (NV ? 1 : 0) + (uv1 ? 1 : 0)));
         bulk_g2s(dst, f.data + (size_t)y0 * f.pitch, copy_bytes, &full[st]);
         if (b1 != 0) bulk_g2s(dst + rb, f.data + (size_t)y1 * f.pitch, copy_bytes, &full[st]);
-        if (NV) bulk_g2s(dst + 2 * rb, f.uv + (size_t)(y0 >> 1) * f.pitch_uv, copy_bytes, &full[st]);
-        if (uv1) bulk_g2s(dst + 3 * rb, f.uv + (size_t)(y1 >> 1) * f.pitch_uv, copy_bytes, &full[st]);
+        if (PL) {
+            const size_t oc0 = (size_t)(y0 >> 1) * f.pitch_uv, oc1 = (size_t)(y1 >> 1) * f.pitch_uv;
+            bulk_g2s(dst + 2 * rb, f.uv + oc0, half_bytes, &full[st]);
+            bulk_g2s(dst + 2 * rb + half, f.v_plane() + oc0, half_bytes, &full[st]);
+            if (uv1) {
+                bulk_g2s(dst + 3 * rb, f.uv + oc1, half_bytes, &full[st]);
+                bulk_g2s(dst + 3 * rb + half, f.v_plane() + oc1, half_bytes, &full[st]);
+            }
+        } else {
+            if (NV) bulk_g2s(dst + 2 * rb, f.uv + (size_t)(y0 >> 1) * f.pitch_uv, copy_bytes, &full[st]);
+            if (uv1) bulk_g2s(dst + 3 * rb, f.uv + (size_t)(y1 >> 1) * f.pitch_uv, copy_bytes, &full[st]);
+        }
     };
     if (tid == 0)
         for (int it = 0; it < PRE2_STAGES - 1 && it < n_content; ++it) issue(it);
@@ -244,6 +271,7 @@ __global__ void __launch_bounds__(256) preprocess_tma_kernel(PreArgs a) {
         const uint8_t *r0 = bufs + (size_t)st * SLOTS * rb;
         const uint8_t *r1 = b1 != 0 ? r0 + rb : r0;
         const uint8_t *c0 = r0 + 2 * rb, *c1 = b1 != 0 && (y1 >> 1) != (y0 >> 1) ? r0 + 3 * rb : c0;   // NV only
+        const uint8_t *v0 = c0 + half, *v1 = c1 + half;                                               // PL only
         mbar_wait(&full[st], (uint32_t)((it / PRE2_STAGES) & 1));
         if (active) {
             float vr[4], vg[4], vb[4];
@@ -253,7 +281,7 @@ __global__ void __launch_bounds__(256) preprocess_tma_kernel(PreArgs a) {
                     if (x0[j] >= 0) {
                         int pb, pg, pr;
                         if (NV) {
-                            const unsigned p = nv12_px24(r0, c0, x0[j]);
+                            const unsigned p = yuv_px24<FMT>(r0, c0, v0, x0[j]);
                             pb = p & 255u; pg = (p >> 8) & 255u; pr = p >> 16;
                         } else {
                             const uint8_t *p = r0 + x0[j];
@@ -273,8 +301,9 @@ __global__ void __launch_bounds__(256) preprocess_tma_kernel(PreArgs a) {
                         const int o0 = x0[j], o1 = x0[j] + (wa1[j] != 0 ? (NV ? 1 : 3) : 0), q0 = wa0[j], q1 = wa1[j];
                         int pb, pg, pr;
                         if (NV) {
-                            const unsigned p = resize_px24(nv12_px24(r0, c0, o0), nv12_px24(r0, c0, o1), b1 != 0 ? nv12_px24(r1, c1, o0) : 0u,
-                                                           b1 != 0 ? nv12_px24(r1, c1, o1) : 0u, q0, q1, b0, b1);
+                            const unsigned p = resize_px24(yuv_px24<FMT>(r0, c0, v0, o0), yuv_px24<FMT>(r0, c0, v0, o1),
+                                                           b1 != 0 ? yuv_px24<FMT>(r1, c1, v1, o0) : 0u,
+                                                           b1 != 0 ? yuv_px24<FMT>(r1, c1, v1, o1) : 0u, q0, q1, b0, b1);
                             pb = p & 255u; pg = (p >> 8) & 255u; pr = p >> 16;
                         } else {
                             pb = resize_px(r0, r1, o0, o1, q0, q1, b0, b1);
@@ -401,10 +430,24 @@ int crops_to_tensor_launch(fd_ctx *ctx, const uint8_t *crops_dev, const int *cou
     return FD_OK;
 }
 
-// max_row_bytes: widest staged row (BGR: 3w, NV12: w); nv12: frames_dev describes NV12 frames
+// launch names by source format (I420 and YV12 share the planar instantiations)
+static const char *const TMA_NAMES[4] = {"preprocess_tma_kernel", "preprocess_tma_kernel_nv12", "preprocess_tma_kernel_nv21",
+                                         "preprocess_tma_kernel_i420"};
+static const char *const PRE_NAMES[4] = {"preprocess_kernel", "preprocess_kernel_nv12", "preprocess_kernel_nv21", "preprocess_kernel_i420"};
+
+template <bool IDENT>
+static void (*tma_kernel_for(int fmt))(PreArgs) {
+    return fmt == SRC_NV12 ? preprocess_tma_kernel<IDENT, SRC_NV12>
+           : fmt == SRC_NV21 ? preprocess_tma_kernel<IDENT, SRC_NV21>
+           : fmt == SRC_PLANAR ? preprocess_tma_kernel<IDENT, SRC_PLANAR> : preprocess_tma_kernel<IDENT, SRC_BGR>;
+}
+
+// max_row_bytes: widest staged row (BGR: 3w, NV12/NV21: w, planar: 2 round16(w/2), a U half and a V half); fmt: the
+// source format of frames_dev (SrcFmt)
 int preprocess_launch(fd_ctx *ctx, const FrameDev *frames_dev, int B, float *out_nchw_dev, int max_row_bytes, bool rows_aligned16,
-                      bool nv12) {
+                      int fmt) {
     constexpr int SLOTS_NV = 4;
+    const bool nv = fmt != SRC_BGR;
     PreArgs a;
     a.frames = frames_dev;
     a.out = out_nchw_dev;
@@ -423,28 +466,29 @@ int preprocess_launch(fd_ctx *ctx, const FrameDev *frames_dev, int B, float *out
     // v2 (bulk-TMA staging): 16-byte aligned source rows, vector stores, one 4-pixel group per thread
     if (rows_aligned16 && a.vec_store && ngroups <= 256) {
         a.row_buf_bytes = (max_row_bytes + 15) & ~15;
-        size_t smem = 64 + 3072 + (size_t)PRE2_STAGES * (nv12 ? SLOTS_NV : 2) * a.row_buf_bytes;
+        size_t smem = 64 + 3072 + (size_t)PRE2_STAGES * (nv ? SLOTS_NV : 2) * a.row_buf_bytes;
         if (smem <= (size_t)ctx->max_smem_optin) {
             int threads = std::max(32, ((ngroups + 31) / 32) * 32);
             dim3 grid((a.out_h + PRE2_ROWS - 1) / PRE2_ROWS, B);
-            void (*kern)(PreArgs) = nv12 ? (ident ? preprocess_tma_kernel<true, true> : preprocess_tma_kernel<false, true>)
-                                         : (ident ? preprocess_tma_kernel<true, false> : preprocess_tma_kernel<false, false>);
+            void (*kern)(PreArgs) = ident ? tma_kernel_for<true>(fmt) : tma_kernel_for<false>(fmt);
             FD_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
             FD_TRY(launch_pdl(ctx, kern, grid, dim3(threads), smem, a));
-            FD_LAUNCH_CHECK_NAMED(ctx, nv12 ? "preprocess_tma_kernel_nv12" : "preprocess_tma_kernel");
+            FD_LAUNCH_CHECK_NAMED(ctx, TMA_NAMES[fmt]);
             return FD_OK;
         }
     }
     size_t tab_bytes = 768 * 4 + (size_t)a.out_w * 12;
     tab_bytes = (tab_bytes + 15) & ~(size_t)15;
-    size_t smem = tab_bytes + (nv12 ? SLOTS_NV : 2) * (size_t)a.row_buf_bytes;
+    size_t smem = tab_bytes + (nv ? SLOTS_NV : 2) * (size_t)a.row_buf_bytes;
     if (smem > (size_t)ctx->max_smem_optin) return fail(FD_ERR_INVALID, "fd_preprocess: source row too wide for shared-memory staging");
-    void (*kern)(PreArgs) = nv12 ? preprocess_kernel<true> : preprocess_kernel<false>;
+    void (*kern)(PreArgs) = fmt == SRC_NV12 ? preprocess_kernel<SRC_NV12>
+                            : fmt == SRC_NV21 ? preprocess_kernel<SRC_NV21>
+                            : fmt == SRC_PLANAR ? preprocess_kernel<SRC_PLANAR> : preprocess_kernel<SRC_BGR>;
     FD_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int threads = std::min(1024, std::max(64, ((ngroups + 31) / 32) * 32));
     dim3 grid((a.out_h + PRE_ROWS - 1) / PRE_ROWS, B);
     FD_TRY(launch_pdl(ctx, kern, grid, dim3(threads), smem, a));
-    FD_LAUNCH_CHECK_NAMED(ctx, nv12 ? "preprocess_kernel_nv12" : "preprocess_kernel");
+    FD_LAUNCH_CHECK_NAMED(ctx, PRE_NAMES[fmt]);
     return FD_OK;
 }
 

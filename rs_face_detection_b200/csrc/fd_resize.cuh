@@ -89,7 +89,7 @@ __device__ __forceinline__ unsigned resize_pixel24(const uint8_t *roi, int pitch
     return pb | (pg << 8) | (pr << 16);
 }
 
-// ---- NV12 sources: every tap is converted as cv::cvtColor(COLOR_YUV2BGR_NV12) would have converted the whole frame ----
+// ---- 4:2:0 sources: every tap is converted as cv::cvtColor(COLOR_YUV2BGR_*) would have converted the whole frame ------
 // OpenCV's BT.601 limited-range conversion (imgproc color_yuv: 20-bit fixed point, round half up, saturate), restated in
 // int32 and equal to cv2 4.13 on all 2^24 (Y,U,V) triples.  Returns b | g << 8 | r << 16.
 __device__ __forceinline__ unsigned yuv_bgr24(int Y, int U, int V) {
@@ -97,9 +97,13 @@ __device__ __forceinline__ unsigned yuv_bgr24(int Y, int U, int V) {
     const int r = (y + 1673527 * v) >> 20, g = (y - 852492 * v - 409993 * u) >> 20, b = (y + 2116026 * u) >> 20;
     return (unsigned)min(max(b, 0), 255) | ((unsigned)min(max(g, 0), 255) << 8) | ((unsigned)min(max(r, 0), 255) << 16);
 }
-// pixel x of an NV12 row: its own Y and the U,V pair of its 2x2 block (uvrow = UV plane row y/2)
-__device__ __forceinline__ unsigned nv12_px24(const uint8_t *yrow, const uint8_t *uvrow, int x) {
-    return yuv_bgr24(yrow[x], uvrow[x & ~1], uvrow[x | 1]);
+// pixel x of a 4:2:0 row (FMT: SRC_NV12, SRC_NV21 or SRC_PLANAR): its own Y and the chroma of its 2x2 block.  crow is the
+// chroma row y/2: interleaved U,V (NV12) or V,U (NV21), or the U row, whose V row is vrow (planar; unused otherwise).
+template <int FMT>
+__device__ __forceinline__ unsigned yuv_px24(const uint8_t *yrow, const uint8_t *crow, const uint8_t *vrow, int x) {
+    if (FMT == SRC_PLANAR) return yuv_bgr24(yrow[x], crow[x >> 1], vrow[x >> 1]);
+    if (FMT == SRC_NV21) return yuv_bgr24(yrow[x], crow[x | 1], crow[x & ~1]);
+    return yuv_bgr24(yrow[x], crow[x & ~1], crow[x | 1]);
 }
 
 // resize_px on the three channels of packed pixels: taps (p00, p01) of the first row, (p10, p11) of the second (read only
@@ -119,13 +123,20 @@ __device__ __forceinline__ unsigned resize_px24(unsigned p00, unsigned p01, unsi
     return out;
 }
 
-// resize_pixel24 of the ROI (rx0, ry0)..(rx0 + rw, ry0 + rh) of an NV12 frame: taps in ROI coordinates, chroma of the
-// frame's own 2x2 blocks (rx0, ry0 may be odd)
-__device__ __forceinline__ unsigned resize_pixel24_nv12(const uint8_t *yp, int pitch, const uint8_t *uvp, int pitch_uv, int rx0, int ry0,
-                                                        int rw, int rh, int ow, int oh, int x, int y) {
+// resize_pixel24 of the ROI (rx0, ry0)..(rx0 + rw, ry0 + rh) of a 4:2:0 frame (chroma plane uvp, and vp the V plane when
+// planar): taps in ROI coordinates, chroma of the frame's own 2x2 blocks (rx0, ry0 may be odd)
+// (The V pointers are formed only for the planar format: vp is null otherwise.)
+template <int FMT>
+__device__ __forceinline__ unsigned resize_pixel24_yuv(const uint8_t *yp, int pitch, const uint8_t *uvp, const uint8_t *vp, int pitch_uv,
+                                                       int rx0, int ry0, int rw, int rh, int ow, int oh, int x, int y) {
     if (rw == ow && rh == oh) {
         const int sy = ry0 + y;
-        return nv12_px24(yp + (size_t)sy * pitch, uvp + (size_t)(sy >> 1) * pitch_uv, rx0 + x);
+        if constexpr (FMT == SRC_PLANAR) {
+            const size_t oc = (size_t)(sy >> 1) * pitch_uv;
+            return yuv_px24<FMT>(yp + (size_t)sy * pitch, uvp + oc, vp + oc, rx0 + x);
+        } else {
+            return yuv_px24<FMT>(yp + (size_t)sy * pitch, uvp + (size_t)(sy >> 1) * pitch_uv, nullptr, rx0 + x);
+        }
     }
     const double scale_x = 1.0 / ((double)ow / rw), scale_y = 1.0 / ((double)oh / rh);
     int o0, o1, y0, y1, b0, b1;
@@ -135,8 +146,13 @@ __device__ __forceinline__ unsigned resize_pixel24_nv12(const uint8_t *yp, int p
     const int x0 = rx0 + o0 / 3, x1 = rx0 + o1 / 3, sy0 = ry0 + y0, sy1 = ry0 + y1;
     const uint8_t *r0 = yp + (size_t)sy0 * pitch, *c0 = uvp + (size_t)(sy0 >> 1) * pitch_uv;
     const uint8_t *r1 = yp + (size_t)sy1 * pitch, *c1 = uvp + (size_t)(sy1 >> 1) * pitch_uv;
-    const unsigned p10 = b1 != 0 ? nv12_px24(r1, c1, x0) : 0u, p11 = b1 != 0 ? nv12_px24(r1, c1, x1) : 0u;
-    return resize_px24(nv12_px24(r0, c0, x0), nv12_px24(r0, c0, x1), p10, p11, a0, a1, b0, b1);
+    const uint8_t *v0 = nullptr, *v1 = nullptr;
+    if constexpr (FMT == SRC_PLANAR) {
+        v0 = vp + (size_t)(sy0 >> 1) * pitch_uv;
+        v1 = vp + (size_t)(sy1 >> 1) * pitch_uv;
+    }
+    const unsigned p10 = b1 != 0 ? yuv_px24<FMT>(r1, c1, v1, x0) : 0u, p11 = b1 != 0 ? yuv_px24<FMT>(r1, c1, v1, x1) : 0u;
+    return resize_px24(yuv_px24<FMT>(r0, c0, v0, x0), yuv_px24<FMT>(r0, c0, v0, x1), p10, p11, a0, a1, b0, b1);
 }
 
 }  // namespace fd

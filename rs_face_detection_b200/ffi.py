@@ -72,6 +72,8 @@ class FdHostBatchOut(C.Structure):
 
 
 FD_UPLOAD_FULL, FD_UPLOAD_ON_DEMAND = 0, 1
+# layouts of a 4:2:0 frame for the *_yuv420 calls (include/fd_b200.h): what an fd_frame_nv12's `uv` points to
+FD_YUV420_NV12, FD_YUV420_NV21, FD_YUV420_I420, FD_YUV420_YV12 = 0, 1, 2, 3
 
 
 class FdPipelineOpts(C.Structure):
@@ -95,6 +97,8 @@ SYMBOLS = [
     "fd_align_detections", "fd_crops_to_tensor", "fd_model_preprocess", "fd_detect_batch_raw", "fd_select_params_default", "fd_face_selection",
     "fd_select_detections", "fd_align_selected", "fd_jpeg_info", "fd_decode_jpeg_batch", "fd_jpeg_last_stats", "fd_imdecode", "fd_pipeline_opts_default", "fd_pipeline_host", "fd_pipeline_host_jpeg", "fd_pipeline_tensor_dev",
     "fd_preprocess_batch_nv12", "fd_align_batch_nv12", "fd_align_detections_nv12", "fd_select_detections_nv12", "fd_align_selected_nv12",
+    "fd_preprocess_batch_yuv420", "fd_align_batch_yuv420", "fd_align_detections_yuv420", "fd_select_detections_yuv420",
+    "fd_align_selected_yuv420",
 ]
 
 _lib = None
@@ -605,6 +609,39 @@ class Context:
         arr = self._frames_nv12(frames)
         _chk(self.lib.fd_align_selected_nv12(self.handle, arr, len(frames), C.c_void_p(_devptr(crops_dev)), C.c_void_p(_devptr(M_dev)),
                                              C.c_void_p(_devptr(ok_dev))))
+
+    # ---- 4:2:0 frames in any FD_YUV420_* layout (descriptors from frame_table_nv12): the results of cv2.cvtColor(
+    # COLOR_YUV2BGR_NV12 / _NV21 / _I420 / _YV12) followed by the BGR call
+    def preprocess_batch_yuv420(self, frames, layout, out_dev):
+        arr = self._frames_nv12(frames)
+        ds = np.empty(len(frames), np.float32)
+        _chk(self.lib.fd_preprocess_batch_yuv420(self.handle, arr, int(layout), len(frames), C.c_void_p(_devptr(out_dev)),
+                                                 _ptr(ds, c_f32p)))
+        return ds
+
+    def align_batch_yuv420(self, frames, layout, landmarks_dev, frame_idx_dev, F, crops_dev, M_dev=None, ok_dev=None, bbox_dev=None):
+        arr = self._frames_nv12(frames)
+        _chk(self.lib.fd_align_batch_yuv420(self.handle, arr, int(layout), len(frames), C.c_void_p(_devptr(landmarks_dev)),
+                                            C.c_void_p(_devptr(frame_idx_dev)), C.c_void_p(_devptr(bbox_dev)), F,
+                                            C.c_void_p(_devptr(crops_dev)), C.c_void_p(_devptr(M_dev)), C.c_void_p(_devptr(ok_dev))))
+
+    def align_detections_yuv420(self, frames, layout, crops_dev, cap_faces, M_dev=None, ok_dev=None):
+        arr = self._frames_nv12(frames)
+        _chk(self.lib.fd_align_detections_yuv420(self.handle, arr, int(layout), len(frames), C.c_void_p(_devptr(crops_dev)), cap_faces,
+                                                 C.c_void_p(_devptr(M_dev)), C.c_void_p(_devptr(ok_dev))))
+
+    def select_detections_yuv420(self, frames, layout, is_enroll=False, params=None, fetch=True):
+        arr = self._frames_nv12(frames)
+        prm = None if params is None else (C.c_float * 4)(*params)
+        sel = np.empty((len(frames), 2), np.int32) if fetch else None
+        _chk(self.lib.fd_select_detections_yuv420(self.handle, arr, int(layout), len(frames), int(bool(is_enroll)), prm,
+                                                  None if sel is None else _ptr(sel, c_i32p)))
+        return sel
+
+    def align_selected_yuv420(self, frames, layout, crops_dev, M_dev=None, ok_dev=None):
+        arr = self._frames_nv12(frames)
+        _chk(self.lib.fd_align_selected_yuv420(self.handle, arr, int(layout), len(frames), C.c_void_p(_devptr(crops_dev)),
+                                               C.c_void_p(_devptr(M_dev)), C.c_void_p(_devptr(ok_dev))))
 
     # ---- N2: Triton raw_output_contents
     def detect_batch_raw(self, raw, shapes, det_scale, conf_thr, iou_thr):

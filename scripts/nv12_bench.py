@@ -1,15 +1,20 @@
 #!/usr/bin/env python
-"""NV12 batch step against the BGR batch step on bench.py's C2 / C5 inputs.
+"""4:2:0 batch steps (NV12, NV21, I420, YV12) against the BGR batch step on bench.py's C2 / C5 inputs.
 
-The frames of bench.py's workload are converted to NV12 the way a decoder hands them over (cv2 COLOR_BGR2YUV_I420, U and V
-interleaved), and the BGR step runs on what cv2.cvtColor(COLOR_YUV2BGR_NV12) gives back (the round trip is lossy, so the
-original BGR frames are never the comparison).  Parity first: tensor, det_scale, detections, crops and modes of
-    NV12 step: preprocess_batch_nv12 -> detect_batch -> align_detections_nv12
-    BGR step:  preprocess_batch      -> detect_batch -> align_detections
-must be byte-identical.  Then both steps are timed with CUDA events, alternating in one process, and profiled per kernel
-(fd_ctx_profile) in a separate pass.  One JSON file per workload goes to --out-dir.
+The frames of bench.py's workload are converted to 4:2:0 the way a decoder hands them over (cv2 COLOR_BGR2YUV_I420), and
+the BGR step runs on what cv2.cvtColor(COLOR_YUV2BGR_I420) gives back (the round trip is lossy, so the original BGR frames
+are never the comparison; every layout of the same chroma converts to the same BGR frame).  Each layout case keeps its
+planes in one layout: nv12 / nv21 (chroma pitch W), i420 / yv12 (tight chroma pitch W/2) and i420_padded / yv12_padded
+(chroma pitch W/2 rounded up to 64 bytes, plus 64).  Parity first: tensor, det_scale, detections, crops and modes of
+    layout step: preprocess_batch_nv12 / _yuv420 -> detect_batch -> align_detections_nv12 / _yuv420
+    BGR step:    preprocess_batch                -> detect_batch -> align_detections
+must be byte-identical.  Then the steps are timed with CUDA events, alternating in one process, and profiled per kernel
+(fd_ctx_profile) in a separate pass.  The NV12 case calls the *_nv12 entry points.  One JSON file per workload goes to
+--out-dir: r4_nv12_<workload>.json for the NV12 case alone (the default), r5_yuv420_<workload>.json otherwise.  'i420' is
+the tight chroma pitch only; name 'i420_padded' as well to measure the padded one.
 
     python scripts/nv12_bench.py --workloads c2,c5 --steps 100 --rounds 3 --out-dir profiles
+    python scripts/nv12_bench.py --layouts nv12,nv21,i420,i420_padded --workloads c2,c5 --out-dir profiles
 """
 import argparse
 import json
@@ -34,16 +39,23 @@ def y_rows(dy, scale_y, h):
     return min(max(sy, 0), h - 1), min(max(sy + 1, 0), h - 1), two
 
 
-def preprocess_bytes(h, w, new_h, nv12):
-    """bytes the preprocess kernel reads per frame (whole staged rows) plus the 640x640x3 f32 tensor it writes"""
+# case -> (FD_YUV420_* layout, chroma pitch from the width)
+LAYOUTS = {"nv12": (0, lambda W: W), "nv21": (1, lambda W: W), "i420": (2, lambda W: W // 2), "yv12": (3, lambda W: W // 2),
+           "i420_padded": (2, lambda W: -(-(W // 2) // 64) * 64 + 64), "yv12_padded": (3, lambda W: -(-(W // 2) // 64) * 64 + 64)}
+KERNEL_SUFFIX = {0: "_nv12", 1: "_nv21", 2: "_i420", 3: "_i420"}   # I420 and YV12 share the planar kernels
+
+
+def preprocess_bytes(h, w, new_h, kind):
+    """bytes the preprocess kernel reads per frame (whole staged rows: Y rows and one or two chroma rows, a planar chroma row
+    as a U and a V row of w/2 bytes) plus the 640x640x3 f32 tensor it writes"""
     scale_y = 1.0 / (new_h / h)
     total = 0
     for dy in range(new_h):
         y0, y1, two = y_rows(dy, scale_y, h)
-        if nv12:
-            total += w * (2 if two else 1) + w * (2 if two and (y1 >> 1) != (y0 >> 1) else 1)
-        else:
+        if kind == "bgr":
             total += 3 * w * (2 if two else 1)
+        else:
+            total += w * (2 if two else 1) + w * (2 if two and (y1 >> 1) != (y0 >> 1) else 1)
     return total + 3 * 640 * 640 * 4
 
 
@@ -65,62 +77,87 @@ def run(wl, args):
     ctx = Context(0)
     w = bench.Workload(ctx, wl, 0, 0)
     B, H, W = w.B, w.H, w.W
-    # NV12 planes and the BGR frames cvtColor makes of them
-    ys, uvs, bgrs = [], [], []
+    cases = args.layouts.split(",")
+    # one I420 conversion per frame; every layout case holds the same Y, U, V bytes
+    ys, us, vs, bgrs = [], [], [], []
     for t in w.frames_t:
-        bgr = t.cpu().numpy()
-        i420 = cv2.cvtColor(bgr, cv2.COLOR_BGR2YUV_I420)
-        uv = np.empty((H // 2, W), np.uint8)
+        i420 = cv2.cvtColor(t.cpu().numpy(), cv2.COLOR_BGR2YUV_I420)
         c, n = i420[H:].reshape(-1), (H // 2) * (W // 2)   # U then V planes
-        uv[:, 0::2] = c[:n].reshape(H // 2, W // 2)
-        uv[:, 1::2] = c[n:2 * n].reshape(H // 2, W // 2)
-        y = i420[:H]
-        back = cv2.cvtColor(np.concatenate([y, uv], 0), cv2.COLOR_YUV2BGR_NV12)
-        ys.append(torch.from_numpy(np.ascontiguousarray(y)).cuda())
-        uvs.append(torch.from_numpy(uv).cuda())
-        bgrs.append(torch.from_numpy(back).cuda())
+        ys.append(np.ascontiguousarray(i420[:H]))
+        us.append(c[:n].reshape(H // 2, W // 2))
+        vs.append(c[n:2 * n].reshape(H // 2, W // 2))
+        bgrs.append(torch.from_numpy(cv2.cvtColor(i420, cv2.COLOR_YUV2BGR_I420)).cuda())
     w.frames_t = bgrs
     w.frames_l = ctx.frame_table([(t.data_ptr(), H, W, W * 3) for t in bgrs])
-    nv_l = ctx.frame_table_nv12([(y.data_ptr(), uv.data_ptr(), H, W, W, W) for y, uv in zip(ys, uvs)])
-    tensor_nv = torch.empty_like(w.tensor_t)
-    crops_nv = torch.empty_like(w.crops_t)
-    mode_bgr = torch.empty(w.cap_faces, dtype=torch.uint8, device="cuda")
-    mode_nv = torch.empty_like(mode_bgr)
+    ys_t = [torch.from_numpy(y).cuda() for y in ys]
+    tables, keep = {}, []
+    for case in cases:
+        layout, pitch_of = LAYOUTS[case]
+        puv = pitch_of(W)
+        desc = []
+        for y_t, u, v in zip(ys_t, us, vs):
+            if layout in (0, 1):
+                c = np.zeros((H // 2, puv), np.uint8)
+                c[:, 0::2], c[:, 1::2] = (u, v) if layout == 0 else (v, u)
+            else:
+                c = np.zeros((H, puv), np.uint8)
+                c[:H // 2, :W // 2], c[H // 2:, :W // 2] = (u, v) if layout == 2 else (v, u)
+            c_t = torch.from_numpy(c).cuda()
+            keep.append(c_t)
+            desc.append((y_t.data_ptr(), c_t.data_ptr(), H, W, W, puv))
+        tables[case] = (layout, ctx.frame_table_nv12(desc), puv)
+    tensors = {k: torch.empty_like(w.tensor_t) for k in ["bgr"] + cases}
+    crops = {k: torch.empty_like(w.crops_t) for k in ["bgr"] + cases}
+    modes = {k: torch.empty(w.cap_faces, dtype=torch.uint8, device="cuda") for k in ["bgr"] + cases}
+    tensors["bgr"], crops["bgr"] = w.tensor_t, w.crops_t
 
     def step_bgr():
         ds = ctx.preprocess_batch(w.frames_l, w.tensor_t)
         ctx.detect_batch(w.heads_c, B, ds, bench.CONF_THR, bench.IOU_THR)
-        ctx.align_detections(w.frames_l, w.crops_t, w.cap_faces, None, mode_bgr)
+        ctx.align_detections(w.frames_l, w.crops_t, w.cap_faces, None, modes["bgr"])
         return ds
 
-    def step_nv():
-        ds = ctx.preprocess_batch_nv12(nv_l, tensor_nv)
-        ctx.detect_batch(w.heads_c, B, ds, bench.CONF_THR, bench.IOU_THR)
-        ctx.align_detections_nv12(nv_l, crops_nv, w.cap_faces, None, mode_nv)
-        return ds
+    def make_step(case):
+        layout, tab, _ = tables[case]
+        if case == "nv12":   # the *_nv12 entry points
+            def step():
+                ds = ctx.preprocess_batch_nv12(tab, tensors[case])
+                ctx.detect_batch(w.heads_c, B, ds, bench.CONF_THR, bench.IOU_THR)
+                ctx.align_detections_nv12(tab, crops[case], w.cap_faces, None, modes[case])
+                return ds
+        else:
+            def step():
+                ds = ctx.preprocess_batch_yuv420(tab, layout, tensors[case])
+                ctx.detect_batch(w.heads_c, B, ds, bench.CONF_THR, bench.IOU_THR)
+                ctx.align_detections_yuv420(tab, layout, crops[case], w.cap_faces, None, modes[case])
+                return ds
+        return step
+
+    steps = [("bgr", step_bgr)] + [(case, make_step(case)) for case in cases]
 
     # ---- parity
-    res = []
-    for fn, tensor, crops, mode in ((step_bgr, w.tensor_t, w.crops_t, mode_bgr), (step_nv, tensor_nv, crops_nv, mode_nv)):
+    res = {}
+    for kind, fn in steps:
         ds = fn()
         counts, det, lmk = ctx.detect_fetch(B)
         ctx.synchronize()
         n = int(counts.sum())
-        res.append(dict(ds=ds, counts=counts, det=det, lmk=lmk, tensor=tensor.cpu().numpy(), crops=crops[:n].cpu().numpy(),
-                        modes=mode[:n].cpu().numpy()))
-    for k in res[0]:
-        if not np.array_equal(res[0][k], res[1][k]):
-            raise SystemExit("%s: NV12 step differs from the BGR step on the converted frames in %s" % (wl, k))
-    faces = int(res[0]["counts"].sum())
+        res[kind] = dict(ds=ds, counts=counts, det=det, lmk=lmk, tensor=tensors[kind].cpu().numpy(), crops=crops[kind][:n].cpu().numpy(),
+                         modes=modes[kind][:n].cpu().numpy())
+    for case in cases:
+        for k in res["bgr"]:
+            if not np.array_equal(res["bgr"][k], res[case][k]):
+                raise SystemExit("%s: %s step differs from the BGR step on the converted frames in %s" % (wl, case, k))
+    faces = int(res["bgr"]["counts"].sum())
 
     # ---- timing: alternating rounds of `steps` steps, CUDA events
     for _ in range(args.warmup):
-        step_bgr()
-        step_nv()
+        for _, fn in steps:
+            fn()
     ctx.synchronize()
-    times = {"bgr": [], "nv12": []}
+    times = {k: [] for k, _ in steps}
     for _ in range(args.rounds):
-        for kind, fn in (("bgr", step_bgr), ("nv12", step_nv)):
+        for kind, fn in steps:
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             s = torch.cuda.ExternalStream(ctx.stream())
             e0.record(s)
@@ -133,7 +170,7 @@ def run(wl, args):
 
     # ---- per-kernel profile, a pass of its own
     prof = {}
-    for kind, fn in (("bgr", step_bgr), ("nv12", step_nv)):
+    for kind, fn in steps:
         ctx.profile(True)
         for _ in range(args.steps):
             fn()
@@ -143,18 +180,22 @@ def run(wl, args):
     ctx.detect_fetch(B)
     name, power = gpu_identity()
     new_h = int(ctx.letterbox_geometry(H, W)[1])
-    pre = {"bgr": preprocess_bytes(H, W, new_h, False) * B, "nv12": preprocess_bytes(H, W, new_h, True) * B}
+    pre = {k: preprocess_bytes(H, W, new_h, k) * B for k, _ in steps}
     conv_us = 4.5 * H * W * B / (HBM_TBS * 1e12) * 1e6    # read 1.5 B + write 3 B per pixel
     best = {k: min(v) for k, v in times.items()}
+    kname = {"bgr": ""}
+    kname.update({c: KERNEL_SUFFIX[tables[c][0]] for c in cases})
     out = {
         "workload": wl, "gpu": name, "power_limit": power, "batch": B, "frame": "%dx%d" % (W, H), "faces": faces,
+        "chroma_pitch": {c: tables[c][2] for c in cases},
         "ms_per_step": times, "frames_per_s": {k: B / (v * 1e-3) for k, v in best.items()},
         "preprocess_bytes_per_step": pre,
-        "preprocess_us": {k: prof[k].get(n, {}).get("us_per_launch") for k, n in (("bgr", "preprocess_tma_kernel"), ("nv12", "preprocess_tma_kernel_nv12"))},
+        "preprocess_us": {k: prof[k].get("preprocess_tma_kernel" + kname[k], {}).get("us_per_launch") for k, _ in steps},
+        "warp_us": {k: prof[k].get("warp_fixed_kernel" + kname[k], {}).get("us_per_launch") for k, _ in steps},
         "profile": prof,
         "least_conversion_pass_us": conv_us,
-        "nv12_beats_bgr_plus_conversion": best["nv12"] * 1e3 < best["bgr"] * 1e3 + conv_us,
-        "parity": "tensor, det_scale, detections, crops and modes byte-identical to the BGR step on the cvtColor frames",
+        "beats_bgr_plus_conversion": {c: best[c] * 1e3 < best["bgr"] * 1e3 + conv_us for c in cases},
+        "parity": "tensor, det_scale, detections, crops and modes of every layout byte-identical to the BGR step on the cvtColor frames",
         "steps": args.steps, "rounds": args.rounds, "warmup": args.warmup,
     }
     ctx.close()
@@ -167,14 +208,18 @@ def main():
     ap.add_argument("--steps", type=int, default=100)
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--rounds", type=int, default=3)
-    ap.add_argument("--out-dir", default=None, help="write r4_nv12_<workload>.json here")
+    ap.add_argument("--layouts", default="nv12", help="comma-separated cases: " + ", ".join(LAYOUTS))
+    ap.add_argument("--out-dir", default=None, help="write --out-name (%%s: the workload) here")
+    ap.add_argument("--out-name", default=None, help="default: r4_nv12_%%s.json for --layouts nv12, else r5_yuv420_%%s.json")
     args = ap.parse_args()
+    if args.out_name is None:
+        args.out_name = "r4_nv12_%s.json" if args.layouts == "nv12" else "r5_yuv420_%s.json"
     for wl in args.workloads.split(","):
         out = run(wl, args)
         print(json.dumps(out))
         if args.out_dir:
             os.makedirs(args.out_dir, exist_ok=True)
-            with open(os.path.join(args.out_dir, "r4_nv12_%s.json" % wl), "w") as f:
+            with open(os.path.join(args.out_dir, args.out_name % wl), "w") as f:
                 json.dump(out, f, indent=1)
 
 
