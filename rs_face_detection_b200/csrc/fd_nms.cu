@@ -19,8 +19,9 @@
 //               rank sort, brute-force predecessor lists, the decision sweeps below (72 us at 4 096 boxes, was 178).
 //   beyond    : nms_big_kernel, ONE cooperative launch: spatially binned exact NMS without a global sort (boxes binned by cell,
 //               ordered inside cells only, predecessor lists + decision sweeps over cell-order positions, kept keys ordered at
-//               the end), or — same launch — a radix sort + the cooperative multi-CTA peel for degenerate inputs.  The round-1
-//               sequence of one kernel per step stays behind FD_NMS_MULTI_KERNEL=1 (A/B reference).
+//               the end), or — same launch — a radix sort + the cooperative multi-CTA peel for degenerate inputs.  A batch image
+//               beyond SMALL_CAP runs the same kernel on the decode kernel's keys (nms_batch_big_image).
+//   argsort_descending beyond SMALL_CAP: argsort_kernel, the same launch's radix sort alone.
 #include <cooperative_groups.h>
 #include <algorithm>
 #include <cmath>
@@ -136,185 +137,11 @@ __global__ void __launch_bounds__(NT, 1) nms_cta_kernel(SmallArgs a) {
 }
 
 // ============================================================================================================
-// Big path: radix sort of u64 keys (own kernels) + cooperative peel
+// Big path: cooperative peel (the fallback of nms_big_kernel)
 // ============================================================================================================
-constexpr int RS_THREADS = 256;
-constexpr int RS_ITEMS = 16;
-constexpr int RS_TILE = RS_THREADS * RS_ITEMS;
-
-__global__ void make_keys_kernel(const float *__restrict__ dets, int n, int stride, u64 *__restrict__ keys, int *status) {
-    int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    float s = __ldg(dets + (size_t)i * stride + 4);
-    if (s != s) atomicExch(&status[0], 1);
-    keys[i] = ((u64)desc_key(s) << 32) | (unsigned)i;
-}
 __global__ void iota_keys_kernel(int n, u64 *__restrict__ keys) {
     int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n) keys[i] = (u64)(unsigned)i;
-}
-
-__global__ void __launch_bounds__(RS_THREADS) radix_hist_kernel(const u64 *__restrict__ keys, int n, int shift,
-                                                                int *__restrict__ hist, int ntiles) {
-    __shared__ int h[256];
-    h[threadIdx.x] = 0;
-    __syncthreads();
-    int base = blockIdx.x * RS_TILE;
-    for (int k = 0; k < RS_ITEMS; ++k) {
-        int e = base + k * RS_THREADS + threadIdx.x;
-        if (e < n) atomicAdd(&h[(int)((keys[e] >> shift) & 0xffull)], 1);
-    }
-    __syncthreads();
-    hist[threadIdx.x * ntiles + blockIdx.x] = h[threadIdx.x];
-}
-
-// exclusive scan over m ints by one CTA
-__global__ void __launch_bounds__(1024) scan_kernel(int *__restrict__ data, int m) {
-    __shared__ int warp_sums[33];
-    __shared__ int carry_s;
-    if (threadIdx.x == 0) carry_s = 0;
-    __syncthreads();
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    for (int base = 0; base < m; base += 1024) {
-        int i = base + threadIdx.x;
-        int v = i < m ? data[i] : 0;
-        int incl = v;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            int nb = __shfl_up_sync(0xffffffffu, incl, o);
-            if (lane >= o) incl += nb;
-        }
-        if (lane == 31) warp_sums[warp] = incl;
-        __syncthreads();
-        if (warp == 0) {
-            int w = warp_sums[lane];
-            int wi = w;
-#pragma unroll
-            for (int o = 1; o < 32; o <<= 1) {
-                int nb = __shfl_up_sync(0xffffffffu, wi, o);
-                if (lane >= o) wi += nb;
-            }
-            warp_sums[lane] = wi - w;
-            if (lane == 31) warp_sums[32] = wi;
-        }
-        __syncthreads();
-        int carry = carry_s;
-        if (i < m) data[i] = carry + warp_sums[warp] + incl - v;
-        __syncthreads();
-        if (threadIdx.x == 0) carry_s = carry + warp_sums[32];
-        __syncthreads();
-    }
-}
-
-// One kernel per radix pass.  hist_cur[d*ntiles + t] = number of keys with digit d in tile t (for this pass's digit and
-// the CURRENT key order).  Every CTA derives its own scatter bases from it (no separate scan launch): for digit d,
-// base = sum over smaller digits of their totals + sum over earlier tiles of digit d.  While scattering, the kernel
-// accumulates the NEXT pass's per-tile histogram (the destination tile of every key is known here), so only the first
-// pass needs a histogram launch.  Stable: element order inside a tile is (warp, round, lane).
-__global__ void __launch_bounds__(RS_THREADS) radix_pass_kernel(const u64 *__restrict__ keys_in, u64 *__restrict__ keys_out, int n,
-                                                                int shift, const int *__restrict__ hist_cur, int *__restrict__ hist_next,
-                                                                int next_shift, int ntiles) {
-    __shared__ int wcount[RS_THREADS / 32][256];
-    __shared__ int gofs[256];
-    __shared__ int wsum[RS_THREADS / 32];
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    for (int i = threadIdx.x; i < (RS_THREADS / 32) * 256; i += RS_THREADS) (&wcount[0][0])[i] = 0;
-    {   // scatter base of digit d = threadIdx.x for this tile
-        const int d = threadIdx.x;
-        const int *row = hist_cur + (size_t)d * ntiles;
-        int before = 0, total = 0;
-        for (int t = 0; t < ntiles; ++t) {
-            const int v = __ldcg(row + t);
-            total += v;
-            if (t < (int)blockIdx.x) before += v;
-        }
-        int incl = total;  // exclusive scan of the digit totals over the 256 threads
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            int nb = __shfl_up_sync(0xffffffffu, incl, o);
-            if (lane >= o) incl += nb;
-        }
-        if (lane == 31) wsum[warp] = incl;
-        __syncthreads();
-        int wbase = 0;
-        for (int w = 0; w < warp; ++w) wbase += wsum[w];
-        gofs[d] = wbase + incl - total + before;
-    }
-    __syncthreads();
-    const int wbase = blockIdx.x * RS_TILE + warp * (32 * RS_ITEMS);
-    u64 key[RS_ITEMS];
-    int rank[RS_ITEMS];
-#pragma unroll
-    for (int r = 0; r < RS_ITEMS; ++r) {
-        int e = wbase + r * 32 + lane;
-        bool valid = e < n;
-        key[r] = valid ? keys_in[e] : 0ull;
-        int d = valid ? (int)((key[r] >> shift) & 0xffull) : 256;
-        unsigned peers = __match_any_sync(0xffffffffu, d);
-        int prior = valid ? wcount[warp][d] : 0;
-        rank[r] = prior + __popc(peers & ((1u << lane) - 1u));
-        __syncwarp();
-        if (valid && lane == (__ffs(peers) - 1)) wcount[warp][d] = prior + __popc(peers);
-        __syncwarp();
-    }
-    __syncthreads();
-    {
-        int d = threadIdx.x, run = 0;
-#pragma unroll
-        for (int w = 0; w < RS_THREADS / 32; ++w) {
-            int c = wcount[w][d];
-            wcount[w][d] = run;
-            run += c;
-        }
-    }
-    __syncthreads();
-#pragma unroll
-    for (int r = 0; r < RS_ITEMS; ++r) {
-        int e = wbase + r * 32 + lane;
-        if (e < n) {
-            int d = (int)((key[r] >> shift) & 0xffull);
-            const int pos = gofs[d] + wcount[warp][d] + rank[r];
-            keys_out[pos] = key[r];
-        }
-        if (hist_next) {  // warp-aggregated: skewed digits (e.g. the exponent byte of scores in [0,1)) would serialise
-            int slot = -1;
-            if (e < n) {
-                int d = (int)((key[r] >> shift) & 0xffull);
-                const int pos = gofs[d] + wcount[warp][d] + rank[r];
-                slot = (int)((key[r] >> next_shift) & 0xffull) * ntiles + pos / RS_TILE;
-            }
-            const unsigned peers = __match_any_sync(0xffffffffu, slot);
-            if (slot >= 0 && lane == (__ffs(peers) - 1)) atomicAdd(&hist_next[slot], __popc(peers));
-        }
-    }
-}
-
-__global__ void gather_sorted_boxes_kernel(const u64 *__restrict__ keys, int n, const float *__restrict__ boxes, int stride,
-                                           float4 *__restrict__ sbox, int *status) {
-    int r = blockIdx.x * blockDim.x + threadIdx.x;
-    bool ok = true;
-    if (r < n) {
-        int idx = (int)(unsigned)keys[r];
-        const float *p = boxes + (size_t)idx * stride;
-        float4 bx = make_float4(__ldg(p), __ldg(p + 1), __ldg(p + 2), __ldg(p + 3));
-        sbox[r] = bx;
-        ok = box_is_fast_ok(bx);
-    }
-    if (!__all_sync(0xffffffffu, ok)) {
-        if ((threadIdx.x & 31) == 0) atomicExch(&status[2], 1);  // not "fast"
-    }
-}
-
-__global__ void map_keep_kernel(const int *__restrict__ keep_ranks, const int *__restrict__ state, const u64 *__restrict__ keys,
-                                int *__restrict__ keep, int *__restrict__ num_keep) {
-    int n = state[1];
-    int k = blockIdx.x * blockDim.x + threadIdx.x;
-    if (k == 0) *num_keep = n;
-    if (k < n) keep[k] = (int)(unsigned)keys[keep_ranks[k]];
-}
-__global__ void low32_kernel(const u64 *__restrict__ keys, int n, int *__restrict__ out) {
-    int k = blockIdx.x * blockDim.x + threadIdx.x;
-    if (k < n) out[k] = (int)(unsigned)keys[k];
 }
 
 struct PeelSmem {
@@ -352,7 +179,7 @@ __device__ __forceinline__ int block_sum(int v, int *red) {
     return t;
 }
 
-// The peel itself: every CTA of a cooperative grid calls it (nms_peel_kernel, and nms_big_kernel when the spatial path does not apply).
+// The peel itself: every CTA of nms_big_kernel's cooperative grid calls it when the spatial path does not apply.
 template <int MODE>
 __device__ __forceinline__ void nms_peel_body(const PeelArgs &a, unsigned char *smem_raw) {
     PeelSmem &sm = *reinterpret_cast<PeelSmem *>(smem_raw);
@@ -465,27 +292,21 @@ __device__ __forceinline__ void nms_peel_body(const PeelArgs &a, unsigned char *
     if (blockIdx.x == 0 && tid == 0) a.state[1] = nk_total;
 }
 
-template <int MODE>
-__global__ void __launch_bounds__(NT, 1) nms_peel_kernel(PeelArgs a) {
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    if (__ldcg(&a.status[3]) != 0) return;  // uniform over the grid: the spatial path owns this problem
-    nms_peel_body<MODE>(a, smem_raw);
-}
-
 // ============================================================================================================
 // Spatial big path: exact greedy NMS with work proportional to the number of OVERLAPPING pairs.
 //
 // IoU(A,B) > t implies the intersection is at least t x the larger box in each axis, hence the box centres are at
-// most (1-t) x max(w) apart per axis.  Boxes are binned by centre into a uniform grid with that cell size (stable
-// radix sort on the cell id: cells come out with their members in rank order), every box collects the EARLIER-ranked
-// boxes of its 3x3 neighbourhood that suppress it (exact predicate) into a short predecessor list, and the keep set is
-// the unique fixed point of   kept(i) = no predecessor kept,   resolved by monotone parallel sweeps inside one
-// cooperative kernel (a box is suppressed as soon as one predecessor is kept, kept as soon as all are suppressed).
-// Same result as the sequential sweep of nms.rs; used when every box is regular (finite, positive area), the
-// threshold is an ordinary one and the grid is fine enough — otherwise the peel kernel above does the job.
+// most (1-t) x max(w) apart per axis.  Boxes are binned by centre into a uniform grid with that cell size (members of
+// a cell ordered by key), every box collects the EARLIER-ranked boxes of its 3x3 neighbourhood that suppress it (exact
+// predicate) into a short predecessor list, and the keep set is the unique fixed point of   kept(i) = no predecessor
+// kept,   resolved by monotone parallel sweeps inside one cooperative kernel (a box is suppressed as soon as one
+// predecessor is kept, kept as soon as all are suppressed).  Same result as the sequential sweep of nms.rs; used when
+// every box is regular (finite, positive area), the threshold is an ordinary one and the grid is fine enough —
+// otherwise the peel above does the job.
 // ============================================================================================================
-constexpr int ADJ_CAP = 96;      // listed predecessors per box (global memory)
-constexpr int ADJ_SMEM = 32;     // of which the first are cached in shared memory across sweeps
+constexpr int ADJ_CAP = 96;      // mid path: listed predecessors per box (global memory)
+constexpr int ADJ_SMEM = 32;     // list entries per box cached in shared memory across sweeps (the big path's lazy lists keep up to 24)
+static_assert(ADJ_SMEM >= 24 && ADJ_SMEM % 4 == 0, "the lazy segment loads and the 128-bit list loads rely on this");
 constexpr int ADJ_SEG = 64;      // one-launch path: a box's list is three segments of this capacity, one per neighbourhood row (three tasks):
 constexpr int ADJ_ROW3 = 3 * ADJ_SEG;   // the first suppressing predecessors of every row.  When all listed ones end up suppressed and there were
                                         // more, the list is refilled (exact; ~40 us each, so the capacity is chosen to make refills rare: at
@@ -512,46 +333,6 @@ __device__ __forceinline__ float box_cy(float4 b) { return __fmul_rn(__fadd_rn(b
 __device__ __forceinline__ int cell_coord(float c, float minc, float cs, int g) {
     int v = (int)floorf(__fdiv_rn(__fsub_rn(c, minc), cs));
     return min(g - 1, max(0, v));
-}
-
-// gs: [0] min cx, [1] min cy (init 0xFFFFFFFF), [2] max cx, [3] max cy, [4] max dim (init 0); ordered-uint encoding
-__global__ void grid_stats_kernel(const float4 *__restrict__ sbox, int N, unsigned *gs) {
-    int r = blockIdx.x * blockDim.x + threadIdx.x;
-    unsigned mincx = 0xFFFFFFFFu, mincy = 0xFFFFFFFFu, maxcx = 0, maxcy = 0, maxd = 0;
-    if (r < N) {
-        float4 b = sbox[r];
-        unsigned cx = f2ord(box_cx(b)), cy = f2ord(box_cy(b));
-        mincx = maxcx = cx;
-        mincy = maxcy = cy;
-        float w = __fadd_rn(__fsub_rn(b.z, b.x), 1.0f), h = __fadd_rn(__fsub_rn(b.w, b.y), 1.0f);
-        maxd = f2ord(fmaxf(fabsf(w), fabsf(h)));
-    }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-        mincx = min(mincx, __shfl_xor_sync(0xffffffffu, mincx, o));
-        mincy = min(mincy, __shfl_xor_sync(0xffffffffu, mincy, o));
-        maxcx = max(maxcx, __shfl_xor_sync(0xffffffffu, maxcx, o));
-        maxcy = max(maxcy, __shfl_xor_sync(0xffffffffu, maxcy, o));
-        maxd = max(maxd, __shfl_xor_sync(0xffffffffu, maxd, o));
-    }
-    __shared__ unsigned red[5][8];
-    const int w = threadIdx.x >> 5;
-    if ((threadIdx.x & 31) == 0) {
-        red[0][w] = mincx; red[1][w] = mincy; red[2][w] = maxcx; red[3][w] = maxcy; red[4][w] = maxd;
-    }
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        const int nw = blockDim.x >> 5;
-        for (int k = 1; k < nw; ++k) {
-            mincx = min(mincx, red[0][k]); mincy = min(mincy, red[1][k]);
-            maxcx = max(maxcx, red[2][k]); maxcy = max(maxcy, red[3][k]); maxd = max(maxd, red[4][k]);
-        }
-        atomicMin(&gs[0], mincx);
-        atomicMin(&gs[1], mincy);
-        atomicMax(&gs[2], maxcx);
-        atomicMax(&gs[3], maxcy);
-        atomicMax(&gs[4], maxd);
-    }
 }
 
 __device__ __forceinline__ GridCfg grid_setup(unsigned g0, unsigned g1, unsigned g2, unsigned g3, unsigned g4, int N, const IouParams &P, int not_fast) {
@@ -582,101 +363,6 @@ __device__ __forceinline__ GridCfg grid_setup(unsigned g0, unsigned g1, unsigned
     }
     return c;
 }
-__global__ void grid_setup_kernel(const unsigned *gs, int N, IouParams P, GridCfg *cfg, int *st) {
-    const GridCfg c = grid_setup(gs[0], gs[1], gs[2], gs[3], gs[4], N, P, st[2]);
-    *cfg = c;
-    st[3] = c.use;
-}
-
-__global__ void cell_keys_kernel(const float4 *__restrict__ sbox, int N, const GridCfg *cfg, u64 *__restrict__ keys) {
-    int r = blockIdx.x * blockDim.x + threadIdx.x;
-    if (r >= N) return;
-    const GridCfg c = *cfg;
-    if (!c.use) { keys[r] = (u64)(unsigned)r; return; }
-    float4 b = sbox[r];
-    int ix = cell_coord(box_cx(b), c.minx, c.cs, c.gx), iy = cell_coord(box_cy(b), c.miny, c.cs, c.gy);
-    keys[r] = ((u64)(unsigned)(iy * c.gx + ix) << 32) | (unsigned)r;
-}
-
-// keys sorted by (cell, rank).  cell_start/cell_end zeroed beforehand.
-__global__ void cell_bounds_kernel(const u64 *__restrict__ keys, int N, const GridCfg *cfg, const float4 *__restrict__ sbox,
-                                   int *__restrict__ cell_start, int *__restrict__ cell_end, float4 *__restrict__ cbox,
-                                   float *__restrict__ carea, int *__restrict__ pos_of_rank) {
-    int k = blockIdx.x * blockDim.x + threadIdx.x;
-    if (k >= N || !cfg->use) return;
-    const u64 key = keys[k];
-    const int cell = (int)(key >> 32), rank = (int)(unsigned)key;
-    if (k == 0 || (int)(keys[k - 1] >> 32) != cell) cell_start[cell] = k;
-    if (k == N - 1 || (int)(keys[k + 1] >> 32) != cell) cell_end[cell] = k + 1;
-    const float4 b = sbox[rank];
-    cbox[k] = b;
-    carea[k] = box_area(b);
-    pos_of_rank[rank] = k;
-}
-
-// visits the earlier-ranked members of the 3x3 neighbourhood of cell-ordered box k that suppress it
-template <class F>
-__device__ __forceinline__ void for_each_predecessor(int k, const u64 *__restrict__ keys, const GridCfg &c,
-                                                     const int *__restrict__ cell_start, const int *__restrict__ cell_end,
-                                                     const float4 *__restrict__ cbox, const float *__restrict__ carea,
-                                                     const IouParams &P, F &&visit, int dy0 = -1, int dy1 = 1) {
-    const u64 key = keys[k];
-    const int cell = (int)(key >> 32), rank = (int)(unsigned)key;
-    const int iy = cell / c.gx, ix = cell - iy * c.gx;
-    const float4 bi = cbox[k];
-    const float ai = carea[k];
-    for (int dy = dy0; dy <= dy1; ++dy) {
-        const int y = iy + dy;
-        if (y < 0 || y >= c.gy) continue;
-        for (int dx = -1; dx <= 1; ++dx) {
-            const int x = ix + dx;
-            if (x < 0 || x >= c.gx) continue;
-            const int c2 = y * c.gx + x;
-            const int e = cell_end[c2];
-            int j = cell_start[c2];
-            // members are in rank order: 4 candidates per step so their loads are in flight together
-            for (; j + 3 < e; j += 4) {
-                int rj[4];
-                float4 bj[4];
-                float aj[4];
-#pragma unroll
-                for (int u = 0; u < 4; ++u) {
-                    rj[u] = (int)(unsigned)keys[j + u];
-                    bj[u] = cbox[j + u];
-                    aj[u] = carea[j + u];
-                }
-                if (rj[0] >= rank) break;
-#pragma unroll
-                for (int u = 0; u < 4; ++u)
-                    if (rj[u] < rank && iou_suppresses_exact(bj[u], aj[u], bi, ai, P))
-                        if (!visit(rj[u])) return;
-                if (rj[3] >= rank) { j = e; break; }
-            }
-            for (; j < e; ++j) {
-                const int rj = (int)(unsigned)keys[j];
-                if (rj >= rank) break;
-                if (iou_suppresses_exact(cbox[j], carea[j], bi, ai, P))
-                    if (!visit(rj)) return;
-            }
-        }
-    }
-}
-
-// predecessor list of cell-ordered box k
-__device__ __forceinline__ void adjacency_of(int k, const u64 *__restrict__ keys, const GridCfg &c, const int *__restrict__ cell_start,
-                                             const int *__restrict__ cell_end, const float4 *__restrict__ cbox, const float *__restrict__ carea,
-                                             const IouParams &P, int *__restrict__ adj, int *__restrict__ adj_cnt) {
-    const int rank = (int)(unsigned)keys[k];
-    int cnt = 0;
-    int *mine = adj + (size_t)rank * ADJ_CAP;
-    for_each_predecessor(k, keys, c, cell_start, cell_end, cbox, carea, P, [&](int rj) {
-        if (cnt < ADJ_CAP) mine[cnt] = rj;
-        ++cnt;
-        return true;
-    });
-    adj_cnt[rank] = cnt;   // may exceed ADJ_CAP: the first ADJ_CAP are listed
-}
-
 // ---- the one-launch path never sorts the boxes globally: boxes are addressed by their position k in
 // cell order, members of a cell are ordered by their FULL key (score desc | source index — the order a stable descending sort
 // gives), "earlier-ranked" is a key comparison, and the cell of a box is recomputed from its centre.  visit(j) gets a position.
@@ -737,17 +423,6 @@ __device__ __forceinline__ void adjacency_row_k(int k, int dy, const u64 *__rest
     cnt3[k * 3 + dy + 1] = cnt;   // ADJ_SEG + 1: more than the segment lists
 }
 
-__global__ void __launch_bounds__(256) adjacency_kernel(const u64 *__restrict__ keys, int N, const GridCfg *cfg,
-                                                        const int *__restrict__ cell_start, const int *__restrict__ cell_end,
-                                                        const float4 *__restrict__ cbox, const float *__restrict__ carea, IouParams P,
-                                                        int *__restrict__ adj, int *__restrict__ adj_cnt) {
-    int k = blockIdx.x * blockDim.x + threadIdx.x;
-    if (k >= N) return;
-    const GridCfg c = *cfg;
-    if (!c.use) return;
-    adjacency_of(k, keys, c, cell_start, cell_end, cbox, carea, P, adj, adj_cnt);
-}
-
 // L2 (cache-global) byte load the compiler may neither cache nor drop: other CTAs update the states concurrently
 __device__ __forceinline__ unsigned ld_state(const unsigned char *p) {
     unsigned v;
@@ -755,35 +430,29 @@ __device__ __forceinline__ unsigned ld_state(const unsigned char *p) {
     return v;
 }
 
+// Two modes (nms_rounds_body<BRUTE>): the big path's (boxes are cell-order positions, three-segment lists, kept keys appended
+// unordered) and the mid path's brute one (boxes are ranks, one list per box from the all-pairs pass, kept source indices
+// written in rank order).
 struct RoundsArgs {
     int N;
-    const u64 *keys;
-    const GridCfg *cfg;
-    const int *cell_start, *cell_end;
+    const u64 *keys;        // keys (score desc | source index) by box: cell order (big path) / rank order (mid path)
+    const int *cell_start, *cell_end;   // big path: the grid's cells, cell-ordered boxes and their areas
     const float4 *cbox;
     const float *carea;
-    const int *pos_of_rank;
     const int *adj, *adj_cnt;
-    unsigned char *state;   // by rank: 0 undecided, 1 kept, 2 suppressed (zeroed)
+    unsigned char *state;   // by box: 0 undecided, 1 kept, 2 suppressed (zeroed)
     int *counters;          // [3] rotating undecided counters (zeroed)
     int *tile_counts;
     unsigned *ballots;
-    int *keep_ranks;
-    int *out_state;         // [0] = this path owns the problem, [1] = total kept
+    int *out_state;         // [1] total kept, [3] grid-wide epochs, [4] list refills (statistics)
     IouParams iou;
     const float4 *sbox;     // brute mode (mid path: no grid): boxes in rank order; a box that exhausts an overflowed list refills it from every earlier box
-    int brute;
     int mode;               // brute mode: 0 nms.rs / 1 cpu_nms.rs comparison for the full IEEE test
     const int *status;      // brute mode: [0] NaN score seen, [2] != 0 -> some box is not "fast ok": full IEEE test
-    int *final_keep;        // brute mode: kept SOURCE indices in rank order (keys[rank] low word) and {count, NaN flag}, written here
-    const u64 *final_keys;  //             instead of keep_ranks + map_keep_kernel
+    int *final_keep;        // brute mode: kept SOURCE indices in rank order (keys[rank] low word) and {count, NaN flag}
     int *final_num;
     long long *dbg;         // FD_NMS_DBG: globaltimer stamps of block 0 (slots 5..7)
-    int adj_smem;           // list entries per box cached in shared memory across sweeps (<= ADJ_SMEM; sadj holds adj_smem x NT ints)
-    int seg3;               // lists are three ADJ_SEG segments with adj_cnt[3 * box + segment] entries each (adjacency_row)
-    int adj_stride;         // ints per box in adj (ADJ_CAP, or ADJ_ROW3 with seg3)
-    int kspace;             // boxes are cell-order positions, keys = full (score | index) keys: for_each_predecessor_k
-    u64 *kept_keys;         // kspace: the kept boxes' keys (in position order) go here instead of final_keep; [1] of out_state = count
+    u64 *kept_keys;         // big path: the kept boxes' keys (unordered) go here; [1] of out_state = count
 };
 
 __device__ __forceinline__ void mid_stamp(long long *dbg, int slot) {
@@ -805,7 +474,7 @@ __device__ __forceinline__ void max_stamp(long long *dbg, int slot) {
 
 constexpr int ROUND_SWEEPS = 24;   // sweeps of a warp between two grid-wide checks
 
-// brute-mode stand-in for for_each_predecessor: every earlier box that suppresses box r
+// brute-mode stand-in for for_each_predecessor_k: every earlier box that suppresses box r
 template <class F>
 __device__ __forceinline__ void for_each_earlier(int r, const float4 *__restrict__ sbox, const IouParams &P, bool fast, int mode, F &&visit) {
     const float4 bi = __ldcg(sbox + r);
@@ -846,9 +515,11 @@ __device__ __forceinline__ int decide_pending(int &pend, GetFn get, PutFn put, c
     return w == 0 ? 1 : 0;
 }
 
-// sadj: [adj_smem][NT] ints of shared memory (head of the pending-predecessor list of each thread's first box, kept across sweeps)
+// sadj: [ADJ_SMEM][NT] ints of shared memory (head of the pending-predecessor list of each thread's first box, kept across sweeps).
+// BRUTE: the mid path's mode (see RoundsArgs).
+template <bool BRUTE>
 __device__ __forceinline__ void nms_rounds_body(const RoundsArgs &a, const GridCfg &c, int *sadj, int *red) {
-    const bool bfast = a.brute && a.iou.fast && __ldcg(&a.status[2]) == 0;
+    const bool bfast = BRUTE && a.iou.fast && __ldcg(&a.status[2]) == 0;
     cg::grid_group grid = cg::this_grid();
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int G = gridDim.x;
@@ -858,12 +529,13 @@ __device__ __forceinline__ void nms_rounds_body(const RoundsArgs &a, const GridC
     //      there are more) — the resident box of this thread keeps the head of its run in shared memory and the count in a
     //      register, the others (N beyond the resident threads) keep both in global memory: adj_cnt[first counter] = count |
     //      overflow << 30.
-    const int cstep = a.seg3 ? 3 : 1;
+    const int cstep = BRUTE ? 1 : 3;
+    const int adj_stride = BRUTE ? ADJ_CAP : ADJ_ROW3;   // ints per box in adj
     int *const acnt = const_cast<int *>(a.adj_cnt);
-    int *const mine0 = const_cast<int *>(a.adj) + (size_t)min(gtid, max(a.N - 1, 0)) * a.adj_stride;   // this thread's resident box
-    auto get0 = [&](int e) { return e < a.adj_smem ? sadj[e * NT + tid] : __ldcg(mine0 + e); };
+    int *const mine0 = const_cast<int *>(a.adj) + (size_t)min(gtid, max(a.N - 1, 0)) * adj_stride;   // this thread's resident box
+    auto get0 = [&](int e) { return e < ADJ_SMEM ? sadj[e * NT + tid] : __ldcg(mine0 + e); };
     auto put0 = [&](int e, int v) {
-        if (e < a.adj_smem) sadj[e * NT + tid] = v;
+        if (e < ADJ_SMEM) sadj[e * NT + tid] = v;
         else mine0[e] = v;
     };
     int pend = 0;
@@ -900,7 +572,7 @@ __device__ __forceinline__ void nms_rounds_body(const RoundsArgs &a, const GridC
         }
         return any;
     };
-    const bool lazy = a.seg3 && a.adj_smem >= 24;
+    const bool lazy = !BRUTE;
     if (lazy && gtid < a.N) {
 #pragma unroll
         for (int sg = 0; sg < 3; ++sg) {
@@ -911,12 +583,12 @@ __device__ __forceinline__ void nms_rounds_body(const RoundsArgs &a, const GridC
         load_more();
     }
     for (int r = gtid + (lazy ? gstride : 0); r < a.N; r += gstride) {
-        int *row = const_cast<int *>(a.adj) + (size_t)r * a.adj_stride;
+        int *row = const_cast<int *>(a.adj) + (size_t)r * adj_stride;
         const int4 *row4 = reinterpret_cast<const int4 *>(row);
         const bool res = r == gtid;
         int total = 0;
         bool ov = false;
-        if (a.seg3) {   // gather the three row segments (typical segment: a few entries, so the three first loads overlap)
+        if (!BRUTE) {   // gather the three row segments (typical segment: a few entries, so the three first loads overlap)
             static_assert(ADJ_SEG % 16 == 0, "the gather below loads a segment four 128-bit words at a time");
             int cs[3];
 #pragma unroll
@@ -926,11 +598,7 @@ __device__ __forceinline__ void nms_rounds_body(const RoundsArgs &a, const GridC
                 cs[sg] = min(cr, ADJ_SEG);
             }
             int w = 0;
-            auto put = [&](int v) {   // w <= the position being read: the gather never overwrites what it has not read
-                if (res) put0(w, v);
-                else row[w] = v;
-                ++w;
-            };
+            auto put = [&](int v) { row[w++] = v; };   // w <= the position being read: the gather never overwrites what it has not read
 #pragma unroll
             for (int sg = 0; sg < 3; ++sg) {
                 for (int g = 0; g * 16 < cs[sg]; ++g) {
@@ -954,7 +622,7 @@ __device__ __forceinline__ void nms_rounds_body(const RoundsArgs &a, const GridC
             ov = cr > ADJ_CAP;                  // (mid path: the counter kept running past the list's capacity)
             total = min(cr, ADJ_CAP);
             if (res)
-                for (int e = 0; e < min(total, a.adj_smem); e += 4) {
+                for (int e = 0; e < min(total, ADJ_SMEM); e += 4) {
                     const int4 q = __ldcg(row4 + (e >> 2));
                     sadj[(e + 0) * NT + tid] = q.x;
                     sadj[(e + 1) * NT + tid] = q.y;
@@ -976,15 +644,14 @@ __device__ __forceinline__ void nms_rounds_body(const RoundsArgs &a, const GridC
             const unsigned sj = ld_state(a.state + j);
             if (sj == 1u) { any_kept = true; return false; }
             if (sj == 0u) {
-                if (w >= a.adj_stride) { more = true; return false; }
+                if (w >= adj_stride) { more = true; return false; }
                 put(w, j);
                 ++w;
             }
             return true;
         };
-        if (a.brute) for_each_earlier(r, a.sbox, a.iou, bfast, a.mode, visit);
-        else if (a.kspace) for_each_predecessor_k(r, a.keys, c, a.cell_start, a.cell_end, a.cbox, a.carea, a.iou, visit);
-        else for_each_predecessor(a.pos_of_rank[r], a.keys, c, a.cell_start, a.cell_end, a.cbox, a.carea, a.iou, visit);
+        if (BRUTE) for_each_earlier(r, a.sbox, a.iou, bfast, a.mode, visit);
+        else for_each_predecessor_k(r, a.keys, c, a.cell_start, a.cell_end, a.cbox, a.carea, a.iou, visit);
         atomicAdd(&a.out_state[4], 1);   // statistics: list refills
         if (any_kept) return 2;
         pn = w;
@@ -1006,7 +673,7 @@ __device__ __forceinline__ void nms_rounds_body(const RoundsArgs &a, const GridC
                 if (d) {
                     state[gtid] = (unsigned char)d;
                     first_done = true;
-                    if (d == 1 && a.kept_keys) a.kept_keys[atomicAdd(&a.out_state[1], 1)] = __ldcg(&a.final_keys[gtid]);   // (the caller orders them)
+                    if (!BRUTE && d == 1) a.kept_keys[atomicAdd(&a.out_state[1], 1)] = __ldcg(&a.keys[gtid]);   // (the caller orders them)
                 }
                 else ++undecided;
             }
@@ -1015,14 +682,14 @@ __device__ __forceinline__ void nms_rounds_body(const RoundsArgs &a, const GridC
                 const int v = __ldcg(&acnt[r * cstep]);
                 int pn = v & 0x3fffffff;
                 bool ov = (v >> 30) & 1;
-                int *row = const_cast<int *>(a.adj) + (size_t)r * a.adj_stride;
+                int *row = const_cast<int *>(a.adj) + (size_t)r * adj_stride;
                 auto putr = [&](int e, int x) { row[e] = x; };
                 int d = pn == 0 ? 1 : (nothing_yet ? 0 : decide_pending(pn, [&](int e) { return __ldcg(row + e); }, putr, a.state));
                 if (d == 1 && ov) d = refill(r, putr, pn, ov);
                 if (d == 0 && !nothing_yet) acnt[r * cstep] = pn | (ov ? (1 << 30) : 0);
                 if (d) {
                     state[r] = (unsigned char)d;
-                    if (d == 1 && a.kept_keys) a.kept_keys[atomicAdd(&a.out_state[1], 1)] = __ldcg(&a.final_keys[r]);
+                    if (!BRUTE && d == 1) a.kept_keys[atomicAdd(&a.out_state[1], 1)] = __ldcg(&a.keys[r]);
                 } else ++undecided;
             }
             // Warps sweep at their own pace — no CTA barrier in here, so a warp with short lists advances one dependency link per
@@ -1043,11 +710,11 @@ __device__ __forceinline__ void nms_rounds_body(const RoundsArgs &a, const GridC
         if (left == 0) break;
     }
     mid_stamp(a.dbg, 5);
-    if (a.kept_keys) {   // every kept box appended its key when it was decided; the epoch's last grid-wide barrier published them
+    if (!BRUTE) {   // every kept box appended its key when it was decided; the epoch's last grid-wide barrier published them
         mid_stamp(a.dbg, 6);
         return;
     }
-    // ordered output of the kept ranks
+    // ordered output of the kept source indices
     const int ntiles = (a.N + NT - 1) / NT;
     for (int t = blockIdx.x; t < ntiles; t += G) {
         const int r = t * NT + tid;
@@ -1073,9 +740,7 @@ __device__ __forceinline__ void nms_rounds_body(const RoundsArgs &a, const GridC
         const unsigned mine = __shfl_sync(0xffffffffu, myb, warp);
         if ((mine >> lane) & 1u) {
             const int pos = offset + wpre + __popc(mine & ((1u << lane) - 1u));
-            if (a.kept_keys) a.kept_keys[pos] = __ldcg(&a.final_keys[t * NT + tid]);
-            else if (a.final_keep) a.final_keep[pos] = (int)(unsigned)__ldcg(&a.final_keys[t * NT + tid]);
-            else a.keep_ranks[pos] = t * NT + tid;
+            a.final_keep[pos] = (int)(unsigned)__ldcg(&a.keys[t * NT + tid]);
         }
     }
     if (blockIdx.x == 0) {
@@ -1084,23 +749,16 @@ __device__ __forceinline__ void nms_rounds_body(const RoundsArgs &a, const GridC
         const int total = block_sum(part, red);
         if (tid == 0) {
             a.out_state[1] = total;
-            if (a.final_num) { a.final_num[0] = total; a.final_num[1] = __ldcg(&a.status[0]); }
+            a.final_num[0] = total;
+            a.final_num[1] = __ldcg(&a.status[0]);
         }
     }
     mid_stamp(a.dbg, 6);
 }
 
-__global__ void __launch_bounds__(NT, 1) nms_rounds_kernel(RoundsArgs a) {
-    extern __shared__ int sadj[];
-    __shared__ int red[32];
-    const GridCfg c = *a.cfg;
-    if (!c.use) return;  // uniform over the grid: the peel kernel handles this problem
-    nms_rounds_body(a, c, sadj, red);
-}
-
 // ---- mid path (one problem of a few thousand boxes) ------------------------------------------------------------------
-// Between the single-CTA path (one SM's latency chain: 229 us at 4 096 boxes) and the spatial path (~25 stream operations of
-// fixed cost, built for 10^5 boxes) a problem of a few thousand boxes is small enough for brute force over ALL SMs, and short
+// Between the single-CTA path (one SM's latency chain: 229 us at 4 096 boxes) and the spatial path (nms_big_kernel, built for
+// 10^5 boxes) a problem of a few thousand boxes is small enough for brute force over ALL SMs, and short
 // enough that launches dominate: separate kernels for these phases measured 103 us at 4 096 boxes, of which ~10 us were
 // work.  So the whole problem is ONE cooperative kernel, phases separated by grid-wide barriers, no memset before it:
 //   0  clear the status block, ranks, list counters and decision states;
@@ -1121,7 +779,7 @@ struct MidArgs {
     u64 *sorted;
     float4 *sbox;
     int *rank;
-    int *st;                // status block (nms_big_impl's slots), followed by everything that must start at zero
+    int *st;                // status block (nms_big_kernel's slots), followed by everything that must start at zero
     int zero_ints;
     RoundsArgs ra;
 };
@@ -1230,15 +888,15 @@ __global__ void __launch_bounds__(NT, 1) nms_mid_kernel(MidArgs m) {
     __threadfence();
     grid.sync();
     mid_stamp(m.ra.dbg, 4);
-    const GridCfg c = *m.ra.cfg;
-    nms_rounds_body(m.ra, c, dyn, red);
+    nms_rounds_body<true>(m.ra, GridCfg{}, dyn, red);   // (brute mode: no grid)
 }
 
 // ---- big path in one launch -------------------------------------------------------------------------------------------
 // The spatial path used to be ~25 stream operations (two radix sorts of one kernel per 8-bit pass, nine small kernels, six
 // memsets): at 100 000 boxes two thirds of its 332 us were launch gaps and latency-bound 25-CTA radix passes.  nms_big_kernel is
 // ONE cooperative kernel, phases separated by grid-wide barriers, and it never sorts the boxes globally:
-//   0  keys (score desc | index) by source index, NaN / regularity flags, grid statistics, the OR / NAND of all score keys;
+//   0  keys (score desc | index) made from the scores or taken from the caller, NaN / regularity flags, grid statistics, the
+//      OR / NAND of all score keys;
 //   1  grid geometry (every CTA, identically); cell of every box and its arrival slot there (atomicAdd);
 //   2  cell bounds: scan of the counts;   3  keys to cell order;
 //   4  key order inside every cell by counting smaller members; cell-ordered boxes and areas;
@@ -1246,31 +904,36 @@ __global__ void __launch_bounds__(NT, 1) nms_mid_kernel(MidArgs m) {
 //   6  decision sweeps (nms_rounds_body) -> the kept boxes' keys, unordered;
 //   7  the kept keys ordered by all-pairs counting (radix passes when there are very many) = the reference's output order.
 // When the grid does not apply (irregular boxes, degenerate thresholds, too crowded) the same launch sorts globally with the
-// cooperative LSD radix sort below (9-bit digits over the differing key bits, tiles of 1024 keys, per-(digit, tile) counts ->
-// row scans -> stable scatter that also counts the next pass's digits) and runs the peel.
+// cooperative LSD radix sort below (9-bit digits over the index bits of caller keys, then the differing score bits, tiles of
+// 1024 keys, per-(digit, tile) counts -> row scans -> stable scatter that also counts the next pass's digits) and runs the peel.
 constexpr int CS_BITS = 9;
 constexpr int CS_D = 1 << CS_BITS;
 constexpr size_t CS_SMEM = sizeof(int) * (size_t)(2 + NWARPS) * CS_D;
 
 struct BigArgs {
-    const float *dets;
+    const float *dets;      // box i at dets + i * stride (x1, y1, x2, y2), its score at column 4 when the keys are made here
     int n, stride, presorted, mode;
-    u64 *key_e;             // keys (score desc | source index) by source index; the fallback's sort ping-pongs it with tmp_key
+    const u64 *keys_in;     // optional: the n keys (score desc | box index), in any order (a batch image's, from the decode kernel)
+    int ibits;              // bits of the largest box index: the radix passes over the index before the score bits
+    u64 *key_e;             // keys by slot e (made: e = the box index); the fallback's sort ping-pongs it with tmp_key
     u64 *tmp_key;           // keys in cell order, arrival order inside a cell
     u64 *ckey;              // keys in cell order, key order inside a cell (final)
     u64 *kept_keys;         // keys of the kept boxes
-    int *cell_e, *slot_e;   // cell and arrival slot of source box e
+    int *cell_e, *slot_e;   // cell and arrival slot of the box of key_e[e]
     int *tmp_cell;          // cell of tmp position k
     int *kept_rank;         // rank of a kept key among the kept keys (zero at its first use)
     int *hist;              // fallback / many kept boxes: [2][CS_D][ntiles] digit counts per tile, then [CS_D] digit totals
     float4 *sbox;           // fallback: boxes in rank order
-    int *st;                // status block (zero at launch): nms_big_impl's slots, [22] NAND / [23] OR of the score keys, [24] ticket
+    int *st;                // status block (zero at launch): [0] NaN score, [2] some box not "fast ok", [3] spatial path used, [4] kept,
+                            // [5] kept of a peel stage, [6] epochs, [7] list refills, [8..12] grid statistics, [13..15] round counters,
+                            // [16..21] GridCfg (statistics), [22] NAND / [23] OR of the score keys, [24] ticket
     int *cell_cnt, *cell_start, *cell_end;
     float4 *cbox;
     float *carea;
     RoundsArgs ra;
     PeelArgs pa;
-    int *keep_dev, *num_keep_dev;
+    int *keep_dev, *keep_count;
+    int *nan_flag;          // optional
     long long *dbg;         // FD_NMS_DBG: globaltimer stamps of block 0
 };
 
@@ -1415,6 +1078,32 @@ __device__ __forceinline__ u64 *cs_sort(u64 *a, u64 *b, int n, int lo_bit, int n
     return in;
 }
 
+// Sorts n unique keys: LSD passes over the index bits [0, ibits) — 0 when the keys are already in index order — then over the
+// score bits that differ (diff: a mask of the high-word bits in which the keys differ).  Returns the sorted array; every CTA must call it.
+__device__ __forceinline__ u64 *cs_sort_keys(u64 *a, u64 *b, int n, int ibits, unsigned diff, int *hist, int *sh, int *red) {
+    cg::grid_group grid = cg::this_grid();
+    const int ntiles = (n + NT - 1) / NT;
+    if (ibits > 0) {
+        cs_tile_hist([&](int e) { return __ldcg(a + e); }, n, 0, hist, ntiles, sh);
+        __threadfence();
+        grid.sync();
+        u64 *r = cs_sort(a, b, n, 0, ibits, hist, ntiles, sh, red);
+        if (r != a) { b = a; a = r; }
+    }
+    const int nbits = diff ? 32 - __clz(diff) : 0;
+    if (nbits > 0) {
+        cs_tile_hist([&](int e) { return __ldcg(a + e); }, n, 32, hist, ntiles, sh);
+        __threadfence();
+        grid.sync();
+        a = cs_sort(a, b, n, 32, nbits, hist, ntiles, sh, red);
+    }
+    return a;
+}
+
+__device__ __forceinline__ unsigned differing_score_bits(const int *nand_or) {   // from the NAND and the OR of all score keys
+    return (~__ldcg(reinterpret_cast<const unsigned *>(nand_or))) ^ __ldcg(reinterpret_cast<const unsigned *>(nand_or) + 1);
+}
+
 constexpr int KEPT_RANK_CAP = 16384;   // kept keys ordered by all-pairs counting up to here (6 357 at 100 000 boxes), by the radix passes beyond
 
 __global__ void __launch_bounds__(NT, 1) nms_big_kernel(BigArgs m) {
@@ -1423,7 +1112,7 @@ __global__ void __launch_bounds__(NT, 1) nms_big_kernel(BigArgs m) {
     __shared__ GridCfg scfg;
     cg::grid_group grid = cg::this_grid();
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, G = gridDim.x, gtid = blockIdx.x * NT + tid, gstride = G * NT;
-    const int n = m.n, ntiles = (n + NT - 1) / NT;
+    const int n = m.n;
     unsigned *gs = reinterpret_cast<unsigned *>(m.st + 8);
     big_stamp(m.dbg, 0);
     // ---- 0. keys, flags, grid statistics; arrays that must start at zero ----
@@ -1432,7 +1121,21 @@ __global__ void __launch_bounds__(NT, 1) nms_big_kernel(BigArgs m) {
         unsigned mincx = 0xFFFFFFFFu, mincy = 0xFFFFFFFFu, maxcx = 0, maxcy = 0, maxd = 0;
         bool nan_seen = false, ok = true;
         for (int e = gtid; e < n; e += gstride) {
-            const float *p = m.dets + (size_t)e * m.stride;
+            u64 key;
+            if (m.keys_in) {
+                key = __ldg(m.keys_in + e);   // (no NaN check: the decode kernel drops NaN scores)
+            } else if (m.presorted) {
+                key = (u64)(unsigned)e;
+            } else {
+                const float sc = __ldg(m.dets + (size_t)e * m.stride + 4);
+                nan_seen |= (sc != sc);
+                key = ((u64)desc_key(sc) << 32) | (unsigned)e;
+            }
+            m.key_e[e] = key;
+            const unsigned k32 = (unsigned)(key >> 32);
+            acc_or |= k32;
+            acc_nand |= ~k32;
+            const float *p = m.dets + (size_t)(unsigned)key * m.stride;
             const float4 b = make_float4(__ldg(p), __ldg(p + 1), __ldg(p + 2), __ldg(p + 3));
             ok &= box_is_fast_ok(b);
             const unsigned cx = f2ord(box_cx(b)), cy = f2ord(box_cy(b));
@@ -1440,16 +1143,6 @@ __global__ void __launch_bounds__(NT, 1) nms_big_kernel(BigArgs m) {
             mincy = min(mincy, cy); maxcy = max(maxcy, cy);
             const float w = __fadd_rn(__fsub_rn(b.z, b.x), 1.0f), h = __fadd_rn(__fsub_rn(b.w, b.y), 1.0f);
             maxd = max(maxd, f2ord(fmaxf(fabsf(w), fabsf(h))));
-            if (m.presorted) {
-                m.key_e[e] = (u64)(unsigned)e;
-            } else {
-                const float sc = __ldg(p + 4);
-                nan_seen |= (sc != sc);
-                const unsigned k32 = desc_key(sc);
-                m.key_e[e] = ((u64)k32 << 32) | (unsigned)e;
-                acc_or |= k32;
-                acc_nand |= ~k32;
-            }
         }
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) {
@@ -1509,7 +1202,7 @@ __global__ void __launch_bounds__(NT, 1) nms_big_kernel(BigArgs m) {
     if (tid == 0) {
         scfg = grid_setup(~__ldcg(gs + 0), ~__ldcg(gs + 1), __ldcg(gs + 2), __ldcg(gs + 3), __ldcg(gs + 4), n, m.ra.iou, __ldcg(&m.st[2]));
         if (blockIdx.x == 0) {
-            *const_cast<GridCfg *>(m.ra.cfg) = scfg;
+            *reinterpret_cast<GridCfg *>(m.st + 16) = scfg;
             m.st[3] = scfg.use;
         }
     }
@@ -1517,17 +1210,9 @@ __global__ void __launch_bounds__(NT, 1) nms_big_kernel(BigArgs m) {
     const GridCfg c = scfg;
     if (!c.use) {
         // ---- the grid does not apply (irregular boxes, degenerate threshold, too crowded; uniform over the launch): global sort by
-        //      key (LSD radix over the differing score bits; the keys are in index order, so ties stay stable), boxes in rank order,
+        //      key (made keys are in index order already, so their sort passes over the score bits only), boxes in rank order,
         //      the peel, and its kept ranks become source indices ----
-        u64 *sorted = m.key_e;
-        if (!m.presorted) {
-            const unsigned diff = (~__ldcg(reinterpret_cast<unsigned *>(m.st) + 22)) ^ __ldcg(reinterpret_cast<unsigned *>(m.st) + 23);
-            const int nbits = diff ? 32 - __clz(diff) : 0;
-            if (nbits > 0) cs_tile_hist([&](int e) { return __ldcg(m.key_e + e); }, n, 32, m.hist, ntiles, dyn);
-            __threadfence();
-            grid.sync();
-            sorted = cs_sort(m.key_e, m.tmp_key, n, 32, nbits, m.hist, ntiles, dyn, red);
-        }
+        u64 *sorted = cs_sort_keys(m.key_e, m.tmp_key, n, m.keys_in ? m.ibits : 0, differing_score_bits(m.st + 22), m.hist, dyn, red);
         for (int r = gtid; r < n; r += gstride) {
             const int idx = (int)(unsigned)__ldcg(sorted + r);
             const float *p = m.dets + (size_t)idx * m.stride;
@@ -1542,15 +1227,15 @@ __global__ void __launch_bounds__(NT, 1) nms_big_kernel(BigArgs m) {
         const int total = __ldcg(&m.pa.state[1]);
         for (int k = gtid; k < total; k += gstride) m.keep_dev[k] = (int)(unsigned)__ldcg(sorted + __ldcg(&m.pa.keep_ranks[k]));
         if (gtid == 0) {
-            m.num_keep_dev[0] = total;
-            m.num_keep_dev[1] = __ldcg(&m.st[0]);
+            *m.keep_count = total;
+            if (m.nan_flag) *m.nan_flag = __ldcg(&m.st[0]);
         }
         return;
     }
     const int ncells = c.gx * c.gy;
     // ---- 1. cell of every box and its arrival slot there (no global sort: only the members of a cell get ordered) ----
     for (int e = gtid; e < n; e += gstride) {
-        const float *p = m.dets + (size_t)e * m.stride;
+        const float *p = m.dets + (size_t)(unsigned)m.key_e[e] * m.stride;   // (key_e[e] was written by this very thread in phase 0)
         const float4 b = make_float4(__ldg(p), __ldg(p + 1), __ldg(p + 2), __ldg(p + 3));
         const int cell = cell_coord(box_cy(b), c.miny, c.cs, c.gy) * c.gx + cell_coord(box_cx(b), c.minx, c.cs, c.gx);
         m.cell_e[e] = cell;
@@ -1648,7 +1333,7 @@ __global__ void __launch_bounds__(NT, 1) nms_big_kernel(BigArgs m) {
     // ---- 6. decision sweeps; the kept boxes' keys come out in position order ----
     RoundsArgs ra = m.ra;
     ra.dbg = m.dbg ? m.dbg + 4 : nullptr;   // its stamps 5 / 6 land in slots 9 / 10
-    nms_rounds_body(ra, c, dyn, red);   // (ends behind the grid-wide barrier of its last epoch: kept keys and their count are visible)
+    nms_rounds_body<false>(ra, c, dyn, red);   // (ends behind the grid-wide barrier of its last epoch: kept keys and their count are visible)
     big_stamp(m.dbg, 7);
     // ---- 7. the kept keys in key order = the reference's output order ----
     const int M = __ldcg(&m.st[4]);
@@ -1682,32 +1367,56 @@ __global__ void __launch_bounds__(NT, 1) nms_big_kernel(BigArgs m) {
         __threadfence();
         grid.sync();
         for (int i = gtid; i < M; i += gstride) m.keep_dev[__ldcg(&m.kept_rank[i])] = (int)(unsigned)__ldcg(&m.kept_keys[i]);
-    } else {                    // very many kept boxes: LSD radix passes over the index bits, then the differing score bits
-        const int mt = (M + NT - 1) / NT;
-        const int ibits = n > 1 ? 32 - __clz(n - 1) : 0;
-        u64 *a = m.kept_keys, *b = m.tmp_key;
-        if (ibits > 0) {
-            cs_tile_hist([&](int e) { return __ldcg(a + e); }, M, 0, m.hist, mt, dyn);
-            __threadfence();
-            grid.sync();
-            u64 *r = cs_sort(a, b, M, 0, ibits, m.hist, mt, dyn, red);
-            if (r != a) { b = a; a = r; }
-        }
-        const unsigned diff = (~__ldcg(reinterpret_cast<unsigned *>(m.st) + 22)) ^ __ldcg(reinterpret_cast<unsigned *>(m.st) + 23);
-        const int nbits = (!m.presorted && diff) ? 32 - __clz(diff) : 0;
-        if (nbits > 0) {
-            cs_tile_hist([&](int e) { return __ldcg(a + e); }, M, 32, m.hist, mt, dyn);
-            __threadfence();
-            grid.sync();
-            a = cs_sort(a, b, M, 32, nbits, m.hist, mt, dyn, red);
-        }
-        for (int i = gtid; i < M; i += gstride) m.keep_dev[i] = (int)(unsigned)__ldcg(a + i);
+    } else {                    // very many kept boxes (appended in no particular order): radix passes over index and score bits
+        const u64 *sorted = cs_sort_keys(m.kept_keys, m.tmp_key, M, m.ibits, differing_score_bits(m.st + 22), m.hist, dyn, red);
+        for (int i = gtid; i < M; i += gstride) m.keep_dev[i] = (int)(unsigned)__ldcg(sorted + i);
     }
     if (gtid == 0) {
-        m.num_keep_dev[0] = M;
-        m.num_keep_dev[1] = __ldcg(&m.st[0]);
+        *m.keep_count = M;
+        if (m.nan_flag) *m.nan_flag = __ldcg(&m.st[0]);
     }
     big_stamp(m.dbg, 8);
+}
+
+// argsort_descending beyond SMALL_CAP: keys (score desc | index) from the score column alone — the caller passes (scores - 4)
+// with stride 1, so any other column would be another score or the pad — sorted by nms_big_kernel's radix passes over the
+// differing score bits (the keys are made in index order, so ties stay stable).  st (zero at launch): [0] NaN score seen,
+// [1] NAND / [2] OR of the score keys.
+__global__ void __launch_bounds__(NT, 1) argsort_kernel(const float *__restrict__ dets, int n, int stride, u64 *keys, u64 *tmp, int *hist,
+                                                        int *st, int *__restrict__ order, int *__restrict__ flag) {
+    extern __shared__ __align__(16) int dyn[];
+    __shared__ int red[32];
+    __shared__ unsigned acc[2];
+    cg::grid_group grid = cg::this_grid();
+    const int tid = threadIdx.x, gtid = blockIdx.x * NT + tid, gstride = gridDim.x * NT;
+    if (tid == 0) acc[0] = acc[1] = 0u;
+    __syncthreads();
+    unsigned acc_or = 0, acc_nand = 0;
+    bool nan_seen = false;
+    for (int e = gtid; e < n; e += gstride) {
+        const float sc = __ldg(dets + (size_t)e * stride + 4);
+        nan_seen |= (sc != sc);
+        const unsigned k32 = desc_key(sc);
+        keys[e] = ((u64)k32 << 32) | (unsigned)e;
+        acc_or |= k32;
+        acc_nand |= ~k32;
+    }
+    acc_or = __reduce_or_sync(0xffffffffu, acc_or);
+    acc_nand = __reduce_or_sync(0xffffffffu, acc_nand);
+    if ((tid & 31) == 0) {   // one pair of global atomics per CTA
+        atomicOr(&acc[0], acc_nand);
+        atomicOr(&acc[1], acc_or);
+    }
+    if (__syncthreads_or(nan_seen) && tid == 0) atomicExch(&st[0], 1);
+    if (tid == 0 && (acc[0] | acc[1])) {
+        atomicOr(reinterpret_cast<unsigned *>(st) + 1, acc[0]);
+        atomicOr(reinterpret_cast<unsigned *>(st) + 2, acc[1]);
+    }
+    __threadfence();
+    grid.sync();
+    const u64 *sorted = cs_sort_keys(keys, tmp, n, 0, differing_score_bits(st + 1), hist, dyn, red);
+    for (int r = gtid; r < n; r += gstride) order[r] = (int)(unsigned)__ldcg(sorted + r);
+    if (gtid == 0) *flag = __ldcg(&st[0]);
 }
 
 // ---- host side ------------------------------------------------------------------------------------------------
@@ -1737,26 +1446,6 @@ IouParams make_iou_params(float thr, int mode) {
         p.fast = 1;
     }
     return p;
-}
-
-// hist: (nbytes + 1) x 256 x ntiles ints.
-static int radix_sort_u64(fd_ctx *ctx, u64 *keys, u64 *tmp, int n, const int *bytes, int nbytes, int *hist, u64 **sorted) {
-    const int ntiles = (n + RS_TILE - 1) / RS_TILE;
-    const size_t hsz = (size_t)256 * ntiles;
-    FD_CUDA(cudaMemsetAsync(hist, 0, sizeof(int) * hsz * (size_t)nbytes, ctx->stream));
-    u64 *in = keys, *out = tmp;
-    radix_hist_kernel<<<ntiles, RS_THREADS, 0, ctx->stream>>>(in, n, bytes[0] * 8, hist, ntiles);
-    FD_LAUNCH_CHECK(ctx);
-    for (int p = 0; p < nbytes; ++p) {
-        int *hcur = hist + hsz * p;
-        int *hnext = p + 1 < nbytes ? hist + hsz * (p + 1) : nullptr;
-        radix_pass_kernel<<<ntiles, RS_THREADS, 0, ctx->stream>>>(in, out, n, bytes[p] * 8, hcur, hnext,
-                                                                 p + 1 < nbytes ? bytes[p + 1] * 8 : 0, ntiles);
-        FD_LAUNCH_CHECK(ctx);
-        std::swap(in, out);
-    }
-    *sorted = in;
-    return FD_OK;
 }
 
 template <int MODE>
@@ -1798,149 +1487,6 @@ static int launch_small(fd_ctx *ctx, const SmallArgs &a_in, int B, bool float4_b
     return FD_OK;
 }
 
-// keys_dev: optional pre-made u64 keys (score desc | source index), else made from dets column 4.
-// key_bytes/nkey_bytes: radix passes to run (LSD order).
-static int nms_big_impl(fd_ctx *ctx, const u64 *keys_in, const int *key_bytes, int nkey_bytes, const float *boxes, int K,
-                        int stride, float thr, int mode, bool presorted, bool sort_only, int32_t *keep_dev,
-                        int32_t *num_keep_dev) {
-    const int ntiles_rs = (K + RS_TILE - 1) / RS_TILE;
-    const int ntiles_peel = (K + NT - 1) / NT;
-    FD_TRY(ctx->nms_ws[0].reserve(sizeof(u64) * (size_t)K));              // keys a
-    FD_TRY(ctx->nms_ws[1].reserve(sizeof(u64) * (size_t)K));              // keys b
-    FD_TRY(ctx->nms_ws[2].reserve(sizeof(int) * (size_t)256 * ntiles_rs * 8)); // per-pass histograms
-    FD_TRY(ctx->nms_ws[3].reserve(sizeof(float4) * (size_t)K));           // sorted boxes
-    FD_TRY(ctx->nms_ws[4].reserve(sizeof(int) * (size_t)K * 3));          // stream a, stream b, keep ranks
-    FD_TRY(ctx->nms_ws[5].reserve(sizeof(float4) * HEAD + sizeof(int) * (size_t)ntiles_peel * 33 + 64));
-    FD_TRY(ctx->nms_ws[6].reserve(sizeof(int) * 32));                     // status/state + grid stats + counters + cfg
-    u64 *ka = ctx->nms_ws[0].as<u64>(), *kb = ctx->nms_ws[1].as<u64>();
-    int *hist = ctx->nms_ws[2].as<int>();
-    float4 *sbox = ctx->nms_ws[3].as<float4>();
-    int *stream_a = ctx->nms_ws[4].as<int>(), *stream_b = stream_a + K, *keep_ranks = stream_b + K;
-    float4 *ks = ctx->nms_ws[5].as<float4>();
-    int *tile_counts = reinterpret_cast<int *>(ks + HEAD);
-    unsigned *ballots = reinterpret_cast<unsigned *>(tile_counts + ntiles_peel);
-    int *st = ctx->nms_ws[6].as<int>();  // [0] nan, [2] not-fast flag, [3] spatial path active, [4] kept total, [5] stage kept,
-                                         // [8..12] grid stats, [13..15] round counters, [16..21] GridCfg
-    FD_CUDA(cudaMemsetAsync(st, 0, sizeof(int) * 32, ctx->stream));
-    FD_CUDA(cudaMemsetAsync(st + 8, 0xFF, sizeof(int) * 2, ctx->stream));   // min cx / min cy
-    const int tb = 256, gb = (K + tb - 1) / tb;
-    u64 *sorted = ka;
-    if (presorted) {
-        iota_keys_kernel<<<gb, tb, 0, ctx->stream>>>(K, ka);
-        FD_LAUNCH_CHECK(ctx);
-    } else {
-        if (keys_in) FD_CUDA(cudaMemcpyAsync(ka, keys_in, sizeof(u64) * (size_t)K, cudaMemcpyDeviceToDevice, ctx->stream));
-        else {
-            make_keys_kernel<<<gb, tb, 0, ctx->stream>>>(boxes, K, stride, ka, st);
-            FD_LAUNCH_CHECK(ctx);
-        }
-        FD_TRY(radix_sort_u64(ctx, ka, kb, K, key_bytes, nkey_bytes, hist, &sorted));
-    }
-    if (sort_only) {
-        low32_kernel<<<gb, tb, 0, ctx->stream>>>(sorted, K, keep_dev);
-        FD_LAUNCH_CHECK(ctx);
-        FD_CUDA(cudaMemcpyAsync(num_keep_dev, st, sizeof(int), cudaMemcpyDeviceToDevice, ctx->stream));  // nan flag
-        return FD_OK;
-    }
-    gather_sorted_boxes_kernel<<<gb, tb, 0, ctx->stream>>>(sorted, K, boxes, stride, sbox, st);
-    FD_LAUNCH_CHECK(ctx);
-    const IouParams iou = make_iou_params(thr, mode);
-    // ---- spatial path (decides on the device whether it applies; the peel kernel below is its complement) ----
-    {
-        FD_TRY(ctx->nms_ws_sp[0].reserve(sizeof(u64) * (size_t)K * 2));                        // cell keys a/b
-        FD_TRY(ctx->nms_ws_sp[1].reserve(sizeof(int) * (size_t)(GRID_MAX_CELLS + 1) * 2));     // cell start / end
-        FD_TRY(ctx->nms_ws_sp[2].reserve((sizeof(float4) + sizeof(float) + sizeof(int) * 2) * (size_t)K + (size_t)K)); // cbox, carea, pos, cnt, state
-        FD_TRY(ctx->nms_ws_sp[3].reserve(sizeof(int) * (size_t)K * ADJ_CAP));                  // predecessor lists
-        u64 *cka = ctx->nms_ws_sp[0].as<u64>(), *ckb = cka + K;
-        int *cell_start = ctx->nms_ws_sp[1].as<int>(), *cell_end = cell_start + (GRID_MAX_CELLS + 1);
-        float4 *cbox = ctx->nms_ws_sp[2].as<float4>();
-        float *carea = reinterpret_cast<float *>(cbox + K);
-        int *pos_of_rank = reinterpret_cast<int *>(carea + K);
-        int *adj_cnt = pos_of_rank + K;
-        unsigned char *state = reinterpret_cast<unsigned char *>(adj_cnt + K);
-        int *adj = ctx->nms_ws_sp[3].as<int>();
-        unsigned *gs = reinterpret_cast<unsigned *>(st + 8);
-        GridCfg *cfg = reinterpret_cast<GridCfg *>(st + 16);
-        grid_stats_kernel<<<gb, tb, 0, ctx->stream>>>(sbox, K, gs);
-        FD_LAUNCH_CHECK(ctx);
-        grid_setup_kernel<<<1, 1, 0, ctx->stream>>>(gs, K, iou, cfg, st);
-        FD_LAUNCH_CHECK(ctx);
-        cell_keys_kernel<<<gb, tb, 0, ctx->stream>>>(sbox, K, cfg, cka);
-        FD_LAUNCH_CHECK(ctx);
-        static const int cell_bytes[2] = {4, 5};
-        u64 *csorted = cka;
-        FD_TRY(radix_sort_u64(ctx, cka, ckb, K, cell_bytes, 2, hist, &csorted));
-        FD_CUDA(cudaMemsetAsync(cell_start, 0, sizeof(int) * (size_t)(GRID_MAX_CELLS + 1) * 2, ctx->stream));
-        FD_CUDA(cudaMemsetAsync(state, 0, (size_t)K, ctx->stream));
-        cell_bounds_kernel<<<gb, tb, 0, ctx->stream>>>(csorted, K, cfg, sbox, cell_start, cell_end, cbox, carea, pos_of_rank);
-        FD_LAUNCH_CHECK(ctx);
-        adjacency_kernel<<<gb, 256, 0, ctx->stream>>>(csorted, K, cfg, cell_start, cell_end, cbox, carea, iou, adj, adj_cnt);
-        FD_LAUNCH_CHECK(ctx);
-        RoundsArgs ra{};
-        ra.N = K;
-        ra.keys = csorted;
-        ra.cfg = cfg;
-        ra.cell_start = cell_start;
-        ra.cell_end = cell_end;
-        ra.cbox = cbox;
-        ra.carea = carea;
-        ra.pos_of_rank = pos_of_rank;
-        ra.adj = adj;
-        ra.adj_cnt = adj_cnt;
-        ra.state = state;
-        ra.counters = st + 13;
-        ra.tile_counts = tile_counts;
-        ra.ballots = ballots;
-        ra.keep_ranks = keep_ranks;
-        ra.out_state = st + 3;
-        ra.iou = iou;
-        ra.sbox = sbox;
-        ra.brute = 0;
-        ra.mode = mode;
-        ra.status = st;
-        ra.adj_smem = ADJ_SMEM;
-        ra.seg3 = 0;
-        ra.adj_stride = ADJ_CAP;
-        ra.kspace = 0;
-        ra.kept_keys = nullptr;
-        void *rargs[] = {&ra};
-        int per_sm_r = 0;
-        const size_t smem_r = sizeof(int) * (size_t)ADJ_SMEM * NT;
-        FD_CUDA(cudaFuncSetAttribute(nms_rounds_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_r));
-        FD_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm_r, nms_rounds_kernel, NT, smem_r));
-        if (per_sm_r < 1) return fail(FD_ERR_CUDA, "nms_rounds_kernel does not fit on an SM");
-        int grid_r = std::min(ctx->num_sms * per_sm_r, std::max(1, ntiles_peel));
-        FD_CUDA(cudaLaunchCooperativeKernel((const void *)nms_rounds_kernel, dim3(grid_r), dim3(NT), rargs, smem_r, ctx->stream));
-        FD_LAUNCH_CHECK(ctx);
-    }
-    PeelArgs pa;
-    pa.sbox = sbox;
-    pa.N = K;
-    pa.stream_a = stream_a;
-    pa.stream_b = stream_b;
-    pa.keep_ranks = keep_ranks;
-    pa.state = st + 3;  // state[1] -> st[4], state[2] -> st[5]
-    pa.ks = ks;
-    pa.tile_counts = tile_counts;
-    pa.ballots = ballots;
-    pa.status = st;
-    pa.iou = iou;
-    const size_t smem = sizeof(PeelSmem);
-    void *kargs[] = {&pa};
-    const void *fn = mode == 0 ? (const void *)nms_peel_kernel<0> : (const void *)nms_peel_kernel<1>;
-    FD_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    int per_sm = 0;
-    if (mode == 0) FD_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, nms_peel_kernel<0>, NT, smem));
-    else FD_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, nms_peel_kernel<1>, NT, smem));
-    if (per_sm < 1) return fail(FD_ERR_CUDA, "nms_peel_kernel does not fit on an SM");
-    int grid = std::min(ctx->num_sms * per_sm, std::max(1, ntiles_peel));
-    FD_CUDA(cudaLaunchCooperativeKernel(fn, dim3(grid), dim3(NT), kargs, smem, ctx->stream));
-    FD_LAUNCH_CHECK(ctx);
-    map_keep_kernel<<<gb, tb, 0, ctx->stream>>>(keep_ranks, st + 3, sorted, keep_dev, num_keep_dev);
-    FD_LAUNCH_CHECK(ctx);
-    return FD_OK;
-}
-
 // One problem of SINGLE_PROBLEM_CROSSOVER < K <= MID_CAP boxes: a single cooperative launch (nms_mid_kernel).
 static int nms_mid_impl(fd_ctx *ctx, const float *boxes, int K, int stride, const IouParams &iou, int mode, bool presorted, int32_t *keep_dev,
                         int32_t *num_keep_dev) {
@@ -1966,27 +1512,19 @@ static int nms_mid_impl(fd_ctx *ctx, const float *boxes, int K, int stride, cons
     m.zero_ints = (int)zero_ints;
     RoundsArgs &ra = m.ra;
     ra.N = K;
-    ra.cfg = reinterpret_cast<GridCfg *>(st + 16);
+    ra.keys = m.sorted;
     ra.adj = ctx->nms_ws_sp[3].as<int>();
     ra.adj_cnt = adj_cnt;
     ra.state = reinterpret_cast<unsigned char *>(rank + K);
     ra.counters = st + 13;
     ra.tile_counts = ctx->nms_ws[5].as<int>();
     ra.ballots = reinterpret_cast<unsigned *>(ra.tile_counts + ntiles);
-    ra.keep_ranks = nullptr;
     ra.out_state = st + 3;
     ra.iou = iou;
     ra.sbox = m.sbox;
-    ra.brute = 1;
     ra.mode = mode;
     ra.status = st;
-    ra.adj_smem = ADJ_SMEM;
-    ra.seg3 = 0;
-    ra.adj_stride = ADJ_CAP;
-    ra.kspace = 0;
-    ra.kept_keys = nullptr;
     ra.final_keep = keep_dev;
-    ra.final_keys = m.sorted;
     ra.final_num = num_keep_dev;
     static int per_sm = 0;                                                 // one device type per process
     const size_t smem = sizeof(int) * (size_t)ADJ_SMEM * NT;
@@ -2019,9 +1557,10 @@ static int nms_mid_impl(fd_ctx *ctx, const float *boxes, int K, int stride, cons
     return FD_OK;
 }
 
-// The big path as ONE cooperative launch (nms_big_kernel); num_keep_dev receives {count, NaN flag}.
-static int nms_big_one_launch(fd_ctx *ctx, const float *boxes, int K, int stride, float thr, int mode, bool presorted, int32_t *keep_dev,
-                              int32_t *num_keep_dev) {
+// The big path as ONE cooperative launch (nms_big_kernel).  keys_in: optional keys (score desc | box index) in any order, else made
+// from column 4 of boxes; box indices are below index_bound.  keep_count receives the count, nan_flag (optional) the NaN flag.
+static int nms_big_one_launch(fd_ctx *ctx, const u64 *keys_in, const float *boxes, int K, int stride, int index_bound, float thr, int mode,
+                              bool presorted, int32_t *keep_dev, int32_t *keep_count, int32_t *nan_flag) {
     const int ntiles = (K + NT - 1) / NT;
     FD_TRY(ctx->nms_ws[0].reserve(sizeof(u64) * (size_t)K));
     FD_TRY(ctx->nms_ws[1].reserve(sizeof(u64) * (size_t)K));
@@ -2043,6 +1582,8 @@ static int nms_big_one_launch(fd_ctx *ctx, const float *boxes, int K, int stride
     m.stride = stride;
     m.presorted = presorted ? 1 : 0;
     m.mode = mode;
+    m.keys_in = keys_in;
+    m.ibits = index_bound > 1 ? 32 - __builtin_clz((unsigned)(index_bound - 1)) : 0;
     m.key_e = ctx->nms_ws[0].as<u64>();
     m.tmp_key = ctx->nms_ws[1].as<u64>();
     m.ckey = ctx->nms_ws_sp[0].as<u64>();
@@ -2067,34 +1608,19 @@ static int nms_big_one_launch(fd_ctx *ctx, const float *boxes, int K, int stride
     RoundsArgs &ra = m.ra;
     ra.N = K;
     ra.keys = m.ckey;
-    ra.cfg = reinterpret_cast<GridCfg *>(st + 16);
     ra.cell_start = m.cell_start;
     ra.cell_end = m.cell_end;
     ra.cbox = m.cbox;
     ra.carea = m.carea;
-    ra.pos_of_rank = nullptr;
     ra.adj = ctx->nms_ws_sp[3].as<int>();
     ra.adj_cnt = adj_cnt;
     ra.state = reinterpret_cast<unsigned char *>(adj_cnt + (size_t)3 * K);
     ra.counters = st + 13;
     ra.tile_counts = tile_counts;
     ra.ballots = ballots;
-    ra.keep_ranks = nullptr;
     ra.out_state = st + 3;
     ra.iou = iou;
-    ra.sbox = m.sbox;
-    ra.brute = 0;
-    ra.mode = mode;
-    ra.status = st;
-    static const int adj_smem = getenv("FD_NMS_ADJ_SMEM") ? std::max(4, std::min(ADJ_SMEM, atoi(getenv("FD_NMS_ADJ_SMEM")) & ~3)) : ADJ_SMEM;
-    ra.adj_smem = adj_smem;
-    ra.seg3 = 1;
-    ra.adj_stride = ADJ_ROW3;
-    ra.kspace = 1;
     ra.kept_keys = m.kept_keys;
-    ra.final_keep = nullptr;
-    ra.final_keys = m.ckey;
-    ra.final_num = nullptr;
     PeelArgs &pa = m.pa;
     pa.sbox = m.sbox;
     pa.N = K;
@@ -2108,9 +1634,10 @@ static int nms_big_one_launch(fd_ctx *ctx, const float *boxes, int K, int stride
     pa.status = st;
     pa.iou = iou;
     m.keep_dev = keep_dev;
-    m.num_keep_dev = num_keep_dev;
+    m.keep_count = keep_count;
+    m.nan_flag = nan_flag;
     static int per_sm = 0;                                                 // one device type per process
-    const size_t smem = std::max(std::max(sizeof(int) * (size_t)adj_smem * NT, sizeof(PeelSmem)), CS_SMEM);
+    const size_t smem = std::max(std::max(sizeof(int) * (size_t)ADJ_SMEM * NT, sizeof(PeelSmem)), CS_SMEM);
     if (!per_sm) {
         FD_CUDA(cudaFuncSetAttribute(nms_big_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         FD_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, nms_big_kernel, NT, smem));
@@ -2137,16 +1664,6 @@ static int nms_big_one_launch(fd_ctx *ctx, const float *boxes, int K, int stride
     return FD_OK;
 }
 
-int nms_big_device(fd_ctx *ctx, const float *dets_dev, int K, int stride, float thr, int mode, bool presorted,
-                   int32_t *keep_dev, int32_t *num_keep_dev) {
-    static const bool multi = getenv("FD_NMS_MULTI_KERNEL") != nullptr && getenv("FD_NMS_MULTI_KERNEL")[0] == '1';   // A/B: the round-1 launch sequence
-    if (!multi) return nms_big_one_launch(ctx, dets_dev, K, stride, thr, mode, presorted, keep_dev, num_keep_dev);
-    static const int bytes[4] = {4, 5, 6, 7};  // score bytes only: the sort is stable, ties keep index order
-    FD_TRY(nms_big_impl(ctx, nullptr, bytes, 4, dets_dev, K, stride, thr, mode, presorted, false, keep_dev, num_keep_dev));
-    FD_CUDA(cudaMemcpyAsync(num_keep_dev + 1, ctx->nms_ws[6].as<int>(), sizeof(int), cudaMemcpyDeviceToDevice, ctx->stream));
-    return FD_OK;
-}
-
 // Statistics of the last big-path NMS: [0] spatial path used, [1] kept, [2] decision epochs, [3] grid w, [4] grid h,
 // [5] cell size (float bits)
 int nms_last_stats(fd_ctx *ctx, int32_t out[8]) {
@@ -2164,8 +1681,8 @@ int nms_last_stats(fd_ctx *ctx, int32_t out[8]) {
 constexpr int SINGLE_PROBLEM_CROSSOVER = 1024;   // = TINY_CAP: beyond it the all-SM mid path is faster (61 vs 68 us at 1 100 boxes)
 int nms_device(fd_ctx *ctx, const float *dets_dev, int K, int stride, float thr, int mode, bool presorted,
                int32_t *keep_dev, int32_t *num_keep_dev) {
-    // ONE problem: a single SM (the barrier-light tiny path) up to 1 024 boxes, one cooperative all-SM kernel up to MID_CAP, the
-    // multi-kernel spatial path beyond (measured: profiles/r2_nms_sizes.json); batched callers keep one CTA per image up to SMALL_CAP
+    // ONE problem: a single SM (the barrier-light tiny path) up to 1 024 boxes, one cooperative all-SM kernel up to MID_CAP,
+    // nms_big_kernel beyond (measured: profiles/r2_nms_sizes.json); batched callers keep one CTA per image up to SMALL_CAP
     static const int single_cross = getenv("FD_NMS_CROSS") ? atoi(getenv("FD_NMS_CROSS")) : SINGLE_PROBLEM_CROSSOVER;
     static const int mid_cap = getenv("FD_NMS_MID_CAP") ? atoi(getenv("FD_NMS_MID_CAP")) : MID_CAP;   // 0: A/B without the mid path
     if (K > std::min(SMALL_CAP, single_cross) && K <= mid_cap)
@@ -2202,7 +1719,7 @@ int nms_device(fd_ctx *ctx, const float *dets_dev, int K, int stride, float thr,
         FD_CUDA(cudaMemcpyAsync(num_keep_dev + 1, status, sizeof(int), cudaMemcpyDeviceToDevice, ctx->stream));
         return FD_OK;
     }
-    return nms_big_device(ctx, dets_dev, K, stride, thr, mode, presorted, keep_dev, num_keep_dev);   // writes {count, NaN flag}
+    return nms_big_one_launch(ctx, nullptr, dets_dev, K, stride, K, thr, mode, presorted, keep_dev, num_keep_dev, num_keep_dev + 1);
 }
 
 // argsort_descending on the device: order_dev (n), flag_dev (1 int: NaN flag)
@@ -2223,8 +1740,23 @@ int argsort_device(fd_ctx *ctx, const float *scores_as_dets, int n, int stride, 
         FD_CUDA(cudaMemcpyAsync(flag_dev, status, sizeof(int), cudaMemcpyDeviceToDevice, ctx->stream));
         return FD_OK;
     }
-    static const int bytes[4] = {4, 5, 6, 7};
-    return nms_big_impl(ctx, nullptr, bytes, 4, scores_as_dets, n, stride, 0.f, 0, false, true, order_dev, flag_dev);
+    const int ntiles = (n + NT - 1) / NT;
+    FD_TRY(ctx->nms_ws[0].reserve(sizeof(u64) * (size_t)n));
+    FD_TRY(ctx->nms_ws[1].reserve(sizeof(u64) * (size_t)n));
+    FD_TRY(ctx->nms_ws[2].reserve(sizeof(int) * ((size_t)2 * CS_D * ntiles + CS_D)));
+    u64 *keys = ctx->nms_ws[0].as<u64>(), *tmp = ctx->nms_ws[1].as<u64>();
+    int *hist = ctx->nms_ws[2].as<int>();
+    static int per_sm = 0;                                                 // one device type per process
+    if (!per_sm) {
+        FD_CUDA(cudaFuncSetAttribute(argsort_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CS_SMEM));
+        FD_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, argsort_kernel, NT, CS_SMEM));
+        if (per_sm < 1) return fail(FD_ERR_CUDA, "argsort_kernel does not fit on an SM");
+    }
+    const int grid = std::min(ctx->num_sms * per_sm, ntiles);             // every CTA owns at least one tile
+    void *args[] = {(void *)&scores_as_dets, &n, &stride, &keys, &tmp, &hist, &status, &order_dev, &flag_dev};
+    FD_CUDA(cudaLaunchCooperativeKernel((const void *)argsort_kernel, dim3(grid), dim3(NT), args, CS_SMEM, ctx->stream));
+    FD_LAUNCH_CHECK_NAMED(ctx, "argsort_kernel");
+    return FD_OK;
 }
 
 // Batched: one CTA per image over the decode kernel's candidate buffers.
@@ -2269,18 +1801,12 @@ int nms_batch_small_image(fd_ctx *ctx, int b, int K, float iou_thr) {
     return launch_small<0>(ctx, a, 1, true);
 }
 
-// Big-path fix-up for one image of the batch (K > SMALL_CAP): radix sort on (anchor id, score) bytes + peel.
+// Big path for one image of the batch (K > SMALL_CAP): nms_big_kernel on the decode kernel's keys, which are in slot (compaction)
+// order and carry anchor ids up to the total anchor count; boxes are float4 by anchor id.
 int nms_batch_big_image(fd_ctx *ctx, int b, int K, float iou_thr) {
     const int TA = ctx->dcfg.total_anchors;
-    int bytes[8], nb = 0;
-    bytes[nb++] = 0;
-    bytes[nb++] = 1;
-    if (TA > 65536) bytes[nb++] = 2;
-    if (TA > (1 << 24)) bytes[nb++] = 3;
-    for (int k = 4; k < 8; ++k) bytes[nb++] = k;
-    return nms_big_impl(ctx, ctx->cand_keys.as<u64>() + (size_t)b * TA, bytes, nb, ctx->cand_box.as<float>() + (size_t)b * TA * 4,
-                        K, 4, iou_thr, 0, false, false, ctx->keep_src.as<int>() + (size_t)b * TA,
-                        ctx->keep_count.as<int>() + b);
+    return nms_big_one_launch(ctx, ctx->cand_keys.as<u64>() + (size_t)b * TA, ctx->cand_box.as<float>() + (size_t)b * TA * 4, K, 4, TA,
+                              iou_thr, 0, false, ctx->keep_src.as<int>() + (size_t)b * TA, ctx->keep_count.as<int>() + b, nullptr);
 }
 
 }  // namespace fd

@@ -1,5 +1,5 @@
 // fd_nms_small.cuh — the general single-CTA NMS (K <= 4096: bitonic sort + peel over a 64-bit earlier-overlap mask) as
-// device code, shared by nms_cta_kernel / nms_peel_kernel (fd_nms.cu) and the fused detect kernel (fd_detect_fused.cu).
+// device code, shared by nms_cta_kernel / nms_big_kernel's peel (fd_nms.cu) and the fused detect kernel (fd_detect_fused.cu).
 #pragma once
 #include "fd_internal.cuh"
 #include "fd_nms_tiny.cuh"

@@ -223,6 +223,22 @@ def _zero_area_batch(seed=7):
     return heads, None
 
 
+@functools.lru_cache(maxsize=None)
+def _big_fallback_batch(seed=8, zero_width=False):
+    """image 0: K = 4097 candidates with one tied score (groups of 4, as in the sweep), so the anchor id decides every order;
+    with zero_width every other group has zero-width boxes.  image 1: 20 faces"""
+    rng = np.random.default_rng(seed)
+    heads = _blank(2, 0.1)
+    K, g = 4097, 4
+    n = -(-K // g)
+    grp = _groups(rng, n, g)
+    grp[-1] = grp[-1][:K - g * (n - 1)]
+    boxes = [(0.0, 4.0) if zero_width and i % 2 == 0 else (4.0, 4.0) for i, members in enumerate(grp) for _ in members]
+    assert _plant(heads, 0, rng, grp, "tied", "tmpl", boxes) == K
+    _plant(heads, 1, rng, _groups(rng, 20, 1, rows=44), "distinct")
+    return heads, n
+
+
 # ---------------------------------------------------------------- running a step
 @functools.lru_cache(maxsize=None)
 def _frames_host(B):
@@ -299,6 +315,12 @@ def _run_empty(c):
     return heads, meta, dict(empty=_aligned_steps(c, warm, heads, sum(m["kept"] for m in meta)))
 
 
+def _run_big_fallback(c):
+    tied, _ = _big_fallback_batch()
+    zero_width, _ = _big_fallback_batch(zero_width=True)
+    return dict(negative_iou=_step(c, tied, 1.0, iou=-1.0), zero_width=_step(c, zero_width, 1.0))
+
+
 def _run_edges(c):
     th, _ = _threshold_batch()
     sz, _ = _signed_zero_batch()
@@ -306,7 +328,7 @@ def _run_edges(c):
     return dict(threshold=_step(c, th, 1.0), signed_zero=_step(c, sz, 1.0, conf=0.0), zero_area=_step(c, za, 1.0))
 
 
-SCENARIOS = dict(sweep=_run_sweep, kept=_run_kept, crowded_kept=_run_crowded_kept, empty=_run_empty)
+SCENARIOS = dict(sweep=_run_sweep, kept=_run_kept, crowded_kept=_run_crowded_kept, empty=_run_empty, big_fallback=_run_big_fallback)
 ARRAYS = ("counts", "det", "lmk", "crops", "modes")
 
 
@@ -442,6 +464,20 @@ def test_zero_area_boxes_take_the_exact_nms(oracle):
     for b, (K, n) in enumerate(got):
         assert K == 100 and n == 31 and area0[off:off + n].sum() == 1, (b, K, n)   # one zero-area box of 60 groups survives
         off += n
+
+
+def test_deferred_image_through_the_big_fallback_with_ties(oracle):
+    """A deferred image with K = 4097 tied candidates runs nms_big_kernel on the decode kernel's keys (slot order, anchor ids
+    up to the total anchor count).  A negative IoU threshold and zero-width boxes each make its grid decline, so it sorts those
+    keys by anchor id, then score, and runs the peel: the anchor id decides which member of a group is kept, and which one
+    zero-width box survives (IoU 0 / 0 suppresses every later one).  The other image's count must stay its own."""
+    outs = _both_builds(_run_big_fallback)
+    n_groups = _big_fallback_batch()[1]
+    neg, zw = outs["negative_iou"], outs["zero_width"]
+    for o in (neg, zw):
+        assert o["stats"]["deferred_images"] == 1 and o["stats"]["max_candidates"] == 4097
+    _check(oracle, _big_fallback_batch()[0], [dict(K=4097, kept=1), dict(K=20, kept=1)], neg, 1.0, iou=-1.0)
+    _check(oracle, _big_fallback_batch(zero_width=True)[0], [dict(K=4097, kept=n_groups // 2 + 1), dict(K=20, kept=20)], zw, 1.0)
 
 
 def test_pipelined_shared_contexts_match_serial(oracle):

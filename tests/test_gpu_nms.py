@@ -153,11 +153,22 @@ def test_nms_sorted_contract(ctx, oracle, n):
     np.testing.assert_array_equal(ctx.nms_sorted(np.ascontiguousarray(srt[:, :4]), 0.4), oracle.nms_sorted(srt, 0.4))
 
 
-@pytest.mark.parametrize("n", [1, 77, 4096, 4097, 100000])
-def test_argsort_descending(ctx, oracle, n):
+@pytest.mark.parametrize("n,kind", [pytest.param(n, "quantised", id=str(n)) for n in (1, 77, 4096, 4097, 100000)]
+                         + [pytest.param(n, k, id="%d-%s" % (n, k)) for n, k in ((4097, "nan"), (100000, "nan"), (100000, "equal"))])
+def test_argsort_descending(ctx, oracle, n, kind):
+    """Above 4 096 scores argsort_kernel sorts over the differing score bits: none when every score is equal."""
+    from rs_face_detection_b200 import FdError, ffi
     rng = np.random.default_rng(n)
     s = (np.round(rng.uniform(0, 1, n) * 1000) / 1000).astype(np.float32)
     s[::17] = -s[::17]
+    if kind == "equal":
+        s[:] = np.float32(0.375)
+    if kind == "nan":
+        s[n // 3] = np.nan
+        with pytest.raises(FdError) as e:
+            ctx.argsort_descending(s)
+        assert e.value.code == ffi.FD_ERR_NAN_SCORE
+        return
     np.testing.assert_array_equal(ctx.argsort_descending(s), oracle.argsort_descending(s))
 
 
@@ -230,7 +241,7 @@ def test_single_cta_and_spatial_paths_behind_the_switches():
 def test_one_launch_big_path_behind_the_switch():
     """FD_NMS_MID_CAP=0 sends every problem above 1 024 boxes through nms_big_kernel (the spatial path as one cooperative launch):
     its sort (0-4 digit passes, several tiles per CTA), the peel fallback for irregular boxes / one-cell grids, the `_nms`
-    (presorted) contract, cpu_nms's comparison, the NaN flag — and the same keep lists as the multi-kernel launch sequence."""
+    (presorted) contract, cpu_nms's comparison, the NaN flag."""
     import subprocess, sys
     code = ("import sys; sys.path.insert(0, %r); sys.path.insert(0, %r); import numpy as np\n"
             "from rs_face_detection_b200 import Context, FdError\n"
@@ -265,7 +276,5 @@ def test_one_launch_big_path_behind_the_switch():
             "d = _random_dets(9000, 2)\n"
             "np.testing.assert_array_equal(c.nms(d, 0.4), O.nms(d, 0.4))\n"          # the flag of the failed call does not stick
             "print('ok')\n" % (ROOT, os.path.join(ROOT, "tests")))
-    for extra in ({}, {"FD_NMS_MULTI_KERNEL": "1"}):
-        out = subprocess.run([sys.executable, "-c", code], env=dict(os.environ, FD_NMS_MID_CAP="0", **extra), capture_output=True, text=True,
-                             timeout=900)
-        assert out.returncode == 0 and "ok" in out.stdout, (extra, out.stderr[-1500:])
+    out = subprocess.run([sys.executable, "-c", code], env=dict(os.environ, FD_NMS_MID_CAP="0"), capture_output=True, text=True, timeout=900)
+    assert out.returncode == 0 and "ok" in out.stdout, out.stderr[-1500:]

@@ -58,6 +58,7 @@ def _preprocess_both(torch, ctx, fr):
     B = len(fr.sizes)
     ta = torch.empty((B, 3, 640, 640), dtype=torch.float32, device="cuda")
     tb = torch.full((B, 3, 640, 640), float("nan"), dtype=torch.float32, device="cuda")
+    torch.cuda.synchronize()   # torch fills on its own stream, which the ctx's stream does not wait for
     dsa = ctx.preprocess_batch(fr.bgr, ta)
     dsb = ctx.preprocess_batch_nv12(fr.nv, tb)
     ctx.synchronize()
@@ -107,6 +108,7 @@ def _detect_align_both(torch, ctx, fr, heads_np, cap=512):
         crops = torch.full((cap, 112, 112, 3), 77, dtype=torch.uint8, device="cuda")
         M = torch.zeros((cap, 6), dtype=torch.float64, device="cuda")
         ok = torch.full((cap,), 9, dtype=torch.uint8, device="cuda")
+        torch.cuda.synchronize()   # torch fills on its own stream, which the ctx's stream does not wait for
         if nv:
             ctx.align_detections_nv12(fr.nv, crops, cap, M, ok)
         else:
@@ -190,6 +192,7 @@ def test_align_batch_caller_faces(torch, oracle, crop, aligned):
                     crops = torch.full((F, crop[1], crop[0], 3), 77, dtype=torch.uint8, device="cuda")
                     M = torch.zeros((F, 6), dtype=torch.float64, device="cuda")
                     ok = torch.full((F,), 9, dtype=torch.uint8, device="cuda")
+                    torch.cuda.synchronize()   # torch fills on its own stream, which the ctx's stream does not wait for
                     fn = c.align_batch_nv12 if nv else c.align_batch
                     fn(fr.nv if nv else fr.bgr, lmk_t, fidx_t, F, crops, M, ok, box_t if with_box else None)
                     c.synchronize()
@@ -222,6 +225,7 @@ def test_select_and_align_selected(torch, ctx, enroll):
         crops = torch.full((B, 112, 112, 3), 77, dtype=torch.uint8, device="cuda")
         M = torch.zeros((B, 6), dtype=torch.float64, device="cuda")
         ok = torch.full((B,), 9, dtype=torch.uint8, device="cuda")
+        torch.cuda.synchronize()   # torch fills on its own stream, which the ctx's stream does not wait for
         (ctx.align_selected_nv12 if nv else ctx.align_selected)(fr.nv if nv else fr.bgr, crops, M, ok)
         ctx.synchronize()
         res.append((sel, crops.cpu().numpy(), M.cpu().numpy(), ok.cpu().numpy()))
@@ -253,6 +257,7 @@ def test_deferred_image_replays_the_nv12_warp(torch):
             cap = 2048
             crops = torch.full((cap, 112, 112, 3), 77, dtype=torch.uint8, device="cuda")
             ok = torch.full((cap,), 9, dtype=torch.uint8, device="cuda")
+            torch.cuda.synchronize()   # torch fills on its own stream, which the ctx's stream does not wait for
             (c.align_detections_nv12 if nv else c.align_detections)(fr.nv if nv else fr.bgr, crops, cap, None, ok)
             assert c.detect_last_stats()["deferred_images"] == 1
             counts, det, _ = c.detect_fetch(2)
@@ -269,6 +274,7 @@ def test_deferred_image_replays_the_nv12_warp(torch):
 def test_bad_descriptors_are_rejected(torch, ctx):
     from rs_face_detection_b200 import FdError, ffi
     buf = torch.zeros(1 << 16, dtype=torch.uint8, device="cuda")
+    torch.cuda.synchronize()   # torch fills on its own stream, which the ctx's stream does not wait for
     p = buf.data_ptr()
     out = torch.empty((1, 3, 640, 640), device="cuda")
     bad = [(p, p + 4096, 11, 16, 16, 16), (p, p + 4096, 12, 15, 16, 16), (p, p + 4096, 12, 16, 15, 16), (p, p + 4096, 12, 16, 16, 15),

@@ -31,6 +31,7 @@ class Batch:
         self.heads_c = ctx.head_table(self.heads_t)
         self.tensor = torch.empty((B, 3, 640, 640), dtype=torch.float32, device="cuda")
         self.crops = torch.zeros((cap, 112, 112, 3), dtype=torch.uint8, device="cuda")
+        torch.cuda.synchronize()   # torch fills on its own stream, which the ctx's stream does not wait for
         self.cap = cap
 
     def preprocess(self):

@@ -68,6 +68,7 @@ def _preprocess_both(torch, ctx, fr):
     B = len(fr.sizes)
     ta = torch.empty((B, 3, 640, 640), dtype=torch.float32, device="cuda")
     tb = torch.full((B, 3, 640, 640), float("nan"), dtype=torch.float32, device="cuda")
+    torch.cuda.synchronize()   # torch fills on its own stream, which the ctx's stream does not wait for
     dsa = ctx.preprocess_batch(fr.bgr, ta)
     dsb = ctx.preprocess_batch_yuv420(fr.yuv, fr.layout, tb)
     ctx.synchronize()
@@ -112,6 +113,7 @@ def _align_detections_both(torch, ctx, fr, cap=512):
         crops = torch.full((cap, 112, 112, 3), 77, dtype=torch.uint8, device="cuda")
         M = torch.zeros((cap, 6), dtype=torch.float64, device="cuda")
         ok = torch.full((cap,), 9, dtype=torch.uint8, device="cuda")
+        torch.cuda.synchronize()   # torch fills on its own stream, which the ctx's stream does not wait for
         if yuv:
             ctx.align_detections_yuv420(fr.yuv, fr.layout, crops, cap, M, ok)
         else:
@@ -201,6 +203,7 @@ def test_align_batch_caller_faces(torch, oracle, crop, layout, mode):
                     crops = torch.full((F, crop[1], crop[0], 3), 77, dtype=torch.uint8, device="cuda")
                     M = torch.zeros((F, 6), dtype=torch.float64, device="cuda")
                     ok = torch.full((F,), 9, dtype=torch.uint8, device="cuda")
+                    torch.cuda.synchronize()   # torch fills on its own stream, which the ctx's stream does not wait for
                     bb = box_t if with_box else None
                     if yuv:
                         c.align_batch_yuv420(fr.yuv, layout, lmk_t, fidx_t, F, crops, M, ok, bb)
@@ -238,6 +241,7 @@ def test_select_and_align_selected(torch, ctx, oracle, layout, mode):
         crops = torch.full((B, 112, 112, 3), 77, dtype=torch.uint8, device="cuda")
         M = torch.zeros((B, 6), dtype=torch.float64, device="cuda")
         ok = torch.full((B,), 9, dtype=torch.uint8, device="cuda")
+        torch.cuda.synchronize()   # torch fills on its own stream, which the ctx's stream does not wait for
         if yuv:
             ctx.align_selected_yuv420(fr.yuv, layout, crops, M, ok)
         else:
@@ -288,6 +292,7 @@ def test_deferred_image_replays_the_warp_in_the_recorded_layout(torch):
                 cap = 2048
                 crops = torch.full((cap, 112, 112, 3), 77, dtype=torch.uint8, device="cuda")
                 ok = torch.full((cap,), 9, dtype=torch.uint8, device="cuda")
+                torch.cuda.synchronize()   # torch fills on its own stream, which the ctx's stream does not wait for
                 if yuv:
                     c.align_detections_yuv420(fr.yuv, layout, crops, cap, None, ok)
                 else:
@@ -317,6 +322,7 @@ def test_same_buffers_as_nv12_then_nv21_back_to_back(torch, ctx):
         out = torch.empty((B, 3, 640, 640), device="cuda")
         crops = torch.full((cap, 112, 112, 3), 77, dtype=torch.uint8, device="cuda")
         ok = torch.full((cap,), 9, dtype=torch.uint8, device="cuda")
+        torch.cuda.synchronize()   # torch fills on its own stream, which the ctx's stream does not wait for
         ds = ctx.preprocess_batch_yuv420(frames, layout, out) if call_yuv else ctx.preprocess_batch(frames, out)
         ctx.detect_batch(ctx.head_table(heads_t), B, ds, CONF, IOU)
         if call_yuv:
@@ -373,6 +379,7 @@ def test_layout_nv12_equals_the_nv12_calls(torch, ctx):
         crops = [torch.full((256, 112, 112, 3), 77, dtype=torch.uint8, device="cuda") for _ in range(3)]
         M = [torch.zeros((256, 6), dtype=torch.float64, device="cuda") for _ in range(3)]
         ok = [torch.full((256,), 9, dtype=torch.uint8, device="cuda") for _ in range(3)]
+        torch.cuda.synchronize()   # torch fills on its own stream, which the ctx's stream does not wait for
         if yuv:
             ctx.align_detections_yuv420(fr.yuv, NV12, crops[0], 256, M[0], ok[0])
             ctx.align_batch_yuv420(fr.yuv, NV12, lmk, fidx, 8, crops[1], M[1], ok[1])
@@ -414,6 +421,7 @@ def test_write_before_preprocess_is_seen(torch, ctx, oracle, layout):
 def test_bad_descriptors_are_rejected(torch, ctx):
     from rs_face_detection_b200 import FdError, ffi
     buf = torch.zeros(1 << 16, dtype=torch.uint8, device="cuda")
+    torch.cuda.synchronize()   # torch fills on its own stream, which the ctx's stream does not wait for
     p = buf.data_ptr()
     out = torch.empty((1, 3, 640, 640), device="cuda")
     u = p + 4096
