@@ -12,7 +12,10 @@
  * qualities 30..100) and on the committed golden vectors tests/golden/jpeg_golden.npz.
  *
  * Scope: baseline / extended-sequential 8-bit Huffman JPEG (SOF0 / SOF1), one interleaved scan, 3 components with luma
- * sampling 1x1, 2x1 or 2x2 and 1x1 chroma (4:4:4, 4:2:2, 4:2:0).  Anything else returns an error code.
+ * sampling 1x1, 2x1 or 2x2 and 1x1 chroma (4:4:4, 4:2:2, 4:2:0), YCbCr or RGB as libjpeg's default_decompress_parms
+ * decides it (JFIF APP0, else the Adobe APP14 transform, else component ids 'R' 'G' 'B'); an RGB stream is upsampled the same
+ * way and written as (comp 2, comp 1, comp 0).  4:1:1, 4:4:0, non-interleaved, progressive, arithmetic, 12-bit, grayscale and
+ * CMYK streams return an error code.
  */
 #include <stdint.h>
 #include <stdlib.h>
@@ -35,6 +38,8 @@ typedef struct {
 typedef struct {
     int h, w, ncomp, restart;
     int id[3], hs[3], vs[3], tq[3], td[3], ta[3];
+    int jfif, adobe, adobe_transform;   /* JFIF APP0 seen, Adobe APP14 seen and its transform byte */
+    int rgb;                            /* the components are R, G, B (no colour conversion) */
     uint16_t qt[4][64];   /* natural (row-major) order */
     int qt_present[4];
     huff_t dc[4], ac[4];
@@ -120,6 +125,10 @@ static int parse(const uint8_t *p, size_t n, jpeg_t *j) {
             have_sof = 1;
         } else if (m >= 0xC2 && m <= 0xCF && m != 0xC4 && m != 0xC8 && m != 0xCC) {
             return FDJ_ERR_UNSUPPORTED;             /* progressive, lossless, arithmetic, hierarchical */
+        } else if (m == 0xE0) {                     /* APP0: JFIF (jdmarker.c examine_app0: >= 14 bytes, "JFIF\0") */
+            if (sl >= 14 && !memcmp(s, "JFIF", 5)) j->jfif = 1;
+        } else if (m == 0xEE) {                     /* APP14: Adobe (examine_app14: >= 12 bytes, "Adobe"), byte 11 = transform */
+            if (sl >= 12 && !memcmp(s, "Adobe", 5)) { j->adobe = 1; j->adobe_transform = s[11]; }
         } else if (m == 0xDD) {                     /* DRI */
             if (sl < 2) return FDJ_ERR_SYNTAX;
             j->restart = (s[0] << 8) | s[1];
@@ -133,6 +142,11 @@ static int parse(const uint8_t *p, size_t n, jpeg_t *j) {
                     return FDJ_ERR_SYNTAX;
             }
             if (s[7] != 0 || s[8] != 63) return FDJ_ERR_UNSUPPORTED;
+            /* jdapimin.c default_decompress_parms, 3 components: JFIF means YCbCr; else an Adobe transform of 0 means RGB (any
+             * other transform YCbCr); else component ids 'R' 'G' 'B' mean RGB, any others YCbCr */
+            if (j->jfif) j->rgb = 0;
+            else if (j->adobe) j->rgb = j->adobe_transform == 0;
+            else j->rgb = j->id[0] == 'R' && j->id[1] == 'G' && j->id[2] == 'B';
             j->scan = p + i + len;
             j->scan_len = n - (i + len);
             return FDJ_OK;
@@ -362,7 +376,8 @@ FDO_API int fdo_jpeg_decode_bgr(const uint8_t *jpeg, size_t n, uint8_t *out, int
                         idct_islow(coef, j.qt[j.tq[c]], plane[c] + (size_t)by * 8 * pw[c] + (size_t)bx * 8, pw[c]);
                     }
         }
-    /* jdcolor.c build_ycc_rgb_table + ycc_rgb_convert (JCS_EXT_BGR ordering) */
+    /* jdcolor.c build_ycc_rgb_table + ycc_rgb_convert (JCS_EXT_BGR ordering); an RGB stream takes rgb_rgb_convert: the
+     * upsampled components are only reordered */
     const int dw = (j.w * 1 + H - 1) / H, dh = (j.h * 1 + V - 1) / V;   /* downsampled_width / _height of the chroma components */
     for (int y = 0; y < j.h; ++y) {
         uint8_t *o = out + (size_t)y * pitch;
@@ -370,6 +385,12 @@ FDO_API int fdo_jpeg_decode_bgr(const uint8_t *jpeg, size_t n, uint8_t *out, int
             const int Y = plane[0][(size_t)y * pw[0] + x];
             const int cb = chroma_at(plane[1], pw[1], dw, dh, H, V, x, y) - 128;
             const int cr = chroma_at(plane[2], pw[2], dw, dh, H, V, x, y) - 128;
+            if (j.rgb) {
+                o[3 * x] = (uint8_t)(cr + 128);
+                o[3 * x + 1] = (uint8_t)(cb + 128);
+                o[3 * x + 2] = (uint8_t)Y;
+                continue;
+            }
             const int r = Y + (int)((91881 * cr + 32768) >> 16);                         /* FIX(1.40200) */
             const int g = Y + (int)(((-22554) * cb + 32768 + (-46802) * cr) >> 16);      /* -FIX(0.34414), -FIX(0.71414) */
             const int bl = Y + (int)((116130 * cb + 32768) >> 16);                       /* FIX(1.77200) */

@@ -20,11 +20,13 @@
 //          range-limit table with its wrap-around), 8 threads per block;
 //          `jpeg_color_kernel`: chroma upsampling (jdsample.c h2v1 / h2v2 "fancy" triangle filters with jdmainct.c's replicated
 //          context rows; plain replication when downsampled_width <= 2, as jinit_upsampler selects) + YCbCr -> BGR with
-//          jdcolor.c's 16-bit fixed-point constants, 8 pixels per thread sharing the filter's column sums.
+//          jdcolor.c's 16-bit fixed-point constants, 8 pixels per thread sharing the filter's column sums.  A stream whose
+//          components are R, G, B (see JpegHeader::rgb) is upsampled the same way and only reordered (jdcolor.c rgb_rgb_convert).
 // Every integer operation follows libjpeg-turbo's decompressor with the defaults OpenCV leaves in place (JDCT_ISLOW,
 // do_fancy_upsampling), so the frames are bit-identical to cv2.imdecode (tests/test_gpu_jpeg.py, golden vectors from cv2 4.13).
-// Scope: SOF0 / SOF1 8-bit, one interleaved 3-component scan, 4:4:4 / 4:2:2 / 4:2:0, DRI/RSTn.  Progressive, arithmetic,
-// grayscale, CMYK streams return FD_ERR_INVALID (the reference would hand them to OpenCV).
+// Scope: SOF0 / SOF1 8-bit, one interleaved 3-component scan, 4:4:4 / 4:2:2 / 4:2:0, DRI/RSTn, YCbCr or RGB components (as
+// libjpeg decides: JFIF APP0, else the Adobe APP14 transform, else component ids 'R' 'G' 'B').  4:1:1, 4:4:0, non-interleaved,
+// progressive, arithmetic, 12-bit, grayscale and CMYK streams return FD_ERR_INVALID (the reference would hand them to OpenCV).
 #include <algorithm>
 #include <atomic>
 #include <chrono>
@@ -83,6 +85,9 @@ struct JpegHuffDev {
 struct JpegHeader {
     int h = 0, w = 0, restart = 0;
     int id[3], hs[3], vs[3], tq[3], td[3], ta[3];
+    bool jfif = false, adobe = false;   // a JFIF APP0 / an Adobe APP14 was seen (jdmarker.c examine_app0 / examine_app14)
+    int adobe_transform = 0;
+    bool rgb = false;                   // the components are R, G, B: no colour conversion (jdapimin.c default_decompress_parms)
     uint16_t qt[4][64];
     bool qt_present[4] = {false, false, false, false};
     HuffTable dc[4], ac[4];
@@ -161,6 +166,12 @@ static const char *parse_jpeg(const uint8_t *p, size_t n, JpegHeader *j) {
                 have_sof = true;
                 break;
             }
+            case 0xE0:   // JFIF: payload >= 14 bytes starting "JFIF\0"
+                if (sl >= 14 && !memcmp(s, "JFIF", 5)) j->jfif = true;
+                break;
+            case 0xEE:   // Adobe: payload >= 12 bytes starting "Adobe"; byte 11 is the colour transform
+                if (sl >= 12 && !memcmp(s, "Adobe", 5)) { j->adobe = true; j->adobe_transform = s[11]; }
+                break;
             case 0xDD:
                 if (sl < 2) return "bad DRI";
                 j->restart = (s[0] << 8) | s[1];
@@ -176,6 +187,11 @@ static const char *parse_jpeg(const uint8_t *p, size_t n, JpegHeader *j) {
                         return "scan refers to a missing table";
                 }
                 if (s[7] != 0 || s[8] != 63) return "unsupported spectral selection";
+                // default_decompress_parms, 3 components: JFIF means YCbCr; else Adobe transform 0 means RGB (1 and any other
+                // value YCbCr); else component ids 'R' 'G' 'B' mean RGB, any others YCbCr
+                if (j->jfif) j->rgb = false;
+                else if (j->adobe) j->rgb = j->adobe_transform == 0;
+                else j->rgb = j->id[0] == 'R' && j->id[1] == 'G' && j->id[2] == 'B';
                 j->scan = p + i + len;
                 j->scan_len = n - (i + len);
                 const int H = j->hs[0], V = j->vs[0];
@@ -388,6 +404,7 @@ struct JpegImageDev {
     int nblk[3];               // blocks per component
     int w, h, pitch;           // output geometry
     int H, V;                  // luma sampling factors (chroma is 1x1)
+    int rgb;                   // the components are R, G, B: jpeg_color_kernel reorders them instead of converting
     uint16_t qt[3][64];        // per COMPONENT quantisation table, natural order
 };
 
@@ -1270,14 +1287,25 @@ __device__ __forceinline__ void jpeg_colsums6(const uint8_t *__restrict__ r0, co
     cs[5] = 3 * r0[rgt] + r1[rgt];
 }
 
+// one output pixel, BGR in the low 24 bits, from the luma / first component and the upsampled other two minus 128.  RGB:
+// jdcolor.c rgb_rgb_convert, the components are R, G, B and only change places.
+template <bool RGB>
+__device__ __forceinline__ unsigned jpeg_to_bgr(int Y, int cb, int cr) {
+    if (RGB) return (unsigned)(cr + 128) | ((unsigned)(cb + 128) << 8) | ((unsigned)Y << 16);
+    return jpeg_ycc_to_bgr(Y, cb, cr);
+}
+
 // grid (ceil(w/8 / 128), h rows, B): 8 pixels per thread -> 24 bytes = six aligned 32-bit stores (pitch % 16 == 0).
 // 4:2:0 with downsampled_width > 2 (the common case) shares the triangle filter's column sums between the 8 pixels and reads
-// the planes by words; the other samplings take the per-pixel form (jpeg_chroma_at).
+// the planes by words; the other samplings take the per-pixel form (jpeg_chroma_at).  One build per colour space: each skips
+// the images of the other (the flag is per image, so the exit is uniform over the CTA) and is launched only for batches that
+// hold such an image.
+template <bool RGB>
 __global__ void __launch_bounds__(128) jpeg_color_kernel(const JpegImageDev *__restrict__ imgs) {
     const JpegImageDev &im = imgs[blockIdx.z];
     const int y = blockIdx.y;
     const int x0 = (blockIdx.x * blockDim.x + threadIdx.x) * 8;
-    if (y >= im.h || x0 >= im.w) return;
+    if (y >= im.h || x0 >= im.w || (im.rgb != 0) != RGB) return;
     const int H = im.H, V = im.V;
     const int dw = (im.w + H - 1) / H, dh = (im.h + V - 1) / V;
     unsigned px[8];
@@ -1298,7 +1326,7 @@ __global__ void __launch_bounds__(128) jpeg_color_kernel(const JpegImageDev *__r
             const int vb = edge ? (cb[t] * 4 + rnd) >> 4 : (cb[t] * 3 + cb[o] + rnd) >> 4;
             const int vr = edge ? (cr[t] * 4 + rnd) >> 4 : (cr[t] * 3 + cr[o] + rnd) >> 4;
             const int Y = (int)(((j < 4 ? yy.x : yy.y) >> (8 * (j & 3))) & 0xFF);
-            px[j] = jpeg_ycc_to_bgr(Y, vb - 128, vr - 128);
+            px[j] = jpeg_to_bgr<RGB>(Y, vb - 128, vr - 128);
         }
     } else {
 #pragma unroll
@@ -1306,7 +1334,7 @@ __global__ void __launch_bounds__(128) jpeg_color_kernel(const JpegImageDev *__r
             const int x = min(x0 + j, im.w - 1);
             const int cb = jpeg_chroma_at(im.plane[1], im.pw[1], dw, dh, H, V, x, y) - 128;
             const int cr = jpeg_chroma_at(im.plane[2], im.pw[2], dw, dh, H, V, x, y) - 128;
-            px[j] = jpeg_ycc_to_bgr(yrow[x], cb, cr);
+            px[j] = jpeg_to_bgr<RGB>(yrow[x], cb, cr);
         }
     }
     uint8_t *row = im.bgr + (size_t)y * im.pitch;
@@ -1408,7 +1436,7 @@ FD_EXPORT int fd_decode_jpeg_batch(fd_ctx *ctx, const uint8_t *const *jpegs, con
     // layout: coefficient arena (device; pinned mirror for host-decoded images), plane arena, frame arena, stream / aux arenas
     std::vector<size_t> coef_off(B), plane_off(B), frame_off(B), stream_off(B), aux_off(B), raw_off(B), sync_off(B);
     size_t coef_total = 0, plane_total = 0, frame_total = 0, stream_total = 0, aux_total = 0, host_coef_total = 0, raw_total = 0, sync_total = 0;
-    int max_blocks = 0, max_h = 0, max_w = 0, max_iv = 0, max_sub = 0, max_chunks = 0, n_rst = 0, n_sync = 0, n_rstsync = 0, n_scan = 0;
+    int max_blocks = 0, max_h = 0, max_w = 0, max_iv = 0, max_sub = 0, max_chunks = 0, n_rst = 0, n_sync = 0, n_rstsync = 0, n_scan = 0, n_rgb = 0;
     for (int i = 0; i < B; ++i) {
         const JpegHeader &j = hdr[i];
         const size_t nblk = j.blocks[0] + j.blocks[1] + j.blocks[2];
@@ -1422,6 +1450,7 @@ FD_EXPORT int fd_decode_jpeg_batch(fd_ctx *ctx, const uint8_t *const *jpegs, con
         max_blocks = std::max<int>(max_blocks, (int)nblk);
         max_h = std::max(max_h, j.h);
         max_w = std::max(max_w, j.w);
+        n_rgb += j.rgb ? 1 : 0;
         if (mode[i] == 1) {
             ++n_rst;
             stream_off[i] = stream_total;
@@ -1539,6 +1568,7 @@ FD_EXPORT int fd_decode_jpeg_batch(fd_ctx *ctx, const uint8_t *const *jpegs, con
         d.bgr = ctx->jpeg_frames.as<uint8_t>() + frame_off[i];
         d.H = j.hs[0];
         d.V = j.vs[0];
+        d.rgb = j.rgb ? 1 : 0;
         d.mcux = j.mcux;
         d.mcuy = j.mcuy;
         d.restart = j.restart;
@@ -1672,8 +1702,14 @@ FD_EXPORT int fd_decode_jpeg_batch(fd_ctx *ctx, const uint8_t *const *jpegs, con
     FD_LAUNCH_CHECK_NAMED(ctx, "jpeg_idct_kernel");
     FD_REQUIRE(max_h <= 65535 && B <= 65535, "fd_decode_jpeg_batch: image too tall / batch too large for one launch");
     dim3 g2(((max_w + 7) / 8 + 127) / 128, max_h, B);
-    jpeg_color_kernel<<<g2, 128, 0, ctx->stream>>>(ddesc);
-    FD_LAUNCH_CHECK_NAMED(ctx, "jpeg_color_kernel");
+    if (n_rgb < B) {
+        jpeg_color_kernel<false><<<g2, 128, 0, ctx->stream>>>(ddesc);
+        FD_LAUNCH_CHECK_NAMED(ctx, "jpeg_color_kernel");
+    }
+    if (n_rgb) {
+        jpeg_color_kernel<true><<<g2, 128, 0, ctx->stream>>>(ddesc);
+        FD_LAUNCH_CHECK_NAMED(ctx, "jpeg_color_kernel");
+    }
     if (dbg)
         fprintf(stderr, "[jpeg dbg] B=%d on-device entropy %d: parse+scan %.2f ms, layout %.2f, wait prev copies %.2f, enqueue copies (+host huffman) %.2f, "
                         "descriptors+launches %.2f, total host %.2f ms\n", B, n_gpu, t_parse - t_begin, t_layout - t_parse, t_wait - t_layout,
