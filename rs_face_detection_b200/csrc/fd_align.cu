@@ -279,23 +279,55 @@ __device__ __forceinline__ void planar_quad_taps(const PlanarQuad &q, unsigned &
     planar_row_taps(__funnelshift_r(q.y1[0], q.y1[1], q.sy_sh), __funnelshift_r(q.u1[0], q.u1[1], q.sc_sh),
                     __funnelshift_r(q.v1[0], q.v1[1], q.sc_sh), q.odd, lo1, hi1);
 }
-// the tap square of a 4:2:0 format (FMT: SRC_NV12, SRC_NV21 or SRC_PLANAR)
-template <int FMT> using YuvQuad = typename std::conditional<FMT == SRC_PLANAR, PlanarQuad, Nv12Quad>::type;
+// The same square of a packed 4:2:2 frame (data and pitch 4-byte aligned): per tap row, the aligned macropixel word of
+// column sx and, when sx is odd, that of column sx+1 (for an even sx both columns share one word).  No byte past the words
+// of the two columns is read.  sel reorders a word to Y0 U Y1 V.
+struct PackedQuad {
+    unsigned r0[2], r1[2];   // words of columns sx, sx+1 in tap rows sy, sy+1
+    unsigned sel;
+    bool odd;
+};
+__device__ __forceinline__ void packed_quad_load(const uint8_t *p, unsigned pitch, unsigned sel, int sx, int sy, PackedQuad &q) {
+    const unsigned o = (unsigned)sy * pitch + 2u * (unsigned)(sx & ~1);
+    const unsigned *w0 = reinterpret_cast<const unsigned *>(p + o), *w1 = reinterpret_cast<const unsigned *>(p + o + pitch);
+    q.odd = (sx & 1) != 0;
+    q.r0[0] = __ldg(w0); q.r1[0] = __ldg(w1);
+    q.r0[1] = q.odd ? __ldg(w0 + 1) : q.r0[0];
+    q.r1[1] = q.odd ? __ldg(w1 + 1) : q.r1[0];
+    q.sel = sel;
+}
+__device__ __forceinline__ void packed_row_taps(unsigned a, unsigned b, unsigned sel, bool odd, unsigned &lo, unsigned &hi) {
+    a = __byte_perm(a, 0u, sel);
+    b = __byte_perm(b, 0u, sel);
+    pack6(packed_bgr24(a, odd ? 1 : 0), packed_bgr24(b, odd ? 0 : 1), lo, hi);
+}
+// the tap square of a YUV format (FMT: SRC_NV12, SRC_NV21, SRC_PLANAR or SRC_PACKED422); sel: packed only
 template <int FMT>
-__device__ __forceinline__ void yuv_quad_load(const uint8_t *yp, unsigned py, const uint8_t *uvp, const uint8_t *vp, unsigned puv, int sx, int sy,
-                                              YuvQuad<FMT> &q) {
+using YuvQuad = typename std::conditional<FMT == SRC_PLANAR, PlanarQuad, typename std::conditional<FMT == SRC_PACKED422, PackedQuad, Nv12Quad>::type>::type;
+template <int FMT>
+__device__ __forceinline__ void yuv_quad_load(const uint8_t *yp, unsigned py, const uint8_t *uvp, const uint8_t *vp, unsigned puv, unsigned sel,
+                                              int sx, int sy, YuvQuad<FMT> &q) {
     if constexpr (FMT == SRC_PLANAR) planar_quad_load(yp, py, uvp, vp, puv, sx, sy, q);
+    else if constexpr (FMT == SRC_PACKED422) packed_quad_load(yp, py, sel, sx, sy, q);
     else nv12_quad_load(yp, py, uvp, puv, sx, sy, q);
 }
 template <int FMT>
 __device__ __forceinline__ void yuv_quad_taps(const YuvQuad<FMT> &q, unsigned &lo0, unsigned &hi0, unsigned &lo1, unsigned &hi1) {
-    if constexpr (FMT == SRC_PLANAR) planar_quad_taps(q, lo0, hi0, lo1, hi1);
-    else nv12_quad_taps<FMT>(q, lo0, hi0, lo1, hi1);
+    if constexpr (FMT == SRC_PLANAR) {
+        planar_quad_taps(q, lo0, hi0, lo1, hi1);
+    } else if constexpr (FMT == SRC_PACKED422) {
+        packed_row_taps(q.r0[0], q.r0[1], q.sel, q.odd, lo0, hi0);
+        packed_row_taps(q.r1[0], q.r1[1], q.sel, q.odd, lo1, hi1);
+    } else {
+        nv12_quad_taps<FMT>(q, lo0, hi0, lo1, hi1);
+    }
 }
-// pixel (xx, yy) of a 4:2:0 frame inside it (vp: the V plane, planar only)
+// pixel (xx, yy) of a YUV frame inside it (vp: the V plane, planar only; sel: packed only)
 template <int FMT>
-__device__ __forceinline__ unsigned yuv_tap(const uint8_t *yp, int py, const uint8_t *uvp, const uint8_t *vp, int puv, int xx, int yy) {
-    if constexpr (FMT == SRC_PLANAR)
+__device__ __forceinline__ unsigned yuv_tap(const uint8_t *yp, int py, const uint8_t *uvp, const uint8_t *vp, int puv, unsigned sel, int xx, int yy) {
+    if constexpr (FMT == SRC_PACKED422)
+        return packed_px24(yp + (ptrdiff_t)yy * py, sel, xx);
+    else if constexpr (FMT == SRC_PLANAR)
         return yuv_bgr24(__ldg(yp + (ptrdiff_t)yy * py + xx), __ldg(uvp + (ptrdiff_t)(yy >> 1) * puv + (xx >> 1)),
                          __ldg(vp + (ptrdiff_t)(yy >> 1) * puv + (xx >> 1)));
     else if constexpr (FMT == SRC_NV21)
@@ -305,10 +337,10 @@ __device__ __forceinline__ unsigned yuv_tap(const uint8_t *yp, int py, const uin
         return yuv_bgr24(__ldg(yp + (ptrdiff_t)yy * py + xx), __ldg(uvp + (ptrdiff_t)(yy >> 1) * puv + (xx & ~1)),
                          __ldg(uvp + (ptrdiff_t)(yy >> 1) * puv + (xx | 1)));
 }
-// border_tap_blend for a 4:2:0 frame: BORDER_CONSTANT(0) applies to the BGR image, so a tap outside the frame is BGR (0,0,0)
+// border_tap_blend for a YUV frame: BORDER_CONSTANT(0) applies to the BGR image, so a tap outside the frame is BGR (0,0,0)
 template <int FMT>
-__device__ __forceinline__ unsigned border_tap_blend_yuv(const uint8_t *yp, int py, const uint8_t *uvp, const uint8_t *vp, int puv, int w, int h,
-                                                         int X, int Y) {
+__device__ __forceinline__ unsigned border_tap_blend_yuv(const uint8_t *yp, int py, const uint8_t *uvp, const uint8_t *vp, int puv, unsigned sel,
+                                                         int w, int h, int X, int Y) {
     const int sx = max(-32768, min(32767, X >> 5)), sy = max(-32768, min(32767, Y >> 5));   // saturate_cast<short>
     unsigned p[2][2];
 #pragma unroll
@@ -316,7 +348,7 @@ __device__ __forceinline__ unsigned border_tap_blend_yuv(const uint8_t *yp, int 
 #pragma unroll
         for (int i = 0; i < 2; ++i) {
             const int xx = sx + i, yy = sy + j;
-            p[j][i] = xx >= 0 && xx < w && yy >= 0 && yy < h ? yuv_tap<FMT>(yp, py, uvp, vp, puv, xx, yy) : 0u;
+            p[j][i] = xx >= 0 && xx < w && yy >= 0 && yy < h ? yuv_tap<FMT>(yp, py, uvp, vp, puv, sel, xx, yy) : 0u;
         }
     unsigned lo0, hi0, lo1, hi1;
     pack6(p[0][0], p[0][1], lo0, hi0);
@@ -330,9 +362,13 @@ __device__ __forceinline__ bool nv12_interior_ok(const FrameDev &f) {
     return ((reinterpret_cast<uintptr_t>(f.data) | reinterpret_cast<uintptr_t>(f.uv)) & 3) == 0 && (f.pitch & 3) == 0 && (f.pitch_uv & 3) == 0 &&
            f.pitch >= 8 && f.pitch_uv >= 8 && (size_t)f.h * f.pitch < 0x7fffffffull && (size_t)f.h * f.pitch_uv < 0x7fffffffull;
 }
+// A packed frame's interior reads stay inside the two tap columns' words (W is even, so a macropixel never straddles the
+// end of a row): only the 4-byte alignment and 32-bit offsets are needed.
 template <int FMT>
 __device__ __forceinline__ bool yuv_interior_ok(const FrameDev &f) {
     if constexpr (FMT == SRC_PLANAR) return nv12_interior_ok(f) && (f.v_off & 3) == 0;   // the V plane too
+    else if constexpr (FMT == SRC_PACKED422)
+        return ((reinterpret_cast<uintptr_t>(f.data) | (uintptr_t)f.pitch) & 3) == 0 && (size_t)f.h * f.pitch < 0x7fffffffull;
     else return nv12_interior_ok(f);
 }
 
@@ -359,6 +395,7 @@ struct WarpItem {
     const uint8_t *uv;   // 4:2:0 only
     int pitch_uv;
     const uint8_t *v;    // planar only
+    unsigned sel;        // packed 4:2:2 only
 };
 
 // N rounds of WARP_THREADS consecutive output pixels starting at p0: all 4N aligned 64-bit loads of a thread are issued
@@ -375,7 +412,7 @@ __device__ __forceinline__ void warp_rounds_interior_yuv(const WarpItem &it, con
         const int2 d = dxy[x], r0 = xy0[row];
         const int X = (int)((unsigned)r0.x + (unsigned)d.x) >> 5, Y = (int)((unsigned)r0.y + (unsigned)d.y) >> 5;
         axy[u] = (X & 31) | ((Y & 31) << 8);
-        yuv_quad_load<FMT>(it.data, (unsigned)it.pitch, it.uv, it.v, (unsigned)it.pitch_uv, X >> 5, Y >> 5, q[u]);
+        yuv_quad_load<FMT>(it.data, (unsigned)it.pitch, it.uv, it.v, (unsigned)it.pitch_uv, it.sel, X >> 5, Y >> 5, q[u]);
     }
 #pragma unroll
     for (int u = 0; u < N; ++u) {
@@ -426,7 +463,7 @@ __device__ __forceinline__ void warp_round_border(const WarpItem &it, const int2
     const int row = cw_magic ? (int)__umulhi((unsigned)p, cw_magic) : p, x = p - row * cw;
     const int2 d = dxy[x], r0 = xy0[row];
     const int X = (int)((unsigned)r0.x + (unsigned)d.x) >> 5, Y = (int)((unsigned)r0.y + (unsigned)d.y) >> 5;
-    const unsigned v = FMT != SRC_BGR ? border_tap_blend_yuv<FMT>(it.data, it.pitch, it.uv, it.v, it.pitch_uv, it.w, it.h, X, Y)
+    const unsigned v = FMT != SRC_BGR ? border_tap_blend_yuv<FMT>(it.data, it.pitch, it.uv, it.v, it.pitch_uv, it.sel, it.w, it.h, X, Y)
                                       : border_tap_blend(it.data, it.w, it.h, it.pitch, it.lo_lim, it.hi_lim, X, Y);
     store_px(band_out, p0, v, p0 < npix, packed);
 }
@@ -438,7 +475,7 @@ __device__ __forceinline__ void warp_round_border(const WarpItem &it, const int2
 // FMT: the source format of the frames (SrcFmt)
 template <int FMT>
 __global__ void __launch_bounds__(WARP_THREADS, 4) warp_kernel(WarpArgs a) {
-    constexpr bool NV = FMT != SRC_BGR;
+    constexpr bool NV = FMT == SRC_NV12 || FMT == SRC_NV21 || FMT == SRC_PLANAR, PK = FMT == SRC_PACKED422;   // NV: 4:2:0
     extern __shared__ int2 wsm[];
     int2 *dxy = wsm;             // [cw]  (adelta, bdelta)
     int2 *xy0 = dxy + a.cw;      // [WARP_BAND]  (X0, Y0) per row
@@ -472,6 +509,8 @@ __global__ void __launch_bounds__(WARP_THREADS, 4) warp_kernel(WarpArgs a) {
                     const int row = p / a.cw, x = p - row * a.cw;
                     const unsigned v = NV ? resize_pixel24_yuv<FMT>(fr.data, fr.pitch, fr.uv, fr.v_plane(), fr.pitch_uv, rx0, ry0, fr.w - rx0, fr.h - ry0, a.cw,
                                                                     a.ch, x, band_y0 + row)
+                                       : PK ? resize_pixel24_packed(fr.data, fr.pitch, (unsigned)fr.v_off, rx0, ry0, fr.w - rx0, fr.h - ry0, a.cw, a.ch, x,
+                                                                    band_y0 + row)
                                           : resize_pixel24(roi, fr.pitch, fr.w - rx0, fr.h - ry0, a.cw, a.ch, x, band_y0 + row);
                     band_out[3 * p] = (uint8_t)v; band_out[3 * p + 1] = (uint8_t)(v >> 8); band_out[3 * p + 2] = (uint8_t)(v >> 16);
                 }
@@ -493,10 +532,10 @@ __global__ void __launch_bounds__(WARP_THREADS, 4) warp_kernel(WarpArgs a) {
         __syncthreads();
         // The map is affine, so the tap coordinates of the band are extremal at its 4 corners: if all 4 corner taps
         // (and their +1 neighbours) are interior, no pixel of the band needs a border test.
-        bool interior = NV ? yuv_interior_ok<FMT>(fr)
-                           : (reinterpret_cast<uintptr_t>(fr.data) & 7) == 0 && (fr.pitch & 7) == 0 && fr.pitch >= 16 &&
-                                 (size_t)fr.h * fr.pitch < 0x7fffffffull;
-        const int bottom = NV ? 2 : 1;   // rows kept from the bottom: the loads over-read past the last tap row
+        bool interior = NV || PK ? yuv_interior_ok<FMT>(fr)
+                                 : (reinterpret_cast<uintptr_t>(fr.data) & 7) == 0 && (fr.pitch & 7) == 0 && fr.pitch >= 16 &&
+                                       (size_t)fr.h * fr.pitch < 0x7fffffffull;
+        const int bottom = NV ? 2 : PK ? 0 : 1;   // rows kept from the bottom: the loads over-read past the last tap row
         {
             const int xs[2] = {0, a.cw - 1}, ys[2] = {0, rows - 1};
 #pragma unroll
@@ -514,8 +553,9 @@ __global__ void __launch_bounds__(WARP_THREADS, 4) warp_kernel(WarpArgs a) {
         it.hi_lim = fr.data + (size_t)(fr.h - 1) * fr.pitch + (size_t)fr.w * 3;  // end of valid pixel bytes
         it.uv = fr.uv; it.pitch_uv = fr.pitch_uv;
         if constexpr (FMT == SRC_PLANAR) it.v = fr.v_plane();
+        it.sel = PK ? (unsigned)fr.v_off : 0u;
         int p0 = tid;
-        if (NV && interior) {
+        if ((NV || PK) && interior) {
             for (int rounds = (npix + WARP_THREADS - 1) / WARP_THREADS; rounds > 0; rounds -= 2, p0 += 2 * WARP_THREADS) {
                 if (rounds >= 2) warp_rounds_interior_yuv<FMT, 2>(it, dxy, xy0, a.cw, a.cw_magic, p0, npix, band_out, packed);
                 else warp_rounds_interior_yuv<FMT, 1>(it, dxy, xy0, a.cw, a.cw_magic, p0, npix, band_out, packed);
@@ -588,8 +628,8 @@ __device__ __forceinline__ void fixed_rounds_interior(const uint8_t *__restrict_
 
 template <int CW, int N, int FMT>
 __device__ __forceinline__ void fixed_rounds_interior_yuv(const uint8_t *__restrict__ yp, unsigned py, const uint8_t *__restrict__ uvp,
-                                                          const uint8_t *__restrict__ vp, unsigned puv, int2 d, const int2 *__restrict__ xy,
-                                                          unsigned *__restrict__ outw, bool store, unsigned pack_sel) {
+                                                          const uint8_t *__restrict__ vp, unsigned puv, unsigned sel, int2 d,
+                                                          const int2 *__restrict__ xy, unsigned *__restrict__ outw, bool store, unsigned pack_sel) {
     YuvQuad<FMT> q[N];
     int axy[N];
 #pragma unroll
@@ -597,7 +637,7 @@ __device__ __forceinline__ void fixed_rounds_interior_yuv(const uint8_t *__restr
         const int2 r0 = xy[2 * u];
         const int X = (int)((unsigned)r0.x + (unsigned)d.x) >> 5, Y = (int)((unsigned)r0.y + (unsigned)d.y) >> 5;
         axy[u] = (X & 31) | ((Y & 31) << 14);   // ax | ay << 6 << 8
-        yuv_quad_load<FMT>(yp, py, uvp, vp, puv, X >> 5, Y >> 5, q[u]);
+        yuv_quad_load<FMT>(yp, py, uvp, vp, puv, sel, X >> 5, Y >> 5, q[u]);
     }
 #pragma unroll
     for (int u = 0; u < N; ++u) {
@@ -612,7 +652,7 @@ __device__ __forceinline__ void fixed_rounds_interior_yuv(const uint8_t *__restr
 // FMT: the source format of the frames (SrcFmt)
 template <int CW, int CH, int IR, int UN, int FMT>
 __global__ void __launch_bounds__(2 * CW) warp_fixed_kernel(WarpArgs a) {
-    constexpr bool NV = FMT != SRC_BGR;
+    constexpr bool NV = FMT == SRC_NV12 || FMT == SRC_NV21 || FMT == SRC_PLANAR, PK = FMT == SRC_PACKED422;   // NV: 4:2:0
     constexpr int T = 2 * CW, ITEMS = CH / IR, ROUNDS = IR / 2;
     static_assert(CH % IR == 0 && IR % 2 == 0 && T % 32 == 0 && (2 * CW * 3) % 4 == 0 && (IR * CW * 3) % 4 == 0, "fixed warp geometry");
     __shared__ int2 xy0[2][IR];
@@ -647,6 +687,7 @@ __global__ void __launch_bounds__(2 * CW) warp_fixed_kernel(WarpArgs a) {
         const int pitch_uv = NV ? frp->pitch_uv : 0;
         const uint8_t *vp = nullptr;   // planar only
         if constexpr (FMT == SRC_PLANAR) vp = frp->v_plane();
+        const unsigned sel = PK ? (unsigned)frp->v_off : 0u;
         int2 d = make_int2(0, 0);
         bool vote = true;
         if (okf) {
@@ -663,13 +704,13 @@ __global__ void __launch_bounds__(2 * CW) warp_fixed_kernel(WarpArgs a) {
                     const long long Xl = (long long)(__double2int_rn((i1 * y + i2) * 1024) + 16) + __double2int_rn(i0 * cx * 1024);
                     const long long Yl = (long long)(__double2int_rn((i4 * y + i5) * 1024) + 16) + __double2int_rn(i3 * cx * 1024);
                     const long long sx = Xl >> 10, sy = Yl >> 10;
-                    vote = sx >= 0 && sx + 1 < fw && sy >= 0 && sy + 1 < fh - (NV ? 2 : 1);   // the over-read stays in the frame
+                    vote = sx >= 0 && sx + 1 < fw && sy >= 0 && sy + 1 < fh - (NV ? 2 : PK ? 0 : 1);   // the over-read stays in the frame
                 }
             }
         }
-        const bool interior = __syncthreads_and(vote) && (NV ? yuv_interior_ok<FMT>(*frp)
-                                                                 : (reinterpret_cast<uintptr_t>(data) & 7) == 0 && (pitch & 7) == 0 && pitch >= 16 &&
-                                                                       (size_t)fh * pitch < 0x7fffffffull);
+        const bool interior = __syncthreads_and(vote) && (NV || PK ? yuv_interior_ok<FMT>(*frp)
+                                                                       : (reinterpret_cast<uintptr_t>(data) & 7) == 0 && (pitch & 7) == 0 && pitch >= 16 &&
+                                                                             (size_t)fh * pitch < 0x7fffffffull);
         const bool store = (tid & 3) != 3;
         unsigned *outw = reinterpret_cast<unsigned *>(band_out) + 3 * (tid >> 2) + (tid & 3);
         if (!okf) {   // estimation failed: bbox-crop fallback (face_alignment.rs:64-116), or a zero crop where the reference errs
@@ -680,6 +721,7 @@ __global__ void __launch_bounds__(2 * CW) warp_fixed_kernel(WarpArgs a) {
                 const uint8_t *roi = data + (size_t)ry0 * pitch + (size_t)rx0 * 3;
                 for (int u = 0; u < ROUNDS; ++u) {
                     const unsigned v = NV ? resize_pixel24_yuv<FMT>(data, pitch, uvp, vp, pitch_uv, rx0, ry0, fw - rx0, fh - ry0, CW, CH, x, y0 + r + 2 * u)
+                                       : PK ? resize_pixel24_packed(data, pitch, sel, rx0, ry0, fw - rx0, fh - ry0, CW, CH, x, y0 + r + 2 * u)
                                           : resize_pixel24(roi, pitch, fw - rx0, fh - ry0, CW, CH, x, y0 + r + 2 * u);
                     const unsigned nv = __shfl_down_sync(0xffffffffu, v, 1);
                     const unsigned word = __funnelshift_r(__byte_perm(v, nv, 0x4210), nv >> 8, 8 * (tid & 3u));
@@ -696,13 +738,13 @@ __global__ void __launch_bounds__(2 * CW) warp_fixed_kernel(WarpArgs a) {
             const unsigned pack_sel = (tid & 3) == 0 ? 0x4210u : ((tid & 3) == 1 ? 0x5421u : 0x6542u);
             int u = 0;
             constexpr int REM = ROUNDS % UN;
-            if (NV) {
+            if (NV || PK) {
 #pragma unroll 1
                 for (; u + UN <= ROUNDS; u += UN)
-                    fixed_rounds_interior_yuv<CW, UN, FMT>(data, (unsigned)pitch, uvp, vp, (unsigned)pitch_uv, d, xy + 2 * u, outw + u * (T * 3 / 4),
-                                                           store, pack_sel);
-                if (REM) fixed_rounds_interior_yuv<CW, REM ? REM : 1, FMT>(data, (unsigned)pitch, uvp, vp, (unsigned)pitch_uv, d, xy + 2 * (ROUNDS - REM),
-                                                                           outw + (ROUNDS - REM) * (T * 3 / 4), store, pack_sel);
+                    fixed_rounds_interior_yuv<CW, UN, FMT>(data, (unsigned)pitch, uvp, vp, (unsigned)pitch_uv, sel, d, xy + 2 * u,
+                                                           outw + u * (T * 3 / 4), store, pack_sel);
+                if (REM) fixed_rounds_interior_yuv<CW, REM ? REM : 1, FMT>(data, (unsigned)pitch, uvp, vp, (unsigned)pitch_uv, sel, d,
+                                                                           xy + 2 * (ROUNDS - REM), outw + (ROUNDS - REM) * (T * 3 / 4), store, pack_sel);
             } else {
 #pragma unroll 1
                 for (; u + UN <= ROUNDS; u += UN)
@@ -714,7 +756,7 @@ __global__ void __launch_bounds__(2 * CW) warp_fixed_kernel(WarpArgs a) {
             for (int u = 0; u < ROUNDS; ++u) {
                 const int2 r0 = xy[2 * u];
                 const int X = (int)((unsigned)r0.x + (unsigned)d.x) >> 5, Y = (int)((unsigned)r0.y + (unsigned)d.y) >> 5;
-                const unsigned v = NV ? border_tap_blend_yuv<FMT>(data, pitch, uvp, vp, pitch_uv, fw, fh, X, Y)
+                const unsigned v = NV || PK ? border_tap_blend_yuv<FMT>(data, pitch, uvp, vp, pitch_uv, sel, fw, fh, X, Y)
                                       : border_tap_blend(data, fw, fh, pitch, lo_lim, hi_lim, X, Y);
                 const unsigned nv = __shfl_down_sync(0xffffffffu, v, 1);
                 const unsigned word = __funnelshift_r(__byte_perm(v, nv, 0x4210), nv >> 8, 8 * (tid & 3u));
@@ -805,11 +847,13 @@ template <int IR>
 static void (*fixed_kernel_for(int fmt))(WarpArgs) {
     return fmt == SRC_NV12 ? warp_fixed_kernel<112, 112, IR, 4, SRC_NV12>
            : fmt == SRC_NV21 ? warp_fixed_kernel<112, 112, IR, 4, SRC_NV21>
-           : fmt == SRC_PLANAR ? warp_fixed_kernel<112, 112, IR, 2, SRC_PLANAR> : warp_fixed_kernel<112, 112, IR, 4, SRC_BGR>;
+           : fmt == SRC_PLANAR ? warp_fixed_kernel<112, 112, IR, 2, SRC_PLANAR>
+           : fmt == SRC_PACKED422 ? warp_fixed_kernel<112, 112, IR, 4, SRC_PACKED422> : warp_fixed_kernel<112, 112, IR, 4, SRC_BGR>;
 }
-// launch names by source format (I420 and YV12 share the planar instantiations)
-static const char *const FIXED_NAMES[4] = {"warp_fixed_kernel", "warp_fixed_kernel_nv12", "warp_fixed_kernel_nv21", "warp_fixed_kernel_i420"};
-static const char *const WARP_NAMES[4] = {"warp_kernel", "warp_kernel_nv12", "warp_kernel_nv21", "warp_kernel_i420"};
+// launch names by source format (I420 and YV12 share the planar instantiations, YUY2, UYVY and YVYU the packed ones)
+static const char *const FIXED_NAMES[5] = {"warp_fixed_kernel", "warp_fixed_kernel_nv12", "warp_fixed_kernel_nv21", "warp_fixed_kernel_i420",
+                                           "warp_fixed_kernel_yuv422"};
+static const char *const WARP_NAMES[5] = {"warp_kernel", "warp_kernel_nv12", "warp_kernel_nv21", "warp_kernel_i420", "warp_kernel_yuv422"};
 
 // fmt: the source format of frames_dev (SrcFmt)
 int warp_launch(fd_ctx *ctx, const FrameDev *frames_dev, const int32_t *frame_idx_dev, const double *M12_dev,
@@ -849,7 +893,7 @@ int warp_launch(fd_ctx *ctx, const FrameDev *frames_dev, const int32_t *frame_id
         static const int ir_env = getenv("FD_WARP_IR") ? atoi(getenv("FD_WARP_IR")) : 14;   // A/B: 16-row items (7 per face, 8 rounds as 4 + 4): 82.0 vs 78.8 us on C2
         const int IR = ir_env == 16 ? 16 : 14;
         void (*kern)(WarpArgs) = IR == 16 ? fixed_kernel_for<16>(fmt) : fixed_kernel_for<14>(fmt);
-        static int per_sm_fixed[4] = {0, 0, 0, 0};
+        static int per_sm_fixed[5] = {0, 0, 0, 0, 0};
         int &per_sm_k = per_sm_fixed[fmt];
         if (!per_sm_k) FD_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm_k, kern, 224, 0));
         const long long items = (long long)F_cap * (112 / IR);
@@ -877,7 +921,8 @@ int warp_launch(fd_ctx *ctx, const FrameDev *frames_dev, const int32_t *frame_id
     int per_sm = 0;
     void (*kern)(WarpArgs) = fmt == SRC_NV12 ? warp_kernel<SRC_NV12>
                              : fmt == SRC_NV21 ? warp_kernel<SRC_NV21>
-                             : fmt == SRC_PLANAR ? warp_kernel<SRC_PLANAR> : warp_kernel<SRC_BGR>;
+                             : fmt == SRC_PLANAR ? warp_kernel<SRC_PLANAR>
+                             : fmt == SRC_PACKED422 ? warp_kernel<SRC_PACKED422> : warp_kernel<SRC_BGR>;
     FD_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, WARP_THREADS, smem));
     const long long items = (long long)F_cap * a.bands;
     const int grid = (int)std::min<long long>(items, (long long)ctx->num_sms * std::max(per_sm, 1));

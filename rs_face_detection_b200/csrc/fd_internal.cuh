@@ -52,18 +52,20 @@ enum SrcFmt : int {
     SRC_NV12 = 1,     // FrameDev::uv: interleaved U,V
     SRC_NV21 = 2,     // FrameDev::uv: interleaved V,U
     SRC_PLANAR = 3,   // I420 and YV12: FrameDev::uv is the U plane, FrameDev::v_plane() the V plane
+    SRC_PACKED422 = 4,   // YUY2, UYVY and YVYU: FrameDev::data is the packed plane, FrameDev::v_off its byte-permute selector
 };
 
 // Per-frame descriptor as the kernels see it.
 struct FrameDev {
-    const uint8_t *data;     // BGR pixels, or the Y plane of a 4:2:0 frame
+    const uint8_t *data;     // BGR pixels, the Y plane of a 4:2:0 frame, or the packed plane of a 4:2:2 frame (h rows of 2w bytes)
     int h, w, pitch;
     int new_w, new_h;        // letterbox content size
     double scale_x, scale_y; // cv::resize inverse scales
     const uint8_t *uv;       // NV12/NV21: the interleaved chroma plane (h/2 rows of w bytes); planar: the U plane (h/2 rows
-                             // of w/2 bytes); nullptr for a BGR frame
+                             // of w/2 bytes); nullptr for a BGR or packed frame
     int pitch_uv;            // of the chroma plane(s)
-    int v_off;               // planar: start of the V plane minus start of the U plane, in bytes; 0 otherwise (fills the
+    int v_off;               // planar: start of the V plane minus start of the U plane, in bytes; packed 4:2:2: the
+                             // __byte_perm selector that reorders a 2-pixel macropixel to Y0 U Y1 V; 0 otherwise (fills the
                              // padding, so the table keeps its size)
     __host__ __device__ const uint8_t *v_plane() const { return uv + v_off; }   // planar only
 };

@@ -97,12 +97,35 @@ static int fill_frame_yuv420(const fd_ctx *ctx, const fd_frame_nv12 &fr, int32_t
     return fill_geometry(ctx, fr.height, fr.width, out, det_scale);
 }
 
-// The frames of a batched call, device pointers: BGR (bgr) or 4:2:0 (yuv, in the FD_YUV420_* layout `layout`); exactly
-// one is set.
+// __byte_perm selector that reorders a macropixel of an FD_YUV422_* layout to Y0 U Y1 V, or -1
+static int yuv422_selector(int32_t layout) {
+    switch (layout) {
+    case FD_YUV422_YUY2: return 0x3210;
+    case FD_YUV422_UYVY: return 0x2301;   // U Y0 V Y1
+    case FD_YUV422_YVYU: return 0x1230;   // Y0 V Y1 U
+    default: return -1;
+    }
+}
+
+// cv::cvtColor(COLOR_YUV2BGR_YUY2 / _UYVY / _YVYU) accepts even widths and any height.
+static int fill_frame_yuv422(const fd_ctx *ctx, const fd_frame &fr, int32_t layout, FrameDev *out, float *det_scale) {
+    FD_REQUIRE(fr.data, "frame (YUV 4:2:2): null data");
+    FD_REQUIRE(fr.height > 0 && fr.width > 0 && fr.width % 2 == 0 && (int64_t)fr.pitch >= 2 * (int64_t)fr.width,
+               "frame (YUV 4:2:2): bad geometry (width must be even, pitch at least twice the width)");
+    out->data = fr.data;
+    out->pitch = fr.pitch;
+    out->v_off = yuv422_selector(layout);
+    return fill_geometry(ctx, fr.height, fr.width, out, det_scale);
+}
+
+// The frames of a batched call, device pointers: BGR (bgr), 4:2:0 (yuv, in the FD_YUV420_* layout `layout`) or packed 4:2:2
+// (packed, in the FD_YUV422_* layout `layout`); exactly one is set.
 struct FrameList {
     const fd_frame *bgr = nullptr;
     const fd_frame_nv12 *yuv = nullptr;
+    const fd_frame *packed = nullptr;
     int32_t layout = FD_YUV420_NV12;
+    bool any() const { return bgr || yuv || packed; }
 };
 
 // the FrameList of a *_yuv420 call; an unknown layout is rejected here, before any call can return early
@@ -113,10 +136,19 @@ static int yuv420_frames(const fd_frame_nv12 *frames, int32_t layout, FrameList 
     return FD_OK;
 }
 
+// the FrameList of a *_yuv422 call; an unknown layout is rejected here, before any call can return early
+static int yuv422_frames(const fd_frame *frames, int32_t layout, FrameList *fl) {
+    FD_REQUIRE(yuv422_selector(layout) >= 0, "frame (YUV 4:2:2): unknown layout");
+    fl->packed = frames;
+    fl->layout = layout;
+    return FD_OK;
+}
+
 // uploads B descriptors and records their source format in ctx->frames_fmt; returns the widest staged source row in bytes
-// (BGR: 3w, NV12/NV21: w, planar: a U and a V half of round16(w/2) bytes each)
+// (BGR: 3w, NV12/NV21: w, planar: a U and a V half of round16(w/2) bytes each, packed 4:2:2: 2w)
 static int upload_frame_table(fd_ctx *ctx, FrameList frames, int B, float *det_scale_host, int *max_row_bytes) {
-    const int fmt = frames.yuv ? yuv420_format(frames.layout) : SRC_BGR;   // a known layout (yuv420_frames)
+    // a known layout (yuv420_frames, yuv422_frames)
+    const int fmt = frames.packed ? SRC_PACKED422 : frames.yuv ? yuv420_format(frames.layout) : SRC_BGR;
     std::vector<FrameDev> tab(B);
     int mrb = 0;
     for (int i = 0; i < B; ++i) {
@@ -126,6 +158,9 @@ static int upload_frame_table(fd_ctx *ctx, FrameList frames, int B, float *det_s
             const int w = frames.yuv[i].width;
             FD_TRY(fill_frame_yuv420(ctx, frames.yuv[i], frames.layout, &tab[i], &ds));
             mrb = std::max(mrb, fmt == SRC_PLANAR ? 2 * ((w / 2 + 15) & ~15) : w);
+        } else if (frames.packed) {
+            FD_TRY(fill_frame_yuv422(ctx, frames.packed[i], frames.layout, &tab[i], &ds));
+            mrb = std::max(mrb, 2 * frames.packed[i].width);
         } else {
             FD_REQUIRE(frames.bgr[i].data != nullptr, "frame: null data");
             FD_TRY(fill_frame(ctx, frames.bgr[i], frames.bgr[i].data, &tab[i], &ds));
@@ -274,7 +309,7 @@ FD_EXPORT int fd_letterbox_geometry(const fd_ctx *ctx, int img_h, int img_w, int
 
 static int preprocess_batch(fd_ctx *ctx, FrameList frames, int B, float *out_nchw_dev, float *det_scale_host) {
     FD_TRY(check_ctx(ctx));
-    FD_REQUIRE(B >= 0 && (B == 0 || ((frames.bgr || frames.yuv) && out_nchw_dev)), "fd_preprocess_batch: bad arguments");
+    FD_REQUIRE(B >= 0 && (B == 0 || (frames.any() && out_nchw_dev)), "fd_preprocess_batch: bad arguments");
     if (B == 0) return FD_OK;
     int mrb = 0;
     FD_TRY(upload_frame_table(ctx, frames, B, det_scale_host, &mrb));
@@ -287,6 +322,8 @@ static int preprocess_batch(fd_ctx *ctx, FrameList frames, int B, float *out_nch
             const fd_frame_nv12 &f = frames.yuv[i];
             const bool planar = ctx->frames_fmt == SRC_PLANAR;
             aligned = aligned && row_ok(f.y, f.pitch_y, f.width) && row_ok(f.uv, f.pitch_uv, planar ? f.width / 2 : f.width);
+        } else if (frames.packed) {
+            aligned = aligned && row_ok(frames.packed[i].data, frames.packed[i].pitch, 2 * frames.packed[i].width);
         } else {
             aligned = aligned && row_ok(frames.bgr[i].data, frames.bgr[i].pitch, frames.bgr[i].width * 3);
         }
@@ -306,6 +343,11 @@ FD_EXPORT int fd_preprocess_batch_yuv420(fd_ctx *ctx, const fd_frame_nv12 *frame
 }
 FD_EXPORT int fd_preprocess_batch_nv12(fd_ctx *ctx, const fd_frame_nv12 *frames, int B, float *out_nchw_dev, float *det_scale_host) {
     return fd_preprocess_batch_yuv420(ctx, frames, FD_YUV420_NV12, B, out_nchw_dev, det_scale_host);
+}
+FD_EXPORT int fd_preprocess_batch_yuv422(fd_ctx *ctx, const fd_frame *frames, int32_t layout, int B, float *out_nchw_dev, float *det_scale_host) {
+    FrameList fl;
+    FD_TRY(yuv422_frames(frames, layout, &fl));
+    return preprocess_batch(ctx, fl, B, out_nchw_dev, det_scale_host);
 }
 
 FD_EXPORT int fd_detect_batch(fd_ctx *ctx, const float *const *heads_dev, int n_heads, int B, const float *det_scale_host,
@@ -375,7 +417,7 @@ FD_EXPORT int fd_detect_last_stats(fd_ctx *ctx, int32_t *out) {
 static int align_batch(fd_ctx *ctx, FrameList frames, int B, const float *landmarks_dev, const int32_t *frame_idx_dev,
                        const float *bbox_dev, int F, uint8_t *crops_dev, double *M_dev, uint8_t *ok_dev) {
     FD_TRY(check_ctx(ctx));
-    FD_REQUIRE(B > 0 && (frames.bgr || frames.yuv) && F >= 0 && (F == 0 || (landmarks_dev && crops_dev)), "fd_align_batch: bad arguments");
+    FD_REQUIRE(B > 0 && frames.any() && F >= 0 && (F == 0 || (landmarks_dev && crops_dev)), "fd_align_batch: bad arguments");
     if (F == 0) return FD_OK;
     FD_TRY(upload_frame_table(ctx, frames, B, nullptr, nullptr));
     WarpFallback fb;
@@ -400,10 +442,16 @@ FD_EXPORT int fd_align_batch_nv12(fd_ctx *ctx, const fd_frame_nv12 *frames, int 
                                   const float *bbox_dev, int F, uint8_t *crops_dev, double *M_dev, uint8_t *ok_dev) {
     return fd_align_batch_yuv420(ctx, frames, FD_YUV420_NV12, B, landmarks_dev, frame_idx_dev, bbox_dev, F, crops_dev, M_dev, ok_dev);
 }
+FD_EXPORT int fd_align_batch_yuv422(fd_ctx *ctx, const fd_frame *frames, int32_t layout, int B, const float *landmarks_dev, const int32_t *frame_idx_dev,
+                                    const float *bbox_dev, int F, uint8_t *crops_dev, double *M_dev, uint8_t *ok_dev) {
+    FrameList fl;
+    FD_TRY(yuv422_frames(frames, layout, &fl));
+    return align_batch(ctx, fl, B, landmarks_dev, frame_idx_dev, bbox_dev, F, crops_dev, M_dev, ok_dev);
+}
 
 static int align_detections(fd_ctx *ctx, FrameList frames, int B, uint8_t *crops_dev, int cap_faces, double *M_dev, uint8_t *ok_dev) {
     FD_TRY(check_ctx(ctx));
-    FD_REQUIRE(B > 0 && (frames.bgr || frames.yuv) && B == ctx->last_B && crops_dev && cap_faces > 0, "fd_align_detections: bad arguments");
+    FD_REQUIRE(B > 0 && frames.any() && B == ctx->last_B && crops_dev && cap_faces > 0, "fd_align_detections: bad arguments");
     // No host synchronisation here: images needing the big NMS path are detected lazily at
     // fd_detect_fetch / fd_detect_view / fd_ctx-level fetch, which replays this align if the detections changed.
     FD_TRY(upload_frame_table(ctx, frames, B, nullptr, nullptr));
@@ -431,6 +479,12 @@ FD_EXPORT int fd_align_detections_yuv420(fd_ctx *ctx, const fd_frame_nv12 *frame
 FD_EXPORT int fd_align_detections_nv12(fd_ctx *ctx, const fd_frame_nv12 *frames, int B, uint8_t *crops_dev, int cap_faces, double *M_dev,
                                        uint8_t *ok_dev) {
     return fd_align_detections_yuv420(ctx, frames, FD_YUV420_NV12, B, crops_dev, cap_faces, M_dev, ok_dev);
+}
+FD_EXPORT int fd_align_detections_yuv422(fd_ctx *ctx, const fd_frame *frames, int32_t layout, int B, uint8_t *crops_dev, int cap_faces, double *M_dev,
+                                         uint8_t *ok_dev) {
+    FrameList fl;
+    FD_TRY(yuv422_frames(frames, layout, &fl));
+    return align_detections(ctx, fl, B, crops_dev, cap_faces, M_dev, ok_dev);
 }
 
 // ---- single-image host wrappers -----------------------------------------------------------------------------------
@@ -694,7 +748,7 @@ FD_EXPORT int fd_face_selection(fd_ctx *ctx, int img_h, int img_w, const float *
 
 static int select_detections(fd_ctx *ctx, FrameList frames, int B, int is_enroll, const fd_select_params *params, int32_t *sel_host) {
     FD_TRY(check_ctx(ctx));
-    FD_REQUIRE((frames.bgr || frames.yuv) && B > 0 && B == ctx->last_B, "fd_select_detections: needs the frames of the last fd_detect_batch");
+    FD_REQUIRE(frames.any() && B > 0 && B == ctx->last_B, "fd_select_detections: needs the frames of the last fd_detect_batch");
     if (sel_host) FD_TRY(detect_resolve(ctx));
     fd_select_params p;
     if (params) p = *params;
@@ -728,10 +782,16 @@ FD_EXPORT int fd_select_detections_nv12(fd_ctx *ctx, const fd_frame_nv12 *frames
                                         int32_t *sel_host) {
     return fd_select_detections_yuv420(ctx, frames, FD_YUV420_NV12, B, is_enroll, params, sel_host);
 }
+FD_EXPORT int fd_select_detections_yuv422(fd_ctx *ctx, const fd_frame *frames, int32_t layout, int B, int is_enroll, const fd_select_params *params,
+                                          int32_t *sel_host) {
+    FrameList fl;
+    FD_TRY(yuv422_frames(frames, layout, &fl));
+    return select_detections(ctx, fl, B, is_enroll, params, sel_host);
+}
 
 static int align_selected(fd_ctx *ctx, FrameList frames, int B, uint8_t *crops_dev, double *M_dev, uint8_t *ok_dev) {
     FD_TRY(check_ctx(ctx));
-    FD_REQUIRE((frames.bgr || frames.yuv) && B > 0 && B == ctx->select_B && crops_dev,
+    FD_REQUIRE(frames.any() && B > 0 && B == ctx->select_B && crops_dev,
                "fd_align_selected: needs the frames of the last fd_select_detections");
     FD_TRY(upload_frame_table(ctx, frames, B, nullptr, nullptr));
     // Images without a selection (or whose selection has no key points) carry NaN key points: the estimate fails there and,
@@ -754,6 +814,11 @@ FD_EXPORT int fd_align_selected_yuv420(fd_ctx *ctx, const fd_frame_nv12 *frames,
 }
 FD_EXPORT int fd_align_selected_nv12(fd_ctx *ctx, const fd_frame_nv12 *frames, int B, uint8_t *crops_dev, double *M_dev, uint8_t *ok_dev) {
     return fd_align_selected_yuv420(ctx, frames, FD_YUV420_NV12, B, crops_dev, M_dev, ok_dev);
+}
+FD_EXPORT int fd_align_selected_yuv422(fd_ctx *ctx, const fd_frame *frames, int32_t layout, int B, uint8_t *crops_dev, double *M_dev, uint8_t *ok_dev) {
+    FrameList fl;
+    FD_TRY(yuv422_frames(frames, layout, &fl));
+    return align_selected(ctx, fl, B, crops_dev, M_dev, ok_dev);
 }
 
 // ---- end-to-end with host buffers ------------------------------------------------------------------------------------

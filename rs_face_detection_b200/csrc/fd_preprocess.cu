@@ -43,12 +43,13 @@ __device__ __forceinline__ const uint8_t *stage_row(uint8_t *buf, const uint8_t 
     return dst;
 }
 
-// FMT: the source format (SrcFmt).  A 4:2:0 frame's taps are converted to BGR (yuv_bgr24) before the resize arithmetic,
-// and the staged rows are the Y rows and the chroma row(s) of the taps; a planar chroma row is staged as its U half and,
-// row_buf_bytes / 2 further, its V half.
+// FMT: the source format (SrcFmt).  A YUV frame's taps are converted to BGR (yuv_bgr24) before the resize arithmetic.  A
+// 4:2:0 frame's staged rows are the Y rows and the chroma row(s) of the taps; a planar chroma row is staged as its U half and,
+// row_buf_bytes / 2 further, its V half.  A packed 4:2:2 frame stages its tap rows (2w bytes) as a BGR frame does.
 template <int FMT>
 __global__ void preprocess_kernel(PreArgs a) {
-    constexpr bool NV = FMT != SRC_BGR, PL = FMT == SRC_PLANAR;
+    constexpr bool NV = FMT == SRC_NV12 || FMT == SRC_NV21 || FMT == SRC_PLANAR, PL = FMT == SRC_PLANAR;   // NV: 4:2:0
+    constexpr bool PK = FMT == SRC_PACKED422;
     extern __shared__ __align__(16) unsigned char smem[];
     const int ow = a.out_w;
     float *lut = reinterpret_cast<float *>(smem);                  // [3][256], indexed by BGR channel
@@ -71,7 +72,7 @@ __global__ void preprocess_kernel(PreArgs a) {
     const FrameDev f = a.frames[blockIdx.y];
     for (int x = threadIdx.x; x < f.new_w; x += blockDim.x) {
         x_taps(x, f.scale_x, f.w, &xo0[x], &xo1[x], &xa0[x], &xa1[x]);
-        if (NV) { xo0[x] /= 3; xo1[x] /= 3; }   // pixel, not byte, offsets
+        if (NV || PK) { xo0[x] /= 3; xo1[x] /= 3; }   // pixel, not byte, offsets
     }
     __syncthreads();
     const float pad_r = lut[2 * 256], pad_g = lut[1 * 256], pad_b = lut[0];
@@ -80,7 +81,8 @@ __global__ void preprocess_kernel(PreArgs a) {
     const int ngroups = (ow + 3) >> 2;
     const int row_begin = blockIdx.x * PRE_ROWS;
     const int row_end = min(row_begin + PRE_ROWS, a.out_h);
-    const int src_row_bytes = NV ? f.w : f.w * 3;
+    const int src_row_bytes = NV ? f.w : PK ? 2 * f.w : f.w * 3;
+    const unsigned sel = PK ? (unsigned)f.v_off : 0u;
 
     for (int dy = row_begin; dy < row_end; ++dy) {
         float *o_r = out_img + (size_t)dy * ow;  // plane 0 = R (BGR channel 2), face_detection.rs:226-227
@@ -115,7 +117,14 @@ __global__ void preprocess_kernel(PreArgs a) {
                 const int x = 4 * g + j;
                 if (content && x < f.new_w) {
                     const int x0 = xo0[x], x1 = xo1[x], a0 = xa0[x], a1 = xa1[x];
-                    if (NV) {
+                    if (PK) {
+                        const unsigned p = resize_px24(packed_px24(r0, sel, x0), packed_px24(r0, sel, x1),
+                                                       b1 != 0 ? packed_px24(r1, sel, x0) : 0u, b1 != 0 ? packed_px24(r1, sel, x1) : 0u,
+                                                       a0, a1, b0, b1);
+                        vb[j] = lut[p & 255u];
+                        vg[j] = lut[256 + ((p >> 8) & 255u)];
+                        vr[j] = lut[512 + (p >> 16)];
+                    } else if (NV) {
                         const unsigned p = resize_px24(yuv_px24<FMT>(r0, c0, v0, x0), yuv_px24<FMT>(r0, c0, v0, x1),
                                                        b1 != 0 ? yuv_px24<FMT>(r1, c1, v1, x0) : 0u, b1 != 0 ? yuv_px24<FMT>(r1, c1, v1, x1) : 0u,
                                                        a0, a1, b0, b1);
@@ -156,6 +165,11 @@ __global__ void preprocess_kernel(PreArgs a) {
 constexpr int PRE2_STAGES = 4;
 constexpr int PRE2_ROWS = 16;
 
+// pixel x of a packed 4:2:2 row staged at a 4-byte aligned address: its macropixel as one aligned word
+__device__ __forceinline__ unsigned packed_tap(const uint8_t *row, unsigned sel, int x) {
+    return packed_bgr24(__byte_perm(*reinterpret_cast<const unsigned *>(row + 4 * (x >> 1)), 0u, sel), x);
+}
+
 __device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ void mbar_init(uint64_t *bar, int count) {
     asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
@@ -181,9 +195,11 @@ __device__ __forceinline__ void bulk_g2s(void *dst_smem, const void *src_gmem, u
 // FMT: the source format (SrcFmt).  4:2:0: a stage holds the Y rows of the taps and their chroma row(s) — one when both
 // taps map to the same chroma row (4K -> 640x360: rows 6y+2 and 6y+3 both read chroma row 3y+1).  A planar chroma row
 // fills its slot as the U half and, row_buf_bytes / 2 further, the V half: bulk copies of round16(w/2) bytes each.
+// Packed 4:2:2: a stage holds the packed tap rows (2w bytes each), and a tap reads its macropixel as one aligned word.
 template <bool IDENT, int FMT>
 __global__ void __launch_bounds__(256) preprocess_tma_kernel(PreArgs a) {
-    constexpr bool NV = FMT != SRC_BGR, PL = FMT == SRC_PLANAR;
+    constexpr bool NV = FMT == SRC_NV12 || FMT == SRC_NV21 || FMT == SRC_PLANAR, PL = FMT == SRC_PLANAR;   // NV: 4:2:0
+    constexpr bool PK = FMT == SRC_PACKED422;
     constexpr int SLOTS = NV ? 4 : 2;                           // rows per stage: Y0, Y1 (BGR: row 0, row 1), UV0, UV1
     extern __shared__ __align__(128) unsigned char smem[];
     uint64_t *full = reinterpret_cast<uint64_t *>(smem);        // [PRE2_STAGES]
@@ -219,7 +235,7 @@ __global__ void __launch_bounds__(256) preprocess_tma_kernel(PreArgs a) {
         if (x < f.new_w) {
             int o1;
             x_taps(x, f.scale_x, f.w, &x0[j], &o1, &wa0[j], &wa1[j]);
-            if (NV) x0[j] /= 3;   // pixel, not byte, offset
+            if (NV || PK) x0[j] /= 3;   // pixel, not byte, offset
             point &= (wa1[j] == 0);
         }
     }
@@ -231,7 +247,8 @@ __global__ void __launch_bounds__(256) preprocess_tma_kernel(PreArgs a) {
     const int row_begin = blockIdx.x * PRE2_ROWS;
     const int row_end = min(row_begin + PRE2_ROWS, a.out_h);
     const int n_content = max(0, min(f.new_h, row_end) - row_begin);
-    const uint32_t copy_bytes = (uint32_t)(((NV ? f.w : f.w * 3) + 15) & ~15);
+    const uint32_t copy_bytes = (uint32_t)(((NV ? f.w : PK ? 2 * f.w : f.w * 3) + 15) & ~15);
+    const unsigned sel = PK ? (unsigned)f.v_off : 0u;
     const uint32_t half_bytes = (uint32_t)(((f.w >> 1) + 15) & ~15);   // PL: one U or V row
     const int half = rb >> 1;
     const bool active = 4 * tid < ow;
@@ -280,7 +297,10 @@ __global__ void __launch_bounds__(256) preprocess_tma_kernel(PreArgs a) {
                 for (int j = 0; j < 4; ++j) {
                     if (x0[j] >= 0) {
                         int pb, pg, pr;
-                        if (NV) {
+                        if (PK) {
+                            const unsigned p = packed_tap(r0, sel, x0[j]);
+                            pb = p & 255u; pg = (p >> 8) & 255u; pr = p >> 16;
+                        } else if (NV) {
                             const unsigned p = yuv_px24<FMT>(r0, c0, v0, x0[j]);
                             pb = p & 255u; pg = (p >> 8) & 255u; pr = p >> 16;
                         } else {
@@ -298,9 +318,14 @@ __global__ void __launch_bounds__(256) preprocess_tma_kernel(PreArgs a) {
 #pragma unroll
                 for (int j = 0; j < 4; ++j) {
                     if (x0[j] >= 0) {
-                        const int o0 = x0[j], o1 = x0[j] + (wa1[j] != 0 ? (NV ? 1 : 3) : 0), q0 = wa0[j], q1 = wa1[j];
+                        const int o0 = x0[j], o1 = x0[j] + (wa1[j] != 0 ? (NV || PK ? 1 : 3) : 0), q0 = wa0[j], q1 = wa1[j];
                         int pb, pg, pr;
-                        if (NV) {
+                        if (PK) {
+                            const unsigned p = resize_px24(packed_tap(r0, sel, o0), packed_tap(r0, sel, o1),
+                                                           b1 != 0 ? packed_tap(r1, sel, o0) : 0u, b1 != 0 ? packed_tap(r1, sel, o1) : 0u,
+                                                           q0, q1, b0, b1);
+                            pb = p & 255u; pg = (p >> 8) & 255u; pr = p >> 16;
+                        } else if (NV) {
                             const unsigned p = resize_px24(yuv_px24<FMT>(r0, c0, v0, o0), yuv_px24<FMT>(r0, c0, v0, o1),
                                                            b1 != 0 ? yuv_px24<FMT>(r1, c1, v1, o0) : 0u,
                                                            b1 != 0 ? yuv_px24<FMT>(r1, c1, v1, o1) : 0u, q0, q1, b0, b1);
@@ -430,24 +455,26 @@ int crops_to_tensor_launch(fd_ctx *ctx, const uint8_t *crops_dev, const int *cou
     return FD_OK;
 }
 
-// launch names by source format (I420 and YV12 share the planar instantiations)
-static const char *const TMA_NAMES[4] = {"preprocess_tma_kernel", "preprocess_tma_kernel_nv12", "preprocess_tma_kernel_nv21",
-                                         "preprocess_tma_kernel_i420"};
-static const char *const PRE_NAMES[4] = {"preprocess_kernel", "preprocess_kernel_nv12", "preprocess_kernel_nv21", "preprocess_kernel_i420"};
+// launch names by source format (I420 and YV12 share the planar instantiations, YUY2, UYVY and YVYU the packed ones)
+static const char *const TMA_NAMES[5] = {"preprocess_tma_kernel", "preprocess_tma_kernel_nv12", "preprocess_tma_kernel_nv21",
+                                         "preprocess_tma_kernel_i420", "preprocess_tma_kernel_yuv422"};
+static const char *const PRE_NAMES[5] = {"preprocess_kernel", "preprocess_kernel_nv12", "preprocess_kernel_nv21", "preprocess_kernel_i420",
+                                         "preprocess_kernel_yuv422"};
 
 template <bool IDENT>
 static void (*tma_kernel_for(int fmt))(PreArgs) {
     return fmt == SRC_NV12 ? preprocess_tma_kernel<IDENT, SRC_NV12>
            : fmt == SRC_NV21 ? preprocess_tma_kernel<IDENT, SRC_NV21>
-           : fmt == SRC_PLANAR ? preprocess_tma_kernel<IDENT, SRC_PLANAR> : preprocess_tma_kernel<IDENT, SRC_BGR>;
+           : fmt == SRC_PLANAR ? preprocess_tma_kernel<IDENT, SRC_PLANAR>
+           : fmt == SRC_PACKED422 ? preprocess_tma_kernel<IDENT, SRC_PACKED422> : preprocess_tma_kernel<IDENT, SRC_BGR>;
 }
 
-// max_row_bytes: widest staged row (BGR: 3w, NV12/NV21: w, planar: 2 round16(w/2), a U half and a V half); fmt: the
-// source format of frames_dev (SrcFmt)
+// max_row_bytes: widest staged row (BGR: 3w, NV12/NV21: w, planar: 2 round16(w/2), a U half and a V half, packed 4:2:2:
+// 2w); fmt: the source format of frames_dev (SrcFmt)
 int preprocess_launch(fd_ctx *ctx, const FrameDev *frames_dev, int B, float *out_nchw_dev, int max_row_bytes, bool rows_aligned16,
                       int fmt) {
     constexpr int SLOTS_NV = 4;
-    const bool nv = fmt != SRC_BGR;
+    const bool nv = fmt == SRC_NV12 || fmt == SRC_NV21 || fmt == SRC_PLANAR;   // 4:2:0: two more row slots for the chroma
     PreArgs a;
     a.frames = frames_dev;
     a.out = out_nchw_dev;
@@ -483,7 +510,8 @@ int preprocess_launch(fd_ctx *ctx, const FrameDev *frames_dev, int B, float *out
     if (smem > (size_t)ctx->max_smem_optin) return fail(FD_ERR_INVALID, "fd_preprocess: source row too wide for shared-memory staging");
     void (*kern)(PreArgs) = fmt == SRC_NV12 ? preprocess_kernel<SRC_NV12>
                             : fmt == SRC_NV21 ? preprocess_kernel<SRC_NV21>
-                            : fmt == SRC_PLANAR ? preprocess_kernel<SRC_PLANAR> : preprocess_kernel<SRC_BGR>;
+                            : fmt == SRC_PLANAR ? preprocess_kernel<SRC_PLANAR>
+                            : fmt == SRC_PACKED422 ? preprocess_kernel<SRC_PACKED422> : preprocess_kernel<SRC_BGR>;
     FD_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int threads = std::min(1024, std::max(64, ((ngroups + 31) / 32) * 32));
     dim3 grid((a.out_h + PRE_ROWS - 1) / PRE_ROWS, B);

@@ -155,4 +155,32 @@ __device__ __forceinline__ unsigned resize_pixel24_yuv(const uint8_t *yp, int pi
     return resize_px24(yuv_px24<FMT>(r0, c0, v0, x0), yuv_px24<FMT>(r0, c0, v0, x1), p10, p11, a0, a1, b0, b1);
 }
 
+// ---- packed 4:2:2 sources (YUY2, UYVY, YVYU): pixel x takes its own Y and the U, V of its pair x & ~1 ------------------
+// A row is w/2 macropixels of 4 bytes.  sel is the __byte_perm selector that reorders a macropixel to Y0 U Y1 V (nibble k:
+// the source byte that lands in byte k): YUY2 0x3210, UYVY 0x2301, YVYU 0x1230.
+// pixel x of a macropixel n already reordered to Y0 U Y1 V
+__device__ __forceinline__ unsigned packed_bgr24(unsigned n, int x) {
+    return yuv_bgr24((x & 1) ? (n >> 16) & 255u : n & 255u, (n >> 8) & 255u, n >> 24);
+}
+// pixel x of a packed row at any alignment: three byte reads
+__device__ __forceinline__ unsigned packed_px24(const uint8_t *row, unsigned sel, int x) {
+    const uint8_t *m = row + 4 * (x >> 1);
+    return yuv_bgr24(m[(sel >> ((x & 1) ? 8 : 0)) & 3u], m[(sel >> 4) & 3u], m[(sel >> 12) & 3u]);
+}
+// resize_pixel24 of the ROI (rx0, ry0)..(rx0 + rw, ry0 + rh) of a packed frame: taps in ROI coordinates, chroma of the
+// frame's own pairs (rx0 may be odd)
+__device__ __forceinline__ unsigned resize_pixel24_packed(const uint8_t *data, int pitch, unsigned sel, int rx0, int ry0, int rw, int rh,
+                                                          int ow, int oh, int x, int y) {
+    if (rw == ow && rh == oh) return packed_px24(data + (size_t)(ry0 + y) * pitch, sel, rx0 + x);
+    const double scale_x = 1.0 / ((double)ow / rw), scale_y = 1.0 / ((double)oh / rh);
+    int o0, o1, y0, y1, b0, b1;
+    short a0, a1;
+    x_taps(x, scale_x, rw, &o0, &o1, &a0, &a1);
+    y_taps(y, scale_y, rh, &y0, &y1, &b0, &b1);
+    const int x0 = rx0 + o0 / 3, x1 = rx0 + o1 / 3;
+    const uint8_t *r0 = data + (size_t)(ry0 + y0) * pitch, *r1 = data + (size_t)(ry0 + y1) * pitch;
+    const unsigned p10 = b1 != 0 ? packed_px24(r1, sel, x0) : 0u, p11 = b1 != 0 ? packed_px24(r1, sel, x1) : 0u;
+    return resize_px24(packed_px24(r0, sel, x0), packed_px24(r0, sel, x1), p10, p11, a0, a1, b0, b1);
+}
+
 }  // namespace fd

@@ -1,20 +1,25 @@
 #!/usr/bin/env python
-"""4:2:0 batch steps (NV12, NV21, I420, YV12) against the BGR batch step on bench.py's C2 / C5 inputs.
+"""4:2:0 (NV12, NV21, I420, YV12) and packed 4:2:2 (YUY2, UYVY, YVYU) batch steps against the BGR batch step on bench.py's
+C2 / C5 inputs.
 
 The frames of bench.py's workload are converted to 4:2:0 the way a decoder hands them over (cv2 COLOR_BGR2YUV_I420), and
 the BGR step runs on what cv2.cvtColor(COLOR_YUV2BGR_I420) gives back (the round trip is lossy, so the original BGR frames
 are never the comparison; every layout of the same chroma converts to the same BGR frame).  Each layout case keeps its
 planes in one layout: nv12 / nv21 (chroma pitch W), i420 / yv12 (tight chroma pitch W/2) and i420_padded / yv12_padded
-(chroma pitch W/2 rounded up to 64 bytes, plus 64).  Parity first: tensor, det_scale, detections, crops and modes of
-    layout step: preprocess_batch_nv12 / _yuv420 -> detect_batch -> align_detections_nv12 / _yuv420
+(chroma pitch W/2 rounded up to 64 bytes, plus 64).  The packed cases yuy2 / uyvy / yvyu (pitch 2W) carry the same bytes:
+each macropixel holds its two Y values and the U, V of its 2x2 block, so cv2.cvtColor(COLOR_YUV2BGR_YUY2 / _UYVY / _YVYU)
+gives the same BGR frame as well.  Parity first: tensor, det_scale, detections, crops and modes of
+    layout step: preprocess_batch_nv12 / _yuv420 / _yuv422 -> detect_batch -> align_detections_nv12 / _yuv420 / _yuv422
     BGR step:    preprocess_batch                -> detect_batch -> align_detections
 must be byte-identical.  Then the steps are timed with CUDA events, alternating in one process, and profiled per kernel
 (fd_ctx_profile) in a separate pass.  The NV12 case calls the *_nv12 entry points.  One JSON file per workload goes to
---out-dir: r4_nv12_<workload>.json for the NV12 case alone (the default), r5_yuv420_<workload>.json otherwise.  'i420' is
-the tight chroma pitch only; name 'i420_padded' as well to measure the padded one.
+--out-dir: r4_nv12_<workload>.json for the NV12 case alone (the default), r6_yuv422_<workload>.json when every case named
+with --layouts is packed, r5_yuv420_<workload>.json otherwise.  'i420' is the tight chroma pitch only; name 'i420_padded' as
+well to measure the padded one.
 
     python scripts/nv12_bench.py --workloads c2,c5 --steps 100 --rounds 3 --out-dir profiles
     python scripts/nv12_bench.py --layouts nv12,nv21,i420,i420_padded --workloads c2,c5 --out-dir profiles
+    python scripts/nv12_bench.py --layouts yuy2,uyvy,yvyu --workloads c2,c5 --out-dir profiles
 """
 import argparse
 import json
@@ -43,17 +48,22 @@ def y_rows(dy, scale_y, h):
 LAYOUTS = {"nv12": (0, lambda W: W), "nv21": (1, lambda W: W), "i420": (2, lambda W: W // 2), "yv12": (3, lambda W: W // 2),
            "i420_padded": (2, lambda W: -(-(W // 2) // 64) * 64 + 64), "yv12_padded": (3, lambda W: -(-(W // 2) // 64) * 64 + 64)}
 KERNEL_SUFFIX = {0: "_nv12", 1: "_nv21", 2: "_i420", 3: "_i420"}   # I420 and YV12 share the planar kernels
+# packed 4:2:2 case -> FD_YUV422_* layout and the byte positions of Y0, U, Y1, V in a macropixel
+PACKED = {"yuy2": (0, (0, 1, 2, 3)), "uyvy": (1, (1, 0, 3, 2)), "yvyu": (2, (0, 3, 2, 1))}
 
 
 def preprocess_bytes(h, w, new_h, kind):
-    """bytes the preprocess kernel reads per frame (whole staged rows: Y rows and one or two chroma rows, a planar chroma row
-    as a U and a V row of w/2 bytes) plus the 640x640x3 f32 tensor it writes"""
+    """bytes the preprocess kernel reads per frame (whole staged rows: BGR rows of 3w bytes, packed 4:2:2 rows of 2w bytes, or
+    Y rows and one or two chroma rows, a planar chroma row as a U and a V row of w/2 bytes) plus the 640x640x3 f32 tensor it
+    writes"""
     scale_y = 1.0 / (new_h / h)
     total = 0
     for dy in range(new_h):
         y0, y1, two = y_rows(dy, scale_y, h)
         if kind == "bgr":
             total += 3 * w * (2 if two else 1)
+        elif kind in PACKED:
+            total += 2 * w * (2 if two else 1)
         else:
             total += w * (2 if two else 1) + w * (2 if two and (y1 >> 1) != (y0 >> 1) else 1)
     return total + 3 * 640 * 640 * 4
@@ -92,6 +102,18 @@ def run(wl, args):
     ys_t = [torch.from_numpy(y).cuda() for y in ys]
     tables, keep = {}, []
     for case in cases:
+        if case in PACKED:   # each macropixel: its two Y values and the U, V of its 2x2 block
+            layout, order = PACKED[case]
+            desc = []
+            for y_t, y, u, v in zip(ys_t, ys, us, vs):
+                m = np.empty((H, W // 2, 4), np.uint8)
+                m[..., order[0]], m[..., order[2]] = y[:, 0::2], y[:, 1::2]
+                m[..., order[1]], m[..., order[3]] = np.repeat(u, 2, 0), np.repeat(v, 2, 0)
+                p_t = torch.from_numpy(m.reshape(H, 2 * W)).cuda()
+                keep.append(p_t)
+                desc.append((p_t.data_ptr(), H, W, 2 * W))
+            tables[case] = (layout, ctx.frame_table(desc), 2 * W)
+            continue
         layout, pitch_of = LAYOUTS[case]
         puv = pitch_of(W)
         desc = []
@@ -119,7 +141,13 @@ def run(wl, args):
 
     def make_step(case):
         layout, tab, _ = tables[case]
-        if case == "nv12":   # the *_nv12 entry points
+        if case in PACKED:
+            def step():
+                ds = ctx.preprocess_batch_yuv422(tab, layout, tensors[case])
+                ctx.detect_batch(w.heads_c, B, ds, bench.CONF_THR, bench.IOU_THR)
+                ctx.align_detections_yuv422(tab, layout, crops[case], w.cap_faces, None, modes[case])
+                return ds
+        elif case == "nv12":   # the *_nv12 entry points
             def step():
                 ds = ctx.preprocess_batch_nv12(tab, tensors[case])
                 ctx.detect_batch(w.heads_c, B, ds, bench.CONF_THR, bench.IOU_THR)
@@ -182,22 +210,26 @@ def run(wl, args):
     new_h = int(ctx.letterbox_geometry(H, W)[1])
     pre = {k: preprocess_bytes(H, W, new_h, k) * B for k, _ in steps}
     conv_us = 4.5 * H * W * B / (HBM_TBS * 1e12) * 1e6    # read 1.5 B + write 3 B per pixel
+    conv_packed_us = 5.0 * H * W * B / (HBM_TBS * 1e12) * 1e6    # read 2 B + write 3 B per pixel
     best = {k: min(v) for k, v in times.items()}
     kname = {"bgr": ""}
-    kname.update({c: KERNEL_SUFFIX[tables[c][0]] for c in cases})
+    kname.update({c: "_yuv422" if c in PACKED else KERNEL_SUFFIX[tables[c][0]] for c in cases})
     out = {
         "workload": wl, "gpu": name, "power_limit": power, "batch": B, "frame": "%dx%d" % (W, H), "faces": faces,
-        "chroma_pitch": {c: tables[c][2] for c in cases},
+        "chroma_pitch": {c: tables[c][2] for c in cases if c not in PACKED},
         "ms_per_step": times, "frames_per_s": {k: B / (v * 1e-3) for k, v in best.items()},
         "preprocess_bytes_per_step": pre,
         "preprocess_us": {k: prof[k].get("preprocess_tma_kernel" + kname[k], {}).get("us_per_launch") for k, _ in steps},
         "warp_us": {k: prof[k].get("warp_fixed_kernel" + kname[k], {}).get("us_per_launch") for k, _ in steps},
         "profile": prof,
         "least_conversion_pass_us": conv_us,
-        "beats_bgr_plus_conversion": {c: best[c] * 1e3 < best["bgr"] * 1e3 + conv_us for c in cases},
+        "beats_bgr_plus_conversion": {c: best[c] * 1e3 < best["bgr"] * 1e3 + (conv_packed_us if c in PACKED else conv_us) for c in cases},
         "parity": "tensor, det_scale, detections, crops and modes of every layout byte-identical to the BGR step on the cvtColor frames",
         "steps": args.steps, "rounds": args.rounds, "warmup": args.warmup,
     }
+    if any(c in PACKED for c in cases):
+        out["packed_pitch"] = {c: tables[c][2] for c in cases if c in PACKED}
+        out["least_conversion_pass_us_packed"] = conv_packed_us
     ctx.close()
     return out
 
@@ -208,12 +240,14 @@ def main():
     ap.add_argument("--steps", type=int, default=100)
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--rounds", type=int, default=3)
-    ap.add_argument("--layouts", default="nv12", help="comma-separated cases: " + ", ".join(LAYOUTS))
+    ap.add_argument("--layouts", default="nv12", help="comma-separated cases: " + ", ".join(list(LAYOUTS) + list(PACKED)))
     ap.add_argument("--out-dir", default=None, help="write --out-name (%%s: the workload) here")
-    ap.add_argument("--out-name", default=None, help="default: r4_nv12_%%s.json for --layouts nv12, else r5_yuv420_%%s.json")
+    ap.add_argument("--out-name", default=None,
+                    help="default: r4_nv12_%%s.json for --layouts nv12, r6_yuv422_%%s.json for packed cases only, else r5_yuv420_%%s.json")
     args = ap.parse_args()
     if args.out_name is None:
-        args.out_name = "r4_nv12_%s.json" if args.layouts == "nv12" else "r5_yuv420_%s.json"
+        packed_only = all(c in PACKED for c in args.layouts.split(","))
+        args.out_name = "r4_nv12_%s.json" if args.layouts == "nv12" else "r6_yuv422_%s.json" if packed_only else "r5_yuv420_%s.json"
     for wl in args.workloads.split(","):
         out = run(wl, args)
         print(json.dumps(out))
