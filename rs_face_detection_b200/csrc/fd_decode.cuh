@@ -57,7 +57,9 @@ __device__ __forceinline__ float4 decode_box(const DecodeCfg &c, const float *ra
     const float dy = __fmul_rn(raw4[1], c.bbox_stds[1]);
     const float dw = __fmul_rn(raw4[2], c.bbox_stds[2]);
     const float dh = __fmul_rn(raw4[3], c.bbox_stds[3]);
-    // :532-535.  exp through fp64 is correctly rounded to <=0.5 ulp; the reference's f32::exp is the platform expf.
+    // :532-535.  exp through fp64, rounded once to f32: correctly rounded for every float.  Only seven floats have a double
+    // exp within 4 double ulps of an f32 rounding midpoint, and the device rounds all seven correctly
+    // (tests/test_gpu_decode_exact.py).  The reference's f32::exp is the platform expf, which is not correctly rounded.
     const float pcx = __fadd_rn(__fmul_rn(dx, g.aw), g.cx), pcy = __fadd_rn(__fmul_rn(dy, g.ah), g.cy);
     const float pw = __fmul_rn((float)exp((double)dw), g.aw), ph = __fmul_rn((float)exp((double)dh), g.ah);
     // :539-542

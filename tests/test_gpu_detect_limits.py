@@ -16,11 +16,11 @@ import sys
 import numpy as np
 import pytest
 
+from detect_ref import assert_rows_exact, decode_rows
 from rs_face_detection_b200.utils import synth
 
 pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REL = 1e-5
 CONF, IOU = 0.7, 0.4
 A = 2
 FEAT = (20, 40, 80)              # feature map side of strides 32, 16, 8 at 640 x 640
@@ -355,7 +355,7 @@ def _both_builds(scenario):
 
 
 def _check(oracle, heads, meta, out, ds, conf=CONF, iou=IOU, frames=None):
-    """rows vs the oracle (scores bit-exact, boxes / landmarks within 1e-5 relative), and with frames every crop and mode vs
+    """rows vs the oracle bit for bit (tests/detect_ref.py: boxes against a correctly rounded exp), and with frames every crop and mode vs
     oracle.align_face(frame, landmark row, bbox=detection row).  Returns the oracle's per-image (K, kept)."""
     cfg = oracle.make_det_cfg(conf_thr=conf, iou_thr=iou)
     B = heads[0].shape[0]
@@ -366,9 +366,7 @@ def _check(oracle, heads, meta, out, ds, conf=CONF, iou=IOU, frames=None):
         n = int(out["counts"][b])
         assert n == len(edet), (b, n, len(edet))
         det, lmk = out["det"][off:off + n], out["lmk"][off:off + n]
-        np.testing.assert_array_equal(det[:, 4].view(np.uint32), edet[:, 4].view(np.uint32))
-        np.testing.assert_allclose(det, edet, rtol=REL, atol=1e-4)
-        np.testing.assert_allclose(lmk, elmk.reshape(-1, 10), rtol=REL, atol=1e-4)
+        assert_rows_exact(det, lmk, (edet, elmk), decode_rows([h[b] for h in heads], cfg, ds, conf, iou), "image %d" % b)
         if meta is not None:
             assert (K, n) == (meta[b]["K"], meta[b]["kept"]), (b, K, n, meta[b])   # the builder planted what it meant to
         if frames is not None:

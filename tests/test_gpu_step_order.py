@@ -7,6 +7,7 @@ with no host synchronisation give the same results as each step run alone."""
 import numpy as np
 import pytest
 
+from detect_ref import assert_rows_exact, decode_rows
 from rs_face_detection_b200.utils import synth
 
 pytestmark = pytest.mark.gpu
@@ -65,14 +66,14 @@ def _heads(seed):
 def _check_vs_oracle(oracle, frames_np, heads_np, res):
     counts, det, lmk, tensor, crops = res
     cfg = oracle.make_det_cfg(conf_thr=CONF, iou_thr=IOU)
+    ds = oracle.letterbox_geometry(H, W)[2]
     off = 0
     for b in range(B):
         etensor, edet, elmk, _ = oracle.pipeline_frame(cfg, frames_np[b], [h[b] for h in heads_np])
         np.testing.assert_array_equal(tensor[b], etensor[0])
         n = int(counts[b])
         assert n == len(edet)
-        np.testing.assert_allclose(det[off:off + n], edet, rtol=1e-5, atol=1e-3)
-        np.testing.assert_allclose(lmk[off:off + n], elmk, rtol=1e-5, atol=1e-3)
+        assert_rows_exact(det[off:off + n], lmk[off:off + n], (edet, elmk), decode_rows([h[b] for h in heads_np], cfg, ds, CONF, IOU))
         for i in range(n):
             crop, _, _ = oracle.align_face(frames_np[b], lmk[off + i], bbox=det[off + i], with_mode=True)
             np.testing.assert_array_equal(crops[off + i], crop if crop is not None else np.zeros((112, 112, 3), np.uint8))
