@@ -55,7 +55,8 @@ typedef struct fd_ctx fd_ctx;
 
 /* Frame descriptor: BGR u8 HWC (an OpenCV CV_8UC3 Mat: face_detection.rs:131, face_alignment.rs:27), pitch >= 3 * width.
  * The *_yuv422 calls describe a packed 4:2:2 frame with it too: `data` is the packed plane, height rows of width / 2
- * macropixels (4 bytes, 2 pixels each), pitch >= 2 * width; width even, any height >= 1. */
+ * macropixels (4 bytes, 2 pixels each), pitch >= 2 * width; width even, any height >= 1.  The *_rgb calls describe an
+ * interleaved RGB24, RGBA, BGRA or GRAY8 frame with it (FD_RGB_* below). */
 typedef struct fd_frame {
     const uint8_t *data; /* dev pointer for *_batch functions */
     int32_t height, width, pitch;
@@ -91,6 +92,16 @@ enum { FD_YUV420_NV12 = 0, FD_YUV420_NV21 = 1, FD_YUV420_I420 = 2, FD_YUV420_YV1
  * The calls give the results of their BGR counterparts on the frame cv::cvtColor(COLOR_YUV2BGR_YUY2 / _UYVY / _YVYU) makes
  * (BT.601 limited range), without building it. */
 enum { FD_YUV422_YUY2 = 0, FD_YUV422_UYVY = 1, FD_YUV422_YVYU = 2 };
+
+/* Layouts of an interleaved RGB-family frame (an fd_frame) for the *_rgb calls; pitch >= bytes per pixel * width, any
+ * width and height >= 1.
+ *   FD_RGB_RGB24  R G B      3 B/pixel
+ *   FD_RGB_RGBA   R G B A    4 B/pixel, the fourth byte is ignored (also RGBX)
+ *   FD_RGB_BGRA   B G R A    4 B/pixel, the fourth byte is ignored (also BGRX)
+ *   FD_RGB_GRAY8  Y          1 B/pixel (B = G = R = Y)
+ * The calls give the results of their BGR counterparts on the frame cv::cvtColor(COLOR_RGB2BGR / COLOR_RGBA2BGR /
+ * COLOR_BGRA2BGR / COLOR_GRAY2BGR) makes, without building it. */
+enum { FD_RGB_RGB24 = 0, FD_RGB_RGBA = 1, FD_RGB_BGRA = 2, FD_RGB_GRAY8 = 3 };
 
 /* ---- library / context ---------------------------------------------------------------------------- */
 int fd_abi_version(void);
@@ -227,6 +238,10 @@ int fd_preprocess_batch_yuv420(fd_ctx *ctx, const fd_frame_nv12 *frames, int32_t
  * FD_ERR_INVALID for a null data pointer, a width that is not positive and even, a height below 1, a pitch below 2 * width or
  * an unknown layout (also when B == 0).  The same for the other *_yuv422 calls. */
 int fd_preprocess_batch_yuv422(fd_ctx *ctx, const fd_frame *frames, int32_t layout, int B, float *out_nchw_dev, float *det_scale_host);
+/* fd_preprocess_batch on interleaved RGB-family frames in an FD_RGB_* layout.  FD_ERR_INVALID for a null data pointer, a
+ * height or width below 1, a pitch below bytes per pixel * width or an unknown layout (also when B == 0).  The same for the
+ * other *_rgb calls. */
+int fd_preprocess_batch_rgb(fd_ctx *ctx, const fd_frame *frames, int32_t layout, int B, float *out_nchw_dev, float *det_scale_host);
 /* heads_dev[3*s+0..2]: (B,2A,H,W), (B,4A,H,W), (B,10A,H,W) dev tensors of stride s.  Results stay on the device
  * inside the ctx until fd_detect_fetch / fd_align_detections.  Asynchronous.  Images with more than 4096 candidates
  * (and, the first time a ctx meets one, images with more than 1024) are completed by fd_detect_fetch / fd_detect_view;
@@ -267,6 +282,9 @@ int fd_align_batch_yuv420(fd_ctx *ctx, const fd_frame_nv12 *frames, int32_t layo
 /* fd_align_batch on packed 4:2:2 frames in an FD_YUV422_* layout (BORDER_CONSTANT is black in BGR). */
 int fd_align_batch_yuv422(fd_ctx *ctx, const fd_frame *frames, int32_t layout, int B, const float *landmarks_dev, const int32_t *frame_idx_dev,
                           const float *bbox_dev, int F, uint8_t *crops_dev, double *M_dev, uint8_t *ok_dev);
+/* fd_align_batch on interleaved RGB-family frames in an FD_RGB_* layout (BORDER_CONSTANT is black in BGR). */
+int fd_align_batch_rgb(fd_ctx *ctx, const fd_frame *frames, int32_t layout, int B, const float *landmarks_dev, const int32_t *frame_idx_dev,
+                       const float *bbox_dev, int F, uint8_t *crops_dev, double *M_dev, uint8_t *ok_dev);
 /* Aligns every detection of the last fd_detect_batch without a host round trip (fallback box = the detection's own box).
  * crops_dev has room for cap_faces crops; detections beyond cap_faces are not aligned (fd_detect_fetch still reports them). */
 int fd_align_detections(fd_ctx *ctx, const fd_frame *frames, int B, uint8_t *crops_dev, int cap_faces, double *M_dev,
@@ -283,6 +301,10 @@ int fd_align_detections_yuv420(fd_ctx *ctx, const fd_frame_nv12 *frames, int32_t
  * frames in the layout given here. */
 int fd_align_detections_yuv422(fd_ctx *ctx, const fd_frame *frames, int32_t layout, int B, uint8_t *crops_dev, int cap_faces, double *M_dev,
                                uint8_t *ok_dev);
+/* fd_align_detections on interleaved RGB-family frames in an FD_RGB_* layout; a replay at fd_detect_fetch / fd_detect_view
+ * reads the frames in the layout given here. */
+int fd_align_detections_rgb(fd_ctx *ctx, const fd_frame *frames, int32_t layout, int B, uint8_t *crops_dev, int cap_faces, double *M_dev,
+                            uint8_t *ok_dev);
 
 /* ---- SURVEY 8(f) N1: post-align model preprocessors, fused onto the aligned crops ----------------------- */
 /* FaceExtraction::_preprocess (face_extraction.rs:38-77: mean 127.5, mul 0.0078125), FaceQuality::call
@@ -332,6 +354,9 @@ int fd_select_detections_yuv420(fd_ctx *ctx, const fd_frame_nv12 *frames, int32_
 /* fd_select_detections on packed 4:2:2 frames in an FD_YUV422_* layout (the selection reads only their sizes). */
 int fd_select_detections_yuv422(fd_ctx *ctx, const fd_frame *frames, int32_t layout, int B, int is_enroll, const fd_select_params *params,
                                 int32_t *sel_host);
+/* fd_select_detections on interleaved RGB-family frames in an FD_RGB_* layout (the selection reads only their sizes). */
+int fd_select_detections_rgb(fd_ctx *ctx, const fd_frame *frames, int32_t layout, int B, int is_enroll, const fd_select_params *params,
+                             int32_t *sel_host);
 /* FaceAlignment::call on the selection of the last fd_select_detections (face_pipeline/pipeline.rs:216-232): one crop per
  * image, crops_dev (B,crop_h,crop_w,3); images without a selection or without key points (the reference's call(.., None)
  * returns Err) get ok = 0 and a zero crop; ok = 2 marks the bbox-crop fallback on the selected box.  M_dev (B,6) / ok_dev (B) optional. */
@@ -343,6 +368,8 @@ int fd_align_selected_yuv420(fd_ctx *ctx, const fd_frame_nv12 *frames, int32_t l
                              uint8_t *ok_dev);
 /* fd_align_selected on packed 4:2:2 frames in an FD_YUV422_* layout. */
 int fd_align_selected_yuv422(fd_ctx *ctx, const fd_frame *frames, int32_t layout, int B, uint8_t *crops_dev, double *M_dev, uint8_t *ok_dev);
+/* fd_align_selected on interleaved RGB-family frames in an FD_RGB_* layout. */
+int fd_align_selected_rgb(fd_ctx *ctx, const fd_frame *frames, int32_t layout, int B, uint8_t *crops_dev, double *M_dev, uint8_t *ok_dev);
 
 /* ---- SURVEY 8(f) N4: utils::byte_data_to_opencv (utils.rs:8-52 = cv::imdecode(bytes, IMREAD_UNCHANGED)), baseline JPEG ------- */
 /* Host-only header parse: image size and luma sampling (11 = 4:4:4, 21 = 4:2:2, 22 = 4:2:0).  FD_ERR_INVALID for streams the

@@ -149,13 +149,17 @@ __device__ __forceinline__ void load6_safe(const uint8_t *p, const uint8_t *lo_l
 // 15-bit table entries are exact multiples of 32).  Integer arithmetic is exact, so the sum is evaluated separably:
 // horizontal 2-tap dot products with 6-bit weights (dp4a on the packed byte pair), then the vertical pair; and
 // (32*S + 2^14) >> 15 == (S + 512) >> 10.  Returns the pixel as b | g << 8 | r << 16.
+// RB: the taps are R,G,B (RGB24), so channels 0 and 2 are taken the other way round.  Bytes 6 and 7 of [lo | hi] contribute
+// nothing (their weights are 0), so a caller may leave them undefined.
+template <bool RB = false>
 __device__ __forceinline__ unsigned blend24(unsigned lo0, unsigned hi0, unsigned lo1, unsigned hi1, int ax, int ay) {
+    constexpr unsigned SB = RB ? 0x7752 : 0x7730, SR = RB ? 0x7730 : 0x7752;
     const unsigned wx = (unsigned)(32 - ax) | ((unsigned)ax << 8);   // bytes: [32-ax, ax, 0, 0]
     const int wy0 = 32 - ay, wy1 = ay;
     // byte pairs (tap0, tap1) per channel: b = bytes (0,3), g = (1,4), r = (2,5) of [lo | hi]
-    const int hb0 = (int)__dp4a(__byte_perm(lo0, hi0, 0x7730), wx, 0u), hb1 = (int)__dp4a(__byte_perm(lo1, hi1, 0x7730), wx, 0u);
+    const int hb0 = (int)__dp4a(__byte_perm(lo0, hi0, SB), wx, 0u), hb1 = (int)__dp4a(__byte_perm(lo1, hi1, SB), wx, 0u);
     const int hg0 = (int)__dp4a(__byte_perm(lo0, hi0, 0x7741), wx, 0u), hg1 = (int)__dp4a(__byte_perm(lo1, hi1, 0x7741), wx, 0u);
-    const int hr0 = (int)__dp4a(__byte_perm(lo0, hi0, 0x7752), wx, 0u), hr1 = (int)__dp4a(__byte_perm(lo1, hi1, 0x7752), wx, 0u);
+    const int hr0 = (int)__dp4a(__byte_perm(lo0, hi0, SR), wx, 0u), hr1 = (int)__dp4a(__byte_perm(lo1, hi1, SR), wx, 0u);
     const unsigned ob = (unsigned)(hb0 * wy0 + hb1 * wy1 + 512) >> 10;
     const unsigned og = (unsigned)(hg0 * wy0 + hg1 * wy1 + 512) >> 10;
     const unsigned orr = (unsigned)(hr0 * wy0 + hr1 * wy1 + 512) >> 10;
@@ -163,20 +167,37 @@ __device__ __forceinline__ unsigned blend24(unsigned lo0, unsigned hi0, unsigned
 }
 
 // blend24 for the fixed-size kernel: ay6 = ay << 6, so each channel's sum lands in byte 2 of its word ((S + 512) << 6 < 2^24) and
-// two byte permutes assemble the pixel instead of three shifts and two merges.
+// two byte permutes assemble the pixel instead of three shifts and two merges.  RB: as for blend24.
+template <bool RB = false>
 __device__ __forceinline__ unsigned blend24_scaled(unsigned lo0, unsigned hi0, unsigned lo1, unsigned hi1, int ax, int ay6) {
+    constexpr unsigned SB = RB ? 0x7752 : 0x7730, SR = RB ? 0x7730 : 0x7752;
     const unsigned wx = (unsigned)(32 - ax) | ((unsigned)ax << 8);
     const int wy0 = 2048 - ay6, wy1 = ay6;
-    const int hb0 = (int)__dp4a(__byte_perm(lo0, hi0, 0x7730), wx, 0u), hb1 = (int)__dp4a(__byte_perm(lo1, hi1, 0x7730), wx, 0u);
+    const int hb0 = (int)__dp4a(__byte_perm(lo0, hi0, SB), wx, 0u), hb1 = (int)__dp4a(__byte_perm(lo1, hi1, SB), wx, 0u);
     const int hg0 = (int)__dp4a(__byte_perm(lo0, hi0, 0x7741), wx, 0u), hg1 = (int)__dp4a(__byte_perm(lo1, hi1, 0x7741), wx, 0u);
-    const int hr0 = (int)__dp4a(__byte_perm(lo0, hi0, 0x7752), wx, 0u), hr1 = (int)__dp4a(__byte_perm(lo1, hi1, 0x7752), wx, 0u);
+    const int hr0 = (int)__dp4a(__byte_perm(lo0, hi0, SR), wx, 0u), hr1 = (int)__dp4a(__byte_perm(lo1, hi1, SR), wx, 0u);
     const unsigned sb = (unsigned)(hb0 * wy0 + hb1 * wy1 + 32768);
     const unsigned sg = (unsigned)(hg0 * wy0 + hg1 * wy1 + 32768);
     const unsigned sr = (unsigned)(hr0 * wy0 + hr1 * wy1 + 32768);
     return __byte_perm(__byte_perm(sb, sg, 0x7762), sr, 0x7610);   // b | g << 8 | r << 16, byte 3 = 0
 }
 
+// blend24 / blend24_scaled of a GRAY8 tap square: the one channel is blended once and replicated.  g0, g1: the tap bytes
+// (sx, sx+1) of rows sy, sy+1 in bytes 0 and 1.
+__device__ __forceinline__ unsigned blend8(unsigned g0, unsigned g1, int ax, int ay) {
+    const unsigned wx = (unsigned)(32 - ax) | ((unsigned)ax << 8);
+    const int h0 = (int)__dp4a(g0, wx, 0u), h1 = (int)__dp4a(g1, wx, 0u);
+    return ((unsigned)(h0 * (32 - ay) + h1 * ay + 512) >> 10) * 0x010101u;
+}
+__device__ __forceinline__ unsigned blend8_scaled(unsigned g0, unsigned g1, int ax, int ay6) {
+    const unsigned wx = (unsigned)(32 - ax) | ((unsigned)ax << 8);
+    const int h0 = (int)__dp4a(g0, wx, 0u), h1 = (int)__dp4a(g1, wx, 0u);
+    return __byte_perm((unsigned)(h0 * (2048 - ay6) + h1 * ay6 + 32768), 0u, 0x4222);   // byte 2 thrice, byte 3 = 0
+}
+
 // One output pixel with per-tap BORDER_CONSTANT(0) tests; X, Y are the 5-bit sub-pixel fixed-point source coordinates.
+// RB: an RGB24 frame (blend24<true>).
+template <bool RB = false>
 __device__ __forceinline__ unsigned border_tap_blend(const uint8_t *data, int w, int h, int pitch, const uint8_t *lo_lim,
                                                      const uint8_t *hi_lim, int X, int Y) {
     unsigned lo0 = 0, hi0 = 0, lo1 = 0, hi1 = 0;
@@ -198,7 +219,7 @@ __device__ __forceinline__ unsigned border_tap_blend(const uint8_t *data, int w,
         if (inx0) { lo0 = t0; lo1 = t1; }              // tap 0 valid, tap 1 (bytes 3..5) zero
         else { lo0 = t0 << 24; hi0 = t0 >> 8; lo1 = t1 << 24; hi1 = t1 >> 8; }  // tap 1 valid
     }
-    return blend24(lo0, hi0, lo1, hi1, X & 31, Y & 31);
+    return blend24<RB>(lo0, hi0, lo1, hi1, X & 31, Y & 31);
 }
 
 // ---- 4:2:0 sources: the four taps are converted to BGR (yuv_bgr24) and blended with the same arithmetic --------------
@@ -301,14 +322,48 @@ __device__ __forceinline__ void packed_row_taps(unsigned a, unsigned b, unsigned
     b = __byte_perm(b, 0u, sel);
     pack6(packed_bgr24(a, odd ? 1 : 0), packed_bgr24(b, odd ? 0 : 1), lo, hi);
 }
-// the tap square of a YUV format (FMT: SRC_NV12, SRC_NV21, SRC_PLANAR or SRC_PACKED422); sel: packed only
+// The same square of an RGBA / BGRA frame (data and pitch 4-byte aligned): per tap row, the words of pixels sx and sx+1
+// (8 bytes at 4-byte alignment).  No byte outside the four tap pixels is read.  sel reorders a word to B,G,R,x.
+struct Px32Quad {
+    unsigned r0[2], r1[2];   // words of columns sx, sx+1 in tap rows sy, sy+1
+    unsigned sel;
+};
+__device__ __forceinline__ void px32_quad_load(const uint8_t *p, unsigned pitch, unsigned sel, int sx, int sy, Px32Quad &q) {
+    const unsigned o = (unsigned)sy * pitch + 4u * (unsigned)sx;
+    const unsigned *w0 = reinterpret_cast<const unsigned *>(p + o), *w1 = reinterpret_cast<const unsigned *>(p + o + pitch);
+    q.r0[0] = __ldg(w0); q.r0[1] = __ldg(w0 + 1);
+    q.r1[0] = __ldg(w1); q.r1[1] = __ldg(w1 + 1);
+    q.sel = sel;
+}
+// blend24's (lo, hi) from the words a, b of two adjacent pixels: lo = B0 G0 R0 B1, hi = G1 R1 and two unused bytes
+__device__ __forceinline__ void px32_row_taps(unsigned a, unsigned b, unsigned sel, unsigned &lo, unsigned &hi) {
+    lo = __byte_perm(a, b, (sel & 0xfffu) | ((4u + (sel & 3u)) << 12));
+    hi = __byte_perm(b, 0u, sel >> 4);
+}
+// The same square of a GRAY8 frame: the four tap bytes, one byte load each (any alignment; nothing else is read).
+struct GrayQuad {
+    unsigned r0, r1;   // bytes (sx, sx+1) of tap rows sy, sy+1 in bytes 0 and 1
+};
+__device__ __forceinline__ void gray_quad_load(const uint8_t *p, unsigned pitch, int sx, int sy, GrayQuad &q) {
+    const uint8_t *t0 = p + (unsigned)sy * pitch + (unsigned)sx, *t1 = t0 + pitch;
+    q.r0 = (unsigned)__ldg(t0) | ((unsigned)__ldg(t0 + 1) << 8);
+    q.r1 = (unsigned)__ldg(t1) | ((unsigned)__ldg(t1 + 1) << 8);
+}
+// the tap square of a format whose taps are converted before the blend (FMT: SRC_NV12, SRC_NV21, SRC_PLANAR, SRC_PACKED422,
+// SRC_PX32 or SRC_GRAY8); sel: packed 4:2:2 and RGBA / BGRA only
 template <int FMT>
-using YuvQuad = typename std::conditional<FMT == SRC_PLANAR, PlanarQuad, typename std::conditional<FMT == SRC_PACKED422, PackedQuad, Nv12Quad>::type>::type;
+using YuvQuad = typename std::conditional<
+    FMT == SRC_PLANAR, PlanarQuad,
+    typename std::conditional<FMT == SRC_PACKED422, PackedQuad,
+                              typename std::conditional<FMT == SRC_PX32, Px32Quad,
+                                                        typename std::conditional<FMT == SRC_GRAY8, GrayQuad, Nv12Quad>::type>::type>::type>::type;
 template <int FMT>
 __device__ __forceinline__ void yuv_quad_load(const uint8_t *yp, unsigned py, const uint8_t *uvp, const uint8_t *vp, unsigned puv, unsigned sel,
                                               int sx, int sy, YuvQuad<FMT> &q) {
     if constexpr (FMT == SRC_PLANAR) planar_quad_load(yp, py, uvp, vp, puv, sx, sy, q);
     else if constexpr (FMT == SRC_PACKED422) packed_quad_load(yp, py, sel, sx, sy, q);
+    else if constexpr (FMT == SRC_PX32) px32_quad_load(yp, py, sel, sx, sy, q);
+    else if constexpr (FMT == SRC_GRAY8) gray_quad_load(yp, py, sx, sy, q);
     else nv12_quad_load(yp, py, uvp, puv, sx, sy, q);
 }
 template <int FMT>
@@ -318,14 +373,21 @@ __device__ __forceinline__ void yuv_quad_taps(const YuvQuad<FMT> &q, unsigned &l
     } else if constexpr (FMT == SRC_PACKED422) {
         packed_row_taps(q.r0[0], q.r0[1], q.sel, q.odd, lo0, hi0);
         packed_row_taps(q.r1[0], q.r1[1], q.sel, q.odd, lo1, hi1);
+    } else if constexpr (FMT == SRC_PX32) {
+        px32_row_taps(q.r0[0], q.r0[1], q.sel, lo0, hi0);
+        px32_row_taps(q.r1[0], q.r1[1], q.sel, lo1, hi1);
     } else {
         nv12_quad_taps<FMT>(q, lo0, hi0, lo1, hi1);
     }
 }
-// pixel (xx, yy) of a YUV frame inside it (vp: the V plane, planar only; sel: packed only)
+// pixel (xx, yy) of a converted-tap frame inside it (vp: the V plane, planar only; sel: packed 4:2:2 and RGBA / BGRA only)
 template <int FMT>
 __device__ __forceinline__ unsigned yuv_tap(const uint8_t *yp, int py, const uint8_t *uvp, const uint8_t *vp, int puv, unsigned sel, int xx, int yy) {
-    if constexpr (FMT == SRC_PACKED422)
+    if constexpr (FMT == SRC_PX32)
+        return px32_px24(yp + (ptrdiff_t)yy * py, sel, xx);
+    else if constexpr (FMT == SRC_GRAY8)
+        return (unsigned)__ldg(yp + (ptrdiff_t)yy * py + xx) * 0x010101u;
+    else if constexpr (FMT == SRC_PACKED422)
         return packed_px24(yp + (ptrdiff_t)yy * py, sel, xx);
     else if constexpr (FMT == SRC_PLANAR)
         return yuv_bgr24(__ldg(yp + (ptrdiff_t)yy * py + xx), __ldg(uvp + (ptrdiff_t)(yy >> 1) * puv + (xx >> 1)),
@@ -337,7 +399,8 @@ __device__ __forceinline__ unsigned yuv_tap(const uint8_t *yp, int py, const uin
         return yuv_bgr24(__ldg(yp + (ptrdiff_t)yy * py + xx), __ldg(uvp + (ptrdiff_t)(yy >> 1) * puv + (xx & ~1)),
                          __ldg(uvp + (ptrdiff_t)(yy >> 1) * puv + (xx | 1)));
 }
-// border_tap_blend for a YUV frame: BORDER_CONSTANT(0) applies to the BGR image, so a tap outside the frame is BGR (0,0,0)
+// border_tap_blend for a converted-tap frame: BORDER_CONSTANT(0) applies to the BGR image, so a tap outside the frame is BGR
+// (0,0,0).  Reads only the bytes of the taps inside the frame (RGBA / BGRA: three bytes of a pixel; GRAY8: one).
 template <int FMT>
 __device__ __forceinline__ unsigned border_tap_blend_yuv(const uint8_t *yp, int py, const uint8_t *uvp, const uint8_t *vp, int puv, unsigned sel,
                                                          int w, int h, int X, int Y) {
@@ -363,12 +426,14 @@ __device__ __forceinline__ bool nv12_interior_ok(const FrameDev &f) {
            f.pitch >= 8 && f.pitch_uv >= 8 && (size_t)f.h * f.pitch < 0x7fffffffull && (size_t)f.h * f.pitch_uv < 0x7fffffffull;
 }
 // A packed frame's interior reads stay inside the two tap columns' words (W is even, so a macropixel never straddles the
-// end of a row): only the 4-byte alignment and 32-bit offsets are needed.
+// end of a row): only the 4-byte alignment and 32-bit offsets are needed.  The same holds for an RGBA / BGRA frame, whose
+// interior reads are the four tap pixels' words, and a GRAY8 frame's interior reads are the four tap bytes (no alignment).
 template <int FMT>
 __device__ __forceinline__ bool yuv_interior_ok(const FrameDev &f) {
     if constexpr (FMT == SRC_PLANAR) return nv12_interior_ok(f) && (f.v_off & 3) == 0;   // the V plane too
-    else if constexpr (FMT == SRC_PACKED422)
+    else if constexpr (FMT == SRC_PACKED422 || FMT == SRC_PX32)
         return ((reinterpret_cast<uintptr_t>(f.data) | (uintptr_t)f.pitch) & 3) == 0 && (size_t)f.h * f.pitch < 0x7fffffffull;
+    else if constexpr (FMT == SRC_GRAY8) return (size_t)f.h * f.pitch < 0x7fffffffull;
     else return nv12_interior_ok(f);
 }
 
@@ -395,7 +460,7 @@ struct WarpItem {
     const uint8_t *uv;   // 4:2:0 only
     int pitch_uv;
     const uint8_t *v;    // planar only
-    unsigned sel;        // packed 4:2:2 only
+    unsigned sel;        // packed 4:2:2 and RGBA / BGRA only
 };
 
 // N rounds of WARP_THREADS consecutive output pixels starting at p0: all 4N aligned 64-bit loads of a thread are issued
@@ -417,14 +482,20 @@ __device__ __forceinline__ void warp_rounds_interior_yuv(const WarpItem &it, con
 #pragma unroll
     for (int u = 0; u < N; ++u) {
         const int p = p0 + u * WARP_THREADS;
-        unsigned lo0, hi0, lo1, hi1;
-        yuv_quad_taps<FMT>(q[u], lo0, hi0, lo1, hi1);
-        const unsigned v = blend24(lo0, hi0, lo1, hi1, axy[u] & 31, axy[u] >> 8);
+        unsigned v;
+        if constexpr (FMT == SRC_GRAY8) {
+            v = blend8(q[u].r0, q[u].r1, axy[u] & 31, axy[u] >> 8);
+        } else {
+            unsigned lo0, hi0, lo1, hi1;
+            yuv_quad_taps<FMT>(q[u], lo0, hi0, lo1, hi1);
+            v = blend24(lo0, hi0, lo1, hi1, axy[u] & 31, axy[u] >> 8);
+        }
         store_px(band_out, p, v, p < npix, packed);
     }
 }
 
-template <int N>
+// RB: an RGB24 frame (blend24<true>)
+template <int N, bool RB = false>
 __device__ __forceinline__ void warp_rounds_interior(const WarpItem &it, const int2 *__restrict__ dxy, const int2 *__restrict__ xy0,
                                                      int cw, unsigned cw_magic, int p0, int npix, uint8_t *band_out, bool packed) {
     uint2 q[N][4];
@@ -450,7 +521,7 @@ __device__ __forceinline__ void warp_rounds_interior(const WarpItem &it, const i
         unsigned lo0, hi0, lo1, hi1;
         extract6(q[u][0], q[u][1], off[u], lo0, hi0);
         extract6(q[u][2], q[u][3], off[u] + pitch, lo1, hi1);
-        const unsigned v = blend24(lo0, hi0, lo1, hi1, axy[u] & 31, axy[u] >> 8);
+        const unsigned v = blend24<RB>(lo0, hi0, lo1, hi1, axy[u] & 31, axy[u] >> 8);
         store_px(band_out, p, v, p < npix, packed);
     }
 }
@@ -463,8 +534,9 @@ __device__ __forceinline__ void warp_round_border(const WarpItem &it, const int2
     const int row = cw_magic ? (int)__umulhi((unsigned)p, cw_magic) : p, x = p - row * cw;
     const int2 d = dxy[x], r0 = xy0[row];
     const int X = (int)((unsigned)r0.x + (unsigned)d.x) >> 5, Y = (int)((unsigned)r0.y + (unsigned)d.y) >> 5;
-    const unsigned v = FMT != SRC_BGR ? border_tap_blend_yuv<FMT>(it.data, it.pitch, it.uv, it.v, it.pitch_uv, it.sel, it.w, it.h, X, Y)
-                                      : border_tap_blend(it.data, it.w, it.h, it.pitch, it.lo_lim, it.hi_lim, X, Y);
+    const unsigned v = FMT != SRC_BGR && FMT != SRC_RGB24
+                           ? border_tap_blend_yuv<FMT>(it.data, it.pitch, it.uv, it.v, it.pitch_uv, it.sel, it.w, it.h, X, Y)
+                           : border_tap_blend<FMT == SRC_RGB24>(it.data, it.w, it.h, it.pitch, it.lo_lim, it.hi_lim, X, Y);
     store_px(band_out, p0, v, p0 < npix, packed);
 }
 
@@ -476,6 +548,8 @@ __device__ __forceinline__ void warp_round_border(const WarpItem &it, const int2
 template <int FMT>
 __global__ void __launch_bounds__(WARP_THREADS, 4) warp_kernel(WarpArgs a) {
     constexpr bool NV = FMT == SRC_NV12 || FMT == SRC_NV21 || FMT == SRC_PLANAR, PK = FMT == SRC_PACKED422;   // NV: 4:2:0
+    constexpr bool RG = FMT == SRC_RGB24, P4 = FMT == SRC_PX32, G1 = FMT == SRC_GRAY8;
+    constexpr bool CV = NV || PK || P4 || G1;   // taps converted to BGR before the blend (the others: 3-byte pixels)
     extern __shared__ int2 wsm[];
     int2 *dxy = wsm;             // [cw]  (adelta, bdelta)
     int2 *xy0 = dxy + a.cw;      // [WARP_BAND]  (X0, Y0) per row
@@ -511,6 +585,9 @@ __global__ void __launch_bounds__(WARP_THREADS, 4) warp_kernel(WarpArgs a) {
                                                                     a.ch, x, band_y0 + row)
                                        : PK ? resize_pixel24_packed(fr.data, fr.pitch, (unsigned)fr.v_off, rx0, ry0, fr.w - rx0, fr.h - ry0, a.cw, a.ch, x,
                                                                     band_y0 + row)
+                                       : P4 || G1 ? resize_pixel24_rgb<FMT>(fr.data, fr.pitch, (unsigned)fr.v_off, rx0, ry0, fr.w - rx0, fr.h - ry0, a.cw,
+                                                                            a.ch, x, band_y0 + row)
+                                       : RG ? swap_rb24(resize_pixel24(roi, fr.pitch, fr.w - rx0, fr.h - ry0, a.cw, a.ch, x, band_y0 + row))
                                           : resize_pixel24(roi, fr.pitch, fr.w - rx0, fr.h - ry0, a.cw, a.ch, x, band_y0 + row);
                     band_out[3 * p] = (uint8_t)v; band_out[3 * p + 1] = (uint8_t)(v >> 8); band_out[3 * p + 2] = (uint8_t)(v >> 16);
                 }
@@ -532,10 +609,10 @@ __global__ void __launch_bounds__(WARP_THREADS, 4) warp_kernel(WarpArgs a) {
         __syncthreads();
         // The map is affine, so the tap coordinates of the band are extremal at its 4 corners: if all 4 corner taps
         // (and their +1 neighbours) are interior, no pixel of the band needs a border test.
-        bool interior = NV || PK ? yuv_interior_ok<FMT>(fr)
-                                 : (reinterpret_cast<uintptr_t>(fr.data) & 7) == 0 && (fr.pitch & 7) == 0 && fr.pitch >= 16 &&
-                                       (size_t)fr.h * fr.pitch < 0x7fffffffull;
-        const int bottom = NV ? 2 : PK ? 0 : 1;   // rows kept from the bottom: the loads over-read past the last tap row
+        bool interior = CV ? yuv_interior_ok<FMT>(fr)
+                           : (reinterpret_cast<uintptr_t>(fr.data) & 7) == 0 && (fr.pitch & 7) == 0 && fr.pitch >= 16 &&
+                                 (size_t)fr.h * fr.pitch < 0x7fffffffull;
+        const int bottom = NV ? 2 : CV ? 0 : 1;   // rows kept from the bottom: the loads over-read past the last tap row
         {
             const int xs[2] = {0, a.cw - 1}, ys[2] = {0, rows - 1};
 #pragma unroll
@@ -553,9 +630,9 @@ __global__ void __launch_bounds__(WARP_THREADS, 4) warp_kernel(WarpArgs a) {
         it.hi_lim = fr.data + (size_t)(fr.h - 1) * fr.pitch + (size_t)fr.w * 3;  // end of valid pixel bytes
         it.uv = fr.uv; it.pitch_uv = fr.pitch_uv;
         if constexpr (FMT == SRC_PLANAR) it.v = fr.v_plane();
-        it.sel = PK ? (unsigned)fr.v_off : 0u;
+        it.sel = PK || P4 ? (unsigned)fr.v_off : 0u;
         int p0 = tid;
-        if ((NV || PK) && interior) {
+        if (CV && interior) {
             for (int rounds = (npix + WARP_THREADS - 1) / WARP_THREADS; rounds > 0; rounds -= 2, p0 += 2 * WARP_THREADS) {
                 if (rounds >= 2) warp_rounds_interior_yuv<FMT, 2>(it, dxy, xy0, a.cw, a.cw_magic, p0, npix, band_out, packed);
                 else warp_rounds_interior_yuv<FMT, 1>(it, dxy, xy0, a.cw, a.cw_magic, p0, npix, band_out, packed);
@@ -563,10 +640,10 @@ __global__ void __launch_bounds__(WARP_THREADS, 4) warp_kernel(WarpArgs a) {
         } else if (interior) {
             int rounds = (npix + WARP_THREADS - 1) / WARP_THREADS;
             while (rounds > 0) {
-                if (rounds >= 4) { warp_rounds_interior<4>(it, dxy, xy0, a.cw, a.cw_magic, p0, npix, band_out, packed); rounds -= 4; p0 += 4 * WARP_THREADS; }
-                else if (rounds == 3) { warp_rounds_interior<3>(it, dxy, xy0, a.cw, a.cw_magic, p0, npix, band_out, packed); rounds = 0; }
-                else if (rounds == 2) { warp_rounds_interior<2>(it, dxy, xy0, a.cw, a.cw_magic, p0, npix, band_out, packed); rounds = 0; }
-                else { warp_rounds_interior<1>(it, dxy, xy0, a.cw, a.cw_magic, p0, npix, band_out, packed); rounds = 0; }
+                if (rounds >= 4) { warp_rounds_interior<4, RG>(it, dxy, xy0, a.cw, a.cw_magic, p0, npix, band_out, packed); rounds -= 4; p0 += 4 * WARP_THREADS; }
+                else if (rounds == 3) { warp_rounds_interior<3, RG>(it, dxy, xy0, a.cw, a.cw_magic, p0, npix, band_out, packed); rounds = 0; }
+                else if (rounds == 2) { warp_rounds_interior<2, RG>(it, dxy, xy0, a.cw, a.cw_magic, p0, npix, band_out, packed); rounds = 0; }
+                else { warp_rounds_interior<1, RG>(it, dxy, xy0, a.cw, a.cw_magic, p0, npix, band_out, packed); rounds = 0; }
             }
         } else {
             for (; p0 - tid < npix; p0 += WARP_THREADS) warp_round_border<FMT>(it, dxy, xy0, a.cw, a.cw_magic, p0, npix, band_out, packed);
@@ -594,8 +671,8 @@ __global__ void __launch_bounds__(WARP_THREADS, 4) warp_kernel(WarpArgs a) {
 #define WARP_LD(p) __ldg(p)
 #endif
 // pack_sel: the byte permute that cuts this lane's word out of (its pixel, the next lane's pixel): lanes 0..2 of a quad store
-// bytes 0-3, 4-7, 8-11 of the quad's 12.
-template <int CW, int N>
+// bytes 0-3, 4-7, 8-11 of the quad's 12.  RB: an RGB24 frame (blend24_scaled<true>).
+template <int CW, int N, bool RB = false>
 __device__ __forceinline__ void fixed_rounds_interior(const uint8_t *__restrict__ data, unsigned pitch, int2 d, const int2 *__restrict__ xy,
                                                       unsigned *__restrict__ outw, bool store, unsigned pack_sel) {
     uint2 q[N][4];
@@ -619,7 +696,7 @@ __device__ __forceinline__ void fixed_rounds_interior(const uint8_t *__restrict_
         const unsigned sft = (off[u] & 3u) * 8;
         const unsigned a0 = up ? q[u][0].y : q[u][0].x, b0 = up ? q[u][1].x : q[u][0].y, c0 = up ? q[u][1].y : q[u][1].x;
         const unsigned a1 = up ? q[u][2].y : q[u][2].x, b1 = up ? q[u][3].x : q[u][2].y, c1 = up ? q[u][3].y : q[u][3].x;
-        const unsigned v = blend24_scaled(__funnelshift_r(a0, b0, sft), __funnelshift_r(b0, c0, sft), __funnelshift_r(a1, b1, sft),
+        const unsigned v = blend24_scaled<RB>(__funnelshift_r(a0, b0, sft), __funnelshift_r(b0, c0, sft), __funnelshift_r(a1, b1, sft),
                                           __funnelshift_r(b1, c1, sft), axy[u] & 31, axy[u] >> 8);
         const unsigned nv = __shfl_down_sync(0xffffffffu, v, 1);
         if (store) outw[u * (2 * CW * 3 / 4)] = __byte_perm(v, nv, pack_sel);
@@ -641,9 +718,14 @@ __device__ __forceinline__ void fixed_rounds_interior_yuv(const uint8_t *__restr
     }
 #pragma unroll
     for (int u = 0; u < N; ++u) {
-        unsigned lo0, hi0, lo1, hi1;
-        yuv_quad_taps<FMT>(q[u], lo0, hi0, lo1, hi1);
-        const unsigned v = blend24_scaled(lo0, hi0, lo1, hi1, axy[u] & 31, axy[u] >> 8);
+        unsigned v;
+        if constexpr (FMT == SRC_GRAY8) {
+            v = blend8_scaled(q[u].r0, q[u].r1, axy[u] & 31, axy[u] >> 8);
+        } else {
+            unsigned lo0, hi0, lo1, hi1;
+            yuv_quad_taps<FMT>(q[u], lo0, hi0, lo1, hi1);
+            v = blend24_scaled(lo0, hi0, lo1, hi1, axy[u] & 31, axy[u] >> 8);
+        }
         const unsigned nv = __shfl_down_sync(0xffffffffu, v, 1);
         if (store) outw[u * (2 * CW * 3 / 4)] = __byte_perm(v, nv, pack_sel);
     }
@@ -653,6 +735,8 @@ __device__ __forceinline__ void fixed_rounds_interior_yuv(const uint8_t *__restr
 template <int CW, int CH, int IR, int UN, int FMT>
 __global__ void __launch_bounds__(2 * CW) warp_fixed_kernel(WarpArgs a) {
     constexpr bool NV = FMT == SRC_NV12 || FMT == SRC_NV21 || FMT == SRC_PLANAR, PK = FMT == SRC_PACKED422;   // NV: 4:2:0
+    constexpr bool RG = FMT == SRC_RGB24, P4 = FMT == SRC_PX32, G1 = FMT == SRC_GRAY8;
+    constexpr bool CV = NV || PK || P4 || G1;   // taps converted to BGR before the blend (the others: 3-byte pixels)
     constexpr int T = 2 * CW, ITEMS = CH / IR, ROUNDS = IR / 2;
     static_assert(CH % IR == 0 && IR % 2 == 0 && T % 32 == 0 && (2 * CW * 3) % 4 == 0 && (IR * CW * 3) % 4 == 0, "fixed warp geometry");
     __shared__ int2 xy0[2][IR];
@@ -687,7 +771,7 @@ __global__ void __launch_bounds__(2 * CW) warp_fixed_kernel(WarpArgs a) {
         const int pitch_uv = NV ? frp->pitch_uv : 0;
         const uint8_t *vp = nullptr;   // planar only
         if constexpr (FMT == SRC_PLANAR) vp = frp->v_plane();
-        const unsigned sel = PK ? (unsigned)frp->v_off : 0u;
+        const unsigned sel = PK || P4 ? (unsigned)frp->v_off : 0u;
         int2 d = make_int2(0, 0);
         bool vote = true;
         if (okf) {
@@ -704,13 +788,13 @@ __global__ void __launch_bounds__(2 * CW) warp_fixed_kernel(WarpArgs a) {
                     const long long Xl = (long long)(__double2int_rn((i1 * y + i2) * 1024) + 16) + __double2int_rn(i0 * cx * 1024);
                     const long long Yl = (long long)(__double2int_rn((i4 * y + i5) * 1024) + 16) + __double2int_rn(i3 * cx * 1024);
                     const long long sx = Xl >> 10, sy = Yl >> 10;
-                    vote = sx >= 0 && sx + 1 < fw && sy >= 0 && sy + 1 < fh - (NV ? 2 : PK ? 0 : 1);   // the over-read stays in the frame
+                    vote = sx >= 0 && sx + 1 < fw && sy >= 0 && sy + 1 < fh - (NV ? 2 : CV ? 0 : 1);   // the over-read stays in the frame
                 }
             }
         }
-        const bool interior = __syncthreads_and(vote) && (NV || PK ? yuv_interior_ok<FMT>(*frp)
-                                                                       : (reinterpret_cast<uintptr_t>(data) & 7) == 0 && (pitch & 7) == 0 && pitch >= 16 &&
-                                                                             (size_t)fh * pitch < 0x7fffffffull);
+        const bool interior = __syncthreads_and(vote) && (CV ? yuv_interior_ok<FMT>(*frp)
+                                                             : (reinterpret_cast<uintptr_t>(data) & 7) == 0 && (pitch & 7) == 0 && pitch >= 16 &&
+                                                                   (size_t)fh * pitch < 0x7fffffffull);
         const bool store = (tid & 3) != 3;
         unsigned *outw = reinterpret_cast<unsigned *>(band_out) + 3 * (tid >> 2) + (tid & 3);
         if (!okf) {   // estimation failed: bbox-crop fallback (face_alignment.rs:64-116), or a zero crop where the reference errs
@@ -722,6 +806,8 @@ __global__ void __launch_bounds__(2 * CW) warp_fixed_kernel(WarpArgs a) {
                 for (int u = 0; u < ROUNDS; ++u) {
                     const unsigned v = NV ? resize_pixel24_yuv<FMT>(data, pitch, uvp, vp, pitch_uv, rx0, ry0, fw - rx0, fh - ry0, CW, CH, x, y0 + r + 2 * u)
                                        : PK ? resize_pixel24_packed(data, pitch, sel, rx0, ry0, fw - rx0, fh - ry0, CW, CH, x, y0 + r + 2 * u)
+                                       : P4 || G1 ? resize_pixel24_rgb<FMT>(data, pitch, sel, rx0, ry0, fw - rx0, fh - ry0, CW, CH, x, y0 + r + 2 * u)
+                                       : RG ? swap_rb24(resize_pixel24(roi, pitch, fw - rx0, fh - ry0, CW, CH, x, y0 + r + 2 * u))
                                           : resize_pixel24(roi, pitch, fw - rx0, fh - ry0, CW, CH, x, y0 + r + 2 * u);
                     const unsigned nv = __shfl_down_sync(0xffffffffu, v, 1);
                     const unsigned word = __funnelshift_r(__byte_perm(v, nv, 0x4210), nv >> 8, 8 * (tid & 3u));
@@ -738,7 +824,7 @@ __global__ void __launch_bounds__(2 * CW) warp_fixed_kernel(WarpArgs a) {
             const unsigned pack_sel = (tid & 3) == 0 ? 0x4210u : ((tid & 3) == 1 ? 0x5421u : 0x6542u);
             int u = 0;
             constexpr int REM = ROUNDS % UN;
-            if (NV || PK) {
+            if (CV) {
 #pragma unroll 1
                 for (; u + UN <= ROUNDS; u += UN)
                     fixed_rounds_interior_yuv<CW, UN, FMT>(data, (unsigned)pitch, uvp, vp, (unsigned)pitch_uv, sel, d, xy + 2 * u,
@@ -748,16 +834,16 @@ __global__ void __launch_bounds__(2 * CW) warp_fixed_kernel(WarpArgs a) {
             } else {
 #pragma unroll 1
                 for (; u + UN <= ROUNDS; u += UN)
-                    fixed_rounds_interior<CW, UN>(data, (unsigned)pitch, d, xy + 2 * u, outw + u * (T * 3 / 4), store, pack_sel);
-                if (REM) fixed_rounds_interior<CW, REM ? REM : 1>(data, (unsigned)pitch, d, xy + 2 * (ROUNDS - REM), outw + (ROUNDS - REM) * (T * 3 / 4), store, pack_sel);
+                    fixed_rounds_interior<CW, UN, RG>(data, (unsigned)pitch, d, xy + 2 * u, outw + u * (T * 3 / 4), store, pack_sel);
+                if (REM) fixed_rounds_interior<CW, REM ? REM : 1, RG>(data, (unsigned)pitch, d, xy + 2 * (ROUNDS - REM), outw + (ROUNDS - REM) * (T * 3 / 4), store, pack_sel);
             }
         } else {
             const uint8_t *lo_lim = data, *hi_lim = data + (size_t)(fh - 1) * pitch + (size_t)fw * 3;  // end of valid pixel bytes
             for (int u = 0; u < ROUNDS; ++u) {
                 const int2 r0 = xy[2 * u];
                 const int X = (int)((unsigned)r0.x + (unsigned)d.x) >> 5, Y = (int)((unsigned)r0.y + (unsigned)d.y) >> 5;
-                const unsigned v = NV || PK ? border_tap_blend_yuv<FMT>(data, pitch, uvp, vp, pitch_uv, sel, fw, fh, X, Y)
-                                      : border_tap_blend(data, fw, fh, pitch, lo_lim, hi_lim, X, Y);
+                const unsigned v = CV ? border_tap_blend_yuv<FMT>(data, pitch, uvp, vp, pitch_uv, sel, fw, fh, X, Y)
+                                      : border_tap_blend<RG>(data, fw, fh, pitch, lo_lim, hi_lim, X, Y);
                 const unsigned nv = __shfl_down_sync(0xffffffffu, v, 1);
                 const unsigned word = __funnelshift_r(__byte_perm(v, nv, 0x4210), nv >> 8, 8 * (tid & 3u));
                 if (store) outw[u * (T * 3 / 4)] = word;
@@ -848,12 +934,18 @@ static void (*fixed_kernel_for(int fmt))(WarpArgs) {
     return fmt == SRC_NV12 ? warp_fixed_kernel<112, 112, IR, 4, SRC_NV12>
            : fmt == SRC_NV21 ? warp_fixed_kernel<112, 112, IR, 4, SRC_NV21>
            : fmt == SRC_PLANAR ? warp_fixed_kernel<112, 112, IR, 2, SRC_PLANAR>
-           : fmt == SRC_PACKED422 ? warp_fixed_kernel<112, 112, IR, 4, SRC_PACKED422> : warp_fixed_kernel<112, 112, IR, 4, SRC_BGR>;
+           : fmt == SRC_PACKED422 ? warp_fixed_kernel<112, 112, IR, 4, SRC_PACKED422>
+           : fmt == SRC_RGB24 ? warp_fixed_kernel<112, 112, IR, 4, SRC_RGB24>
+           : fmt == SRC_PX32 ? warp_fixed_kernel<112, 112, IR, 4, SRC_PX32>
+           : fmt == SRC_GRAY8 ? warp_fixed_kernel<112, 112, IR, 4, SRC_GRAY8> : warp_fixed_kernel<112, 112, IR, 4, SRC_BGR>;
 }
-// launch names by source format (I420 and YV12 share the planar instantiations, YUY2, UYVY and YVYU the packed ones)
-static const char *const FIXED_NAMES[5] = {"warp_fixed_kernel", "warp_fixed_kernel_nv12", "warp_fixed_kernel_nv21", "warp_fixed_kernel_i420",
-                                           "warp_fixed_kernel_yuv422"};
-static const char *const WARP_NAMES[5] = {"warp_kernel", "warp_kernel_nv12", "warp_kernel_nv21", "warp_kernel_i420", "warp_kernel_yuv422"};
+// launch names by source format (I420 and YV12 share the planar instantiations, YUY2, UYVY and YVYU the packed ones, RGBA
+// and BGRA the 4-byte ones)
+static const char *const FIXED_NAMES[SRC_FMT_COUNT] = {"warp_fixed_kernel",       "warp_fixed_kernel_nv12",   "warp_fixed_kernel_nv21",
+                                                       "warp_fixed_kernel_i420",  "warp_fixed_kernel_yuv422", "warp_fixed_kernel_rgb24",
+                                                       "warp_fixed_kernel_rgba",  "warp_fixed_kernel_gray8"};
+static const char *const WARP_NAMES[SRC_FMT_COUNT] = {"warp_kernel",      "warp_kernel_nv12",   "warp_kernel_nv21", "warp_kernel_i420",
+                                                      "warp_kernel_yuv422", "warp_kernel_rgb24", "warp_kernel_rgba", "warp_kernel_gray8"};
 
 // fmt: the source format of frames_dev (SrcFmt)
 int warp_launch(fd_ctx *ctx, const FrameDev *frames_dev, const int32_t *frame_idx_dev, const double *M12_dev,
@@ -893,7 +985,7 @@ int warp_launch(fd_ctx *ctx, const FrameDev *frames_dev, const int32_t *frame_id
         static const int ir_env = getenv("FD_WARP_IR") ? atoi(getenv("FD_WARP_IR")) : 14;   // A/B: 16-row items (7 per face, 8 rounds as 4 + 4): 82.0 vs 78.8 us on C2
         const int IR = ir_env == 16 ? 16 : 14;
         void (*kern)(WarpArgs) = IR == 16 ? fixed_kernel_for<16>(fmt) : fixed_kernel_for<14>(fmt);
-        static int per_sm_fixed[5] = {0, 0, 0, 0, 0};
+        static int per_sm_fixed[SRC_FMT_COUNT] = {};
         int &per_sm_k = per_sm_fixed[fmt];
         if (!per_sm_k) FD_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm_k, kern, 224, 0));
         const long long items = (long long)F_cap * (112 / IR);
@@ -922,7 +1014,10 @@ int warp_launch(fd_ctx *ctx, const FrameDev *frames_dev, const int32_t *frame_id
     void (*kern)(WarpArgs) = fmt == SRC_NV12 ? warp_kernel<SRC_NV12>
                              : fmt == SRC_NV21 ? warp_kernel<SRC_NV21>
                              : fmt == SRC_PLANAR ? warp_kernel<SRC_PLANAR>
-                             : fmt == SRC_PACKED422 ? warp_kernel<SRC_PACKED422> : warp_kernel<SRC_BGR>;
+                             : fmt == SRC_PACKED422 ? warp_kernel<SRC_PACKED422>
+                             : fmt == SRC_RGB24 ? warp_kernel<SRC_RGB24>
+                             : fmt == SRC_PX32 ? warp_kernel<SRC_PX32>
+                             : fmt == SRC_GRAY8 ? warp_kernel<SRC_GRAY8> : warp_kernel<SRC_BGR>;
     FD_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, WARP_THREADS, smem));
     const long long items = (long long)F_cap * a.bands;
     const int grid = (int)std::min<long long>(items, (long long)ctx->num_sms * std::max(per_sm, 1));

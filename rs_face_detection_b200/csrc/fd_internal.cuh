@@ -53,11 +53,16 @@ enum SrcFmt : int {
     SRC_NV21 = 2,     // FrameDev::uv: interleaved V,U
     SRC_PLANAR = 3,   // I420 and YV12: FrameDev::uv is the U plane, FrameDev::v_plane() the V plane
     SRC_PACKED422 = 4,   // YUY2, UYVY and YVYU: FrameDev::data is the packed plane, FrameDev::v_off its byte-permute selector
+    SRC_RGB24 = 5,       // R,G,B: the BGR layout with channels 0 and 2 exchanged
+    SRC_PX32 = 6,        // RGBA and BGRA: 4 bytes a pixel, FrameDev::v_off the byte-permute selector to B,G,R,x
+    SRC_GRAY8 = 7,       // one byte a pixel, B = G = R
 };
+constexpr int SRC_FMT_COUNT = 8;
 
 // Per-frame descriptor as the kernels see it.
 struct FrameDev {
-    const uint8_t *data;     // BGR pixels, the Y plane of a 4:2:0 frame, or the packed plane of a 4:2:2 frame (h rows of 2w bytes)
+    const uint8_t *data;     // BGR pixels, the Y plane of a 4:2:0 frame, the packed plane of a 4:2:2 frame (h rows of 2w bytes),
+                             // or the interleaved pixels of an RGB24 / RGBA / BGRA / GRAY8 frame
     int h, w, pitch;
     int new_w, new_h;        // letterbox content size
     double scale_x, scale_y; // cv::resize inverse scales
@@ -65,7 +70,8 @@ struct FrameDev {
                              // of w/2 bytes); nullptr for a BGR or packed frame
     int pitch_uv;            // of the chroma plane(s)
     int v_off;               // planar: start of the V plane minus start of the U plane, in bytes; packed 4:2:2: the
-                             // __byte_perm selector that reorders a 2-pixel macropixel to Y0 U Y1 V; 0 otherwise (fills the
+                             // __byte_perm selector that reorders a 2-pixel macropixel to Y0 U Y1 V; RGBA / BGRA: the
+                             // selector that reorders a pixel word to B,G,R,x; 0 otherwise (fills the
                              // padding, so the table keeps its size)
     __host__ __device__ const uint8_t *v_plane() const { return uv + v_off; }   // planar only
 };

@@ -118,14 +118,42 @@ static int fill_frame_yuv422(const fd_ctx *ctx, const fd_frame &fr, int32_t layo
     return fill_geometry(ctx, fr.height, fr.width, out, det_scale);
 }
 
-// The frames of a batched call, device pointers: BGR (bgr), 4:2:0 (yuv, in the FD_YUV420_* layout `layout`) or packed 4:2:2
-// (packed, in the FD_YUV422_* layout `layout`); exactly one is set.
+// the kernels' source format of an FD_RGB_* layout, or -1
+static int rgb_format(int32_t layout) {
+    switch (layout) {
+    case FD_RGB_RGB24: return SRC_RGB24;
+    case FD_RGB_RGBA:
+    case FD_RGB_BGRA: return SRC_PX32;
+    case FD_RGB_GRAY8: return SRC_GRAY8;
+    default: return -1;
+    }
+}
+
+// bytes per pixel of a known FD_RGB_* layout
+static int rgb_bpp(int32_t layout) { return layout == FD_RGB_RGB24 ? 3 : layout == FD_RGB_GRAY8 ? 1 : 4; }
+
+// cv::cvtColor(COLOR_RGB2BGR / RGBA2BGR / BGRA2BGR / GRAY2BGR) accepts any size.  An RGBA / BGRA frame carries the
+// __byte_perm selector that reorders its pixel word to B,G,R,x.
+static int fill_frame_rgb(const fd_ctx *ctx, const fd_frame &fr, int32_t layout, FrameDev *out, float *det_scale) {
+    FD_REQUIRE(fr.data, "frame (RGB): null data");
+    FD_REQUIRE(fr.height > 0 && fr.width > 0 && (int64_t)fr.pitch >= rgb_bpp(layout) * (int64_t)fr.width,
+               "frame (RGB): bad geometry (pitch at least the bytes per pixel times the width)");
+    out->data = fr.data;
+    out->pitch = fr.pitch;
+    out->v_off = layout == FD_RGB_RGBA ? 0x3012 : layout == FD_RGB_BGRA ? 0x3210 : 0;
+    return fill_geometry(ctx, fr.height, fr.width, out, det_scale);
+}
+
+// The frames of a batched call, device pointers: BGR (bgr), 4:2:0 (yuv, in the FD_YUV420_* layout `layout`), packed 4:2:2
+// (packed, in the FD_YUV422_* layout `layout`) or interleaved RGB-family (rgb, in the FD_RGB_* layout `layout`); exactly one
+// is set.
 struct FrameList {
     const fd_frame *bgr = nullptr;
     const fd_frame_nv12 *yuv = nullptr;
     const fd_frame *packed = nullptr;
+    const fd_frame *rgb = nullptr;
     int32_t layout = FD_YUV420_NV12;
-    bool any() const { return bgr || yuv || packed; }
+    bool any() const { return bgr || yuv || packed || rgb; }
 };
 
 // the FrameList of a *_yuv420 call; an unknown layout is rejected here, before any call can return early
@@ -144,11 +172,20 @@ static int yuv422_frames(const fd_frame *frames, int32_t layout, FrameList *fl) 
     return FD_OK;
 }
 
-// uploads B descriptors and records their source format in ctx->frames_fmt; returns the widest staged source row in bytes
-// (BGR: 3w, NV12/NV21: w, planar: a U and a V half of round16(w/2) bytes each, packed 4:2:2: 2w)
+// the FrameList of an *_rgb call; an unknown layout is rejected here, before any call can return early
+static int rgb_frames(const fd_frame *frames, int32_t layout, FrameList *fl) {
+    FD_REQUIRE(rgb_format(layout) >= 0, "frame (RGB): unknown layout");
+    fl->rgb = frames;
+    fl->layout = layout;
+    return FD_OK;
+}
+
+// uploads B descriptors and records their source format in ctx->frames_fmt (the same buffers described as BGR and as RGB24
+// give byte-identical tables: only the format tells them apart); returns the widest staged source row in bytes (BGR and
+// RGB24: 3w, NV12/NV21: w, planar: a U and a V half of round16(w/2) bytes each, packed 4:2:2: 2w, RGBA / BGRA: 4w, GRAY8: w)
 static int upload_frame_table(fd_ctx *ctx, FrameList frames, int B, float *det_scale_host, int *max_row_bytes) {
-    // a known layout (yuv420_frames, yuv422_frames)
-    const int fmt = frames.packed ? SRC_PACKED422 : frames.yuv ? yuv420_format(frames.layout) : SRC_BGR;
+    // a known layout (yuv420_frames, yuv422_frames, rgb_frames)
+    const int fmt = frames.rgb ? rgb_format(frames.layout) : frames.packed ? SRC_PACKED422 : frames.yuv ? yuv420_format(frames.layout) : SRC_BGR;
     std::vector<FrameDev> tab(B);
     int mrb = 0;
     for (int i = 0; i < B; ++i) {
@@ -161,6 +198,9 @@ static int upload_frame_table(fd_ctx *ctx, FrameList frames, int B, float *det_s
         } else if (frames.packed) {
             FD_TRY(fill_frame_yuv422(ctx, frames.packed[i], frames.layout, &tab[i], &ds));
             mrb = std::max(mrb, 2 * frames.packed[i].width);
+        } else if (frames.rgb) {
+            FD_TRY(fill_frame_rgb(ctx, frames.rgb[i], frames.layout, &tab[i], &ds));
+            mrb = std::max(mrb, rgb_bpp(frames.layout) * frames.rgb[i].width);
         } else {
             FD_REQUIRE(frames.bgr[i].data != nullptr, "frame: null data");
             FD_TRY(fill_frame(ctx, frames.bgr[i], frames.bgr[i].data, &tab[i], &ds));
@@ -324,6 +364,8 @@ static int preprocess_batch(fd_ctx *ctx, FrameList frames, int B, float *out_nch
             aligned = aligned && row_ok(f.y, f.pitch_y, f.width) && row_ok(f.uv, f.pitch_uv, planar ? f.width / 2 : f.width);
         } else if (frames.packed) {
             aligned = aligned && row_ok(frames.packed[i].data, frames.packed[i].pitch, 2 * frames.packed[i].width);
+        } else if (frames.rgb) {
+            aligned = aligned && row_ok(frames.rgb[i].data, frames.rgb[i].pitch, rgb_bpp(frames.layout) * frames.rgb[i].width);
         } else {
             aligned = aligned && row_ok(frames.bgr[i].data, frames.bgr[i].pitch, frames.bgr[i].width * 3);
         }
@@ -347,6 +389,11 @@ FD_EXPORT int fd_preprocess_batch_nv12(fd_ctx *ctx, const fd_frame_nv12 *frames,
 FD_EXPORT int fd_preprocess_batch_yuv422(fd_ctx *ctx, const fd_frame *frames, int32_t layout, int B, float *out_nchw_dev, float *det_scale_host) {
     FrameList fl;
     FD_TRY(yuv422_frames(frames, layout, &fl));
+    return preprocess_batch(ctx, fl, B, out_nchw_dev, det_scale_host);
+}
+FD_EXPORT int fd_preprocess_batch_rgb(fd_ctx *ctx, const fd_frame *frames, int32_t layout, int B, float *out_nchw_dev, float *det_scale_host) {
+    FrameList fl;
+    FD_TRY(rgb_frames(frames, layout, &fl));
     return preprocess_batch(ctx, fl, B, out_nchw_dev, det_scale_host);
 }
 
@@ -448,6 +495,12 @@ FD_EXPORT int fd_align_batch_yuv422(fd_ctx *ctx, const fd_frame *frames, int32_t
     FD_TRY(yuv422_frames(frames, layout, &fl));
     return align_batch(ctx, fl, B, landmarks_dev, frame_idx_dev, bbox_dev, F, crops_dev, M_dev, ok_dev);
 }
+FD_EXPORT int fd_align_batch_rgb(fd_ctx *ctx, const fd_frame *frames, int32_t layout, int B, const float *landmarks_dev, const int32_t *frame_idx_dev,
+                                 const float *bbox_dev, int F, uint8_t *crops_dev, double *M_dev, uint8_t *ok_dev) {
+    FrameList fl;
+    FD_TRY(rgb_frames(frames, layout, &fl));
+    return align_batch(ctx, fl, B, landmarks_dev, frame_idx_dev, bbox_dev, F, crops_dev, M_dev, ok_dev);
+}
 
 static int align_detections(fd_ctx *ctx, FrameList frames, int B, uint8_t *crops_dev, int cap_faces, double *M_dev, uint8_t *ok_dev) {
     FD_TRY(check_ctx(ctx));
@@ -484,6 +537,12 @@ FD_EXPORT int fd_align_detections_yuv422(fd_ctx *ctx, const fd_frame *frames, in
                                          uint8_t *ok_dev) {
     FrameList fl;
     FD_TRY(yuv422_frames(frames, layout, &fl));
+    return align_detections(ctx, fl, B, crops_dev, cap_faces, M_dev, ok_dev);
+}
+FD_EXPORT int fd_align_detections_rgb(fd_ctx *ctx, const fd_frame *frames, int32_t layout, int B, uint8_t *crops_dev, int cap_faces, double *M_dev,
+                                      uint8_t *ok_dev) {
+    FrameList fl;
+    FD_TRY(rgb_frames(frames, layout, &fl));
     return align_detections(ctx, fl, B, crops_dev, cap_faces, M_dev, ok_dev);
 }
 
@@ -788,6 +847,12 @@ FD_EXPORT int fd_select_detections_yuv422(fd_ctx *ctx, const fd_frame *frames, i
     FD_TRY(yuv422_frames(frames, layout, &fl));
     return select_detections(ctx, fl, B, is_enroll, params, sel_host);
 }
+FD_EXPORT int fd_select_detections_rgb(fd_ctx *ctx, const fd_frame *frames, int32_t layout, int B, int is_enroll, const fd_select_params *params,
+                                       int32_t *sel_host) {
+    FrameList fl;
+    FD_TRY(rgb_frames(frames, layout, &fl));
+    return select_detections(ctx, fl, B, is_enroll, params, sel_host);
+}
 
 static int align_selected(fd_ctx *ctx, FrameList frames, int B, uint8_t *crops_dev, double *M_dev, uint8_t *ok_dev) {
     FD_TRY(check_ctx(ctx));
@@ -818,6 +883,11 @@ FD_EXPORT int fd_align_selected_nv12(fd_ctx *ctx, const fd_frame_nv12 *frames, i
 FD_EXPORT int fd_align_selected_yuv422(fd_ctx *ctx, const fd_frame *frames, int32_t layout, int B, uint8_t *crops_dev, double *M_dev, uint8_t *ok_dev) {
     FrameList fl;
     FD_TRY(yuv422_frames(frames, layout, &fl));
+    return align_selected(ctx, fl, B, crops_dev, M_dev, ok_dev);
+}
+FD_EXPORT int fd_align_selected_rgb(fd_ctx *ctx, const fd_frame *frames, int32_t layout, int B, uint8_t *crops_dev, double *M_dev, uint8_t *ok_dev) {
+    FrameList fl;
+    FD_TRY(rgb_frames(frames, layout, &fl));
     return align_selected(ctx, fl, B, crops_dev, M_dev, ok_dev);
 }
 

@@ -45,11 +45,14 @@ __device__ __forceinline__ const uint8_t *stage_row(uint8_t *buf, const uint8_t 
 
 // FMT: the source format (SrcFmt).  A YUV frame's taps are converted to BGR (yuv_bgr24) before the resize arithmetic.  A
 // 4:2:0 frame's staged rows are the Y rows and the chroma row(s) of the taps; a planar chroma row is staged as its U half and,
-// row_buf_bytes / 2 further, its V half.  A packed 4:2:2 frame stages its tap rows (2w bytes) as a BGR frame does.
+// row_buf_bytes / 2 further, its V half.  A packed 4:2:2 frame stages its tap rows (2w bytes) as a BGR frame does, and so
+// do the RGB-family frames (RGB24 3w, RGBA / BGRA 4w, GRAY8 w bytes).  Rows staged here keep the source's 16-byte phase, so
+// a 4-byte pixel is read as three bytes at any frame alignment.
 template <int FMT>
 __global__ void preprocess_kernel(PreArgs a) {
     constexpr bool NV = FMT == SRC_NV12 || FMT == SRC_NV21 || FMT == SRC_PLANAR, PL = FMT == SRC_PLANAR;   // NV: 4:2:0
     constexpr bool PK = FMT == SRC_PACKED422;
+    constexpr bool RG = FMT == SRC_RGB24, P4 = FMT == SRC_PX32, G1 = FMT == SRC_GRAY8;
     extern __shared__ __align__(16) unsigned char smem[];
     const int ow = a.out_w;
     float *lut = reinterpret_cast<float *>(smem);                  // [3][256], indexed by BGR channel
@@ -72,7 +75,7 @@ __global__ void preprocess_kernel(PreArgs a) {
     const FrameDev f = a.frames[blockIdx.y];
     for (int x = threadIdx.x; x < f.new_w; x += blockDim.x) {
         x_taps(x, f.scale_x, f.w, &xo0[x], &xo1[x], &xa0[x], &xa1[x]);
-        if (NV || PK) { xo0[x] /= 3; xo1[x] /= 3; }   // pixel, not byte, offsets
+        if (NV || PK || P4 || G1) { xo0[x] /= 3; xo1[x] /= 3; }   // pixel, not byte, offsets
     }
     __syncthreads();
     const float pad_r = lut[2 * 256], pad_g = lut[1 * 256], pad_b = lut[0];
@@ -81,8 +84,8 @@ __global__ void preprocess_kernel(PreArgs a) {
     const int ngroups = (ow + 3) >> 2;
     const int row_begin = blockIdx.x * PRE_ROWS;
     const int row_end = min(row_begin + PRE_ROWS, a.out_h);
-    const int src_row_bytes = NV ? f.w : PK ? 2 * f.w : f.w * 3;
-    const unsigned sel = PK ? (unsigned)f.v_off : 0u;
+    const int src_row_bytes = NV || G1 ? f.w : PK ? 2 * f.w : P4 ? 4 * f.w : f.w * 3;
+    const unsigned sel = PK || P4 ? (unsigned)f.v_off : 0u;
 
     for (int dy = row_begin; dy < row_end; ++dy) {
         float *o_r = out_img + (size_t)dy * ow;  // plane 0 = R (BGR channel 2), face_detection.rs:226-227
@@ -131,10 +134,22 @@ __global__ void preprocess_kernel(PreArgs a) {
                         vb[j] = lut[p & 255u];
                         vg[j] = lut[256 + ((p >> 8) & 255u)];
                         vr[j] = lut[512 + (p >> 16)];
-                    } else {
-                        vb[j] = lut[resize_px(r0, r1, x0, x1, a0, a1, b0, b1)];
+                    } else if (P4) {
+                        const unsigned p = resize_px24(px32_px24(r0, sel, x0), px32_px24(r0, sel, x1),
+                                                       b1 != 0 ? px32_px24(r1, sel, x0) : 0u, b1 != 0 ? px32_px24(r1, sel, x1) : 0u,
+                                                       a0, a1, b0, b1);
+                        vb[j] = lut[p & 255u];
+                        vg[j] = lut[256 + ((p >> 8) & 255u)];
+                        vr[j] = lut[512 + (p >> 16)];
+                    } else if (G1) {   // one resize indexes the three planes
+                        const int p = resize_px(r0, r1, x0, x1, a0, a1, b0, b1);
+                        vb[j] = lut[p];
+                        vg[j] = lut[256 + p];
+                        vr[j] = lut[512 + p];
+                    } else {   // BGR, or RGB24 with channels 0 and 2 exchanged
+                        vb[j] = lut[resize_px(r0, r1, x0 + (RG ? 2 : 0), x1 + (RG ? 2 : 0), a0, a1, b0, b1)];
                         vg[j] = lut[256 + resize_px(r0, r1, x0 + 1, x1 + 1, a0, a1, b0, b1)];
-                        vr[j] = lut[512 + resize_px(r0, r1, x0 + 2, x1 + 2, a0, a1, b0, b1)];
+                        vr[j] = lut[512 + resize_px(r0, r1, x0 + (RG ? 0 : 2), x1 + (RG ? 0 : 2), a0, a1, b0, b1)];
                     }
                 } else {
                     vb[j] = pad_b; vg[j] = pad_g; vr[j] = pad_r;
@@ -163,11 +178,19 @@ __global__ void preprocess_kernel(PreArgs a) {
 // (exact integer scales such as 1080p -> 640x360: scale 3, fractions 0) reduce to byte gathers; identity normalisation
 // skips the table.  Requires 16-byte aligned rows (base, pitch) — otherwise the v1 kernel above is used.
 constexpr int PRE2_STAGES = 4;
+// RGBA / BGRA rows are a third longer than BGR ones: with three stages a 4K frame's ring (94 KB) still leaves room for two
+// CTAs per SM, which four stages (123 KB) do not.
+template <int FMT> constexpr int PRE2_STAGES_OF = FMT == SRC_PX32 ? 3 : PRE2_STAGES;
 constexpr int PRE2_ROWS = 16;
 
 // pixel x of a packed 4:2:2 row staged at a 4-byte aligned address: its macropixel as one aligned word
 __device__ __forceinline__ unsigned packed_tap(const uint8_t *row, unsigned sel, int x) {
     return packed_bgr24(__byte_perm(*reinterpret_cast<const unsigned *>(row + 4 * (x >> 1)), 0u, sel), x);
+}
+// pixel x of an RGBA / BGRA row staged at a 4-byte aligned address: one aligned word reordered to B,G,R,x (byte 3 is then
+// the alpha, which the callers mask off)
+__device__ __forceinline__ unsigned px32_tap(const uint8_t *row, unsigned sel, int x) {
+    return __byte_perm(*reinterpret_cast<const unsigned *>(row + 4 * x), 0u, sel);
 }
 
 __device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -196,22 +219,27 @@ __device__ __forceinline__ void bulk_g2s(void *dst_smem, const void *src_gmem, u
 // taps map to the same chroma row (4K -> 640x360: rows 6y+2 and 6y+3 both read chroma row 3y+1).  A planar chroma row
 // fills its slot as the U half and, row_buf_bytes / 2 further, the V half: bulk copies of round16(w/2) bytes each.
 // Packed 4:2:2: a stage holds the packed tap rows (2w bytes each), and a tap reads its macropixel as one aligned word.
+// RGB family: a stage holds the tap rows (RGB24 3w, RGBA / BGRA 4w, GRAY8 w bytes); a 4-byte tap is one aligned word, and a
+// GRAY8 tap is resized once and indexes the three planes.
 template <bool IDENT, int FMT>
 __global__ void __launch_bounds__(256) preprocess_tma_kernel(PreArgs a) {
     constexpr bool NV = FMT == SRC_NV12 || FMT == SRC_NV21 || FMT == SRC_PLANAR, PL = FMT == SRC_PLANAR;   // NV: 4:2:0
     constexpr bool PK = FMT == SRC_PACKED422;
+    constexpr bool RG = FMT == SRC_RGB24, P4 = FMT == SRC_PX32, G1 = FMT == SRC_GRAY8;
+    constexpr bool PXO = NV || PK || P4 || G1;   // taps in pixels, not bytes
+    constexpr int STAGES = PRE2_STAGES_OF<FMT>;
     constexpr int SLOTS = NV ? 4 : 2;                           // rows per stage: Y0, Y1 (BGR: row 0, row 1), UV0, UV1
     extern __shared__ __align__(128) unsigned char smem[];
-    uint64_t *full = reinterpret_cast<uint64_t *>(smem);        // [PRE2_STAGES]
+    uint64_t *full = reinterpret_cast<uint64_t *>(smem);        // [STAGES]
     float *lut = reinterpret_cast<float *>(smem + 64);          // [3][256]
-    uint8_t *bufs = smem + 64 + 3072;                           // [PRE2_STAGES][SLOTS][row_buf_bytes]
+    uint8_t *bufs = smem + 64 + 3072;                           // [STAGES][SLOTS][row_buf_bytes]
     const int tid = threadIdx.x;
     const int ow = a.out_w;
     const int rb = a.row_buf_bytes;
 
     if (tid == 0) {
 #pragma unroll
-        for (int s = 0; s < PRE2_STAGES; ++s) mbar_init(&full[s], 1);
+        for (int s = 0; s < STAGES; ++s) mbar_init(&full[s], 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     if (!IDENT) {
@@ -235,7 +263,7 @@ __global__ void __launch_bounds__(256) preprocess_tma_kernel(PreArgs a) {
         if (x < f.new_w) {
             int o1;
             x_taps(x, f.scale_x, f.w, &x0[j], &o1, &wa0[j], &wa1[j]);
-            if (NV || PK) x0[j] /= 3;   // pixel, not byte, offset
+            if (PXO) x0[j] /= 3;   // pixel, not byte, offset
             point &= (wa1[j] == 0);
         }
     }
@@ -247,8 +275,8 @@ __global__ void __launch_bounds__(256) preprocess_tma_kernel(PreArgs a) {
     const int row_begin = blockIdx.x * PRE2_ROWS;
     const int row_end = min(row_begin + PRE2_ROWS, a.out_h);
     const int n_content = max(0, min(f.new_h, row_end) - row_begin);
-    const uint32_t copy_bytes = (uint32_t)(((NV ? f.w : PK ? 2 * f.w : f.w * 3) + 15) & ~15);
-    const unsigned sel = PK ? (unsigned)f.v_off : 0u;
+    const uint32_t copy_bytes = (uint32_t)(((NV || G1 ? f.w : PK ? 2 * f.w : P4 ? 4 * f.w : f.w * 3) + 15) & ~15);
+    const unsigned sel = PK || P4 ? (unsigned)f.v_off : 0u;
     const uint32_t half_bytes = (uint32_t)(((f.w >> 1) + 15) & ~15);   // PL: one U or V row
     const int half = rb >> 1;
     const bool active = 4 * tid < ow;
@@ -256,7 +284,7 @@ __global__ void __launch_bounds__(256) preprocess_tma_kernel(PreArgs a) {
     auto issue = [&](int it) {
         int y0, y1, b0, b1;
         y_taps(row_begin + it, f.scale_y, f.h, &y0, &y1, &b0, &b1);
-        const int st = it % PRE2_STAGES;
+        const int st = it % STAGES;
         uint8_t *dst = bufs + (size_t)st * SLOTS * rb;
         const bool uv1 = NV && b1 != 0 && (y1 >> 1) != (y0 >> 1);
         if (PL) mbar_expect_tx(&full[st], copy_bytes * (b1 != 0 ? 2 : 1) + half_bytes * (uv1 ? 4 : 2));
@@ -277,19 +305,19 @@ __global__ void __launch_bounds__(256) preprocess_tma_kernel(PreArgs a) {
         }
     };
     if (tid == 0)
-        for (int it = 0; it < PRE2_STAGES - 1 && it < n_content; ++it) issue(it);
+        for (int it = 0; it < STAGES - 1 && it < n_content; ++it) issue(it);
 
     for (int it = 0; it < n_content; ++it) {
-        if (tid == 0 && it + PRE2_STAGES - 1 < n_content) issue(it + PRE2_STAGES - 1);
+        if (tid == 0 && it + STAGES - 1 < n_content) issue(it + STAGES - 1);
         const int dy = row_begin + it;
         int y0, y1, b0, b1;
         y_taps(dy, f.scale_y, f.h, &y0, &y1, &b0, &b1);
-        const int st = it % PRE2_STAGES;
+        const int st = it % STAGES;
         const uint8_t *r0 = bufs + (size_t)st * SLOTS * rb;
         const uint8_t *r1 = b1 != 0 ? r0 + rb : r0;
         const uint8_t *c0 = r0 + 2 * rb, *c1 = b1 != 0 && (y1 >> 1) != (y0 >> 1) ? r0 + 3 * rb : c0;   // NV only
         const uint8_t *v0 = c0 + half, *v1 = c1 + half;                                               // PL only
-        mbar_wait(&full[st], (uint32_t)((it / PRE2_STAGES) & 1));
+        mbar_wait(&full[st], (uint32_t)((it / STAGES) & 1));
         if (active) {
             float vr[4], vg[4], vb[4];
             if (hpoint && b1 == 0) {
@@ -303,9 +331,14 @@ __global__ void __launch_bounds__(256) preprocess_tma_kernel(PreArgs a) {
                         } else if (NV) {
                             const unsigned p = yuv_px24<FMT>(r0, c0, v0, x0[j]);
                             pb = p & 255u; pg = (p >> 8) & 255u; pr = p >> 16;
-                        } else {
+                        } else if (P4) {
+                            const unsigned p = px32_tap(r0, sel, x0[j]);
+                            pb = p & 255u; pg = (p >> 8) & 255u; pr = (p >> 16) & 255u;
+                        } else if (G1) {
+                            pb = pg = pr = r0[x0[j]];
+                        } else {   // BGR, or RGB24 with channels 0 and 2 exchanged
                             const uint8_t *p = r0 + x0[j];
-                            pb = p[0]; pg = p[1]; pr = p[2];
+                            pb = p[RG ? 2 : 0]; pg = p[1]; pr = p[RG ? 0 : 2];
                         }
                         vb[j] = IDENT ? (float)pb : lut[pb];
                         vg[j] = IDENT ? (float)pg : lut[256 + pg];
@@ -318,7 +351,7 @@ __global__ void __launch_bounds__(256) preprocess_tma_kernel(PreArgs a) {
 #pragma unroll
                 for (int j = 0; j < 4; ++j) {
                     if (x0[j] >= 0) {
-                        const int o0 = x0[j], o1 = x0[j] + (wa1[j] != 0 ? (NV || PK ? 1 : 3) : 0), q0 = wa0[j], q1 = wa1[j];
+                        const int o0 = x0[j], o1 = x0[j] + (wa1[j] != 0 ? (PXO ? 1 : 3) : 0), q0 = wa0[j], q1 = wa1[j];
                         int pb, pg, pr;
                         if (PK) {
                             const unsigned p = resize_px24(packed_tap(r0, sel, o0), packed_tap(r0, sel, o1),
@@ -330,10 +363,17 @@ __global__ void __launch_bounds__(256) preprocess_tma_kernel(PreArgs a) {
                                                            b1 != 0 ? yuv_px24<FMT>(r1, c1, v1, o0) : 0u,
                                                            b1 != 0 ? yuv_px24<FMT>(r1, c1, v1, o1) : 0u, q0, q1, b0, b1);
                             pb = p & 255u; pg = (p >> 8) & 255u; pr = p >> 16;
-                        } else {
-                            pb = resize_px(r0, r1, o0, o1, q0, q1, b0, b1);
+                        } else if (P4) {   // resize_px24 keeps only bytes 0..2 of the taps: the alpha byte drops out
+                            const unsigned p = resize_px24(px32_tap(r0, sel, o0), px32_tap(r0, sel, o1),
+                                                           b1 != 0 ? px32_tap(r1, sel, o0) : 0u, b1 != 0 ? px32_tap(r1, sel, o1) : 0u,
+                                                           q0, q1, b0, b1);
+                            pb = p & 255u; pg = (p >> 8) & 255u; pr = p >> 16;
+                        } else if (G1) {
+                            pb = pg = pr = resize_px(r0, r1, o0, o1, q0, q1, b0, b1);
+                        } else {   // BGR, or RGB24 with channels 0 and 2 exchanged
+                            pb = resize_px(r0, r1, o0 + (RG ? 2 : 0), o1 + (RG ? 2 : 0), q0, q1, b0, b1);
                             pg = resize_px(r0, r1, o0 + 1, o1 + 1, q0, q1, b0, b1);
-                            pr = resize_px(r0, r1, o0 + 2, o1 + 2, q0, q1, b0, b1);
+                            pr = resize_px(r0, r1, o0 + (RG ? 0 : 2), o1 + (RG ? 0 : 2), q0, q1, b0, b1);
                         }
                         vb[j] = IDENT ? (float)pb : lut[pb];
                         vg[j] = IDENT ? (float)pg : lut[256 + pg];
@@ -455,22 +495,29 @@ int crops_to_tensor_launch(fd_ctx *ctx, const uint8_t *crops_dev, const int *cou
     return FD_OK;
 }
 
-// launch names by source format (I420 and YV12 share the planar instantiations, YUY2, UYVY and YVYU the packed ones)
-static const char *const TMA_NAMES[5] = {"preprocess_tma_kernel", "preprocess_tma_kernel_nv12", "preprocess_tma_kernel_nv21",
-                                         "preprocess_tma_kernel_i420", "preprocess_tma_kernel_yuv422"};
-static const char *const PRE_NAMES[5] = {"preprocess_kernel", "preprocess_kernel_nv12", "preprocess_kernel_nv21", "preprocess_kernel_i420",
-                                         "preprocess_kernel_yuv422"};
+// launch names by source format (I420 and YV12 share the planar instantiations, YUY2, UYVY and YVYU the packed ones, RGBA
+// and BGRA the 4-byte ones)
+static const char *const TMA_NAMES[SRC_FMT_COUNT] = {"preprocess_tma_kernel",      "preprocess_tma_kernel_nv12",  "preprocess_tma_kernel_nv21",
+                                                     "preprocess_tma_kernel_i420", "preprocess_tma_kernel_yuv422", "preprocess_tma_kernel_rgb24",
+                                                     "preprocess_tma_kernel_rgba", "preprocess_tma_kernel_gray8"};
+static const char *const PRE_NAMES[SRC_FMT_COUNT] = {"preprocess_kernel",      "preprocess_kernel_nv12",   "preprocess_kernel_nv21",
+                                                     "preprocess_kernel_i420", "preprocess_kernel_yuv422", "preprocess_kernel_rgb24",
+                                                     "preprocess_kernel_rgba", "preprocess_kernel_gray8"};
 
 template <bool IDENT>
 static void (*tma_kernel_for(int fmt))(PreArgs) {
     return fmt == SRC_NV12 ? preprocess_tma_kernel<IDENT, SRC_NV12>
            : fmt == SRC_NV21 ? preprocess_tma_kernel<IDENT, SRC_NV21>
            : fmt == SRC_PLANAR ? preprocess_tma_kernel<IDENT, SRC_PLANAR>
-           : fmt == SRC_PACKED422 ? preprocess_tma_kernel<IDENT, SRC_PACKED422> : preprocess_tma_kernel<IDENT, SRC_BGR>;
+           : fmt == SRC_PACKED422 ? preprocess_tma_kernel<IDENT, SRC_PACKED422>
+           : fmt == SRC_RGB24 ? preprocess_tma_kernel<IDENT, SRC_RGB24>
+           : fmt == SRC_PX32 ? preprocess_tma_kernel<IDENT, SRC_PX32>
+           : fmt == SRC_GRAY8 ? preprocess_tma_kernel<IDENT, SRC_GRAY8> : preprocess_tma_kernel<IDENT, SRC_BGR>;
 }
 
-// max_row_bytes: widest staged row (BGR: 3w, NV12/NV21: w, planar: 2 round16(w/2), a U half and a V half, packed 4:2:2:
-// 2w); fmt: the source format of frames_dev (SrcFmt)
+// max_row_bytes: widest staged row (BGR and RGB24: 3w, NV12/NV21: w, planar: 2 round16(w/2), a U half and a V half, packed
+// 4:2:2: 2w, RGBA / BGRA: 4w, GRAY8: w); fmt: the source format of frames_dev (SrcFmt).  A row too wide for the bulk-copy
+// ring (PRE2_STAGES_OF x 2 rows: a 4K RGBA row of 15 360 B fits, an 8K one does not) takes the row-staging kernel.
 int preprocess_launch(fd_ctx *ctx, const FrameDev *frames_dev, int B, float *out_nchw_dev, int max_row_bytes, bool rows_aligned16,
                       int fmt) {
     constexpr int SLOTS_NV = 4;
@@ -493,7 +540,8 @@ int preprocess_launch(fd_ctx *ctx, const FrameDev *frames_dev, int B, float *out
     // v2 (bulk-TMA staging): 16-byte aligned source rows, vector stores, one 4-pixel group per thread
     if (rows_aligned16 && a.vec_store && ngroups <= 256) {
         a.row_buf_bytes = (max_row_bytes + 15) & ~15;
-        size_t smem = 64 + 3072 + (size_t)PRE2_STAGES * (nv ? SLOTS_NV : 2) * a.row_buf_bytes;
+        const int stages = fmt == SRC_PX32 ? PRE2_STAGES_OF<SRC_PX32> : PRE2_STAGES;
+        size_t smem = 64 + 3072 + (size_t)stages * (nv ? SLOTS_NV : 2) * a.row_buf_bytes;
         if (smem <= (size_t)ctx->max_smem_optin) {
             int threads = std::max(32, ((ngroups + 31) / 32) * 32);
             dim3 grid((a.out_h + PRE2_ROWS - 1) / PRE2_ROWS, B);
@@ -511,7 +559,10 @@ int preprocess_launch(fd_ctx *ctx, const FrameDev *frames_dev, int B, float *out
     void (*kern)(PreArgs) = fmt == SRC_NV12 ? preprocess_kernel<SRC_NV12>
                             : fmt == SRC_NV21 ? preprocess_kernel<SRC_NV21>
                             : fmt == SRC_PLANAR ? preprocess_kernel<SRC_PLANAR>
-                            : fmt == SRC_PACKED422 ? preprocess_kernel<SRC_PACKED422> : preprocess_kernel<SRC_BGR>;
+                            : fmt == SRC_PACKED422 ? preprocess_kernel<SRC_PACKED422>
+                            : fmt == SRC_RGB24 ? preprocess_kernel<SRC_RGB24>
+                            : fmt == SRC_PX32 ? preprocess_kernel<SRC_PX32>
+                            : fmt == SRC_GRAY8 ? preprocess_kernel<SRC_GRAY8> : preprocess_kernel<SRC_BGR>;
     FD_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int threads = std::min(1024, std::max(64, ((ngroups + 31) / 32) * 32));
     dim3 grid((a.out_h + PRE_ROWS - 1) / PRE_ROWS, B);

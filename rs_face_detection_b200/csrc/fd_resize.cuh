@@ -183,4 +183,37 @@ __device__ __forceinline__ unsigned resize_pixel24_packed(const uint8_t *data, i
     return resize_px24(packed_px24(r0, sel, x0), packed_px24(r0, sel, x1), p10, p11, a0, a1, b0, b1);
 }
 
+// ---- interleaved RGB-family sources: each tap is the pixel cv::cvtColor(COLOR_RGB2BGR / RGBA2BGR / BGRA2BGR / GRAY2BGR)
+// would have made, and the resize arithmetic is the BGR one ---------------------------------------------------------------
+// b | g << 8 | r << 16 of a packed pixel read as b, g, r (RGB24: channels 0 and 2 exchanged)
+__device__ __forceinline__ unsigned swap_rb24(unsigned p) { return __byte_perm(p, 0u, 0x3012); }
+// pixel x of a 4-byte row (RGBA / BGRA) at any alignment: three byte reads; sel reorders a pixel word to B,G,R,x (nibble k:
+// the source byte that lands in byte k): RGBA 0x3012, BGRA 0x3210
+__device__ __forceinline__ unsigned px32_px24(const uint8_t *row, unsigned sel, int x) {
+    const uint8_t *p = row + 4 * x;
+    return (unsigned)p[sel & 3u] | ((unsigned)p[(sel >> 4) & 3u] << 8) | ((unsigned)p[(sel >> 8) & 3u] << 16);
+}
+// pixel x of a GRAY8 row as BGR
+__device__ __forceinline__ unsigned gray_px24(const uint8_t *row, int x) { return (unsigned)row[x] * 0x010101u; }
+// resize_pixel24 of the ROI (rx0, ry0)..(rx0 + rw, ry0 + rh) of an RGBA / BGRA (FMT = SRC_PX32) or GRAY8 frame.  A GRAY8
+// pixel is resized once: the three channels of its BGR image are equal.
+template <int FMT>
+__device__ __forceinline__ unsigned resize_pixel24_rgb(const uint8_t *data, int pitch, unsigned sel, int rx0, int ry0, int rw, int rh, int ow,
+                                                       int oh, int x, int y) {
+    if (rw == ow && rh == oh) {
+        const uint8_t *row = data + (size_t)(ry0 + y) * pitch;
+        return FMT == SRC_GRAY8 ? gray_px24(row, rx0 + x) : px32_px24(row, sel, rx0 + x);
+    }
+    const double scale_x = 1.0 / ((double)ow / rw), scale_y = 1.0 / ((double)oh / rh);
+    int o0, o1, y0, y1, b0, b1;
+    short a0, a1;
+    x_taps(x, scale_x, rw, &o0, &o1, &a0, &a1);
+    y_taps(y, scale_y, rh, &y0, &y1, &b0, &b1);
+    const int x0 = rx0 + o0 / 3, x1 = rx0 + o1 / 3;
+    const uint8_t *r0 = data + (size_t)(ry0 + y0) * pitch, *r1 = data + (size_t)(ry0 + y1) * pitch;
+    if constexpr (FMT == SRC_GRAY8) return (unsigned)resize_px(r0, r1, x0, x1, a0, a1, b0, b1) * 0x010101u;
+    const unsigned p10 = b1 != 0 ? px32_px24(r1, sel, x0) : 0u, p11 = b1 != 0 ? px32_px24(r1, sel, x1) : 0u;
+    return resize_px24(px32_px24(r0, sel, x0), px32_px24(r0, sel, x1), p10, p11, a0, a1, b0, b1);
+}
+
 }  // namespace fd

@@ -76,6 +76,8 @@ FD_UPLOAD_FULL, FD_UPLOAD_ON_DEMAND = 0, 1
 FD_YUV420_NV12, FD_YUV420_NV21, FD_YUV420_I420, FD_YUV420_YV12 = 0, 1, 2, 3
 # layouts of a packed 4:2:2 frame (an fd_frame) for the *_yuv422 calls: the byte order of a 2-pixel macropixel
 FD_YUV422_YUY2, FD_YUV422_UYVY, FD_YUV422_YVYU = 0, 1, 2
+# layouts of an interleaved RGB-family frame (an fd_frame) for the *_rgb calls: R,G,B / R,G,B,A / B,G,R,A / one grey byte
+FD_RGB_RGB24, FD_RGB_RGBA, FD_RGB_BGRA, FD_RGB_GRAY8 = 0, 1, 2, 3
 
 
 class FdPipelineOpts(C.Structure):
@@ -103,6 +105,7 @@ SYMBOLS = [
     "fd_align_selected_yuv420",
     "fd_preprocess_batch_yuv422", "fd_align_batch_yuv422", "fd_align_detections_yuv422", "fd_select_detections_yuv422",
     "fd_align_selected_yuv422",
+    "fd_preprocess_batch_rgb", "fd_align_batch_rgb", "fd_align_detections_rgb", "fd_select_detections_rgb", "fd_align_selected_rgb",
 ]
 
 _lib = None
@@ -679,6 +682,38 @@ class Context:
         arr = self._frames(frames)
         _chk(self.lib.fd_align_selected_yuv422(self.handle, arr, int(layout), len(frames), C.c_void_p(_devptr(crops_dev)),
                                                C.c_void_p(_devptr(M_dev)), C.c_void_p(_devptr(ok_dev))))
+
+    # ---- interleaved RGB-family frames in any FD_RGB_* layout (descriptors from frame_table: (dev_ptr, h, w, pitch)): the
+    # results of cv2.cvtColor(COLOR_RGB2BGR / COLOR_RGBA2BGR / COLOR_BGRA2BGR / COLOR_GRAY2BGR) followed by the BGR call
+    def preprocess_batch_rgb(self, frames, layout, out_dev):
+        arr = self._frames(frames)
+        ds = np.empty(len(frames), np.float32)
+        _chk(self.lib.fd_preprocess_batch_rgb(self.handle, arr, int(layout), len(frames), C.c_void_p(_devptr(out_dev)), _ptr(ds, c_f32p)))
+        return ds
+
+    def align_batch_rgb(self, frames, layout, landmarks_dev, frame_idx_dev, F, crops_dev, M_dev=None, ok_dev=None, bbox_dev=None):
+        arr = self._frames(frames)
+        _chk(self.lib.fd_align_batch_rgb(self.handle, arr, int(layout), len(frames), C.c_void_p(_devptr(landmarks_dev)),
+                                         C.c_void_p(_devptr(frame_idx_dev)), C.c_void_p(_devptr(bbox_dev)), F,
+                                         C.c_void_p(_devptr(crops_dev)), C.c_void_p(_devptr(M_dev)), C.c_void_p(_devptr(ok_dev))))
+
+    def align_detections_rgb(self, frames, layout, crops_dev, cap_faces, M_dev=None, ok_dev=None):
+        arr = self._frames(frames)
+        _chk(self.lib.fd_align_detections_rgb(self.handle, arr, int(layout), len(frames), C.c_void_p(_devptr(crops_dev)), cap_faces,
+                                              C.c_void_p(_devptr(M_dev)), C.c_void_p(_devptr(ok_dev))))
+
+    def select_detections_rgb(self, frames, layout, is_enroll=False, params=None, fetch=True):
+        arr = self._frames(frames)
+        prm = None if params is None else (C.c_float * 4)(*params)
+        sel = np.empty((len(frames), 2), np.int32) if fetch else None
+        _chk(self.lib.fd_select_detections_rgb(self.handle, arr, int(layout), len(frames), int(bool(is_enroll)), prm,
+                                               None if sel is None else _ptr(sel, c_i32p)))
+        return sel
+
+    def align_selected_rgb(self, frames, layout, crops_dev, M_dev=None, ok_dev=None):
+        arr = self._frames(frames)
+        _chk(self.lib.fd_align_selected_rgb(self.handle, arr, int(layout), len(frames), C.c_void_p(_devptr(crops_dev)),
+                                            C.c_void_p(_devptr(M_dev)), C.c_void_p(_devptr(ok_dev))))
 
     # ---- N2: Triton raw_output_contents
     def detect_batch_raw(self, raw, shapes, det_scale, conf_thr, iou_thr):
