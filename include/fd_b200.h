@@ -425,6 +425,18 @@ int fd_pipeline_opts_default(fd_pipeline_opts *opts);   /* select 0, FD_UPLOAD_F
  * opts NULL = defaults.  Blocks until the outputs are in host memory. */
 int fd_pipeline_host(fd_ctx *ctx, const fd_frame *frames, int B, const float *const *heads_host, int n_heads,
                      float conf_thr, float iou_thr, const fd_pipeline_opts *opts, fd_host_batch_out *out);
+/* fd_pipeline_host on HOST frames in another layout: the descriptors of fd_preprocess_batch_yuv420 / _yuv422 / _rgb, with
+ * host pointers, and the same FD_ERR_INVALID rules (an I420 / YV12 frame's second chroma plane starts (H/2) * pitch_uv after
+ * uv, as av_image_alloc and av_frame_get_buffer lay it out).  Every output equals fd_pipeline_host's on cv::cvtColor(
+ * COLOR_YUV2BGR_<layout> / RGB2BGR / RGBA2BGR / BGRA2BGR / GRAY2BGR) of the frames, for both upload modes and both flows; only
+ * the layout's own bytes cross PCIe (1080p: NV12 / I420 half of BGR's, YUY2 two thirds, GRAY8 one third), and
+ * FD_UPLOAD_ON_DEMAND sends per plane only the rows the resize reads and the rectangles the warps read. */
+int fd_pipeline_host_yuv420(fd_ctx *ctx, const fd_frame_nv12 *frames, int32_t layout, int B, const float *const *heads_host,
+                            int n_heads, float conf_thr, float iou_thr, const fd_pipeline_opts *opts, fd_host_batch_out *out);
+int fd_pipeline_host_yuv422(fd_ctx *ctx, const fd_frame *frames, int32_t layout, int B, const float *const *heads_host,
+                            int n_heads, float conf_thr, float iou_thr, const fd_pipeline_opts *opts, fd_host_batch_out *out);
+int fd_pipeline_host_rgb(fd_ctx *ctx, const fd_frame *frames, int32_t layout, int B, const float *const *heads_host,
+                         int n_heads, float conf_thr, float iou_thr, const fd_pipeline_opts *opts, fd_host_batch_out *out);
 /* The same with the frames given as JPEG streams — FacePipeline::extract's real input (face_pipeline/pipeline.rs:188-196,
  * byte_data_to_opencv): fd_decode_jpeg_batch (host Huffman on n_threads threads, CUDA IDCT / upsampling / colour) on the way in,
  * then the path above with the frames already on the device.  h2d_bytes counts the coefficient upload.  opts->upload is ignored. */

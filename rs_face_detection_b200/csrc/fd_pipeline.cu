@@ -180,32 +180,44 @@ static int rgb_frames(const fd_frame *frames, int32_t layout, FrameList *fl) {
     return FD_OK;
 }
 
-// uploads B descriptors and records their source format in ctx->frames_fmt (the same buffers described as BGR and as RGB24
-// give byte-identical tables: only the format tells them apart); returns the widest staged source row in bytes (BGR and
+// the kernels' source format of a FrameList whose layout is known (yuv420_frames, yuv422_frames, rgb_frames)
+static int frames_format(const FrameList &frames) {
+    return frames.rgb ? rgb_format(frames.layout) : frames.packed ? SRC_PACKED422 : frames.yuv ? yuv420_format(frames.layout) : SRC_BGR;
+}
+
+// validates frame i of `frames` and fills its table entry; *row_bytes: the staged source row of the frame in bytes (BGR and
 // RGB24: 3w, NV12/NV21: w, planar: a U and a V half of round16(w/2) bytes each, packed 4:2:2: 2w, RGBA / BGRA: 4w, GRAY8: w)
+static int fill_frame_of(const fd_ctx *ctx, const FrameList &frames, int i, FrameDev *out, float *ds, int *row_bytes) {
+    memset(out, 0, sizeof(FrameDev));
+    if (frames.yuv) {
+        const int w = frames.yuv[i].width;
+        FD_TRY(fill_frame_yuv420(ctx, frames.yuv[i], frames.layout, out, ds));
+        *row_bytes = yuv420_format(frames.layout) == SRC_PLANAR ? 2 * ((w / 2 + 15) & ~15) : w;
+    } else if (frames.packed) {
+        FD_TRY(fill_frame_yuv422(ctx, frames.packed[i], frames.layout, out, ds));
+        *row_bytes = 2 * frames.packed[i].width;
+    } else if (frames.rgb) {
+        FD_TRY(fill_frame_rgb(ctx, frames.rgb[i], frames.layout, out, ds));
+        *row_bytes = rgb_bpp(frames.layout) * frames.rgb[i].width;
+    } else {
+        FD_REQUIRE(frames.bgr[i].data != nullptr, "frame: null data");
+        FD_TRY(fill_frame(ctx, frames.bgr[i], frames.bgr[i].data, out, ds));
+        *row_bytes = frames.bgr[i].width * 3;
+    }
+    return FD_OK;
+}
+
+// uploads B descriptors and records their source format in ctx->frames_fmt (the same buffers described as BGR and as RGB24
+// give byte-identical tables: only the format tells them apart); returns the widest staged source row in bytes
 static int upload_frame_table(fd_ctx *ctx, FrameList frames, int B, float *det_scale_host, int *max_row_bytes) {
-    // a known layout (yuv420_frames, yuv422_frames, rgb_frames)
-    const int fmt = frames.rgb ? rgb_format(frames.layout) : frames.packed ? SRC_PACKED422 : frames.yuv ? yuv420_format(frames.layout) : SRC_BGR;
+    const int fmt = frames_format(frames);
     std::vector<FrameDev> tab(B);
     int mrb = 0;
     for (int i = 0; i < B; ++i) {
         float ds;
-        memset(&tab[i], 0, sizeof(FrameDev));
-        if (frames.yuv) {
-            const int w = frames.yuv[i].width;
-            FD_TRY(fill_frame_yuv420(ctx, frames.yuv[i], frames.layout, &tab[i], &ds));
-            mrb = std::max(mrb, fmt == SRC_PLANAR ? 2 * ((w / 2 + 15) & ~15) : w);
-        } else if (frames.packed) {
-            FD_TRY(fill_frame_yuv422(ctx, frames.packed[i], frames.layout, &tab[i], &ds));
-            mrb = std::max(mrb, 2 * frames.packed[i].width);
-        } else if (frames.rgb) {
-            FD_TRY(fill_frame_rgb(ctx, frames.rgb[i], frames.layout, &tab[i], &ds));
-            mrb = std::max(mrb, rgb_bpp(frames.layout) * frames.rgb[i].width);
-        } else {
-            FD_REQUIRE(frames.bgr[i].data != nullptr, "frame: null data");
-            FD_TRY(fill_frame(ctx, frames.bgr[i], frames.bgr[i].data, &tab[i], &ds));
-            mrb = std::max(mrb, frames.bgr[i].width * 3);
-        }
+        int rb;
+        FD_TRY(fill_frame_of(ctx, frames, i, &tab[i], &ds, &rb));
+        mrb = std::max(mrb, rb);
         if (det_scale_host) det_scale_host[i] = ds;
     }
     if (max_row_bytes) *max_row_bytes = mrb;
@@ -936,33 +948,129 @@ static bool warp_source_rect(const double *iM, int cw, int ch, int fw, int fh, i
     return true;
 }
 
-struct HostFrame {
-    size_t off;     // offset of the frame in the device arena
-    int dpitch;     // device pitch (16-byte multiple)
-    bool full;      // every row is on the device
-    // rows already uploaded for the preprocess when !full: a0 + k*j (and a1 + k*j when two), j < n
-    int a0, a1, k, n;
-    bool two;
+// rows first + step * j, j < count, of one plane
+struct RowRun {
+    int first, step, count;
 };
 
-// whole frame, one copy
-static int upload_full(fd_ctx *ctx, const fd_frame &fr, uint8_t *dst, int dpitch, int64_t *h2d) {
-    const size_t row = (size_t)fr.width * 3;
-    if (fr.pitch == dpitch)
-        FD_CUDA(cudaMemcpyAsync(dst, fr.data, (size_t)dpitch * (fr.height - 1) + row, cudaMemcpyHostToDevice, ctx->stream));
+// One plane of a host frame and its copy in the device arena.  Frame row y lies in plane row y >> ys; frame columns
+// [x0, x1] lie in plane bytes [unit * (x0 >> xs), unit * ((x1 >> xs) + 1)).
+struct HostPlane {
+    const uint8_t *src;
+    int spitch;
+    size_t off;                 // offset in the device arena
+    int dpitch;                 // 16-byte multiple
+    int row_bytes, rows, xs, unit, ys;
+    bool joined;                // the next plane follows this one, in host and in device memory: a whole-frame copy takes both
+    std::vector<RowRun> have;   // rows on the device when the frame is not full (disjoint runs of one step)
+};
+
+struct HostFrame {
+    int h, w;
+    bool full;   // every plane is on the device
+    int np;
+    HostPlane pl[3];
+};
+
+static HostPlane host_plane(const uint8_t *src, int spitch, int row_bytes, int rows, int xs, int unit, int ys, size_t *arena) {
+    HostPlane p;
+    p.src = src;
+    p.spitch = spitch;
+    p.dpitch = (row_bytes + 15) & ~15;
+    p.off = *arena;
+    p.row_bytes = row_bytes;
+    p.rows = rows;
+    p.xs = xs;
+    p.unit = unit;
+    p.ys = ys;
+    p.joined = false;
+    *arena += ((size_t)p.dpitch * rows + 255) & ~(size_t)255;
+    return p;
+}
+
+// the planes of host frame i (validated by fill_frame_of) and their places in the arena, each plane at a 256-byte aligned
+// start with a 16-byte multiple pitch (bulk-copy preprocess, interior warp reads): BGR / RGB24 3w, RGBA / BGRA 4w, GRAY8 w,
+// packed 4:2:2 2w (whole macropixels), NV12 / NV21 a Y plane of w and h/2 chroma rows of w (U,V pairs), I420 / YV12 a Y plane
+// of w and the two chroma planes at round16(w/2), the second (h/2) pitches after the first as the descriptor wants it.
+static void host_planes(const FrameList &frames, int i, HostFrame *hf, size_t *arena) {
+    hf->full = false;
+    if (frames.yuv) {
+        const fd_frame_nv12 &f = frames.yuv[i];
+        hf->h = f.height;
+        hf->w = f.width;
+        hf->np = 2;
+        hf->pl[0] = host_plane(f.y, f.pitch_y, f.width, f.height, 0, 1, 0, arena);
+        if (yuv420_format(frames.layout) != SRC_PLANAR) {
+            hf->pl[1] = host_plane(f.uv, f.pitch_uv, f.width, f.height / 2, 1, 2, 1, arena);
+            return;
+        }
+        HostPlane both = host_plane(f.uv, f.pitch_uv, f.width / 2, f.height, 1, 1, 1, arena);
+        both.rows = f.height / 2;
+        both.joined = true;
+        hf->pl[1] = hf->pl[2] = both;
+        hf->pl[2].src += (size_t)both.rows * f.pitch_uv;
+        hf->pl[2].off += (size_t)both.rows * both.dpitch;
+        hf->pl[2].joined = false;
+        hf->np = 3;
+        return;
+    }
+    const fd_frame &f = frames.packed ? frames.packed[i] : frames.rgb ? frames.rgb[i] : frames.bgr[i];
+    hf->h = f.height;
+    hf->w = f.width;
+    hf->np = 1;
+    if (frames.packed) hf->pl[0] = host_plane(f.data, f.pitch, 2 * f.width, f.height, 1, 4, 0, arena);
+    else {
+        const int bpp = frames.rgb ? rgb_bpp(frames.layout) : 3;
+        hf->pl[0] = host_plane(f.data, f.pitch, bpp * f.width, f.height, 0, bpp, 0, arena);
+    }
+}
+
+// rows first + step * j (j < count) of plane p, host to device: one copy
+static int upload_rows(fd_ctx *ctx, const HostPlane &p, uint8_t *arena, int first, int step, int count, int64_t *h2d) {
+    if (count <= 0) return FD_OK;
+    uint8_t *dst = arena + p.off + (size_t)first * p.dpitch;
+    const uint8_t *src = p.src + (size_t)first * p.spitch;
+    if (step == 1 && p.spitch == p.dpitch)
+        FD_CUDA(cudaMemcpyAsync(dst, src, (size_t)p.dpitch * (count - 1) + p.row_bytes, cudaMemcpyHostToDevice, ctx->stream));
     else
-        FD_CUDA(cudaMemcpy2DAsync(dst, dpitch, fr.data, fr.pitch, row, fr.height, cudaMemcpyHostToDevice, ctx->stream));
-    *h2d += (int64_t)row * fr.height;
+        FD_CUDA(cudaMemcpy2DAsync(dst, (size_t)step * p.dpitch, src, (size_t)step * p.spitch, p.row_bytes, count, cudaMemcpyHostToDevice,
+                                  ctx->stream));
+    *h2d += (int64_t)p.row_bytes * count;
     return FD_OK;
 }
 
+// whole frame: one copy a plane (the two chroma planes of I420 / YV12 as one)
+static int upload_full(fd_ctx *ctx, HostFrame &hf, uint8_t *arena, int64_t *h2d) {
+    for (int q = 0; q < hf.np; ++q) {
+        HostPlane p = hf.pl[q];
+        if (p.joined) p.rows += hf.pl[++q].rows;
+        FD_TRY(upload_rows(ctx, p, arena, 0, 1, p.rows, h2d));
+    }
+    hf.full = true;
+    return FD_OK;
+}
+
+// adds the run to p.have; false when it overlaps a run already there without being the same
+static bool add_run(HostPlane &p, RowRun r) {
+    if (r.count <= 0) return true;
+    for (const RowRun &o : p.have) {
+        if (o.first == r.first && o.count == r.count && o.step == r.step) return true;
+        if (o.step != r.step) return false;
+        const bool same_rows = (o.first - r.first) % r.step == 0;
+        if (same_rows && r.first <= o.first + o.step * (o.count - 1) && o.first <= r.first + r.step * (r.count - 1)) return false;
+    }
+    p.have.push_back(r);
+    return true;
+}
+
 // Only the source rows the letterbox resize reads (face_detection.rs:156): for an integer down-scale k they form at most two
-// arithmetic progressions of stride k (1080p -> 640x360: rows 3y+1; 4K: rows 6y+2 and 6y+3), each ONE strided 2-D copy.
-// Returns *done = false when the pattern is not worth it (most rows needed, or no short description): caller uploads the frame.
-static int upload_preprocess_rows(fd_ctx *ctx, const fd_frame &fr, int new_h, double scale_y, uint8_t *dst, int dpitch, int64_t *h2d,
-                                  HostFrame *hfr, bool *done) {
+// arithmetic progressions of stride k (1080p -> 640x360: rows 3y+1; 4K: rows 6y+2 and 6y+3), each ONE strided 2-D copy a
+// plane.  A 4:2:0 chroma plane holds rows y >> 1 of them: two progressions of stride k for an odd k (1080p: chroma rows 3m and
+// 3m+2), one of stride k/2 for an even k (4K: chroma rows 3y+1).  Returns *done = false when the pattern is not worth it (most
+// rows needed, or no short description): the caller uploads the frame.
+static int upload_preprocess_rows(fd_ctx *ctx, HostFrame &hf, int new_h, double scale_y, uint8_t *arena, int64_t *h2d, bool *done) {
     *done = false;
-    const int h = fr.height;
+    const int h = hf.h;
     const long long k = llround(scale_y);
     if (k < 2 || fabs(scale_y - (double)k) > 1e-12 || new_h < 2) return FD_OK;
     // rows of dy = 0 and their stride-k continuation must reproduce every dy's rows
@@ -974,41 +1082,64 @@ static int upload_preprocess_rows(fd_ctx *ctx, const fd_frame &fr, int new_h, do
         if (two != two0 || c0 != a0 + (int)k * dy || (two && c1 != a1 + (int)k * dy)) return FD_OK;
     }
     if (two0 && k < 3) return FD_OK;
-    const size_t row = (size_t)fr.width * 3;
-    FD_CUDA(cudaMemcpy2DAsync(dst + (size_t)a0 * dpitch, (size_t)k * dpitch, fr.data + (size_t)a0 * fr.pitch, (size_t)k * fr.pitch, row, new_h,
-                              cudaMemcpyHostToDevice, ctx->stream));
-    *h2d += (int64_t)row * new_h;
-    if (two0) {
-        FD_CUDA(cudaMemcpy2DAsync(dst + (size_t)a1 * dpitch, (size_t)k * dpitch, fr.data + (size_t)a1 * fr.pitch, (size_t)k * fr.pitch, row, new_h,
-                                  cudaMemcpyHostToDevice, ctx->stream));
-        *h2d += (int64_t)row * new_h;
+    const RowRun luma[2] = {{a0, (int)k, new_h}, {a1, (int)k, new_h}};
+    for (int q = 0; q < hf.np; ++q) {
+        HostPlane &p = hf.pl[q];
+        p.have.clear();
+        for (int t = 0; t < (two0 ? 2 : 1); ++t) {
+            const RowRun &r = luma[t];
+            bool ok;
+            if (!p.ys) ok = add_run(p, r);
+            else if (r.step % 2 == 0) ok = add_run(p, {r.first >> 1, r.step / 2, r.count});
+            else ok = add_run(p, {r.first >> 1, r.step, (r.count + 1) / 2}) && add_run(p, {(r.first + r.step) >> 1, r.step, r.count / 2});
+            if (!ok) return FD_OK;
+        }
     }
-    hfr->a0 = a0; hfr->a1 = a1; hfr->k = (int)k; hfr->n = new_h; hfr->two = two0;
+    for (int q = 0; q < hf.np; ++q)
+        for (const RowRun &r : hf.pl[q].have) FD_TRY(upload_rows(ctx, hf.pl[q], arena, r.first, r.step, r.count, h2d));
     *done = true;
     return FD_OK;
 }
 
-// the rows upload_preprocess_rows left out: the other residues mod k, and the tail of the uploaded residues
-static int upload_complement_rows(fd_ctx *ctx, const fd_frame &fr, const HostFrame &hfr, uint8_t *dst, int64_t *h2d) {
-    const size_t row = (size_t)fr.width * 3;
-    const int k = hfr.k, h = fr.height;
-    auto strided = [&](int first, int step, int count) -> int {
-        if (count <= 0) return FD_OK;
-        FD_CUDA(cudaMemcpy2DAsync(dst + (size_t)first * hfr.dpitch, (size_t)step * hfr.dpitch, fr.data + (size_t)first * fr.pitch,
-                                  (size_t)step * fr.pitch, row, count, cudaMemcpyHostToDevice, ctx->stream));
-        *h2d += (int64_t)row * count;
-        return FD_OK;
-    };
-    for (int r = 0; r < k; ++r) {
-        if (r == hfr.a0 % k || (hfr.two && r == hfr.a1 % k)) continue;
-        FD_TRY(strided(r, k, (h - r + k - 1) / k));
+// bytes of the frame's rows already on the device (upload_preprocess_rows)
+static int64_t have_bytes(const HostFrame &hf) {
+    int64_t n = 0;
+    for (int q = 0; q < hf.np; ++q)
+        for (const RowRun &r : hf.pl[q].have) n += (int64_t)hf.pl[q].row_bytes * r.count;
+    return n;
+}
+
+// the rows upload_preprocess_rows left out: per plane and residue of the runs' step, the gaps between the runs
+static int upload_complement_rows(fd_ctx *ctx, HostFrame &hf, uint8_t *arena, int64_t *h2d) {
+    for (int q = 0; q < hf.np; ++q) {
+        const HostPlane &p = hf.pl[q];
+        const int s = p.have[0].step;
+        std::vector<RowRun> runs = p.have;
+        std::sort(runs.begin(), runs.end(), [](const RowRun &a, const RowRun &b) { return a.first < b.first; });
+        for (int res = 0; res < s && res < p.rows; ++res) {
+            int next = res;   // the first row of this residue not yet accounted for
+            for (const RowRun &r : runs) {
+                if (r.first % s != res) continue;
+                FD_TRY(upload_rows(ctx, p, arena, next, s, (r.first - next) / s, h2d));
+                next = r.first + s * r.count;
+            }
+            FD_TRY(upload_rows(ctx, p, arena, next, s, (p.rows - next + s - 1) / s, h2d));
+        }
     }
-    const int firsts[2] = {hfr.a0, hfr.a1};
-    for (int t = 0; t < (hfr.two ? 2 : 1); ++t) {
-        const int r = firsts[t] % k;
-        if (firsts[t] > r) FD_TRY(strided(r, k, (firsts[t] - r) / k));                   // rows of this residue before the first one
-        const int next = firsts[t] + k * hfr.n;
-        if (next < h) FD_TRY(strided(next, k, (h - next + k - 1) / k));                   // ... and after the last one
+    hf.full = true;
+    return FD_OK;
+}
+
+// Plane bytes the warp of pixel rectangle [x0,x1] x [y0,y1] reads; upload them when `arena` is given
+static int upload_rect(fd_ctx *ctx, const HostFrame &hf, int x0, int y0, int x1, int y1, uint8_t *arena, int64_t *bytes) {
+    for (int q = 0; q < hf.np; ++q) {
+        const HostPlane &p = hf.pl[q];
+        const int r0 = y0 >> p.ys, rows = (y1 >> p.ys) - r0 + 1;
+        const size_t b0 = (size_t)p.unit * (x0 >> p.xs), wbytes = (size_t)p.unit * ((x1 >> p.xs) + 1) - b0;
+        if (arena)
+            FD_CUDA(cudaMemcpy2DAsync(arena + p.off + (size_t)r0 * p.dpitch + b0, p.dpitch, p.src + (size_t)r0 * p.spitch + b0, p.spitch,
+                                      wbytes, rows, cudaMemcpyHostToDevice, ctx->stream));
+        *bytes += (int64_t)wbytes * rows;
     }
     return FD_OK;
 }
@@ -1021,8 +1152,9 @@ FD_EXPORT int fd_pipeline_opts_default(fd_pipeline_opts *o) {
     return fd_select_params_default(&o->select_params);
 }
 
-// frames: HOST pixel frames, or (dev_frames != nullptr) frames already resident on the device (fd_decode_jpeg_batch)
-static int pipeline_host_impl(fd_ctx *ctx, const fd_frame *frames, const fd_frame *dev_frames, int B, const float *const *heads_host, int n_heads,
+// frames: HOST pixel frames in any layout, or (dev_frames != nullptr) BGR frames already resident on the device
+// (fd_decode_jpeg_batch)
+static int pipeline_host_impl(fd_ctx *ctx, FrameList frames, const fd_frame *dev_frames, int B, const float *const *heads_host, int n_heads,
                               float conf_thr, float iou_thr, const fd_pipeline_opts *opts, fd_host_batch_out *out, int64_t h2d_so_far) {
     FD_REQUIRE(heads_host && out && B > 0, "fd_pipeline_host: bad arguments");
     FD_REQUIRE(n_heads == 3 * ctx->dcfg.n_strides, "fd_pipeline_host: n_heads must be 3 * n_strides");
@@ -1040,50 +1172,48 @@ static int pipeline_host_impl(fd_ctx *ctx, const fd_frame *frames, const fd_fram
     const DecodeCfg &d = ctx->dcfg;
     const int cw = ctx->cfg.crop_w, ch = ctx->cfg.crop_h;
     int64_t h2d = h2d_so_far, d2h = 0;
-    // 1. frames H2D into one device arena (16-byte aligned rows).  FD_UPLOAD_ON_DEMAND: only the rows the letterbox resize
-    //    reads now; the pixels the warps read follow after detection (step 4).
-    std::vector<HostFrame> hf(B);
+    // 1. frames H2D into one device arena (host_planes).  FD_UPLOAD_ON_DEMAND: only the rows the letterbox resize reads now;
+    //    the pixels the warps read follow after detection (step 4).  dfl describes the frames on the device, in their layout.
+    std::vector<HostFrame> hf(dev_frames ? 0 : B);
     std::vector<fd_frame> dframes(B);
+    std::vector<fd_frame_nv12> dyuv(frames.yuv ? B : 0);
     std::vector<float> ds(B);
+    FrameList dfl = frames;
     if (dev_frames) {
         for (int i = 0; i < B; ++i) {
             dframes[i] = dev_frames[i];
-            hf[i].full = true;
-            hf[i].dpitch = dev_frames[i].pitch;
-            hf[i].off = 0;
             FrameDev geo;
             FD_TRY(fill_frame(ctx, dframes[i], dframes[i].data, &geo, &ds[i]));
-            if (out->det_scale) out->det_scale[i] = ds[i];
         }
+        dfl.bgr = dframes.data();
     } else {
-    size_t arena = 0;
-    for (int i = 0; i < B; ++i) {
-        FD_REQUIRE(frames[i].data && frames[i].height > 0 && frames[i].width > 0 && frames[i].pitch >= frames[i].width * 3,
-                   "fd_pipeline_host: bad frame");
-        hf[i].dpitch = (frames[i].width * 3 + 15) & ~15;
-        hf[i].off = arena;
-        hf[i].full = false;
-        arena += ((size_t)hf[i].dpitch * frames[i].height + 255) & ~(size_t)255;
-    }
-    FD_TRY(ctx->pipe_frames.reserve(arena + 256));
-    for (int i = 0; i < B; ++i) {
-        uint8_t *dst = ctx->pipe_frames.as<uint8_t>() + hf[i].off;
-        dframes[i] = fd_frame{dst, frames[i].height, frames[i].width, hf[i].dpitch};
-        FrameDev geo;
-        FD_TRY(fill_frame(ctx, dframes[i], dst, &geo, &ds[i]));
-        if (out->det_scale) out->det_scale[i] = ds[i];
-        bool sparse = false;
-        if (demand) FD_TRY(upload_preprocess_rows(ctx, frames[i], geo.new_h, geo.scale_y, dst, hf[i].dpitch, &h2d, &hf[i], &sparse));
-        if (!sparse) {
-            FD_TRY(upload_full(ctx, frames[i], dst, hf[i].dpitch, &h2d));
-            hf[i].full = true;
+        size_t arena = 0;
+        std::vector<FrameDev> geo(B);
+        for (int i = 0; i < B; ++i) {
+            int rb;
+            FD_TRY(fill_frame_of(ctx, frames, i, &geo[i], &ds[i], &rb));
+            host_planes(frames, i, &hf[i], &arena);
         }
+        FD_TRY(ctx->pipe_frames.reserve(arena + 256));
+        uint8_t *base = ctx->pipe_frames.as<uint8_t>();
+        for (int i = 0; i < B; ++i) {
+            const HostPlane *p = hf[i].pl;
+            if (frames.yuv) dyuv[i] = fd_frame_nv12{base + p[0].off, base + p[1].off, hf[i].h, hf[i].w, p[0].dpitch, p[1].dpitch};
+            else dframes[i] = fd_frame{base + p[0].off, hf[i].h, hf[i].w, p[0].dpitch};
+            bool sparse = false;
+            if (demand) FD_TRY(upload_preprocess_rows(ctx, hf[i], geo[i].new_h, geo[i].scale_y, base, &h2d, &sparse));
+            if (!sparse) FD_TRY(upload_full(ctx, hf[i], base, &h2d));
+        }
+        if (frames.yuv) dfl.yuv = dyuv.data();
+        else if (frames.packed) dfl.packed = dframes.data();
+        else if (frames.rgb) dfl.rgb = dframes.data();
+        else dfl.bgr = dframes.data();
     }
-    }
+    if (out->det_scale) std::copy(ds.begin(), ds.end(), out->det_scale);
     // 2. preprocess -> CNN input tensor (stays on the device unless out->tensor is given)
     const size_t tn = (size_t)B * 3 * ctx->cfg.image_h * ctx->cfg.image_w;
     FD_TRY(ctx->pipe_tensor.reserve(sizeof(float) * tn));
-    FD_TRY(fd_preprocess_batch(ctx, dframes.data(), B, ctx->pipe_tensor.as<float>(), nullptr));
+    FD_TRY(preprocess_batch(ctx, dfl, B, ctx->pipe_tensor.as<float>(), nullptr));
     // 3. heads (the CNN outputs), decode + NMS.  The score planes are dense reads: the A foreground channels of each image go
     //    to the device by DMA (face_detection.rs:322 never reads the background half).  The bbox / landmark tensors are read
     //    only at the anchors that pass the threshold (~450 of 16 800 per image): when the caller's buffers are pinned, the
@@ -1128,20 +1258,19 @@ static int pipeline_host_impl(fd_ctx *ctx, const fd_frame *frames, const fd_fram
     int total = 0, n_crops = 0;
     if (!demand && !select) {
         // 4a. whole frames are on the device: align every detection without a host round trip, then fetch
-        FD_TRY(fd_align_detections(ctx, dframes.data(), B, crops_dev, out->cap_rows, nullptr, mode_dev));
+        FD_TRY(align_detections(ctx, dfl, B, crops_dev, out->cap_rows, nullptr, mode_dev));
         FD_TRY(fd_detect_fetch(ctx, out->counts, out->det, out->landmarks, out->cap_rows, &total));
         n_crops = total;
     } else {
         // 4b. fetch the detections first (the reference has a host round trip here too: gRPC response, face_detection.rs:279,
         //     then FaceSelection / FaceAlignment on the host, face_pipeline/pipeline.rs:208-216)
         FD_TRY(fd_detect_fetch(ctx, out->counts, out->det, out->landmarks, out->cap_rows, &total));
-        const FrameDev *frames_dev = ctx->frames_dev.as<FrameDev>();
         const int F = select ? B : total;
         n_crops = F;
         WarpFallback fb = detect_fallback(ctx);
         const int32_t *fidx_dev = ctx->out_frame_idx.as<int32_t>();
         if (select) {   // FaceSelection::call per image on the device, then the estimate of the B selected faces
-            FD_TRY(fd_select_detections(ctx, dframes.data(), B, o.is_enroll, &o.select_params, nullptr));
+            FD_TRY(select_detections(ctx, dfl, B, o.is_enroll, &o.select_params, nullptr));
             fb.sel = ctx->select_sel.as<int>();
             fidx_dev = ctx->select_fidx.as<int32_t>();
             ctx->est_valid = false;
@@ -1178,37 +1307,28 @@ static int pipeline_host_impl(fd_ctx *ctx, const fd_frame *frames, const fd_fram
                             rect_bytes[b] = INT64_MAX / 4;
                             continue;
                         }
-                        if (!warp_source_rect(&M12[(size_t)f * 12 + 6], cw, ch, frames[b].width, frames[b].height, &r.x0, &r.y0, &r.x1, &r.y1))
+                        if (!warp_source_rect(&M12[(size_t)f * 12 + 6], cw, ch, hf[b].w, hf[b].h, &r.x0, &r.y0, &r.x1, &r.y1))
                             continue;
                         rects[b].push_back(r);
-                        rect_bytes[b] += (int64_t)(r.x1 - r.x0 + 1) * 3 * (r.y1 - r.y0 + 1);
+                        FD_TRY(upload_rect(ctx, hf[b], r.x0, r.y0, r.x1, r.y1, nullptr, &rect_bytes[b]));
                     }
                 }
+                uint8_t *base = ctx->pipe_frames.as<uint8_t>();
                 for (int b = 0; b < B; ++b) {
                     if (hf[b].full || rect_bytes[b] == 0) continue;
-                    uint8_t *dst = ctx->pipe_frames.as<uint8_t>() + hf[b].off;
-                    const int64_t frame_bytes = (int64_t)frames[b].width * 3 * frames[b].height;
-                    const int64_t sent = (int64_t)frames[b].width * 3 * hf[b].n * (hf[b].two ? 2 : 1);
-                    if (rect_bytes[b] >= frame_bytes - sent) {   // many overlapping faces: the rest of the frame is cheaper
-                        FD_TRY(upload_complement_rows(ctx, frames[b], hf[b], dst, &h2d));
-                        hf[b].full = true;
+                    int64_t frame_bytes = 0;
+                    for (int q = 0; q < hf[b].np; ++q) frame_bytes += (int64_t)hf[b].pl[q].row_bytes * hf[b].pl[q].rows;
+                    if (rect_bytes[b] >= frame_bytes - have_bytes(hf[b])) {   // many overlapping faces: the rest of the frame is cheaper
+                        FD_TRY(upload_complement_rows(ctx, hf[b], base, &h2d));
                         continue;
                     }
-                    for (const Rect &r : rects[b]) {
-                        const size_t wbytes = (size_t)(r.x1 - r.x0 + 1) * 3, rows = (size_t)(r.y1 - r.y0 + 1);
-                        FD_CUDA(cudaMemcpy2DAsync(dst + (size_t)r.y0 * hf[b].dpitch + (size_t)r.x0 * 3, hf[b].dpitch,
-                                                  frames[b].data + (size_t)r.y0 * frames[b].pitch + (size_t)r.x0 * 3, frames[b].pitch, wbytes, rows,
-                                                  cudaMemcpyHostToDevice, ctx->stream));
-                        h2d += (int64_t)(wbytes * rows);
-                    }
+                    for (const Rect &r : rects[b]) FD_TRY(upload_rect(ctx, hf[b], r.x0, r.y0, r.x1, r.y1, base, &h2d));
                 }
             }
-            FrameList fl;
-            fl.bgr = dframes.data();
-            FD_TRY(upload_frame_table(ctx, fl, B, nullptr, nullptr));
+            FD_TRY(upload_frame_table(ctx, dfl, B, nullptr, nullptr));
             fb.mode_out = mode_dev;
-            FD_TRY(warp_launch(ctx, frames_dev, fidx_dev, ctx->align_M.as<double>(), ctx->align_ok.as<uint8_t>(), nullptr,
-                               std::min(F, (int)out->cap_rows), crops_dev, cw, ch, fb, SRC_BGR));
+            FD_TRY(warp_launch(ctx, ctx->frames_dev.as<FrameDev>(), fidx_dev, ctx->align_M.as<double>(), ctx->align_ok.as<uint8_t>(), nullptr,
+                               std::min(F, (int)out->cap_rows), crops_dev, cw, ch, fb, ctx->frames_fmt));
             ctx->align_replay = false;
         }
         if (select && out->sel) {
@@ -1248,7 +1368,33 @@ FD_EXPORT int fd_pipeline_host(fd_ctx *ctx, const fd_frame *frames, int B, const
                                float conf_thr, float iou_thr, const fd_pipeline_opts *opts, fd_host_batch_out *out) {
     FD_TRY(check_ctx(ctx));
     FD_REQUIRE(frames, "fd_pipeline_host: null frames");
-    return pipeline_host_impl(ctx, frames, nullptr, B, heads_host, n_heads, conf_thr, iou_thr, opts, out, 0);
+    FrameList fl;
+    fl.bgr = frames;
+    return pipeline_host_impl(ctx, fl, nullptr, B, heads_host, n_heads, conf_thr, iou_thr, opts, out, 0);
+}
+FD_EXPORT int fd_pipeline_host_yuv420(fd_ctx *ctx, const fd_frame_nv12 *frames, int32_t layout, int B, const float *const *heads_host,
+                                      int n_heads, float conf_thr, float iou_thr, const fd_pipeline_opts *opts, fd_host_batch_out *out) {
+    FD_TRY(check_ctx(ctx));
+    FrameList fl;
+    FD_TRY(yuv420_frames(frames, layout, &fl));
+    FD_REQUIRE(frames, "fd_pipeline_host_yuv420: null frames");
+    return pipeline_host_impl(ctx, fl, nullptr, B, heads_host, n_heads, conf_thr, iou_thr, opts, out, 0);
+}
+FD_EXPORT int fd_pipeline_host_yuv422(fd_ctx *ctx, const fd_frame *frames, int32_t layout, int B, const float *const *heads_host,
+                                      int n_heads, float conf_thr, float iou_thr, const fd_pipeline_opts *opts, fd_host_batch_out *out) {
+    FD_TRY(check_ctx(ctx));
+    FrameList fl;
+    FD_TRY(yuv422_frames(frames, layout, &fl));
+    FD_REQUIRE(frames, "fd_pipeline_host_yuv422: null frames");
+    return pipeline_host_impl(ctx, fl, nullptr, B, heads_host, n_heads, conf_thr, iou_thr, opts, out, 0);
+}
+FD_EXPORT int fd_pipeline_host_rgb(fd_ctx *ctx, const fd_frame *frames, int32_t layout, int B, const float *const *heads_host,
+                                   int n_heads, float conf_thr, float iou_thr, const fd_pipeline_opts *opts, fd_host_batch_out *out) {
+    FD_TRY(check_ctx(ctx));
+    FrameList fl;
+    FD_TRY(rgb_frames(frames, layout, &fl));
+    FD_REQUIRE(frames, "fd_pipeline_host_rgb: null frames");
+    return pipeline_host_impl(ctx, fl, nullptr, B, heads_host, n_heads, conf_thr, iou_thr, opts, out, 0);
 }
 
 // FacePipeline::extract's real input (face_pipeline/pipeline.rs:188-196): encoded image bytes.  byte_data_to_opencv (N4) on the
@@ -1260,7 +1406,7 @@ FD_EXPORT int fd_pipeline_host_jpeg(fd_ctx *ctx, const uint8_t *const *jpegs, co
     FD_REQUIRE(jpegs && nbytes && B > 0, "fd_pipeline_host_jpeg: bad arguments");
     std::vector<fd_frame> dev((size_t)B);
     FD_TRY(fd_decode_jpeg_batch(ctx, jpegs, nbytes, B, n_threads, dev.data()));
-    return pipeline_host_impl(ctx, nullptr, dev.data(), B, heads_host, n_heads, conf_thr, iou_thr, opts, out, ctx->jpeg_last_h2d);
+    return pipeline_host_impl(ctx, FrameList(), dev.data(), B, heads_host, n_heads, conf_thr, iou_thr, opts, out, ctx->jpeg_last_h2d);
 }
 
 FD_EXPORT int fd_pipeline_tensor_dev(fd_ctx *ctx, const float **out_nchw_dev) {

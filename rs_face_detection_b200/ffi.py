@@ -106,6 +106,7 @@ SYMBOLS = [
     "fd_preprocess_batch_yuv422", "fd_align_batch_yuv422", "fd_align_detections_yuv422", "fd_select_detections_yuv422",
     "fd_align_selected_yuv422",
     "fd_preprocess_batch_rgb", "fd_align_batch_rgb", "fd_align_detections_rgb", "fd_select_detections_rgb", "fd_align_selected_rgb",
+    "fd_pipeline_host_yuv420", "fd_pipeline_host_yuv422", "fd_pipeline_host_rgb",
 ]
 
 _lib = None
@@ -797,13 +798,44 @@ class Context:
         upload: FD_UPLOAD_FULL | FD_UPLOAD_ON_DEMAND.  -> (bufs, total detections, h2d bytes, d2h bytes); bufs also
         holds "n_crops"."""
         B = len(frames_host)
+        hp, ct, it, opts, out, bufs = self._host_batch(B, heads_host, cap_rows, conf_thr, iou_thr, want_tensor, bufs, select, is_enroll,
+                                                       upload, select_params, heads_zero_copy)
         if jpeg:     # frames_host: list of 1-D u8 arrays holding JPEG streams (fd_pipeline_host_jpeg)
             jp = (C.c_void_p * B)(*[f.ctypes.data for f in frames_host])
             jl = (C.c_size_t * B)(*[f.size for f in frames_host])
+            _chk(self.lib.fd_pipeline_host_jpeg(self.handle, jp, jl, B, int(jpeg_threads), hp, len(heads_host), ct, it, C.byref(opts), C.byref(out)))
         else:
             arr = (FdFrame * B)()
             for i, f in enumerate(frames_host):
                 arr[i].data, arr[i].height, arr[i].width, arr[i].pitch = f.ctypes.data, f.shape[0], f.shape[1], f.strides[0]
+            _chk(self.lib.fd_pipeline_host(self.handle, arr, B, hp, len(heads_host), ct, it, C.byref(opts), C.byref(out)))
+        return self._host_result(bufs, out)
+
+    # ---- fd_pipeline_host on host frames in another layout: frames are the descriptors of the *_yuv420 / *_yuv422 / *_rgb
+    # device calls with HOST addresses (e.g. numpy_array.ctypes.data; pinned memory for full PCIe rate), as tuples or as the
+    # array frame_table / frame_table_nv12 built.  Keyword arguments and results are pipeline_host's (jpeg aside); the results
+    # are fd_pipeline_host's on cv2.cvtColor(COLOR_YUV2BGR_<layout> / RGB2BGR / RGBA2BGR / BGRA2BGR / GRAY2BGR) of the frames.
+    def pipeline_host_yuv420(self, frames, layout, heads_host, cap_rows, **kw):
+        arr = self._frames_nv12(frames)
+        hp, ct, it, opts, out, bufs = self._host_batch(len(arr), heads_host, cap_rows, **kw)
+        _chk(self.lib.fd_pipeline_host_yuv420(self.handle, arr, int(layout), len(arr), hp, len(heads_host), ct, it, C.byref(opts), C.byref(out)))
+        return self._host_result(bufs, out)
+
+    def pipeline_host_yuv422(self, frames, layout, heads_host, cap_rows, **kw):
+        arr = self._frames(frames)
+        hp, ct, it, opts, out, bufs = self._host_batch(len(arr), heads_host, cap_rows, **kw)
+        _chk(self.lib.fd_pipeline_host_yuv422(self.handle, arr, int(layout), len(arr), hp, len(heads_host), ct, it, C.byref(opts), C.byref(out)))
+        return self._host_result(bufs, out)
+
+    def pipeline_host_rgb(self, frames, layout, heads_host, cap_rows, **kw):
+        arr = self._frames(frames)
+        hp, ct, it, opts, out, bufs = self._host_batch(len(arr), heads_host, cap_rows, **kw)
+        _chk(self.lib.fd_pipeline_host_rgb(self.handle, arr, int(layout), len(arr), hp, len(heads_host), ct, it, C.byref(opts), C.byref(out)))
+        return self._host_result(bufs, out)
+
+    def _host_batch(self, B, heads_host, cap_rows, conf_thr=None, iou_thr=None, want_tensor=False, bufs=None, select=False,
+                    is_enroll=False, upload=FD_UPLOAD_FULL, select_params=None, heads_zero_copy=False):
+        """the head table, thresholds, options, fd_host_batch_out and output buffers of an fd_pipeline_host family call"""
         hp = (C.c_void_p * len(heads_host))(*[h.ctypes.data for h in heads_host])
         if bufs is None:
             bufs = dict(counts=np.empty(B, np.int32), det=np.empty((cap_rows, 5), np.float32),
@@ -827,9 +859,9 @@ class Context:
             opts.select_params = FdSelectParams(*select_params)
         ct = C.c_float(self.cfg.conf_thr if conf_thr is None else conf_thr)
         it = C.c_float(self.cfg.iou_thr if iou_thr is None else iou_thr)
-        if jpeg:
-            _chk(self.lib.fd_pipeline_host_jpeg(self.handle, jp, jl, B, int(jpeg_threads), hp, len(heads_host), ct, it, C.byref(opts), C.byref(out)))
-        else:
-            _chk(self.lib.fd_pipeline_host(self.handle, arr, B, hp, len(heads_host), ct, it, C.byref(opts), C.byref(out)))
+        return hp, ct, it, opts, out, bufs
+
+    @staticmethod
+    def _host_result(bufs, out):
         bufs["n_crops"] = out.n_crops
         return bufs, out.total, out.h2d_bytes, out.d2h_bytes
